@@ -62,7 +62,13 @@ def parse():
     ap.add_argument("--dropout", type=float, default=0.0, help="train: dropout probability (configs/tante.yaml:29 uses 0.1)")
     ap.add_argument("--global-batch", type=int, default=None,
                     help="strong scaling: total samples / trajectories per step, split evenly over the ranks")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if a.shape is None:
         a.shape = "active_matter" if a.workload == "train" else "rayleigh_benard"
     if a.batch is None:
@@ -167,7 +173,7 @@ def run_reference(args):
     if rank != 0:
         return
     warm = max(args.warmup, 1)
-    steps = max(args.steps, 1)
+    steps = args.steps
     import torch
     O, cfg = oracle_setup(args)
     torch.set_num_threads(os.cpu_count() or 1)
@@ -307,10 +313,34 @@ def load_peaks():
         return {}
 
 
+DUMP_MAX_ELEMS = 6 << 20      # per array: a dump holds at most two arrays this large, so it stays under 64 MB
+
+
+def flat(tensors):
+    """One 1-D tensor of the given tensors' elements; complex tensors contribute (re, im) pairs."""
+    import torch
+    return torch.cat([(torch.view_as_real(t) if t.is_complex() else t).detach().reshape(-1) for t in tensors])
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy in float32.  A tensor of more than DUMP_MAX_ELEMS elements is replaced by
+    the same seeded sample of its flattened elements on every run, so that two builds run with the same arguments can be
+    compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 AMP_MIX = (0.25, 1.0, 2.0, 4.0)      # per-trajectory input amplitudes of the `adaptive` rollout record
 
 
-def rollout_measure(args, dev, world, rank, with_cpu_baseline=True):
+def rollout_measure(args, dev, world, rank, with_cpu_baseline=True, dump_dir=None):
     """BASELINE configs[2]: per-sample adaptive rollout, `args.batch` trajectories per GPU per step.  Returns the JSON
     record on rank 0 (None elsewhere).  args.rt_bias shifts the interprators' last bias (SURVEY F7); args.amp_mix scales
     trajectory i's window by AMP_MIX[i % 4] so that trajectories of one batch take different step sequences."""
@@ -353,7 +383,7 @@ def rollout_measure(args, dev, world, rank, with_cpu_baseline=True):
         calib = {"first_call_Rt_before": [float(r0.min()), float(r0.median()), float(r0.max())], "bias_shift": shift}
     cpu_sd = {k: v.detach().cpu().clone() for k, v in model.state_dict().items()}
 
-    W_, K_ = max(args.warmup, 3), max(args.steps, 1)
+    W_, K_ = max(args.warmup, 3), args.steps
     with torch.inference_mode():
         for _ in range(W_):
             y, rts, ns, steps = model.rollout(dev_in, n_roll, per_sample=True, sync=False)
@@ -372,6 +402,8 @@ def rollout_measure(args, dev, world, rank, with_cpu_baseline=True):
         ms_total = max_over_ranks(e0.elapsed_time(e1))
         launches = model.launch_count() - l0
         clocks = sampler.stop()
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, {"frames": y, "rts": rts, "frames_per_call": ns, "model_calls": steps})
         steps_h = steps.tolist()
         model_calls = int(max(steps_h))
         ns_first = ns[0].tolist()
@@ -457,7 +489,7 @@ def run_b200(args):
     dev = torch.device("cuda", local)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    line = rollout_measure(args, dev, world, rank)
+    line = rollout_measure(args, dev, world, rank, dump_dir=args.dump_outputs)
     if rank == 0:
         if world == 1 and not args.no_eager:
             try:
@@ -731,7 +763,7 @@ def run_reference_train(args):
     if rank != 0:
         return
     import torch
-    steps = max(args.steps, 1)
+    steps = args.steps
     warm = max(args.warmup, 1)
     O, cfg = oracle_train_setup(args)
     torch.set_num_threads(os.cpu_count() or 1)
@@ -825,7 +857,7 @@ def run_b200_train(args):
             return float(t.item())
         return ms
 
-    W_, K_ = max(args.warmup, 3), max(args.steps, 1)
+    W_, K_ = max(args.warmup, 3), args.steps
     for _ in range(W_):
         train_step(model, opt, dev_x, dev_y, n_out, bucket)
     barrier()
@@ -844,6 +876,10 @@ def run_b200_train(args):
     launches = model.launch_count() - l0
     clocks = sampler.stop()
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:
+        # the caller of train_step receives the loss; the step leaves the updated weights and their gradients in the module
+        params = [p for _, p in model.named_parameters()]
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1), "params": flat(params), "grads": flat(p.grad for p in params)})
 
     # ---- timed region 2: end to end with HOST batches (H2D of inputs+targets, D2H of the loss every step) ----
     # Every step copies its pinned HOST batch to the device and its loss back; tante_b200.pipeline.HostPrefetcher (the
@@ -956,6 +992,9 @@ def run_b200_train(args):
 
 
 def main():
+    # the benchmark writes nothing into the source tree: it imports modules that build() does not (tante_b200.pipeline,
+    # oracle.eager_module), whose bytecode caches would otherwise appear there
+    sys.dont_write_bytecode = True
     args = parse()
     if args.workload == "train":
         if args.impl == "reference":

@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz from the LIVE upstream reference (TEST INFRASTRUCTURE).
 
-Run in the build container only (needs /root/reference):
+Needs an upstream TANTE checkout:
 
-    python -m oracle.make_golden
+    TANTE_REFERENCE_ROOT=<upstream checkout> python -m oracle.make_golden
 
 The reference ships no golden vectors (SURVEY.md §4); these files are outputs of the
 reference's own `models.TANTE` (+ the `deg=False` repair in oracle/ref_shim.py) and
@@ -311,10 +311,66 @@ def main_fno(ns):
                  B=1, out_T=1, rt_bias=0.0, n_roll=2, stride=5)
 
 
+# ---- the live-reference comparisons of tests/test_oracle_vs_reference.py and tests/test_abi_cpu.py, stored --------------
+LIVE_CASES = {   # name -> (cfg, B, out_T, rt_bias); weights O.make_state_dict(cfg, 7, rt_bias), input O.make_input(cfg, B, 8)
+    "ref_live_deg_k1": (O.OracleConfig(n_fields=4, H=64, W=64, taylor_order=1, deg=True), 2, 1, 0.0),
+    "ref_live_adp_k2_lya": (O.OracleConfig(n_fields=3, H=32, W=32, taylor_order=2, attn_axes="THWLA-TYW", deg=False,
+                                           patch_scale=4, frame_interval=0.5), 2, 8, 5.2),
+    "ref_live_adp_k1_p16": (O.OracleConfig(n_fields=2, H=64, W=128, taylor_order=1, attn_axes="THW", deg=False,
+                                           patch_scale=16), 1, 8, 1.3),
+}
+LIVE_STRIDE = 7
+# default initialisation under torch.manual_seed(211): in_T 4, 3 fields on 64x96, patch_scale 8, dropout 0.1
+INIT_CASES = (dict(taylor_order=1, attn_axes="THWTHW", deg=True), dict(taylor_order=2, attn_axes="THW-HW", deg=False),
+              dict(taylor_order=2, attn_axes="TH-W", deg=False, enc_dec_type="fno", modes1=16, modes2=16),
+              dict(taylor_order=2, attn_axes="TCW-CH", deg=False, expanded_channel=256, mlp_ratio=2.0))
+INIT_SAMPLE = 128   # values stored per tensor (evenly strided); the float64 sum and sum of squares cover every element
+
+
+def init_summary(t: torch.Tensor):
+    """(strided sample, float64 sum, float64 sum of squares) of one state_dict tensor (complex as (re, im) pairs)."""
+    a = (torch.view_as_real(t) if t.is_complex() else t).detach().reshape(-1).numpy().astype(np.float64)
+    step = max(1, a.size // INIT_SAMPLE)
+    return a[::step][:INIT_SAMPLE].astype(np.float32), float(a.sum()), float(np.square(a).sum())
+
+
+def main_live(ns, source="the live reference module"):
+    """tests/golden/ref_live_*.npz (the reference's frames / R_t for LIVE_CASES) and ref_init.npz (the reference module's
+    default initialisation for INIT_CASES)."""
+    for name, (cfg, B, out_T, bias) in LIVE_CASES.items():
+        sd = O.make_state_dict(cfg, 7, bias)
+        m = build_ref(ns, cfg, sd).eval()
+        with torch.inference_mode():
+            out = m(O.make_input(cfg, B, 8), out_T)
+        y, rt = (out, None) if cfg.deg else out
+        arrays = {"frames": sub(y, LIVE_STRIDE)}
+        if rt is not None:
+            arrays["R_t"] = rt
+        save(name, cfg, {"B": B, "out_T": out_T, "rt_bias": bias, "seed": 7, "input_seed": 8, "stride": LIVE_STRIDE,
+                         "frames_shape": list(y.shape), "keys": sorted(m.state_dict().keys()), "source": source}, arrays)
+    arrays, cases = {}, []
+    md = ref_shim.make_metadata(3, 64, 96)
+    for i, kw in enumerate(INIT_CASES):
+        torch.manual_seed(211)
+        sd = ns.TANTE(in_T=4, dset_metadata=md, patch_scale=8, dropout=0.1, **kw).state_dict()
+        sums = {}
+        for j, (k, v) in enumerate(sd.items()):
+            arrays[f"c{i}_{j}"], s, s2 = init_summary(v)
+            sums[k] = [list(v.shape), s, s2]
+        cases.append({"kw": kw, "keys": list(sd.keys()), "sums": sums})
+    arrays["meta_json"] = np.frombuffer(json.dumps({"source": source, "init": cases}).encode(), dtype=np.uint8)
+    path = os.path.join(OUT, "ref_init.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"wrote {path}: {os.path.getsize(path)/1024:.1f} KiB")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 1)
     ns = ref_shim.load_reference()
+    if "--live" in sys.argv:
+        main_live(ns)
+        return
     if "--round2" in sys.argv:
         main_round2(ns)
         return

@@ -1,16 +1,17 @@
 """Import shim for the upstream TANTE reference (TEST INFRASTRUCTURE ONLY).
 
-The reference at /root/reference cannot be imported as published in this
-container: `torchinfo`, `h5py`, `matplotlib`, `hydra`, `timm`, `neuralop` are
-missing (SURVEY.md F9).  This module registers stub modules for the three that
-the hot-path files import but never use, bypasses `models/__init__.py` (which
+The reference is an upstream TANTE checkout that is not part of this repository;
+point TANTE_REFERENCE_ROOT at it.  It cannot be imported as published without
+`torchinfo`, `h5py`, `matplotlib`, `hydra`, `timm`, `neuralop` (SURVEY.md F9).
+This module registers stub modules for the three that the hot-path files
+import but never use, bypasses `models/__init__.py` (which
 pulls in the baselines), and applies the *minimal repair* of the adaptive
 (`deg=False`) branch of `TANTE.forward` (reference models/tante.py:147-153,
 SURVEY.md F5 / §8(c)) as a monkey-patch -- the reference tree is never edited.
 
 It is used only by `oracle/make_golden.py` (to generate tests/golden/*) and by
-`tests/test_oracle_vs_reference.py` (skipped when /root/reference is absent,
-e.g. on the GPU box).  Nothing in the product path imports it.
+the tests that compare with the live reference (skipped when TANTE_REFERENCE_ROOT
+is unset).  Nothing in the product path imports it.
 """
 from __future__ import annotations
 
@@ -20,11 +21,12 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("TANTE_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("TANTE_REFERENCE_ROOT", "")
+SKIP_REASON = "upstream reference not found: set TANTE_REFERENCE_ROOT to an upstream TANTE checkout"
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF_ROOT, "models", "tante.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "models", "tante.py"))
 
 
 def _stub(name: str, **attrs):
@@ -46,7 +48,7 @@ def load_reference():
     if _loaded is not None:
         return _loaded
     if not reference_available():
-        raise RuntimeError(f"reference not found under {REF_ROOT}")
+        raise RuntimeError(SKIP_REASON)
     _stub("torchinfo", summary=lambda *a, **k: None)
     _stub("h5py")
     mpl = _stub("matplotlib")

@@ -6,10 +6,11 @@ import os
 import re
 import subprocess
 
+import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import ROOT, load_golden
 from tante_b200 import TANTE, TanteMetadata, _abi
 
 
@@ -103,10 +104,30 @@ def test_ctor_errors_match_reference():
             m(torch.zeros(1, 4, 2, 64, 64))
 
 
+def test_default_init_and_state_dict_equal_the_stored_reference():
+    """Parameter order and seeded default init against the reference module's, as stored in tests/golden/ref_init.npz
+    (`python -m oracle.make_golden --live`): every key in order, shapes, a strided sample of each tensor bitwise, and
+    the float64 sum and sum of squares over all of its elements."""
+    from oracle.make_golden import INIT_CASES, init_summary
+    z, meta = load_golden("ref_init")
+    assert len(meta["init"]) == len(INIT_CASES)
+    for i, (kw, case) in enumerate(zip(INIT_CASES, meta["init"])):
+        assert case["kw"] == kw
+        torch.manual_seed(211)
+        sd = TANTE(4, TanteMetadata(spatial_resolution=(64, 96), n_fields=3), patch_scale=8, dropout=0.1, **kw).state_dict()
+        assert list(sd.keys()) == case["keys"]
+        for j, (k, v) in enumerate(sd.items()):
+            sample, s, s2 = init_summary(v)
+            shape, ref_s, ref_s2 = case["sums"][k]
+            assert list(v.shape) == shape, k
+            np.testing.assert_array_equal(sample, z[f"c{i}_{j}"], err_msg=k)
+            assert s == pytest.approx(ref_s, rel=1e-12, abs=1e-12) and s2 == pytest.approx(ref_s2, rel=1e-12), k
+
+
 def test_default_init_and_state_dict_equal_the_reference():
     from oracle import ref_shim
     if not ref_shim.reference_available():
-        pytest.skip("upstream reference not mounted")
+        pytest.skip(ref_shim.SKIP_REASON)
     ns = ref_shim.load_reference()
     md = ref_shim.make_metadata(3, 64, 96)
     for kw in (dict(taylor_order=1, attn_axes="THWTHW", deg=True), dict(taylor_order=2, attn_axes="THW-HW", deg=False),

@@ -11,7 +11,7 @@ from conftest import GOLDEN, golden_cfg, load_golden, rel_l2
 from oracle import tante_oracle as O
 
 FWD = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, "*.npz"))
-             if not os.path.basename(p).startswith("train_"))
+             if not os.path.basename(p).startswith(("train_", "ref_")))
 FAST = [n for n in FWD if not n.startswith("trl_")] + ["trl_k1_b52", "trl_k2_b13"]
 TOL = 2e-6   # fp32 CPU restatement vs fp32 CPU reference: measured <= 6e-7 (summation order only)
 

@@ -1,13 +1,34 @@
-"""Oracle restatement vs the LIVE upstream module (only where /root/reference exists)."""
+"""Oracle restatement vs the upstream module: against its outputs stored in tests/golden/ref_live_*.npz (always), and
+against the LIVE module where TANTE_REFERENCE_ROOT names an upstream checkout (`python -m oracle.make_golden --live`
+rewrites the stored outputs from it)."""
+import numpy as np
 import pytest
 import torch
 
-from conftest import rel_l2
+from conftest import load_golden, rel_l2
 from oracle import ref_shim, tante_oracle as O
+from oracle.make_golden import LIVE_CASES
 
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="upstream reference not mounted")
+live = pytest.mark.skipif(not ref_shim.reference_available(), reason=ref_shim.SKIP_REASON)
 
 
+@pytest.mark.parametrize("name", sorted(LIVE_CASES))
+def test_oracle_equals_stored_reference(name):
+    cfg, B, out_T, bias = LIVE_CASES[name]
+    z, meta = load_golden(name)
+    sd = O.make_state_dict(cfg, meta["seed"], bias)
+    assert sorted(sd.keys()) == meta["keys"]
+    x = O.make_input(cfg, B, meta["input_seed"])
+    with torch.inference_mode():
+        o = O.forward(sd, cfg, x, out_T)
+    y = o if cfg.deg else o[0]
+    if not cfg.deg:
+        np.testing.assert_allclose(o[1].numpy(), z["R_t"], rtol=0, atol=5e-6)
+    assert list(y.shape) == meta["frames_shape"]
+    assert rel_l2(y.reshape(-1)[::meta["stride"]].numpy(), z["frames"]) < 2e-6
+
+
+@live
 @pytest.mark.parametrize("cfg,B,out_T,bias", [
     (O.OracleConfig(n_fields=4, H=64, W=64, taylor_order=1, deg=True), 2, 1, 0.0),
     (O.OracleConfig(n_fields=3, H=32, W=32, taylor_order=2, attn_axes="THWLA-TYW", deg=False, patch_scale=4,
@@ -33,6 +54,7 @@ def test_oracle_equals_live_reference(cfg, B, out_T, bias):
     assert rel_l2(yo.numpy(), y.numpy()) < 2e-6
 
 
+@live
 def test_unrepaired_adaptive_branch_crashes_as_published():
     """SURVEY.md F5: documents why the oracle is 'reference + minimal repair'."""
     from oracle.make_golden import build_ref
