@@ -169,6 +169,25 @@ TANTE_API int tante_backward_win(tante_handle_t h, int32_t slot, const float* gr
                                  const float* grad_Rt, float* const* grad_frame_ptrs, const int64_t* grad_bstride,
                                  float* grad_params, void* stream);
 
+/* Per-sample cursor variants of the pair above for the adaptive BPTT rollout of R_Trainer (trainer/r_trainer.py:117-133, each
+ * sample its own step sequence, the window NOT detached), the whole batch in one call.  Sample b's history is its input window
+ * input = f32 (B, in_T, D, H, W) (contiguous, 16-byte aligned) followed by its predictions pred + b * pred_bstride (+ j * D * H * W
+ * for prediction j).  cursor = device i32[B], the frames each sample has emitted (zero before the first call): window frame t of
+ * sample b is history frame cursor[b] + t.  The call emits n_b = min(floor(R_t), n_cap) frames of sample b (n_cap = floor(out_T +
+ * 0.001) as in tante_forward) to pred[b, cursor[b] ..], or none once cursor[b] >= n_steps; pred must hold n_steps + n_cap - 1
+ * frames per sample so that an overshooting last call stays inside it.  Then it advances the cursor by n_b and, all on the
+ * device: R_t = f32[B] the call's R_t (0 where n_b = 0), ns = i32[B] n_b, steps = i32[B] += (n_b > 0), n_active (nullable, device
+ * i32[1]) = samples still short of n_steps.  Nothing is synchronised.  The tape keeps the cursor the call saw.
+ * tante_backward_hist reads the gradient of this call's frames from grad_pred (batch stride gp_bstride, same frame positions as
+ * pred; positions past n_steps must hold zeros), takes grad_Rt = f32[B] (nullable; entries with n_b = 0 must be zero), and
+ * ACCUMULATES (+=) the window gradient into grad_pred (predictions) and grad_input (input window, f32 (B, in_T, D, H, W);
+ * NULL: not wanted).  Coverage as the _win pair. */
+TANTE_API int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input, float* pred, int64_t pred_bstride,
+                                       int32_t* cursor, int32_t B, float out_T, int32_t n_cap, int32_t n_steps, float* R_t,
+                                       int32_t* ns, int32_t* steps, int32_t* n_active, void* stream);
+TANTE_API int tante_backward_hist(tante_handle_t h, int32_t slot, float* grad_pred, int64_t gp_bstride, const float* grad_Rt,
+                                  float* grad_input, float* grad_params, void* stream);
+
 /* ---- introspection for tests / profiling ------------------------------------------ */
 /* Copy an internal stage tensor of the last tante_forward into `dst` (f32, device).
  * stage: "latent_in" (after embed), "latent" (after the last backbone), "deriv<k>"

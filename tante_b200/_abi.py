@@ -87,6 +87,11 @@ SIGNATURES = {
                                           C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),
     "tante_backward_win": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.POINTER(C.c_void_p),
                                      C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
+    "tante_train_forward_hist": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32,
+                                           C.c_float, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]),
+    "tante_backward_hist": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_void_p]),
     "tante_test_wgrad": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                    C.c_int32, C.c_int32, C.c_void_p]),
     "tante_bench_head": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,

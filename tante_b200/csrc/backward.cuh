@@ -910,13 +910,20 @@ struct HeadBwdParams {
     const int* n_arr;               // [B]
     float* gi_last;                 // gradient of the LAST window frame (u0 path) of sample 0, += ; null: not needed
     long long gi_bs;                // its batch stride in elements
+    // per-sample cursor mode (tante_backward_hist; null: off): gframes is the gradient of the whole prediction buffer, sample b's
+    // frame i at (cur[b] + i - 1); once cur[b] > 0 the u0 of the call is prediction cur[b] - 1, whose gradient goes to gpred
+    const int* cur;
+    float* gpred;
 };
 
 // Window of a training call given as T separate frames (the chained BPTT rollout of the training drivers slides its window over
 // ONE history instead of torch.cat-ing a new tensor per call, trainer/trainer.py:151-157): frame t of sample b lives at
 // base + off[t] + b * bs[t] (elements, relative to the base pointer the kernel is given).  off[t] = kFrameSkip: no gradient wanted.
+// Per-sample cursor mode (cur != null; tante_train_forward_hist / tante_backward_hist): every sample slides over its own history at
+// its own pace -- window frame t of sample b is history frame i = cur[b] + t, the caller's input frame (off[i], bs[i]) below T, else
+// prediction i - T at hoff + (i - T) * D * H * W + b * hbs.
 constexpr long long kFrameSkip = (long long)(-0x7fffffffffffffffLL - 1);
-struct FrameTab { long long off[16]; long long bs[16]; int on; };
+struct FrameTab { long long off[16]; long long bs[16]; int on; const int* cur; long long hoff, hbs; };
 
 // thread = (stage-1 row, group of 4 consecutive outputs): 16 threads per row, coalesced 128-byte row writes
 __device__ __forceinline__ void patch_pixel(const PatchGeom& g, int h1, int w1, int oo, int& d, size_t& pix) {
@@ -958,8 +965,9 @@ __device__ __forceinline__ void patch_tile_frames(PatchTile& pt, const PatchGeom
         const long long e = pt.img[threadIdx.x];
         if (e >= 0) {
             const long long b = e / g.T;
-            const int t = (int)(e - b * g.T);
-            if (ft.off[t] == kFrameSkip) pt.img[threadIdx.x] = -1;
+            const int t = (int)(e - b * g.T) + (ft.cur ? ft.cur[b] : 0);
+            if (t >= g.T) pt.base[threadIdx.x] = ft.hoff + (long long)(t - g.T) * g.D * g.H * g.W + b * ft.hbs;
+            else if (ft.off[t] == kFrameSkip) pt.img[threadIdx.x] = -1;
             else pt.base[threadIdx.x] = ft.off[t] + b * ft.bs[t];
         }
     }
@@ -1068,12 +1076,13 @@ __global__ void __launch_bounds__(128) head_gather_kernel(HeadBwdParams hp, Patc
         if (!patch_item<VEC>(pt, g, item, tok, d, pix, soff)) continue;
         const long long b = pt.img[tok];
         const int n = min(hp.n_arr[b], hp.n_cap);
+        const int c = hp.cur ? hp.cur[b] : 0;
         float Gk[4][VEC], du[VEC];
 #pragma unroll
         for (int e = 0; e < VEC; ++e) { du[e] = 0.f; Gk[0][e] = Gk[1][e] = Gk[2][e] = Gk[3][e] = 0.f; }
         for (int i = 1; i <= n; ++i) {
             float gv[VEC];
-            VecN<VEC>::load(hp.gframes + (size_t)b * hp.gf_bs + ((size_t)(i - 1) * g.D + d) * HW + pix, gv);
+            VecN<VEC>::load(hp.gframes + (size_t)b * hp.gf_bs + ((size_t)(c + i - 1) * g.D + d) * HW + pix, gv);
             const float dt = (float)i * hp.fi;
             float coef = 1.f;
 #pragma unroll
@@ -1085,8 +1094,10 @@ __global__ void __launch_bounds__(128) head_gather_kernel(HeadBwdParams hp, Patc
 #pragma unroll
             for (int e = 0; e < VEC; ++e) du[e] += gv[e];
         }
-        if (hp.gi_last && n > 0) {
-            float* gp = hp.gi_last + (size_t)b * hp.gi_bs + (size_t)d * HW + pix;
+        float* gu0 = c > 0 ? hp.gpred + (size_t)b * hp.gf_bs + (size_t)(c - 1) * g.D * HW
+                           : (hp.gi_last ? hp.gi_last + (size_t)b * hp.gi_bs : nullptr);
+        if (gu0 && n > 0) {
+            float* gp = gu0 + (size_t)d * HW + pix;
             float cur[VEC];
             VecN<VEC>::load(gp, cur);
 #pragma unroll

@@ -147,13 +147,13 @@ taylor_head_mma_kernel(HeadParams hp, PatchGeom g, long long rows_total, int B) 
         const int bt = hp.act ? hp.act[b] : b;                       // trajectory of ring / counters / history (compaction)
         const int n = hp.n_arr[bt];
         const int fc = hp.fcount ? hp.fcount[bt] : g.T;
+        const int f0 = hp.cur ? hp.cur[bt] : 0;
         const size_t pix0 = (size_t)hpp * P * g.W + (size_t)wpc * XW;
         // u0 of this thread's items: in flight during phase 1  (requesting them one tile ahead was measured SLOWER on B200:
         // K = 1, n = 1 on the TRL shape 45.7 -> 63 us -- the extra per-tile index chain costs more than the latency it hides)
         float4 u0r[NJ];
         {
-            const float* u0p = (hp.u0_base ? hp.u0_base + (size_t)bt * hp.u0_bs
-                                           : hp.u_ring + (size_t)(bt * g.T + (fc + g.T - 1) % g.T) * g.D * HW) + pix0;
+            const float* u0p = head_u0(hp, g, bt, fc, HW) + pix0;
 #pragma unroll
             for (int j = 0; j < NJ; ++j) {
                 u0r[j] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -243,7 +243,7 @@ taylor_head_mma_kernel(HeadParams hp, PatchGeom g, long long rows_total, int B) 
                 v.x += u0.x; v.y += u0.y; v.z += u0.z; v.w += u0.w;
                 if (hp.frames)
                     *reinterpret_cast<float4*>(hp.frames + (size_t)b * (hp.frames_bs ? (size_t)hp.frames_bs : (size_t)hp.n_cap * g.D * HW) +
-                                               (size_t)(i - 1) * g.D * HW + goff) = v;
+                                               (size_t)(f0 + i - 1) * g.D * HW + goff) = v;
                 if (y_out && i > n - g.T) {
                     const int slot = (fc + i - 1) % g.T;
                     *reinterpret_cast<float4*>(hp.ring_out + (size_t)(bt * g.T + slot) * g.D * HW + goff) = v;

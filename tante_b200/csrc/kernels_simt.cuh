@@ -532,11 +532,15 @@ __global__ void set_rollout_ptrs_kernel(RolloutPtrs* dst, float* y, float* rts, 
 
 __global__ void select_step_kernel(const float* __restrict__ rt /* [K][Bstride] */, int K, int Bstride, int B,
                                    int deg, int output_length, int per_sample, int n_cap,
-                                   float* __restrict__ R_t, int* __restrict__ n_out, RolloutState rs, int rollout) {
+                                   float* __restrict__ R_t, int* __restrict__ n_out, RolloutState rs, int rollout,
+                                   const int* __restrict__ cur = nullptr, int n_lim = 0) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;      // compact index (rt / R_t / n_out are compact)
     if (b >= B) return;
     const int bt = (rollout && rs.act) ? rs.act[b] : b;       // trajectory
     const int Bs = (rollout && rs.B_full > 0) ? rs.B_full : B;
+    // per-sample cursor mode of the training rollout (cur != null): a sample that already holds its n_lim frames emits nothing
+    // and its R_t is unused (0)
+    const bool done = cur && cur[b] >= n_lim;
     int n;
     float Rb = 0.f;
     if (deg) {
@@ -551,9 +555,9 @@ __global__ void select_step_kernel(const float* __restrict__ rt /* [K][Bstride] 
         Rb /= (float)K;
         sg /= (float)K;
         n = (int)floorf(sg);
-        if (R_t) R_t[b] = Rb;
+        if (R_t) R_t[b] = done ? 0.f : Rb;
     }
-    n = max(1, min(n, n_cap));
+    n = done ? 0 : max(1, min(n, n_cap));
     if (rollout) {
         const bool active = rs.cum[bt] < rs.n_roll;
         if (!active) n = 0;
@@ -567,6 +571,25 @@ __global__ void select_step_kernel(const float* __restrict__ rt /* [K][Bstride] 
         rs.n_cur[bt] = n;
     }
     if (n_out) n_out[b] = n;
+}
+
+// Per-sample cursor mode of the training rollout (tante_train_forward_hist), after the head: sample b emitted n_arr[b] frames
+// (0 once it holds n_lim).  Records them in ns, advances its cursor and call count, and counts the samples still short of n_lim
+// into *n_active (nullable).  One CTA.
+__global__ void hist_advance_kernel(const int* __restrict__ n_arr, int* __restrict__ cur, int* __restrict__ ns,
+                                    int* __restrict__ steps, int* __restrict__ n_active, int B, int n_lim) {
+    __shared__ int cnt;
+    if (threadIdx.x == 0) cnt = 0;
+    __syncthreads();
+    for (int b = threadIdx.x; b < B; b += blockDim.x) {
+        const int n = n_arr[b];
+        ns[b] = n;
+        const int c = cur[b] + n;
+        if (n > 0) { cur[b] = c; steps[b] += 1; }
+        if (c < n_lim) atomicAdd(&cnt, 1);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && n_active) *n_active = cnt;
 }
 
 __global__ void advance_state_kernel(RolloutState rs, int B, cudaGraphConditionalHandle cond, int use_cond) {
@@ -672,7 +695,17 @@ struct HeadParams {
     // training over a frame table: u0 = last window frame of sample b at u0_base + b * u0_bs (null: u_ring); frame i of sample b is
     // written to frames + b * frames_bs + i * D * H * W (0: contiguous (B, n_cap, D, H, W))
     const float* u0_base; long long u0_bs; long long frames_bs;
+    // per-sample cursor mode (tante_train_forward_hist; null: off): frames is the prediction buffer and sample b has emitted cur[b]
+    // frames into it so far -- its window ends with prediction cur[b] - 1 once cur[b] > 0, and frame i goes to cur[b] + i - 1
+    const int* cur;
 };
+
+// u0 (the last window frame) of sample bt
+__device__ __forceinline__ const float* head_u0(const HeadParams& hp, const PatchGeom& g, int bt, int fc, size_t HW) {
+    const int c = hp.cur ? hp.cur[bt] : 0;
+    if (c > 0) return hp.frames + (size_t)bt * hp.frames_bs + (size_t)(c - 1) * g.D * HW;
+    return hp.u0_base ? hp.u0_base + (size_t)bt * hp.u0_bs : hp.u_ring + (size_t)(bt * g.T + (fc + g.T - 1) % g.T) * g.D * HW;
+}
 
 // Exact-mode (FFMA) variant: one thread per stage-1 row; the thread streams its own C1-long row(s)
 // from global/L1 (each row is one or two full 128 B lines), weights of all K orders sit in shared
@@ -706,8 +739,8 @@ __global__ void __launch_bounds__(128) taylor_head_kernel(HeadParams hp, PatchGe
     if (n <= 0 && !hp.deriv_dbg) return;
     const size_t HW = (size_t)g.H * g.W;
     const int fc = hp.fcount ? hp.fcount[bt] : g.T;
-    const int u_slot = (fc + g.T - 1) % g.T;
-    const float* u0p = hp.u0_base ? hp.u0_base + (size_t)bt * hp.u0_bs : hp.u_ring + ((size_t)(bt * g.T + u_slot) * g.D) * HW;
+    const float* u0p = head_u0(hp, g, bt, fc, HW);
+    const int f0 = hp.cur ? hp.cur[bt] : 0;
     const int cum = hp.cum ? hp.cum[bt] : 0;
     float* y_out = hp.ptrs ? hp.ptrs->y_out : nullptr;
 
@@ -751,7 +784,7 @@ __global__ void __launch_bounds__(128) taylor_head_kernel(HeadParams hp, PatchGe
                 for (int k = KORD; k >= 1; --k) v = (acc[k - 1][o] + v) * (dt / (float)k);
                 const float val = v + u0;
                 if (hp.frames)
-                    hp.frames[(size_t)b * (hp.frames_bs ? (size_t)hp.frames_bs : (size_t)hp.n_cap * g.D * HW) + ((size_t)(i - 1) * g.D + d) * HW + pix] = val;
+                    hp.frames[(size_t)b * (hp.frames_bs ? (size_t)hp.frames_bs : (size_t)hp.n_cap * g.D * HW) + ((size_t)(f0 + i - 1) * g.D + d) * HW + pix] = val;
                 if (y_out) {
                     const int fidx = cum + i - 1;
                     if (fidx < hp.n_roll) y_out[(((size_t)bt * hp.n_roll + fidx) * HW + pix) * g.D + d] = val;

@@ -126,11 +126,14 @@ struct OrderTape {
 };
 struct Tape {
     DevBuf cols, a1pre, a1act, a2pre, a2act, v, n_arr;
+    DevBuf cur;                         // per-sample cursor mode: the cursor this call saw (its backward addresses the same frames)
     DevBuf f0pre, f0act;                // fno encoder: [B*T][H][W][C/8] grid behind enc_spectral_1 (a1* = [..][H1][W1][C/4], a2* = [..][H1][W1][C/2])
     std::vector<OrderTape> ord;
     int B = 0;          // allocated batch
     int B_used = 0;     // batch of the taped forward
     float out_T = 1.f;
+    int n_cap = 0;      // frames per sample the taped call could emit
+    bool hist = false;  // taped by tante_train_forward_hist
     bool valid = false;
     DropCfg drop;       // dropout of this taped call (p = 0: none); the backward regenerates the forward's masks from it
 };
@@ -1700,7 +1703,7 @@ void launch_propagator_bwd(tante_handle_s* h, const float* xin, float* dy, int B
 }
 
 void free_tape(Tape& tp) {
-    DevBuf* bufs[] = {&tp.cols, &tp.a1pre, &tp.a1act, &tp.a2pre, &tp.a2act, &tp.v, &tp.n_arr, &tp.f0pre, &tp.f0act};
+    DevBuf* bufs[] = {&tp.cols, &tp.a1pre, &tp.a1act, &tp.a2pre, &tp.a2act, &tp.v, &tp.n_arr, &tp.cur, &tp.f0pre, &tp.f0act};
     for (DevBuf* b : bufs) b->free();
     for (OrderTape& ot : tp.ord) {
         DevBuf* ob[] = {&ot.P[0], &ot.P[1], &ot.P[2], &ot.dl, &ot.d32, &ot.dmod, &ot.i1, &ot.i2, &ot.rt, &ot.film, &ot.z1pre,
@@ -1735,6 +1738,7 @@ void tape_alloc(tante_handle_s* h, Tape& tp, int B) {
     }
     dev_alloc(h, tp.v, tokens * C * 4);
     dev_alloc(h, tp.n_arr, (size_t)B * 4);
+    dev_alloc(h, tp.cur, (size_t)B * 4);
     tp.ord.resize(h->K);
     for (int o = 0; o < h->K; ++o) {
         OrderTape& ot = tp.ord[o];
@@ -1848,6 +1852,7 @@ void backward_alloc(tante_handle_s* h, int B) {
 struct TrainWin {
     FrameTab in;                  // forward: the T window frames, offsets relative to `input`
     long long frames_bs = 0;      // batch stride of the emitted frames (0: contiguous)
+    int n_lim = 0;                // per-sample cursor mode (in.cur != null): frames a sample needs; it emits nothing once it has them
 };
 
 template <typename TA>
@@ -2151,8 +2156,9 @@ void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, floa
         launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z2pre), TP<TA>(ot.z2act), (long long)B * L * g.R1 * C1, st);
     }
     RolloutState rs{};
-    select_step_kernel<<<(B + 127) / 128, 128, 0, st>>>(rt, K, h->max_batch, B, h->cfg.deg, h->cfg.output_length, 0, n_cap,
-                                                        R_t, reinterpret_cast<int*>(h->nbuf.p), rs, 0);
+    const int* cur = win ? win->in.cur : nullptr;
+    select_step_kernel<<<(B + 127) / 128, 128, 0, st>>>(rt, K, h->max_batch, B, h->cfg.deg, h->cfg.output_length, cur ? 1 : 0, n_cap,
+                                                        R_t, reinterpret_cast<int*>(h->nbuf.p), rs, 0, cur, win ? win->n_lim : 0);
     CK(cudaGetLastError());
     h->launches++;
     CK(cudaMemcpyAsync(tp.n_arr.p, h->nbuf.p, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
@@ -2179,7 +2185,7 @@ void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, floa
         }
         hp.K = K; hp.fi = h->cfg.frame_interval; hp.u_ring = input; hp.fcount = nullptr;
         hp.n_arr = reinterpret_cast<int*>(h->nbuf.p); hp.frames = frames; hp.n_cap = n_cap;
-        if (win) { hp.u0_base = input + win->in.off[T - 1]; hp.u0_bs = win->in.bs[T - 1]; hp.frames_bs = win->frames_bs; }
+        if (win) { hp.u0_base = input + win->in.off[T - 1]; hp.u0_bs = win->in.bs[T - 1]; hp.frames_bs = win->frames_bs; hp.cur = cur; }
         const long long rows = (long long)B * L * g.R1;
         bool done = false;
         if (kTensor) {
@@ -2198,6 +2204,8 @@ void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, floa
         h->launches++;
     }
     tp.out_T = out_T;
+    tp.n_cap = n_cap;
+    tp.hist = cur != nullptr;
     tp.B_used = B;
     tp.valid = true;
 }
@@ -2338,6 +2346,8 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             const bool want = grad_input && win->gin.off[T - 1] != kFrameSkip;
             hp.gi_last = want ? grad_input + win->gin.off[T - 1] : nullptr;
             hp.gi_bs = win->gin.bs[T - 1];
+            hp.cur = win->gin.cur;
+            if (hp.cur) hp.gpred = grad_input + win->gin.hoff;
         } else {
             hp.gi_last = grad_input ? grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
             hp.gi_bs = (long long)T * D * h->cfg.H * h->cfg.W;
@@ -3359,6 +3369,83 @@ int tante_backward_win(tante_handle_t h, int32_t slot, const float* grad_frames,
             run_backward<float>(h, tp, nullptr, grad_frames, n_frames, grad_Rt, gbase, grad_params, st, &win);
         else
             run_backward<__nv_bfloat16>(h, tp, nullptr, grad_frames, n_frames, grad_Rt, gbase, grad_params, st, &win);
+        tp.valid = false;
+    });
+}
+
+// Per-sample cursor variants: every sample slides over its own history (input window, then its predictions) at its own pace.
+static long long elem_offset(const float* p, const float* base) {
+    const intptr_t d = reinterpret_cast<intptr_t>(p) - reinterpret_cast<intptr_t>(base);
+    REQUIRE(d % 16 == 0, "buffers must be 16-byte aligned");
+    return (long long)(d / 4);
+}
+
+int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input, float* pred, int64_t pred_bstride, int32_t* cursor,
+                             int32_t B, float out_T, int32_t n_cap, int32_t n_steps, float* R_t, int32_t* ns, int32_t* steps,
+                             int32_t* n_active, void* stream) {
+    return guarded([&] {
+        REQUIRE(h && input && pred && cursor && R_t && ns && steps, "null argument");
+        REQUIRE(n_cap >= 1 && n_steps >= 1, "n_cap and n_steps must be >= 1");
+        REQUIRE(slot >= 0 && slot < (int)h->tapes.size(), "tape slot out of range: call tante_reserve(.., training = slots)");
+        REQUIRE(h->T <= 16, "training supports in_T <= 16");
+        REQUIRE(!h->wide && !h->fno && !h->chan, "the windowed BPTT entry points cover patch_scale <= 8 with the CNN encoder and the axes T H W L Y A");
+        const long long DHW = (long long)h->D * h->cfg.H * h->cfg.W;
+        REQUIRE(pred_bstride % 4 == 0 && pred_bstride >= (long long)(n_steps + n_cap - 1) * DHW,
+                "pred_bstride must be a multiple of 4 elements and hold n_steps + n_cap - 1 frames");
+        REQUIRE(reinterpret_cast<uintptr_t>(input) % 16 == 0, "input must be 16-byte aligned");
+        CK(cudaSetDevice(h->device));
+        ensure_ready(h, B);
+        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+        Tape& tp = *h->tapes[slot];
+        tape_alloc(h, tp, B);
+        CK(cudaMemcpyAsync(tp.cur.p, cursor, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+        TrainWin win;
+        win.in = FrameTab{};
+        win.in.on = 1;
+        for (int t = 0; t < h->T; ++t) { win.in.off[t] = t * DHW; win.in.bs[t] = h->T * DHW; }
+        win.in.cur = reinterpret_cast<const int*>(tp.cur.p);
+        win.in.hoff = elem_offset(pred, input);
+        win.in.hbs = pred_bstride;
+        win.frames_bs = pred_bstride;
+        win.n_lim = n_steps;
+        if (h->cfg.precision == TANTE_PREC_FP32) run_step_train<float>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
+        else run_step_train<__nv_bfloat16>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
+        hist_advance_kernel<<<1, 256, 0, st>>>(reinterpret_cast<const int*>(tp.n_arr.p), cursor, ns, steps, n_active, B, n_steps);
+        CK(cudaGetLastError());
+        h->launches++;
+        h->last_B = B;
+    });
+}
+
+int tante_backward_hist(tante_handle_t h, int32_t slot, float* grad_pred, int64_t gp_bstride, const float* grad_Rt,
+                        float* grad_input, float* grad_params, void* stream) {
+    return guarded([&] {
+        REQUIRE(h && grad_pred && grad_params, "null argument");
+        REQUIRE(slot >= 0 && slot < (int)h->tapes.size(), "tape slot out of range");
+        REQUIRE(gp_bstride % 4 == 0, "gp_bstride must be a multiple of 4 elements");
+        Tape& tp = *h->tapes[slot];
+        if (!tp.valid) throw Error(TANTE_ERR_STATE, "tape slot holds no forward (or was already consumed)");
+        REQUIRE(tp.hist, "tape slot was not written by tante_train_forward_hist");
+        CK(cudaSetDevice(h->device));
+        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+        backward_alloc(h, tp.B_used);
+        const long long DHW = (long long)h->D * h->cfg.H * h->cfg.W;
+        BackwardWin win;
+        win.gf_bs = gp_bstride;
+        win.gin = FrameTab{};
+        win.gin.on = 1;
+        const long long gi = grad_input ? elem_offset(grad_input, grad_pred) : 0;
+        for (int t = 0; t < h->T; ++t) {
+            win.gin.off[t] = grad_input ? gi + t * DHW : kFrameSkip;
+            win.gin.bs[t] = h->T * DHW;
+        }
+        win.gin.cur = reinterpret_cast<const int*>(tp.cur.p);
+        win.gin.hoff = 0;
+        win.gin.hbs = gp_bstride;
+        if (h->cfg.precision == TANTE_PREC_FP32)
+            run_backward<float>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_pred, grad_params, st, &win);
+        else
+            run_backward<__nv_bfloat16>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_pred, grad_params, st, &win);
         tp.valid = false;
     });
 }

@@ -440,6 +440,93 @@ class _TanteBPTT(torch.autograd.Function):
         return (None, g_x, None, *grads)
 
 
+class _TanteHistBPTT(torch.autograd.Function):
+    """The per-sample adaptive BPTT rollout of R_Trainer (r_trainer.py:117-133: each sample its own while-loop of
+    `y, rt = model(window_b, out_T)`, the window sliding by floor(R_t) frames over its own predictions, NOT detached) for the
+    whole batch as ONE autograd node.  Every call is one batched tante_train_forward_hist: the library keeps a device cursor per
+    sample (frames emitted so far), reads each sample's window at its cursor and writes its frames behind it; a sample that has
+    its n_steps frames emits nothing.  The backward walks the calls in reverse (tante_backward_hist), accumulating each call's
+    window gradient into the gradient of the earlier predictions in place."""
+
+    @staticmethod
+    def forward(ctx, model, x, n_steps, out_T, *params):
+        eng = model._engine(x.device)
+        B = x.shape[0]
+        D, (H, W) = model.n_channel, model.shape
+        DHW = D * H * W
+        n_cap = max(1, int(math.floor(out_T + 0.001)))
+        n_hist = n_steps + n_cap - 1          # an overshooting last call writes past n_steps, into this slack
+        eng.reserve(B)
+        dev = x.device
+        pred = torch.empty((B, n_hist, D, H, W), device=dev, dtype=torch.float32)
+        cursor = torch.zeros((B,), device=dev, dtype=torch.int32)
+        steps = torch.zeros((B,), device=dev, dtype=torch.int32)
+        rts = torch.zeros((n_steps, B), device=dev, dtype=torch.float32)
+        ns = torch.zeros((n_steps, B), device=dev, dtype=torch.int32)
+        # one frame per call (R_Trainer's out_T = 1.5): every sample makes exactly n_steps calls, no need to ask the device
+        n_active = torch.zeros((1,), device=dev, dtype=torch.int32) if n_cap > 1 else None
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        p_drop = float(model.dropout) if model.training else 0.0
+        slots = []
+        try:
+            for k in range(n_steps):
+                slot = eng.acquire_slot()
+                slots.append(slot)
+                seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if p_drop > 0 else 0
+                _abi.check(eng.lib.tante_set_dropout(eng.handle, p_drop, seed))
+                _abi.check(eng.lib.tante_train_forward_hist(
+                    eng.handle, slot, x.data_ptr(), pred.data_ptr(), n_hist * DHW, cursor.data_ptr(), B, float(out_T), n_cap,
+                    n_steps, rts[k].data_ptr(), ns[k].data_ptr(), steps.data_ptr(),
+                    None if n_active is None else n_active.data_ptr(), stream))
+                if n_active is not None and int(n_active.item()) == 0:
+                    break
+        except Exception:
+            for sl in slots:
+                eng.release_slot(sl)
+            raise
+        n_calls = len(slots)
+        ctx.eng, ctx.model, ctx.slots, ctx.n_steps, ctx.n_hist = eng, model, slots, n_steps, n_hist
+        ctx.guards = [_SlotGuard(eng, sl) for sl in slots]
+        ctx.x_shape = tuple(x.shape)
+        ns = ns[:n_calls].clone()
+        ctx.save_for_backward(ns)
+        ctx.mark_non_differentiable(ns, steps)
+        out = pred if n_hist == n_steps else pred[:, :n_steps].contiguous()
+        return out, rts[:n_calls].clone(), ns, steps
+
+    @staticmethod
+    def backward(ctx, g_pred, g_rts, g_ns, g_steps):
+        eng, model, n_steps, n_hist = ctx.eng, ctx.model, ctx.n_steps, ctx.n_hist
+        (ns,) = ctx.saved_tensors
+        B, T, D, H, W = ctx.x_shape
+        DHW = D * H * W
+        dev = ns.device
+        # gradient of the whole prediction buffer: accumulated in place below; the slack past n_steps stays zero
+        g_acc = torch.zeros((B, n_hist, D, H, W), device=dev, dtype=torch.float32)
+        if g_pred is not None:
+            g_acc[:, :n_steps] = g_pred
+        g_r = None
+        if g_rts is not None:      # R_t of a call a sample did not take part in is unused
+            g_r = torch.where(ns > 0, g_rts.to(torch.float32), 0.0).contiguous()
+        g_x = torch.zeros(ctx.x_shape, device=dev, dtype=torch.float32) if ctx.needs_input_grad[1] else None
+        acc = model._flat_grad_view(eng) if all(ctx.needs_input_grad[4:]) else None
+        flat_sum = None
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        for k in range(len(ctx.slots) - 1, -1, -1):
+            flat = torch.empty((eng.grad_numel,), device=dev, dtype=torch.float32)
+            _abi.check(eng.lib.tante_backward_hist(eng.handle, ctx.slots[k], g_acc.data_ptr(), n_hist * DHW,
+                                                   None if g_r is None else g_r[k].data_ptr(),
+                                                   None if g_x is None else g_x.data_ptr(), flat.data_ptr(), stream))
+            ctx.guards[k].release()
+            if acc is not None:
+                acc.add_(flat)
+            else:
+                flat_sum = flat if flat_sum is None else flat_sum.add_(flat)
+        if acc is not None:
+            return (None, g_x, None, None, *([None] * len(eng.names)))
+        return (None, g_x, None, None, *model._grad_views(eng, flat_sum))
+
+
 import weakref
 
 _LIVE_MODELS: "weakref.WeakSet" = weakref.WeakSet()
@@ -687,12 +774,28 @@ class TANTE(nn.Module):
         """The windowed BPTT entry points (frame tables) exist for the nested-order patch stages (patch_scale <= 8, cnn) without axis-C layers."""
         return self.patch_scale <= 8 and self.enc_dec_type == "cnn" and "C" not in self.attn_axes and self.overlap_ratio == 0.0
 
-    def rollout_train(self, window, n_steps: int):
-        """Fixed-step BPTT rollout of the training drivers (trainer/trainer.py:144-159) for the `deg=True`, `output_length=1`
-        model: (B, T, D, H, W) -> predictions (B, n_steps, D, H, W), one autograd node, no window concatenation.  Same
-        arithmetic as n_steps chained `forward` calls on `cat(window[:, 1:], y)`."""
-        if not (self.deg and int(self.output_length) == 1):
-            raise ValueError("rollout_train covers the fixed-step model (deg=True, output_length=1)")
+    def rollout_train(self, window, n_steps: int, out_T: float = 1.5):
+        """BPTT rollout of the training drivers as one autograd node, no window concatenation.
+
+        Fixed-step model (`deg=True`, `output_length=1`; trainer/trainer.py:144-159): (B, T, D, H, W) -> predictions
+        (B, n_steps, D, H, W), the arithmetic of n_steps chained `forward` calls on `cat(window[:, 1:], y)`.
+
+        Adaptive model (`deg=False`; r_trainer.py:117-133): what the per-sample B=1 loops `y, rt = model(window_b, out_T)`
+        compute, each sample with its own step sequence -> pred (B, n_steps, D, H, W), rts (n_calls, B) R_t of every call,
+        ns (n_calls, B) frames each call emitted per sample (0 once the sample had its n_steps frames; its rts entry is then
+        unused), steps (B,) calls per sample.  With floor(out_T + 0.001) == 1 (R_Trainer's out_T = 1.5) every sample makes
+        n_steps calls and nothing is synchronised; otherwise one 4-byte count is read after each call."""
+        if not self.deg:
+            if not self.bptt_windows_ok:
+                raise ValueError("rollout_train for deg=False covers patch_scale <= 8 with the cnn encoder, no overlap and no axis C")
+            if out_T < 1:
+                raise ValueError("out_T must be >= 1")
+            x = self._prep_input(window)
+            eng = self._engine(x.device)
+            params = dict(self.named_parameters())
+            return _TanteHistBPTT.apply(self, x, int(n_steps), float(out_T), *[params[n] for n in eng.names])
+        if int(self.output_length) != 1:
+            raise ValueError("rollout_train covers the fixed-step model with output_length=1 and the adaptive model")
         x = self._prep_input(window)
         eng = self._engine(x.device)
         params = dict(self.named_parameters())

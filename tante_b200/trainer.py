@@ -12,6 +12,7 @@ from __future__ import annotations
 
 from typing import Optional
 
+import math
 import os
 
 import torch
@@ -87,10 +88,16 @@ def mse_loss_frames(frames, y_ref, n_steps: int):
     return _FusedMSE.apply(y_ref, int(n_steps), *frames)
 
 
+def _bptt_windows(model, window) -> bool:
+    """The module's one-node BPTT rollout (TANTE.rollout_train) applies: CUDA input, the windowed entry points cover the
+    configuration, grad mode, and TANTE_BPTT_WINDOWS is not 0."""
+    return (hasattr(model, "rollout_train") and window.is_cuda and getattr(model, "bptt_windows_ok", True)
+            and torch.is_grad_enabled() and os.environ.get("TANTE_BPTT_WINDOWS", "1") != "0")
+
+
 def _roll_frames(model, window, n_steps: int):
     """`_roll` for the fixed-step model without the formatter permute and the cat over calls."""
-    if (hasattr(model, "rollout_train") and window.is_cuda and int(getattr(model, "output_length", 0)) == 1
-            and getattr(model, "bptt_windows_ok", True) and torch.is_grad_enabled() and os.environ.get("TANTE_BPTT_WINDOWS", "1") != "0"):
+    if int(getattr(model, "output_length", 0)) == 1 and _bptt_windows(model, window):
         return [model.rollout_train(window, n_steps)]      # one autograd node, the window slides over one history buffer
     moving, ys, cum = window, [], 0
     while cum < n_steps:
@@ -118,10 +125,22 @@ def _roll(model, window, n_steps: int, out_T):
     return torch.cat(ys, dim=1)[:, :n_steps], (torch.cat(rts, dim=0) if rts else None)
 
 
+def flat_rts(rts, ns, every_call: bool = False):
+    """Per-call R_t (n_calls, B) and frames per call (n_calls, B) of the batched adaptive rollout -> the flat Rts of the
+    per-sample loops (r_trainer.py:118-131): sample 0's calls in order, then sample 1's, ...; entries of calls a sample did
+    not take part in (ns == 0) are left out.  every_call: every sample took part in every call (no mask, no host sync)."""
+    rt = rts.t()
+    return rt.reshape(-1) if every_call else rt[ns.t() > 0]
+
+
 def rollout_train(model, x, n_steps: int, out_T: float = 1.5):
     """x (B,T,D,H,W) channels-first -> (y_pred (B,n_steps,H,W,D), Rts or None)."""
     if model.deg:
         return _roll(model, x, n_steps, out_T)
+    if _bptt_windows(model, x):
+        # the per-sample loops below as one batched device-resident rollout (TANTE.rollout_train, deg=False)
+        pred, rts, ns, _ = model.rollout_train(x, n_steps, out_T=out_T)
+        return pred.permute(0, 1, 3, 4, 2), flat_rts(rts, ns, every_call=int(math.floor(out_T + 0.001)) <= 1)
     outs, rts = [], []
     for b in range(x.shape[0]):                                         # r_trainer.py:118 ("TODO: batch size > 1")
         y, r = _roll(model, x[b:b + 1], n_steps, out_T)
@@ -418,7 +437,8 @@ def rt_analyse(rt):
 
 class R_Trainer(_TrainerBase):
     """Drop-in for trainer.R_Trainer (r_trainer.py:43-231): adaptive model, per-sample B=1 rollouts with out_T = 1.5 and
-    BPTT through the chained calls, MSE + rt penalty, `clip_grad_value_(1.0)`."""
+    BPTT through the chained calls, MSE + rt penalty, `clip_grad_value_(1.0)`.  On the CUDA module the per-sample loops run
+    as one batched rollout (`rollout_train`); `train_out_T` (default 1.5, the reference's) sets the out_T of training."""
 
     adaptive = True
 
@@ -426,7 +446,8 @@ class R_Trainer(_TrainerBase):
                  optimizer=None, train_loss_fn=None, eval_loss_fn=None, max_epoch: int = 1, lr_scheduler=None,
                  device=torch.device("cuda"), is_distributed: bool = False, enable_amp: bool = False,
                  amp_type: str = "float16", checkpoint_path: str = "", n_steps_output: int = 4, n_steps_rollout: int = 8,
-                 rt_eps: float = 0.5, rt_n: int = 2):
+                 rt_eps: float = 0.5, rt_n: int = 2, train_out_T: float = 1.5):
+        # train_out_T: out_T of the training rollout (the reference always uses 1.5, r_trainer.py:117-133)
         self._init_common(dict(locals()))
 
     def rollout_model(self, model, batch, formatter, mode="train"):
@@ -438,7 +459,7 @@ class R_Trainer(_TrainerBase):
             from .rollout import rollout_eval
             y, Rts, _, _ = rollout_eval(model, batch, n_steps, out_T=1.5, per_sample=True)
             return y, y_ref.to(self.device), Rts
-        y_pred_out, Rts = rollout_train(model, batch, n_steps, 1.5)
+        y_pred_out, Rts = rollout_train(model, batch, n_steps, self.train_out_T)
         return y_pred_out, y_ref.to(self.device), Rts
 
     def train_one_epoch(self, epoch: int, dataloader):
