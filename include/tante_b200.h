@@ -154,34 +154,23 @@ TANTE_API int tante_train_forward(tante_handle_t h, int32_t slot, const float* i
 TANTE_API int tante_backward(tante_handle_t h, int32_t slot, const float* input, const float* grad_frames,
                    int32_t n_frames, const float* grad_Rt, float* grad_input, float* grad_params, void* stream);
 
-/* Frame-table variants of the two calls above for the chained BPTT rollout of the training drivers (trainer/trainer.py:144-159,
- * trainer/r_trainer.py:122-126: window = cat(window[:, n:], y), NOT detached): the window of a call is given as in_T separate
- * frames -- frame_ptrs[t] = device pointer of frame t of sample 0 (a contiguous (D, H, W) plane set, 16-byte aligned),
- * sample b at + b * frame_bstride[t] elements -- so that consecutive calls slide over ONE history buffer and no window is ever
- * concatenated; the emitted frames go to frames + b * frames_bstride (+ i * D * H * W).  tante_backward_win reads the frame
- * gradients with batch stride gf_bstride and ACCUMULATES (+=) the window gradient into grad_frame_ptrs[t] + b * grad_bstride[t]
- * (NULL entry: that frame needs no gradient; grad_frame_ptrs == NULL: none does), which is how BPTT sums the contributions of
- * later calls into the gradient of an earlier prediction in place. */
-TANTE_API int tante_train_forward_win(tante_handle_t h, int32_t slot, const float* const* frame_ptrs,
-                                      const int64_t* frame_bstride, int32_t B, float out_T, int32_t n_cap, float* frames,
-                                      int64_t frames_bstride, float* R_t, int32_t* n_host, void* stream);
-TANTE_API int tante_backward_win(tante_handle_t h, int32_t slot, const float* grad_frames, int64_t gf_bstride, int32_t n_frames,
-                                 const float* grad_Rt, float* const* grad_frame_ptrs, const int64_t* grad_bstride,
-                                 float* grad_params, void* stream);
-
-/* Per-sample cursor variants of the pair above for the adaptive BPTT rollout of R_Trainer (trainer/r_trainer.py:117-133, each
- * sample its own step sequence, the window NOT detached), the whole batch in one call.  Sample b's history is its input window
+/* The chained BPTT rollout of both training drivers, the whole batch in one call per model call: the fixed-step model
+ * (trainer/trainer.py:144-159) and the adaptive model (trainer/r_trainer.py:117-133, each sample its own step sequence), the
+ * window = cat(window[:, n:], y) NOT detached in either.  No window is ever concatenated: sample b's history is its input window
  * input = f32 (B, in_T, D, H, W) (contiguous, 16-byte aligned) followed by its predictions pred + b * pred_bstride (+ j * D * H * W
  * for prediction j).  cursor = device i32[B], the frames each sample has emitted (zero before the first call): window frame t of
- * sample b is history frame cursor[b] + t.  The call emits n_b = min(floor(R_t), n_cap) frames of sample b (n_cap = floor(out_T +
- * 0.001) as in tante_forward) to pred[b, cursor[b] ..], or none once cursor[b] >= n_steps; pred must hold n_steps + n_cap - 1
- * frames per sample so that an overshooting last call stays inside it.  Then it advances the cursor by n_b and, all on the
- * device: R_t = f32[B] the call's R_t (0 where n_b = 0), ns = i32[B] n_b, steps = i32[B] += (n_b > 0), n_active (nullable, device
- * i32[1]) = samples still short of n_steps.  Nothing is synchronised.  The tape keeps the cursor the call saw.
+ * sample b is history frame cursor[b] + t.  The call emits n_b frames of sample b to pred[b, cursor[b] ..], or none once
+ * cursor[b] >= n_steps: n_b = output_length for the fixed-step model (pass n_cap = output_length), the same for every sample;
+ * n_b = min(floor(R_t), n_cap) for the adaptive model (n_cap = floor(out_T + 0.001) as in tante_forward).
+ * pred must hold n_steps + n_cap - 1 frames per sample so that an overshooting last call stays inside it.  Then it advances the
+ * cursor by n_b and, all on the device: R_t = f32[B] the call's R_t (0 where n_b = 0; the fixed-step model has no R_t: NULL
+ * allowed, never written), ns = i32[B] n_b, steps = i32[B] += (n_b > 0), n_active (nullable, device i32[1]) = samples still short
+ * of n_steps.  Nothing is synchronised.  The tape keeps the cursor the call saw.
  * tante_backward_hist reads the gradient of this call's frames from grad_pred (batch stride gp_bstride, same frame positions as
  * pred; positions past n_steps must hold zeros), takes grad_Rt = f32[B] (nullable; entries with n_b = 0 must be zero), and
  * ACCUMULATES (+=) the window gradient into grad_pred (predictions) and grad_input (input window, f32 (B, in_T, D, H, W);
- * NULL: not wanted).  Coverage as the _win pair. */
+ * NULL: not wanted), which is how BPTT sums the contributions of later calls into the gradient of an earlier prediction in
+ * place.  Covers patch_scale <= 8 with the CNN encoder, no overlap, no axis C, and in_T <= 16. */
 TANTE_API int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input, float* pred, int64_t pred_bstride,
                                        int32_t* cursor, int32_t B, float out_T, int32_t n_cap, int32_t n_steps, float* R_t,
                                        int32_t* ns, int32_t* steps, int32_t* n_active, void* stream);

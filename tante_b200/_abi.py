@@ -83,10 +83,6 @@ SIGNATURES = {
                                       C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),
     "tante_backward": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_void_p]),
-    "tante_train_forward_win": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.c_int32, C.c_float,
-                                          C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),
-    "tante_backward_win": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.POINTER(C.c_void_p),
-                                     C.POINTER(C.c_int64), C.c_void_p, C.c_void_p]),
     "tante_train_forward_hist": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32,
                                            C.c_float, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p]),

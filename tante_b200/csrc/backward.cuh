@@ -916,14 +916,13 @@ struct HeadBwdParams {
     float* gpred;
 };
 
-// Window of a training call given as T separate frames (the chained BPTT rollout of the training drivers slides its window over
-// ONE history instead of torch.cat-ing a new tensor per call, trainer/trainer.py:151-157): frame t of sample b lives at
-// base + off[t] + b * bs[t] (elements, relative to the base pointer the kernel is given).  off[t] = kFrameSkip: no gradient wanted.
-// Per-sample cursor mode (cur != null; tante_train_forward_hist / tante_backward_hist): every sample slides over its own history at
-// its own pace -- window frame t of sample b is history frame i = cur[b] + t, the caller's input frame (off[i], bs[i]) below T, else
-// prediction i - T at hoff + (i - T) * D * H * W + b * hbs.
-constexpr long long kFrameSkip = (long long)(-0x7fffffffffffffffLL - 1);
-struct FrameTab { long long off[16]; long long bs[16]; int on; const int* cur; long long hoff, hbs; };
+// Per-sample cursor mode of the training rollout (cur != null; tante_train_forward_hist / tante_backward_hist): the chained BPTT
+// rollout of the training drivers slides every sample's window over its own history instead of torch.cat-ing a new tensor per
+// call (trainer/trainer.py:151-157, r_trainer.py:126).  Window frame t of sample b is history frame i = cur[b] + t: below T the
+// input frame at (b * T + i) * D * H * W, the contiguous (B, T, D, H, W) layout of the plain path (skip_in: no input frame is
+// wanted, their tokens are skipped), else prediction i - T at hoff + b * hbs + (i - T) * D * H * W.  Element offsets, relative to
+// the pointer the kernel is given.
+struct FrameTab { const int* cur; long long hoff, hbs; int skip_in; };
 
 // thread = (stage-1 row, group of 4 consecutive outputs): 16 threads per row, coalesced 128-byte row writes
 __device__ __forceinline__ void patch_pixel(const PatchGeom& g, int h1, int w1, int oo, int& d, size_t& pix) {
@@ -957,18 +956,19 @@ struct PatchTile {
     int stab[32];                             // RH[8], RW[8], OH[8], OW[8]   (see taylor_head_mma_kernel)
     long long pix0[kPatchRows];               // per token: pixel offset of its top-left corner in a plane
     long long img[kPatchRows];                // per token: image index (-1 = past the end)
-    long long base[kPatchRows];               // per token: element offset of its image (frame tables only)
+    long long base[kPatchRows];               // per token: element offset of its image (cursor mode only)
 };
-// image index b * T + t -> address through a frame table (call after patch_tile_init, before a __syncthreads)
+// image index b * T + t -> address of history frame cur[b] + t (call after patch_tile_init, before a __syncthreads)
 __device__ __forceinline__ void patch_tile_frames(PatchTile& pt, const PatchGeom& g, const FrameTab& ft) {
     if (threadIdx.x < kPatchRows / g.R1) {
         const long long e = pt.img[threadIdx.x];
         if (e >= 0) {
             const long long b = e / g.T;
-            const int t = (int)(e - b * g.T) + (ft.cur ? ft.cur[b] : 0);
-            if (t >= g.T) pt.base[threadIdx.x] = ft.hoff + (long long)(t - g.T) * g.D * g.H * g.W + b * ft.hbs;
-            else if (ft.off[t] == kFrameSkip) pt.img[threadIdx.x] = -1;
-            else pt.base[threadIdx.x] = ft.off[t] + b * ft.bs[t];
+            const int i = (int)(e - b * g.T) + ft.cur[b];       // history frame
+            const long long DHW = (long long)g.D * g.H * g.W;
+            if (i >= g.T) pt.base[threadIdx.x] = ft.hoff + b * ft.hbs + (long long)(i - g.T) * DHW;
+            else if (ft.skip_in) pt.img[threadIdx.x] = -1;
+            else pt.base[threadIdx.x] = (b * g.T + i) * DHW;
         }
     }
 }
@@ -1150,7 +1150,7 @@ __global__ void __launch_bounds__(128) conv1_im2col_kernel(const float* __restri
         }
     }
     if (enc_list || fcount) __syncthreads();
-    if (ft.on) { patch_tile_frames(pt, g, ft); __syncthreads(); }
+    if (ft.cur) { patch_tile_frames(pt, g, ft); __syncthreads(); }
     const size_t HW = (size_t)g.H * g.W;
     const int nitems = (g.D * pt.P * pt.NT) << (pt.lP - (VEC == 4 ? 2 : 1));
     bool any = false;
@@ -1159,7 +1159,7 @@ __global__ void __launch_bounds__(128) conv1_im2col_kernel(const float* __restri
         size_t pix;
         if (!patch_item<VEC>(pt, g, item, tok, d, pix, soff)) continue;
         float v[VEC];
-        const long long ib = ft.on ? pt.base[tok] : pt.img[tok] * (long long)(g.D * HW);
+        const long long ib = ft.cur ? pt.base[tok] : pt.img[tok] * (long long)(g.D * HW);
         VecN<VEC>::load(x + ib + (size_t)d * HW + pix, v);
 #pragma unroll
         for (int e = 0; e < VEC; ++e) S[soff[e]] = v[e];
@@ -1179,7 +1179,12 @@ __global__ void __launch_bounds__(128) conv1_col2im_kernel(const TA* __restrict_
     __shared__ PatchTile pt;
     const long long row0 = (long long)blockIdx.x * kPatchRows;
     patch_tile_init(pt, g, row0, rows_total);
-    if (ft.on) { __syncthreads(); patch_tile_frames(pt, g, ft); }
+    if (ft.cur) {
+        __syncthreads();
+        patch_tile_frames(pt, g, ft);
+        // a tile none of whose tokens wants a gradient (input frames without grad_input) has nothing to add
+        if (!__syncthreads_or(threadIdx.x < kPatchRows / g.R1 && pt.img[threadIdx.x] >= 0)) return;
+    }
     patch_rows_load<TA>(S, dpatch, row0, rows_total);
     __syncthreads();
     const size_t HW = (size_t)g.H * g.W;
@@ -1188,7 +1193,7 @@ __global__ void __launch_bounds__(128) conv1_col2im_kernel(const TA* __restrict_
         int tok, d, soff[VEC];
         size_t pix;
         if (!patch_item<VEC>(pt, g, item, tok, d, pix, soff)) continue;
-        const long long ib = ft.on ? pt.base[tok] : pt.img[tok] * (long long)(g.D * HW);
+        const long long ib = ft.cur ? pt.base[tok] : pt.img[tok] * (long long)(g.D * HW);
         float* gp = grad_input + ib + (size_t)d * HW + pix;
         float cur[VEC];
         VecN<VEC>::load(gp, cur);

@@ -574,16 +574,17 @@ __global__ void select_step_kernel(const float* __restrict__ rt /* [K][Bstride] 
 }
 
 // Per-sample cursor mode of the training rollout (tante_train_forward_hist), after the head: sample b emitted n_arr[b] frames
-// (0 once it holds n_lim).  Records them in ns, advances its cursor and call count, and counts the samples still short of n_lim
-// into *n_active (nullable).  One CTA.
-__global__ void hist_advance_kernel(const int* __restrict__ n_arr, int* __restrict__ cur, int* __restrict__ ns,
-                                    int* __restrict__ steps, int* __restrict__ n_active, int B, int n_lim) {
+// (0 once it holds n_lim).  Keeps the cursor the call saw in cur_seen (the tape's, for the backward), records the frames in ns,
+// advances the cursor and call count, and counts the samples still short of n_lim into *n_active (nullable).  One CTA.
+__global__ void hist_advance_kernel(const int* __restrict__ n_arr, int* __restrict__ cur, int* __restrict__ cur_seen,
+                                    int* __restrict__ ns, int* __restrict__ steps, int* __restrict__ n_active, int B, int n_lim) {
     __shared__ int cnt;
     if (threadIdx.x == 0) cnt = 0;
     __syncthreads();
     for (int b = threadIdx.x; b < B; b += blockDim.x) {
         const int n = n_arr[b];
         ns[b] = n;
+        cur_seen[b] = cur[b];
         const int c = cur[b] + n;
         if (n > 0) { cur[b] = c; steps[b] += 1; }
         if (c < n_lim) atomicAdd(&cnt, 1);
@@ -692,9 +693,8 @@ struct HeadParams {
     float* deriv_dbg;
     // rollout compaction: sample index of the stage-1 rows (compact) -> trajectory of ring / counters / history (null: identity)
     const int* act;
-    // training over a frame table: u0 = last window frame of sample b at u0_base + b * u0_bs (null: u_ring); frame i of sample b is
-    // written to frames + b * frames_bs + i * D * H * W (0: contiguous (B, n_cap, D, H, W))
-    const float* u0_base; long long u0_bs; long long frames_bs;
+    // batch stride of frames (0: contiguous (B, n_cap, D, H, W))
+    long long frames_bs;
     // per-sample cursor mode (tante_train_forward_hist; null: off): frames is the prediction buffer and sample b has emitted cur[b]
     // frames into it so far -- its window ends with prediction cur[b] - 1 once cur[b] > 0, and frame i goes to cur[b] + i - 1
     const int* cur;
@@ -704,7 +704,7 @@ struct HeadParams {
 __device__ __forceinline__ const float* head_u0(const HeadParams& hp, const PatchGeom& g, int bt, int fc, size_t HW) {
     const int c = hp.cur ? hp.cur[bt] : 0;
     if (c > 0) return hp.frames + (size_t)bt * hp.frames_bs + (size_t)(c - 1) * g.D * HW;
-    return hp.u0_base ? hp.u0_base + (size_t)bt * hp.u0_bs : hp.u_ring + (size_t)(bt * g.T + (fc + g.T - 1) % g.T) * g.D * HW;
+    return hp.u_ring + (size_t)(bt * g.T + (fc + g.T - 1) % g.T) * g.D * HW;
 }
 
 // Exact-mode (FFMA) variant: one thread per stage-1 row; the thread streams its own C1-long row(s)

@@ -1848,11 +1848,11 @@ void backward_alloc(tante_handle_s* h, int B) {
 }
 
 // One TANTE step in training mode: same arithmetic as run_step, every activation the backward needs is kept.
-// Window of a training call as a frame table (tante_train_forward_win / tante_backward_win)
+// Per-sample cursor mode (tante_train_forward_hist): the window frames relative to `input`; `frames` is the prediction buffer
+// (batch stride in.hbs) and a sample that has its n_lim frames emits nothing.
 struct TrainWin {
-    FrameTab in;                  // forward: the T window frames, offsets relative to `input`
-    long long frames_bs = 0;      // batch stride of the emitted frames (0: contiguous)
-    int n_lim = 0;                // per-sample cursor mode (in.cur != null): frames a sample needs; it emits nothing once it has them
+    FrameTab in;
+    int n_lim;
 };
 
 template <typename TA>
@@ -2185,7 +2185,7 @@ void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, floa
         }
         hp.K = K; hp.fi = h->cfg.frame_interval; hp.u_ring = input; hp.fcount = nullptr;
         hp.n_arr = reinterpret_cast<int*>(h->nbuf.p); hp.frames = frames; hp.n_cap = n_cap;
-        if (win) { hp.u0_base = input + win->in.off[T - 1]; hp.u0_bs = win->in.bs[T - 1]; hp.frames_bs = win->frames_bs; hp.cur = cur; }
+        if (win) { hp.frames_bs = win->in.hbs; hp.cur = cur; }
         const long long rows = (long long)B * L * g.R1;
         bool done = false;
         if (kTensor) {
@@ -2213,8 +2213,9 @@ void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, floa
 // Backward of one taped step.  gframes: f32 (B, n_g, D, H, W) gradient of the emitted frames; gRt: f32 [B] or null;
 // grad_input: f32 (B, T, D, H, W) or null (written, not accumulated; but see `win`); flat: f32 [sum numel] parameter gradients in
 // tante_param order (written, not accumulated).
-// win (frame-table mode): gframes has batch stride win->gf_bs; the input gradient is ACCUMULATED into the frames of win->gin
-// (offsets relative to grad_input; kFrameSkip entries are not computed) instead of written to a contiguous (B, T, D, H, W).
+// win (per-sample cursor mode, tante_backward_hist): gframes is win->gpred, the gradient of the whole prediction buffer (batch
+// stride win->gin.hbs), and the window gradient is ACCUMULATED into it and into grad_input (nullable) through win->gin, whose
+// offsets are relative to grad_input, or to gpred when there is no grad_input (gin.skip_in).
 // Backward of one axis-'C' layer (channel_axis.cuh): dxs [tokens][C] holds the gradient of the layer output on entry and of its
 // input on return (the layer REPLACES the latent: no residual around it).  Per chunk of h->chanb_tokens latent tokens the block is
 // recomputed from the saved fp32 input (lift, LN1, QKV, attention, out-proj, LN2, MLP -- everything the backward reads stays in
@@ -2296,7 +2297,7 @@ void run_channel_layer_bwd(tante_handle_s* h, const LayerPlan& lp, const float* 
     }
 }
 
-struct BackwardWin { long long gf_bs; FrameTab gin; };
+struct BackwardWin { FrameTab gin; float* gpred; };
 template <typename TA>
 void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* gframes, int n_g, const float* gRt,
                   float* grad_input, float* flat, cudaStream_t st, const BackwardWin* win = nullptr) {
@@ -2340,18 +2341,11 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
         HeadBwdParams hp{};
         for (int k = 0; k < K; ++k) hp.G[k] = TP<TA>(h->hG) + (size_t)k * rows1 * kHeadPad;
         hp.K = K; hp.fi = h->cfg.frame_interval; hp.gframes = gframes; hp.n_cap = n_g;
-        hp.gf_bs = win ? win->gf_bs : (long long)n_g * D * h->cfg.H * h->cfg.W;
+        hp.gf_bs = win ? win->gin.hbs : (long long)n_g * D * h->cfg.H * h->cfg.W;
         hp.n_arr = reinterpret_cast<const int*>(tp.n_arr.p);
-        if (win) {
-            const bool want = grad_input && win->gin.off[T - 1] != kFrameSkip;
-            hp.gi_last = want ? grad_input + win->gin.off[T - 1] : nullptr;
-            hp.gi_bs = win->gin.bs[T - 1];
-            hp.cur = win->gin.cur;
-            if (hp.cur) hp.gpred = grad_input + win->gin.hoff;
-        } else {
-            hp.gi_last = grad_input ? grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
-            hp.gi_bs = (long long)T * D * h->cfg.H * h->cfg.W;
-        }
+        hp.gi_last = grad_input ? grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
+        hp.gi_bs = (long long)T * D * h->cfg.H * h->cfg.W;
+        if (win) { hp.cur = win->gin.cur; hp.gpred = win->gpred; }
         const size_t hsmem = (size_t)K * kPatchRows * kPatchPitch * sizeof(float);
         if (g.k0 * g.k1 * g.k2 >= 4) head_gather_kernel<TA, 4><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
         else head_gather_kernel<TA, 2><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
@@ -2684,13 +2678,14 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
     (void)input;      // the patches were kept by the forward (tape im2col)
     TA* cols = TP<TA>(h->cols);
     wgrad_pad<TA>(h, ga1, C1, C1, TP<TA>(tp.cols), kHeadPad, kHeadPad, GA(h, h->enc_w[0]), NO, NO, rows_in, st, GA(h, h->enc_b[0]));
-    if (grad_input) {
+    if (grad_input || win) {
         // dpatch[rows, 64 (K1 padded)] = da1[rows, C1] * W1[C1][K1]  (thin GEMM), then scatter-add into the pixels
         REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv backward GEMM");
         gemm_dx<TA>(h, ga1, C1, h->enc_wT[0], cols, kHeadPad, (int)rows_in, kHeadPad, C1, st);
         const FrameTab gt = win ? win->gin : FrameTab();
-        if (g.k0 * g.k1 * g.k2 >= 4) conv1_col2im_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, grad_input, rows_in, gt);
-        else conv1_col2im_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, grad_input, rows_in, gt);
+        float* gbase = grad_input ? grad_input : win->gpred;
+        if (g.k0 * g.k1 * g.k2 >= 4) conv1_col2im_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, gt);
+        else conv1_col2im_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, gt);
         CK(cudaGetLastError());
         h->launches++;
     }
@@ -3300,80 +3295,7 @@ int tante_backward(tante_handle_t h, int32_t slot, const float* input, const flo
     });
 }
 
-// Frame-table variants: the window of a call is T separate frames (device pointer of sample 0 + batch stride each).
-static FrameTab make_frame_tab(const float* base, const float* const* ptrs, const int64_t* bs, int T) {
-    FrameTab ft{};
-    ft.on = 1;
-    for (int t = 0; t < T; ++t) {
-        if (!ptrs[t]) { ft.off[t] = kFrameSkip; ft.bs[t] = 0; continue; }
-        const intptr_t d = reinterpret_cast<intptr_t>(ptrs[t]) - reinterpret_cast<intptr_t>(base);
-        REQUIRE(d % 4 == 0 && reinterpret_cast<uintptr_t>(ptrs[t]) % 16 == 0 && bs[t] % 4 == 0,
-                "frame pointers must be 16-byte aligned and batch strides multiples of 4 elements");
-        ft.off[t] = (long long)(d / 4);
-        ft.bs[t] = (long long)bs[t];
-    }
-    return ft;
-}
-
-int tante_train_forward_win(tante_handle_t h, int32_t slot, const float* const* frame_ptrs, const int64_t* frame_bstride,
-                            int32_t B, float out_T, int32_t n_cap, float* frames, int64_t frames_bstride, float* R_t,
-                            int32_t* n_host, void* stream) {
-    return guarded([&] {
-        REQUIRE(h && frame_ptrs && frame_bstride && frames, "null argument");
-        REQUIRE(n_cap >= 1, "n_cap must be >= 1");
-        REQUIRE(slot >= 0 && slot < (int)h->tapes.size(), "tape slot out of range: call tante_reserve(.., training = slots)");
-        REQUIRE(h->T <= 16, "training supports in_T <= 16");
-        REQUIRE(!h->wide && !h->fno && !h->chan, "the windowed BPTT entry points cover patch_scale <= 8 with the CNN encoder and the axes T H W L Y A");
-        for (int t = 0; t < h->T; ++t) REQUIRE(frame_ptrs[t], "null frame pointer");
-        REQUIRE(frames_bstride % 4 == 0, "frames_bstride must be a multiple of 4 elements");
-        CK(cudaSetDevice(h->device));
-        ensure_ready(h, B);
-        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-        Tape& tp = *h->tapes[slot];
-        tape_alloc(h, tp, B);
-        const float* base = frame_ptrs[0];
-        TrainWin win;
-        win.in = make_frame_tab(base, frame_ptrs, frame_bstride, h->T);
-        win.frames_bs = frames_bstride;
-        if (h->cfg.precision == TANTE_PREC_FP32) run_step_train<float>(h, tp, base, B, out_T, n_cap, frames, R_t, st, &win);
-        else run_step_train<__nv_bfloat16>(h, tp, base, B, out_T, n_cap, frames, R_t, st, &win);
-        h->last_B = B;
-        if (n_host) {
-            CK(cudaMemcpyAsync(h->h_flag + 8, h->nbuf.p, 4, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            *n_host = h->h_flag[8];
-        }
-    });
-}
-
-int tante_backward_win(tante_handle_t h, int32_t slot, const float* grad_frames, int64_t gf_bstride, int32_t n_frames,
-                       const float* grad_Rt, float* const* grad_frame_ptrs, const int64_t* grad_bstride, float* grad_params,
-                       void* stream) {
-    return guarded([&] {
-        REQUIRE(h && grad_frames && grad_params, "null argument");
-        REQUIRE(slot >= 0 && slot < (int)h->tapes.size(), "tape slot out of range");
-        REQUIRE(n_frames >= 1 && gf_bstride % 4 == 0, "bad gradient frame layout");
-        Tape& tp = *h->tapes[slot];
-        if (!tp.valid) throw Error(TANTE_ERR_STATE, "tape slot holds no forward (or was already consumed)");
-        CK(cudaSetDevice(h->device));
-        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-        backward_alloc(h, tp.B_used);
-        BackwardWin win;
-        win.gf_bs = gf_bstride;
-        float* gbase = nullptr;
-        if (grad_frame_ptrs)
-            for (int t = 0; t < h->T && !gbase; ++t) gbase = grad_frame_ptrs[t];
-        if (gbase) win.gin = make_frame_tab(gbase, grad_frame_ptrs, grad_bstride, h->T);
-        else { win.gin = FrameTab{}; win.gin.on = 1; for (int t = 0; t < 16; ++t) win.gin.off[t] = kFrameSkip; }
-        if (h->cfg.precision == TANTE_PREC_FP32)
-            run_backward<float>(h, tp, nullptr, grad_frames, n_frames, grad_Rt, gbase, grad_params, st, &win);
-        else
-            run_backward<__nv_bfloat16>(h, tp, nullptr, grad_frames, n_frames, grad_Rt, gbase, grad_params, st, &win);
-        tp.valid = false;
-    });
-}
-
-// Per-sample cursor variants: every sample slides over its own history (input window, then its predictions) at its own pace.
+// Per-sample cursor pair: every sample slides over its own history (input window, then its predictions) at its own pace.
 static long long elem_offset(const float* p, const float* base) {
     const intptr_t d = reinterpret_cast<intptr_t>(p) - reinterpret_cast<intptr_t>(base);
     REQUIRE(d % 16 == 0, "buffers must be 16-byte aligned");
@@ -3384,7 +3306,8 @@ int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input,
                              int32_t B, float out_T, int32_t n_cap, int32_t n_steps, float* R_t, int32_t* ns, int32_t* steps,
                              int32_t* n_active, void* stream) {
     return guarded([&] {
-        REQUIRE(h && input && pred && cursor && R_t && ns && steps, "null argument");
+        REQUIRE(h && input && pred && cursor && ns && steps, "null argument");
+        REQUIRE(R_t || h->cfg.deg, "R_t is required for the adaptive model");
         REQUIRE(n_cap >= 1 && n_steps >= 1, "n_cap and n_steps must be >= 1");
         REQUIRE(slot >= 0 && slot < (int)h->tapes.size(), "tape slot out of range: call tante_reserve(.., training = slots)");
         REQUIRE(h->T <= 16, "training supports in_T <= 16");
@@ -3398,19 +3321,14 @@ int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input,
         cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
         Tape& tp = *h->tapes[slot];
         tape_alloc(h, tp, B);
-        CK(cudaMemcpyAsync(tp.cur.p, cursor, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+        // the kernels of the call read the caller's cursor; the advance stores the value they saw in the tape
         TrainWin win;
-        win.in = FrameTab{};
-        win.in.on = 1;
-        for (int t = 0; t < h->T; ++t) { win.in.off[t] = t * DHW; win.in.bs[t] = h->T * DHW; }
-        win.in.cur = reinterpret_cast<const int*>(tp.cur.p);
-        win.in.hoff = elem_offset(pred, input);
-        win.in.hbs = pred_bstride;
-        win.frames_bs = pred_bstride;
+        win.in = FrameTab{cursor, elem_offset(pred, input), pred_bstride, 0};
         win.n_lim = n_steps;
         if (h->cfg.precision == TANTE_PREC_FP32) run_step_train<float>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
         else run_step_train<__nv_bfloat16>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
-        hist_advance_kernel<<<1, 256, 0, st>>>(reinterpret_cast<const int*>(tp.n_arr.p), cursor, ns, steps, n_active, B, n_steps);
+        hist_advance_kernel<<<1, 256, 0, st>>>(reinterpret_cast<const int*>(tp.n_arr.p), cursor, reinterpret_cast<int*>(tp.cur.p), ns,
+                                               steps, n_active, B, n_steps);
         CK(cudaGetLastError());
         h->launches++;
         h->last_B = B;
@@ -3429,23 +3347,14 @@ int tante_backward_hist(tante_handle_t h, int32_t slot, float* grad_pred, int64_
         CK(cudaSetDevice(h->device));
         cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
         backward_alloc(h, tp.B_used);
-        const long long DHW = (long long)h->D * h->cfg.H * h->cfg.W;
         BackwardWin win;
-        win.gf_bs = gp_bstride;
-        win.gin = FrameTab{};
-        win.gin.on = 1;
-        const long long gi = grad_input ? elem_offset(grad_input, grad_pred) : 0;
-        for (int t = 0; t < h->T; ++t) {
-            win.gin.off[t] = grad_input ? gi + t * DHW : kFrameSkip;
-            win.gin.bs[t] = h->T * DHW;
-        }
-        win.gin.cur = reinterpret_cast<const int*>(tp.cur.p);
-        win.gin.hoff = 0;
-        win.gin.hbs = gp_bstride;
+        win.gin = FrameTab{reinterpret_cast<const int*>(tp.cur.p), grad_input ? elem_offset(grad_pred, grad_input) : 0, gp_bstride,
+                           grad_input ? 0 : 1};
+        win.gpred = grad_pred;
         if (h->cfg.precision == TANTE_PREC_FP32)
-            run_backward<float>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_pred, grad_params, st, &win);
+            run_backward<float>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_input, grad_params, st, &win);
         else
-            run_backward<__nv_bfloat16>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_pred, grad_params, st, &win);
+            run_backward<__nv_bfloat16>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_input, grad_params, st, &win);
         tp.valid = false;
     });
 }

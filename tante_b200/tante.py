@@ -364,89 +364,15 @@ class _TanteStep(torch.autograd.Function):
 
 
 class _TanteBPTT(torch.autograd.Function):
-    """The chained fixed-step rollout of the training drivers (trainer/trainer.py:144-159: `window = cat(window[:, 1:], y)`, NOT
-    detached) as ONE autograd node: every call reads its window as a frame table over the input window and the prediction
-    buffer (tante_train_forward_win), so no window is ever concatenated, and the backward walks the calls in reverse,
-    ACCUMULATING each call's window gradient into the gradient of the earlier predictions in place (tante_backward_win) --
-    what autograd does with a cat / slice / add chain per call."""
-
-    @staticmethod
-    def forward(ctx, model, x, n_steps, *params):
-        eng = model._engine(x.device)
-        B, T = x.shape[0], model.T
-        D, (H, W) = model.n_channel, model.shape
-        DHW = D * H * W
-        eng.reserve(B)
-        pred = torch.empty((B, n_steps, D, H, W), device=x.device, dtype=torch.float32)
-        stream = torch.cuda.current_stream(x.device).cuda_stream
-        p_drop = float(model.dropout) if model.training else 0.0
-        slots = []
-        PT, I64 = ctypes.c_void_p * T, ctypes.c_int64 * T
-        try:
-            for k in range(n_steps):
-                slot = eng.acquire_slot()
-                slots.append(slot)
-                seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if p_drop > 0 else 0
-                _abi.check(eng.lib.tante_set_dropout(eng.handle, p_drop, seed))
-                ptrs, bss = PT(), I64()
-                for t in range(T):
-                    i = k + t
-                    if i < T:
-                        ptrs[t], bss[t] = x.data_ptr() + 4 * i * DHW, T * DHW
-                    else:
-                        ptrs[t], bss[t] = pred.data_ptr() + 4 * (i - T) * DHW, n_steps * DHW
-                _abi.check(eng.lib.tante_train_forward_win(eng.handle, slot, ptrs, bss, B, 1.0, 1, pred.data_ptr() + 4 * k * DHW,
-                                                           n_steps * DHW, None, None, stream))
-        except Exception:
-            for sl in slots:
-                eng.release_slot(sl)
-            raise
-        ctx.eng, ctx.model, ctx.slots, ctx.n_steps = eng, model, slots, n_steps
-        ctx.guards = [_SlotGuard(eng, sl) for sl in slots]
-        ctx.x_shape = tuple(x.shape)
-        return pred
-
-    @staticmethod
-    def backward(ctx, g_pred):
-        eng, model, n_steps = ctx.eng, ctx.model, ctx.n_steps
-        B, T, D, H, W = ctx.x_shape
-        DHW = D * H * W
-        dev = g_pred.device
-        g_acc = g_pred.to(torch.float32).contiguous().clone()        # accumulated in place below: never autograd's own tensor
-        g_x = torch.zeros(ctx.x_shape, device=dev, dtype=torch.float32) if ctx.needs_input_grad[1] else None
-        acc = model._flat_grad_view(eng) if all(ctx.needs_input_grad[3:]) else None
-        flat_sum = None
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        PT, I64 = ctypes.c_void_p * T, ctypes.c_int64 * T
-        for k in range(n_steps - 1, -1, -1):
-            ptrs, bss = PT(), I64()
-            for t in range(T):
-                i = k + t
-                if i < T:
-                    ptrs[t], bss[t] = (g_x.data_ptr() + 4 * i * DHW if g_x is not None else None), T * DHW
-                else:
-                    ptrs[t], bss[t] = g_acc.data_ptr() + 4 * (i - T) * DHW, n_steps * DHW
-            flat = torch.empty((eng.grad_numel,), device=dev, dtype=torch.float32)
-            _abi.check(eng.lib.tante_backward_win(eng.handle, ctx.slots[k], g_acc.data_ptr() + 4 * k * DHW, n_steps * DHW, 1, None,
-                                                  ptrs, bss, flat.data_ptr(), stream))
-            ctx.guards[k].release()
-            if acc is not None:
-                acc.add_(flat)
-            else:
-                flat_sum = flat if flat_sum is None else flat_sum.add_(flat)
-        if acc is not None:
-            return (None, g_x, None, *([None] * len(eng.names)))
-        grads = model._grad_views(eng, flat_sum)
-        return (None, g_x, None, *grads)
-
-
-class _TanteHistBPTT(torch.autograd.Function):
-    """The per-sample adaptive BPTT rollout of R_Trainer (r_trainer.py:117-133: each sample its own while-loop of
-    `y, rt = model(window_b, out_T)`, the window sliding by floor(R_t) frames over its own predictions, NOT detached) for the
-    whole batch as ONE autograd node.  Every call is one batched tante_train_forward_hist: the library keeps a device cursor per
-    sample (frames emitted so far), reads each sample's window at its cursor and writes its frames behind it; a sample that has
-    its n_steps frames emits nothing.  The backward walks the calls in reverse (tante_backward_hist), accumulating each call's
-    window gradient into the gradient of the earlier predictions in place."""
+    """The chained BPTT rollout of both training drivers as ONE autograd node: the fixed-step model (trainer/trainer.py:144-159:
+    `window = cat(window[:, 1:], y)`) and the per-sample adaptive loops of R_Trainer (r_trainer.py:117-133: each sample its own
+    while-loop of `y, rt = model(window_b, out_T)`, the window sliding by floor(R_t) frames over its own predictions), NOT
+    detached in either.  Every call is one batched tante_train_forward_hist: the library keeps a device cursor per sample
+    (frames emitted so far), reads each sample's window at its cursor and writes its frames behind it, so no window is ever
+    concatenated; a sample that has its n_steps frames emits nothing.  The backward walks the calls in reverse
+    (tante_backward_hist), ACCUMULATING each call's window gradient into the gradient of the earlier predictions in place --
+    what autograd does with a cat / slice / add chain per call.  Returns pred for the fixed-step model, (pred, rts, ns, steps)
+    for the adaptive one."""
 
     @staticmethod
     def forward(ctx, model, x, n_steps, out_T, *params):
@@ -454,16 +380,18 @@ class _TanteHistBPTT(torch.autograd.Function):
         B = x.shape[0]
         D, (H, W) = model.n_channel, model.shape
         DHW = D * H * W
-        n_cap = max(1, int(math.floor(out_T + 0.001)))
+        # the fixed-step model emits output_length frames per call and sample, and has no R_t
+        n_cap = int(model.output_length) if model.deg else max(1, int(math.floor(out_T + 0.001)))
         n_hist = n_steps + n_cap - 1          # an overshooting last call writes past n_steps, into this slack
         eng.reserve(B)
         dev = x.device
         pred = torch.empty((B, n_hist, D, H, W), device=dev, dtype=torch.float32)
         cursor = torch.zeros((B,), device=dev, dtype=torch.int32)
         steps = torch.zeros((B,), device=dev, dtype=torch.int32)
-        rts = torch.zeros((n_steps, B), device=dev, dtype=torch.float32)
+        rts = None if model.deg else torch.zeros((n_steps, B), device=dev, dtype=torch.float32)
         ns = torch.zeros((n_steps, B), device=dev, dtype=torch.int32)
-        # one frame per call (R_Trainer's out_T = 1.5): every sample makes exactly n_steps calls, no need to ask the device
+        # one frame per call (the fixed-step model, R_Trainer's out_T = 1.5): every sample makes exactly n_steps calls, no need
+        # to ask the device
         n_active = torch.zeros((1,), device=dev, dtype=torch.int32) if n_cap > 1 else None
         stream = torch.cuda.current_stream(dev).cuda_stream
         p_drop = float(model.dropout) if model.training else 0.0
@@ -476,7 +404,7 @@ class _TanteHistBPTT(torch.autograd.Function):
                 _abi.check(eng.lib.tante_set_dropout(eng.handle, p_drop, seed))
                 _abi.check(eng.lib.tante_train_forward_hist(
                     eng.handle, slot, x.data_ptr(), pred.data_ptr(), n_hist * DHW, cursor.data_ptr(), B, float(out_T), n_cap,
-                    n_steps, rts[k].data_ptr(), ns[k].data_ptr(), steps.data_ptr(),
+                    n_steps, None if rts is None else rts[k].data_ptr(), ns[k].data_ptr(), steps.data_ptr(),
                     None if n_active is None else n_active.data_ptr(), stream))
                 if n_active is not None and int(n_active.item()) == 0:
                     break
@@ -488,25 +416,28 @@ class _TanteHistBPTT(torch.autograd.Function):
         ctx.eng, ctx.model, ctx.slots, ctx.n_steps, ctx.n_hist = eng, model, slots, n_steps, n_hist
         ctx.guards = [_SlotGuard(eng, sl) for sl in slots]
         ctx.x_shape = tuple(x.shape)
+        out = pred if n_hist == n_steps else pred[:, :n_steps].contiguous()
+        if model.deg:
+            return out
         ns = ns[:n_calls].clone()
         ctx.save_for_backward(ns)
         ctx.mark_non_differentiable(ns, steps)
-        out = pred if n_hist == n_steps else pred[:, :n_steps].contiguous()
         return out, rts[:n_calls].clone(), ns, steps
 
     @staticmethod
-    def backward(ctx, g_pred, g_rts, g_ns, g_steps):
+    def backward(ctx, g_pred, g_rts=None, *_):
         eng, model, n_steps, n_hist = ctx.eng, ctx.model, ctx.n_steps, ctx.n_hist
-        (ns,) = ctx.saved_tensors
         B, T, D, H, W = ctx.x_shape
         DHW = D * H * W
-        dev = ns.device
-        # gradient of the whole prediction buffer: accumulated in place below; the slack past n_steps stays zero
-        g_acc = torch.zeros((B, n_hist, D, H, W), device=dev, dtype=torch.float32)
-        if g_pred is not None:
-            g_acc[:, :n_steps] = g_pred
+        dev = eng.device
+        # gradient of the whole prediction buffer: accumulated in place below (never autograd's own tensor); the slack past
+        # n_steps stays zero
+        g_acc = torch.empty((B, n_hist, D, H, W), device=dev, dtype=torch.float32)
+        g_acc[:, :n_steps] = 0.0 if g_pred is None else g_pred
+        g_acc[:, n_steps:] = 0.0
         g_r = None
         if g_rts is not None:      # R_t of a call a sample did not take part in is unused
+            (ns,) = ctx.saved_tensors
             g_r = torch.where(ns > 0, g_rts.to(torch.float32), 0.0).contiguous()
         g_x = torch.zeros(ctx.x_shape, device=dev, dtype=torch.float32) if ctx.needs_input_grad[1] else None
         acc = model._flat_grad_view(eng) if all(ctx.needs_input_grad[4:]) else None
@@ -771,35 +702,31 @@ class TANTE(nn.Module):
 
     @property
     def bptt_windows_ok(self) -> bool:
-        """The windowed BPTT entry points (frame tables) exist for the nested-order patch stages (patch_scale <= 8, cnn) without axis-C layers."""
+        """The windowed BPTT entry points (per-sample cursors) exist for the nested-order patch stages (patch_scale <= 8, cnn) without axis-C layers."""
         return self.patch_scale <= 8 and self.enc_dec_type == "cnn" and "C" not in self.attn_axes and self.overlap_ratio == 0.0
 
     def rollout_train(self, window, n_steps: int, out_T: float = 1.5):
         """BPTT rollout of the training drivers as one autograd node, no window concatenation.
 
         Fixed-step model (`deg=True`, `output_length=1`; trainer/trainer.py:144-159): (B, T, D, H, W) -> predictions
-        (B, n_steps, D, H, W), the arithmetic of n_steps chained `forward` calls on `cat(window[:, 1:], y)`.
+        (B, n_steps, D, H, W), the arithmetic of n_steps chained `forward` calls on `cat(window[:, 1:], y)`.  out_T is unused.
 
         Adaptive model (`deg=False`; r_trainer.py:117-133): what the per-sample B=1 loops `y, rt = model(window_b, out_T)`
         compute, each sample with its own step sequence -> pred (B, n_steps, D, H, W), rts (n_calls, B) R_t of every call,
         ns (n_calls, B) frames each call emitted per sample (0 once the sample had its n_steps frames; its rts entry is then
         unused), steps (B,) calls per sample.  With floor(out_T + 0.001) == 1 (R_Trainer's out_T = 1.5) every sample makes
         n_steps calls and nothing is synchronised; otherwise one 4-byte count is read after each call."""
+        if self.deg and int(self.output_length) != 1:
+            raise ValueError("rollout_train covers the fixed-step model with output_length=1 and the adaptive model")
         if not self.deg:
             if not self.bptt_windows_ok:
                 raise ValueError("rollout_train for deg=False covers patch_scale <= 8 with the cnn encoder, no overlap and no axis C")
             if out_T < 1:
                 raise ValueError("out_T must be >= 1")
-            x = self._prep_input(window)
-            eng = self._engine(x.device)
-            params = dict(self.named_parameters())
-            return _TanteHistBPTT.apply(self, x, int(n_steps), float(out_T), *[params[n] for n in eng.names])
-        if int(self.output_length) != 1:
-            raise ValueError("rollout_train covers the fixed-step model with output_length=1 and the adaptive model")
         x = self._prep_input(window)
         eng = self._engine(x.device)
         params = dict(self.named_parameters())
-        return _TanteBPTT.apply(self, x, int(n_steps), *[params[n] for n in eng.names])
+        return _TanteBPTT.apply(self, x, int(n_steps), float(out_T), *[params[n] for n in eng.names])
 
     @torch.no_grad()
     def rollout(self, window, n_steps_rollout: int, out_T=None, per_sample: bool = False, sync: bool = True):

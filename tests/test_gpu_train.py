@@ -414,8 +414,8 @@ def test_fused_mse_matches_reference_loss_and_gradient(n_steps):
 @pytest.mark.parametrize("prec,tol", [("fp32", 2e-5), ("bf16", 2e-2)])
 @pytest.mark.parametrize("n_steps", [2, 5])
 def test_windowed_bptt_rollout_equals_chained_calls(prec, tol, n_steps):
-    """`TANTE.rollout_train` (one autograd node over frame tables: tante_train_forward_win / tante_backward_win, no torch.cat)
-    against the reference-style chain `y = model(win); win = cat(win[:, 1:], y)` (trainer/trainer.py:144-159) on the same
+    """`TANTE.rollout_train` (one autograd node, every sample's window read at its device cursor over the input window and the
+    prediction buffer: tante_train_forward_hist / tante_backward_hist, no torch.cat) against the reference-style chain `y = model(win); win = cat(win[:, 1:], y)` (trainer/trainer.py:144-159) on the same
     module: identical predictions, equal parameter gradients and input gradient.  n_steps = 5 > in_T: the last window holds
     predictions only."""
     from gpu_util import make_model
