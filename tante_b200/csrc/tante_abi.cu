@@ -538,6 +538,11 @@ struct StepIO {
     bool rollout = false;
     int per_sample = 0;
     float out_T = 1.f;
+    Tape* tape = nullptr;           // taped training call: every activation the backward reads is kept here (null: inference)
+    // Per-sample cursor mode (tante_train_forward_hist; ft.cur null: off): window frames relative to `input`; `frames` is the
+    // prediction buffer (batch stride ft.hbs) and a sample that has its n_lim frames emits nothing.
+    FrameTab ft{};
+    int n_lim = 0;
 };
 
 RolloutState make_state(tante_handle_s* h, int B, int n_roll) {
@@ -560,6 +565,9 @@ RolloutState make_state(tante_handle_s* h, int B, int n_roll) {
 }
 
 inline __nv_bfloat16* AH(tante_handle_s* h, int64_t off) { return reinterpret_cast<__nv_bfloat16*>(h->arena_bf16.p) + off; }
+
+template <typename TA> inline TA* TP(DevBuf& b) { return reinterpret_cast<TA*>(b.p); }
+inline float* FP(DevBuf& b) { return reinterpret_cast<float*>(b.p); }
 
 // C = epi(A * W^T): fp32 mode -> FFMA GEMM; bf16 mode -> tcgen05 GEMM (C is fp32 when out_f32, else bf16).
 template <typename TA>
@@ -615,27 +623,47 @@ void launch_layernorm(tante_handle_s* h, const float* x, int64_t w, int64_t b, T
     h->launches++;
 }
 
+// Destinations of one transformer block: in place on the residual stream and the shared scratch buffers (inference, `ot`
+// null), or out of place into the tape slots of layer li, so that every input of a later derivative survives (training).
+// hpre is null in inference: the MLP GELU rides in the GEMM epilogue there.
+template <typename TA>
+struct LayerBufs {
+    float *x_in, *x_mid, *x_out;
+    TA *ln1, *qkv, *att, *ln2, *hpre, *hact, *ln_next;
+    uint32_t site[3];      // dropout sites: attention probabilities, residual after the out-projection, residual after the MLP
+};
+template <typename TA>
+LayerBufs<TA> layer_bufs(tante_handle_s* h, OrderTape* ot, int o, size_t li) {
+    if (!ot) {
+        float* x = FP(h->x);
+        TA* ln = TP<TA>(h->ln);
+        return {x, x, x, ln, TP<TA>(h->qkv), TP<TA>(h->att), ln, nullptr, TP<TA>(h->hid), ln, {0, 0, 0}};
+    }
+    const int i = (int)li;
+    return {FP(ot->X[2 * li]), FP(ot->X[2 * li + 1]), FP(ot->X[2 * li + 2]), TP<TA>(ot->ln1[li]), TP<TA>(ot->qkv[li]),
+            TP<TA>(ot->att[li]), TP<TA>(ot->ln2[li]), TP<TA>(ot->hpre[li]), TP<TA>(ot->hact[li]),
+            li + 1 < ot->ln1.size() ? TP<TA>(ot->ln1[li + 1]) : nullptr, {drop_site(o, i, 0), drop_site(o, i, 1), drop_site(o, i, 2)}};
+}
+
 // Fused tail of a transformer block (block_tail_tc.cuh): out-projection + residual + LN2 + MLP + residual + the next layer's
 // LN1 in one tcgen05 kernel.  `nx` = the next layer of the backbone (null for the last one: no LayerNorm output).
-// Training (x_mid != null) also stores x_mid, the LN2 output, the MLP pre-activation and the hidden activation.
-void launch_tail(tante_handle_s* h, const LayerPlan& lp, const LayerPlan* nx, const __nv_bfloat16* att, const float* x_in,
-                 float* x_out, __nv_bfloat16* ln_out, int tokens, cudaStream_t st, float* x_mid = nullptr,
-                 __nv_bfloat16* ln2 = nullptr, __nv_bfloat16* hpre = nullptr, __nv_bfloat16* hact = nullptr,
-                 const DropCfg& drop = DropCfg(), uint32_t site1 = 0, uint32_t site2 = 0) {
-    const bool train = x_mid != nullptr;
+// Training (b.hpre != null) also stores x_mid, the LN2 output, the MLP pre-activation and the hidden activation.
+void launch_tail(tante_handle_s* h, const LayerPlan& lp, const LayerPlan* nx, const LayerBufs<__nv_bfloat16>& b, int tokens,
+                 const DropCfg& drop, cudaStream_t st) {
+    const bool train = b.hpre != nullptr;
     const double C = h->C;
     // class 3: HBM-bound by construction -- att (2C) + x in (4C) + x out (4C) [+ ln out (2C)] per token; training adds
     // x_mid (4C) and the three saved bf16 activations (6C)
     ProfScope ps(h, st, 3.0 * 2.0 * tokens * C * C, 3,
                  (double)tokens * (2 * C + 4 * C + 4 * C + (nx ? 2 * C : 0) + (train ? 4 * C + 6 * C : 0)));
     BlockTailArgs a;
-    a.att = att;
+    a.att = b.att;
     a.Wo = AH(h, lp.outw); a.W1 = AH(h, lp.m0w); a.W2 = AH(h, lp.m2w);
     a.bo = AF(h, lp.outb); a.g2 = AF(h, lp.ln2w); a.be2 = AF(h, lp.ln2b); a.b1 = AF(h, lp.m0b); a.b2 = AF(h, lp.m2b);
     a.gn = nx ? AF(h, nx->ln1w) : nullptr; a.ben = nx ? AF(h, nx->ln1b) : nullptr;
-    a.x_in = x_in; a.x_out = x_out; a.ln_out = nx ? ln_out : nullptr;
-    a.x_mid = x_mid; a.ln2 = ln2; a.hpre = hpre; a.hact = hact;
-    a.drop = drop; a.site1 = site1; a.site2 = site2;
+    a.x_in = b.x_in; a.x_out = b.x_out; a.ln_out = nx ? b.ln_next : nullptr;
+    if (train) { a.x_mid = b.x_mid; a.ln2 = b.ln2; a.hpre = b.hpre; a.hact = b.hact; }
+    a.drop = drop; a.site1 = b.site[1]; a.site2 = b.site[2];
     CK(launch_block_tail_any(a, tokens, train, h->num_sms, st));
     h->launches++;
 }
@@ -772,11 +800,63 @@ void launch_propagator(tante_handle_s* h, const float* xin, float* x, int B, int
 
 inline unsigned blocks_for(long long n, int per) { return (unsigned)((n + per - 1) / per); }
 
+template <typename TA, int ACT>
+void launch_act_fwd(tante_handle_s* h, const TA* pre, TA* out, long long n, cudaStream_t st) {
+    act_fwd_kernel<TA, ACT><<<blocks_for(n / 4, 256), 256, 0, st>>>(pre, out, n / 4);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+
+// Activation producers.  With `pre` null the GELU is fused into the pass that produces its input (inference); otherwise that
+// pass writes the pre-activation into `pre`, which the backward reads, and act_fwd_kernel writes the activation (training).
+// GEMM, activation epilogue: out[M][N] = act(A W^T + bias)
+template <typename TA, int ACT>
+void gemm_act(tante_handle_s* h, const TA* A, int lda, int64_t w_off, TA* pre, TA* out, int M, int N, int K, const EpiParams& ep,
+              cudaStream_t st) {
+    if (!pre) {
+        gemm<TA>(h, ACT == ACT_GELU_TANH ? EPI_BIAS_GELU_TANH : EPI_BIAS_GELU_ERF, A, lda, w_off, out, N, false, M, N, K, ep, st);
+        return;
+    }
+    gemm<TA>(h, EPI_BIAS, A, lda, w_off, pre, N, false, M, N, K, ep, st);
+    launch_act_fwd<TA, ACT>(h, pre, out, (long long)M * N, st);
+}
+// overlap: adaptive average pooling of a conv grid [n_img][Hc][Wc][Cc] to the patch grid [n_img][Ho][Wo][Cc], then GELU
+template <typename TA>
+void pool_act(tante_handle_s* h, const TA* in, long long n_img, int Hc, int Wc, int Cc, int Ho, int Wo, TA* pre, TA* out,
+              cudaStream_t st) {
+    const long long n4 = n_img * Ho * Wo * Cc / 4;
+    if (pre) wide_pool_kernel<TA, false, false><<<blocks_for(n4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, pre, nullptr, n4);
+    else wide_pool_kernel<TA, true, false><<<blocks_for(n4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, out, nullptr, n4);
+    CK(cudaGetLastError());
+    h->launches++;
+    if (pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, out, n4 * 4, st);
+}
+// decoder stage: sub-pixel matrix S [B*hi*wi][ldS] -> crop + resample (+ bias) to the grid [B][hi*k][wi*k][Cout], then GELU
+template <typename TA>
+void post_act(tante_handle_s* h, const TA* S, int ldS, int B, int hi, int wi, int Cout, int k, int sd, const float* bias, TA* pre,
+              TA* out, cudaStream_t st) {
+    const long long n = (long long)B * (hi * k) * (wi * k) * Cout;
+    if (pre) wide_deconv_post_kernel<TA, false, false><<<blocks_for(n, 256), 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, pre, nullptr, n, sd);
+    else wide_deconv_post_kernel<TA, true, false><<<blocks_for(n, 256), 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, out, nullptr, n, sd);
+    CK(cudaGetLastError());
+    h->launches++;
+    if (pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, out, n, st);
+}
+
+// t_encode FiLM + s_emb + t_emb of the fp32 pre-embedding v [tokens][C] -> residual stream x
+void launch_embed(tante_handle_s* h, const float* v, float* x, int tokens, cudaStream_t st) {
+    const int C = h->C;
+    embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(v, AF(h, h->film_t_off), AF(h, h->s_emb),
+                                                                              AF(h, h->t_emb), x, tokens, h->T, h->L, C);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+
 template <typename TA>
 void launch_head(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, float* deriv_dbg, cudaStream_t st) {
     HeadParams hp{};
     for (int k = 0; k < h->K; ++k) {
-        hp.z[k] = h->z2[k].p;
+        hp.z[k] = io.tape ? io.tape->ord[k].z2act.p : h->z2[k].p;
         hp.w3[k] = AF(h, h->orders[k].decw[2]);
         hp.b3[k] = AF(h, h->orders[k].decb[2]);
     }
@@ -789,6 +869,7 @@ void launch_head(tante_handle_s* h, const StepIO& io, int B, const RolloutState&
     hp.ptrs = io.rollout ? rs.ptrs : nullptr; hp.ring_out = io.ring_out; hp.cum = io.rollout ? rs.cum : nullptr; hp.n_roll = io.n_roll;
     hp.deriv_dbg = deriv_dbg;
     hp.act = io.rollout ? rs.act : nullptr;
+    hp.frames_bs = io.ft.hbs; hp.cur = io.ft.cur;
     const long long rows = (long long)B * h->L * h->geom.R1;
     if (sizeof(TA) == 2) {
         cudaError_t e = cudaSuccess;
@@ -856,129 +937,101 @@ inline void gemm_bigk_f32(tante_handle_s* h, const __nv_bfloat16* A, int lda, in
 
 template <typename TA>
 void run_encoder_wide(tante_handle_s* h, const StepIO& io, int B, cudaStream_t st) {
-    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L;
+    REQUIRE(!io.ft.cur, "windowed BPTT is not available at patch_scale >= 16 / with overlap");
+    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T;
     const PatchGeom& g = h->geom;
-    const int tokens = B * T * L;
-    const int H = h->cfg.H, W = h->cfg.W, D = h->D;
-    TA* wb = reinterpret_cast<TA*>(h->wbuf.p);
-    TA* a1 = reinterpret_cast<TA*>(h->a1.p);
-    TA* a2 = reinterpret_cast<TA*>(h->a2.p);
-    float* x = reinterpret_cast<float*>(h->x.p);
-    const int H1 = H / g.k0, W1 = W / g.k0, H2 = H1 / g.k1, W2 = W1 / g.k1;
+    const int tokens = B * T * h->L;
     const long long NI = (long long)B * T;
-    // conv grid of a stage (kernel k, stride s, pad (k - 1) / 2 over an Hin x Win grid); == the patch grid without overlap
-    auto cdim = [](int n, int k, int s) { return (n + 2 * ((k - 1) / 2) - k) / s + 1; };
-    const int Hc1 = cdim(H, g.k0, h->st[0]), Wc1 = cdim(W, g.k0, h->st[0]);
-    const int Hc2 = cdim(H1, g.k1, h->st[1]), Wc2 = cdim(W1, g.k1, h->st[1]);
-    const int Hc3 = cdim(H2, g.k2, h->st[2]), Wc3 = cdim(W2, g.k2, h->st[2]);
-    const bool pool1 = Hc1 != H1 || Wc1 != W1, pool2 = Hc2 != H2 || Wc2 != W2, pool3 = Hc3 != h->Hp || Wc3 != h->Wp;
-    const long long rows1 = NI * Hc1 * Wc1, rows2 = NI * Hc2 * Wc2, rows3 = NI * Hc3 * Wc3;
-    REQUIRE(rows1 * h->K1pad < (1LL << 40) && rows1 < (1LL << 31) && rows2 < (1LL << 31) && rows3 < (1LL << 31),
+    const WideDims d = wide_dims(h, B);
+    REQUIRE(d.rows1 * h->K1pad < (1LL << 40) && d.rows1 < (1LL << 31) && d.rows2 < (1LL << 31) && d.rows3 < (1LL << 31),
             "input too large for the wide conv GEMMs");
-    TA* cg = reinterpret_cast<TA*>(h->cgrid.p);
-    auto pool = [&](const TA* in, int Hc, int Wc, int Cc, int Ho, int Wo, TA* out, float* out32, bool act) {
-        const long long total4 = NI * Ho * Wo * Cc / 4;
-        const unsigned nb = blocks_for(total4, 256);
-        if (out32) wide_pool_kernel<TA, false, true><<<nb, 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, nullptr, out32, total4);
-        else if (act) wide_pool_kernel<TA, true, false><<<nb, 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, out, nullptr, total4);
-        else wide_pool_kernel<TA, false, false><<<nb, 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, out, nullptr, total4);
-        CK(cudaGetLastError());
-        h->launches++;
+    Tape* tp = io.tape;
+    TA* wb = TP<TA>(h->wbuf);
+    TA* cg = TP<TA>(h->cgrid);
+    TA* cols = tp ? TP<TA>(tp->cols) : wb;      // first patch matrix (training keeps it for the weight gradient)
+    TA* a1 = tp ? TP<TA>(tp->a1act) : TP<TA>(h->a1);
+    TA* a2 = tp ? TP<TA>(tp->a2act) : TP<TA>(h->a2);
+    TA* a1pre = tp ? TP<TA>(tp->a1pre) : nullptr;
+    TA* a2pre = tp ? TP<TA>(tp->a2pre) : nullptr;
+    float* v = tp ? FP(tp->v) : FP(h->qkv);     // fp32 pre-embedding (inference: the QKV scratch, free until the first QKV GEMM)
+    float* x = tp ? FP(tp->ord[0].P[0]) : FP(h->x);
+    // conv stage + GELU: GEMM over the patch matrix; with overlap onto the conv grid, then adaptive average pooling
+    auto stage = [&](const TA* A, int Kc, int64_t w_off, const float* bias, int Cc, long long rows, bool pooled, int Hc, int Wc,
+                     int Ho, int Wo, TA* pre, TA* out) {
+        EpiParams e; e.bias = bias;
+        if (!pooled) {
+            gemm_act<TA, ACT_GELU_ERF>(h, A, Kc, w_off, pre, out, (int)rows, Cc, Kc, e, st);
+            return;
+        }
+        gemm<TA>(h, EPI_BIAS, A, Kc, w_off, cg, Cc, false, (int)rows, Cc, Kc, e, st);
+        pool_act<TA>(h, cg, NI, Hc, Wc, Cc, Ho, Wo, pre, out, st);
     };
-    // conv1: (shifted / strided) windows of the ring frames -> [rows1][K1pad] -> GEMM (+ pooling) + GELU -> grid [BT][H1][W1][C1]
-    {
-        const long long total = rows1 * h->K1pad;
-        wide_im2col_cf_kernel<TA><<<blocks_for(total, 256), 256, 0, st>>>(io.input, io.fcount, T, D, H, W, g.k0, (g.k0 - 1) / 2,
-                                                                         h->K1pad, wb, total, h->st[0], Hc1, Wc1);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-        if (pool1) {
-            gemm<TA>(h, EPI_BIAS, wb, h->K1pad, h->enc_w1wide, cg, C1, false, (int)rows1, C1, h->K1pad, e1, st);
-            pool(cg, Hc1, Wc1, C1, H1, W1, a1, nullptr, true);
-        } else {
-            gemm<TA>(h, EPI_BIAS_GELU_ERF, wb, h->K1pad, h->enc_w1wide, a1, C1, false, (int)rows1, C1, h->K1pad, e1, st);
-        }
-    }
+    // conv1: (shifted / strided) windows of the ring frames -> [rows1][K1pad] -> grid [BT][H1][W1][C1]
+    const long long total = d.rows1 * h->K1pad;
+    wide_im2col_cf_kernel<TA><<<blocks_for(total, 256), 256, 0, st>>>(io.input, io.fcount, T, h->D, h->cfg.H, h->cfg.W, g.k0,
+                                                                     (g.k0 - 1) / 2, h->K1pad, cols, total, h->st[0], d.Hc1, d.Wc1);
+    CK(cudaGetLastError());
+    h->launches++;
+    stage(cols, h->K1pad, h->enc_w1wide, AF(h, h->enc_b[0]), C1, d.rows1, d.pool1, d.Hc1, d.Wc1, d.H1, d.W1, a1pre, a1);
     // conv2
-    {
-        const int K2 = g.k1 * g.k1 * C1;
-        const long long total4 = rows2 * K2 / 4;
-        wide_im2col_cl_kernel<TA><<<blocks_for(total4, 256), 256, 0, st>>>(a1, H1, W1, C1, g.k1, (g.k1 - 1) / 2, wb, total4, h->st[1], Hc2, Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-        if (pool2) {
-            gemm<TA>(h, EPI_BIAS, wb, K2, h->enc_w[1], cg, C2, false, (int)rows2, C2, K2, e2, st);
-            pool(cg, Hc2, Wc2, C2, H2, W2, a2, nullptr, true);
-        } else {
-            gemm<TA>(h, EPI_BIAS_GELU_ERF, wb, K2, h->enc_w[1], a2, C2, false, (int)rows2, C2, K2, e2, st);
-        }
-    }
+    const int K2 = g.k1 * g.k1 * C1, K3 = g.k2 * g.k2 * C2;
+    wide_im2col_cl_kernel<TA><<<blocks_for(d.rows2 * K2 / 4, 256), 256, 0, st>>>(a1, d.H1, d.W1, C1, g.k1, (g.k1 - 1) / 2, wb,
+                                                                                d.rows2 * K2 / 4, h->st[1], d.Hc2, d.Wc2);
+    CK(cudaGetLastError());
+    h->launches++;
+    stage(wb, K2, h->enc_w[1], AF(h, h->enc_b[1]), C2, d.rows2, d.pool2, d.Hc2, d.Wc2, d.H2, d.W2, a2pre, a2);
     // conv3 + t_encode FiLM + embeddings -> residual stream
-    {
-        const int K3 = g.k2 * g.k2 * C2;
-        const long long total4 = rows3 * K3 / 4;
-        wide_im2col_cl_kernel<TA><<<blocks_for(total4, 256), 256, 0, st>>>(a2, H2, W2, C2, g.k2, (g.k2 - 1) / 2, wb, total4, h->st[2], Hc3, Wc3);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
-        if (pool3) {
-            // overlap: conv grid -> adaptive average pooling -> fp32 pre-embedding -> embed pass
-            float* v = reinterpret_cast<float*>(h->qkv.p);
-            if (sizeof(TA) == 2 && K3 > 1024) {
-                REQUIRE((size_t)rows3 * C * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
-                float* acc = reinterpret_cast<float*>(h->kscratch.p);
-                gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], acc, (int)rows3, C, K3, e3.bias, st);
-                f32_to_ta_kernel<TA, false><<<blocks_for(rows3 * C / 4, 256), 256, 0, st>>>(acc, cg, rows3 * C / 4);
-                CK(cudaGetLastError());
-                h->launches++;
-            } else {
-                gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], cg, C, false, (int)rows3, C, K3, e3, st);
-            }
-            pool(cg, Hc3, Wc3, C, h->Hp, h->Wp, nullptr, v, false);
-            embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(v, AF(h, h->film_t_off), AF(h, h->s_emb),
-                                                                                      AF(h, h->t_emb), x, tokens, T, L, C);
-            CK(cudaGetLastError());
-            h->launches++;
-        } else if (sizeof(TA) == 2 && K3 > 1024) {
-            // K = 2048 (patch_scale 64) exceeds the resident weight slice of the tcgen05 GEMM: K blocks through an fp32
-            // scratch, then the embed pass
-            float* v = reinterpret_cast<float*>(h->qkv.p);
-            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], v, tokens, C, K3, e3.bias, st);
-            embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(v, AF(h, h->film_t_off), AF(h, h->s_emb),
-                                                                                      AF(h, h->t_emb), x, tokens, T, L, C);
+    wide_im2col_cl_kernel<TA><<<blocks_for(d.rows3 * K3 / 4, 256), 256, 0, st>>>(a2, d.H2, d.W2, C2, g.k2, (g.k2 - 1) / 2, wb,
+                                                                                d.rows3 * K3 / 4, h->st[2], d.Hc3, d.Wc3);
+    CK(cudaGetLastError());
+    h->launches++;
+    EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
+    // K = 2048 (patch_scale 64) exceeds the resident weight slice of the tcgen05 GEMM: K blocks through an fp32 scratch
+    const bool bigk = sizeof(TA) == 2 && K3 > 1024;
+    if (!d.pool3 && !bigk && !tp) {      // the embed epilogue writes the residual stream directly
+        e3.film = AF(h, h->film_t_off); e3.s_emb = AF(h, h->s_emb); e3.t_emb = AF(h, h->t_emb);
+        e3.T = T; e3.L = h->L; e3.ldr = C;
+        gemm<TA>(h, EPI_EMBED, wb, K3, h->enc_w[2], x, C, true, tokens, C, K3, e3, st);
+        return;
+    }
+    if (d.pool3) {
+        // overlap: conv grid -> adaptive average pooling -> fp32 pre-embedding
+        if (bigk) {
+            REQUIRE((size_t)d.rows3 * C * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
+            float* acc = FP(h->kscratch);
+            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], acc, (int)d.rows3, C, K3, e3.bias, st);
+            f32_to_ta_kernel<TA, false><<<blocks_for(d.rows3 * C / 4, 256), 256, 0, st>>>(acc, cg, d.rows3 * C / 4);
             CK(cudaGetLastError());
             h->launches++;
         } else {
-            e3.film = AF(h, h->film_t_off); e3.s_emb = AF(h, h->s_emb); e3.t_emb = AF(h, h->t_emb);
-            e3.T = T; e3.L = L; e3.ldr = C;
-            gemm<TA>(h, EPI_EMBED, wb, K3, h->enc_w[2], x, C, true, tokens, C, K3, e3, st);
+            gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], cg, C, false, (int)d.rows3, C, K3, e3, st);
         }
+        const long long n4 = NI * h->Hp * h->Wp * C / 4;
+        wide_pool_kernel<TA, false, true><<<blocks_for(n4, 256), 256, 0, st>>>(cg, d.Hc3, d.Wc3, C, h->Hp, h->Wp, nullptr, v, n4);
+        CK(cudaGetLastError());
+        h->launches++;
+    } else if (bigk) {
+        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], v, tokens, C, K3, e3.bias, st);
+    } else {
+        gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], v, C, true, tokens, C, K3, e3, st);
     }
+    launch_embed(h, v, x, tokens, st);
 }
 
-// decoder of order o on the (modified) last-frame latent dmod [B*L][C] -> derivative field dfield[o] (B, D, H, W)
+// decoder of order o on the (modified) last-frame latent dmod [B*L][C] -> derivative field dfield[o] (B, D, H, W); the stage
+// grids go to the shared scratch (inference) or to the tape of the order (`ot`, training)
 template <typename TA>
-void run_decoder_wide(tante_handle_s* h, int o, const TA* dmod, int B, cudaStream_t st) {
+void run_decoder_wide(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape* ot, cudaStream_t st) {
     const OrderPlan& op = h->orders[o];
     const int C = h->C, C1 = h->C1, C2 = h->C2, L = h->L, D = h->D, Hp = h->Hp, Wp = h->Wp;
     const PatchGeom& g = h->geom;
-    const int H = h->cfg.H, W = h->cfg.W;
-    TA* wb = reinterpret_cast<TA*>(h->wbuf.p);
-    TA* z1 = reinterpret_cast<TA*>(h->z1.p);
-    TA* z2 = reinterpret_cast<TA*>(h->z2[o].p);
-    float* field = reinterpret_cast<float*>(h->dfield.p) + (size_t)o * B * D * H * W;
+    TA* wb = TP<TA>(h->wbuf);
+    TA* z1 = ot ? TP<TA>(ot->z1act) : TP<TA>(h->z1);
+    TA* z2 = ot ? TP<TA>(ot->z2act) : TP<TA>(h->z2[o]);
+    TA* z1pre = ot ? TP<TA>(ot->z1pre) : nullptr;
+    TA* z2pre = ot ? TP<TA>(ot->z2pre) : nullptr;
+    float* field = FP(h->dfield) + (size_t)o * B * D * h->cfg.H * h->cfg.W;
     const int H2 = Hp * g.k2, W2 = Wp * g.k2, H1 = H2 * g.k1, W1 = W2 * g.k1;
-    auto post = [&](const TA* S, int ldS, int hi, int wi, int Cout, int k, int sd, const float* bias, TA* out, float* fld, bool act) {
-        const long long total = (long long)B * (hi * k) * (wi * k) * Cout;
-        const unsigned blocks = blocks_for(total, 256);
-        if (fld) wide_deconv_post_kernel<TA, false, true><<<blocks, 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, nullptr, fld, total, sd);
-        else if (act) wide_deconv_post_kernel<TA, true, false><<<blocks, 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, out, nullptr, total, sd);
-        else wide_deconv_post_kernel<TA, false, false><<<blocks, 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, out, nullptr, total, sd);
-        CK(cudaGetLastError());
-        h->launches++;
-    };
     // With stride == kernel every output sample has ONE tap, so the (replicated) bias rides in the GEMM epilogue; with overlap
     // (stride < kernel) several taps are summed per sample: the GEMM runs bias-free and the pass after it adds bias[co] once (the
     // first Cout entries of the replicated vector are the raw bias).
@@ -987,15 +1040,19 @@ void run_decoder_wide(tante_handle_s* h, int o, const TA* dmod, int B, cudaStrea
     const int N1 = g.k2 * g.k2 * C2, N2 = g.k1 * g.k1 * C1;
     EpiParams ed; ed.bias = ov1 ? AF(h, h->zero_off) : AF(h, op.decb[0]);
     gemm<TA>(h, EPI_BIAS, dmod, C, op.decw[0], wb, N1, false, B * L, N1, C, ed, st);
-    post(wb, N1, Hp, Wp, C2, g.k2, h->st[2], ov1 ? AF(h, op.decb[0]) : nullptr, z1, nullptr, true);
+    post_act<TA>(h, wb, N1, B, Hp, Wp, C2, g.k2, h->st[2], ov1 ? AF(h, op.decb[0]) : nullptr, z1pre, z1, st);
     // dec_conv_2 (k1)
     ed.bias = ov2 ? AF(h, h->zero_off) : AF(h, op.decb[1]);
     gemm<TA>(h, EPI_BIAS, z1, C2, op.decw[1], wb, N2, false, B * H2 * W2, N2, C2, ed, st);
-    post(wb, N2, H2, W2, C1, g.k1, h->st[1], ov2 ? AF(h, op.decb[1]) : nullptr, z2, nullptr, true);
+    post_act<TA>(h, wb, N2, B, H2, W2, C1, g.k1, h->st[1], ov2 ? AF(h, op.decb[1]) : nullptr, z2pre, z2, st);
     // dec_conv_3 (k0): output width k0*k0*D padded to NOpad, bias added after the resample (its weights sum to one)
     EpiParams e3; e3.bias = AF(h, h->zero_off);
     gemm<TA>(h, EPI_BIAS, z2, C1, op.w3nk, wb, h->NOpad, false, B * H1 * W1, h->NOpad, C1, e3, st);
-    post(wb, h->NOpad, H1, W1, D, g.k0, h->st[0], AF(h, op.decb[2]), nullptr, field, false);
+    const long long n = (long long)B * (H1 * g.k0) * (W1 * g.k0) * D;
+    wide_deconv_post_kernel<TA, false, true><<<blocks_for(n, 256), 256, 0, st>>>(wb, h->NOpad, H1, W1, D, g.k0, AF(h, op.decb[2]),
+                                                                               nullptr, field, n, h->st[0]);
+    CK(cudaGetLastError());
+    h->launches++;
 }
 
 // ---- enc_dec_type = 'fno' (fno.cuh) ----
@@ -1055,6 +1112,14 @@ void run_spectral(tante_handle_s* h, const SpecPlan& sp, const SpecView& in, lon
     else spec_out_kernel<TA, false, false><<<nb, 256, 0, st>>>(Bc, in, AF(h, sp.w0), AF(h, sp.b0), sp.Cin, sp.Cout, H, W, m2, twW, out, nullptr, to, conv_done);
     CK(cudaGetLastError());
     h->launches += 5;
+}
+
+// one SpectralLayer + GELU (activation producer, see gemm_act)
+template <typename TA>
+void spectral_act(tante_handle_s* h, const SpecPlan& sp, const SpecView& in, long long N, int H, int W, int level, TA* pre, TA* out,
+                  cudaStream_t st) {
+    run_spectral<TA>(h, sp, in, N, H, W, level, !pre, pre ? pre : out, nullptr, st);
+    if (pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, out, N * H * W * sp.Cout, st);
 }
 
 // conv over a channels-last grid as gather + GEMM; K beyond the tcgen05 GEMM's resident slice (1024) runs in K blocks
@@ -1123,71 +1188,74 @@ void conv_cl_gemm(tante_handle_s* h, int epi, const TA* grid, int Hs, int Ws, in
 
 template <typename TA>
 void run_encoder_fno(tante_handle_s* h, const StepIO& io, int B, cudaStream_t st) {
-    const int C = h->C, C1 = h->C1, C2 = h->C2, C8 = h->C / 8, T = h->T, L = h->L, D = h->D;
+    REQUIRE(!io.ft.cur, "windowed BPTT is not available with enc_dec_type='fno'");
+    const int C = h->C, C1 = h->C1, C2 = h->C2, C8 = h->C / 8, T = h->T, L = h->L;
     const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0;
     const int tokens = B * T * L;
     const long long NI = (long long)B * T;
-    float* x = reinterpret_cast<float*>(h->x.p);
-    TA* g0 = reinterpret_cast<TA*>(h->fg0.p);      // [NI][H][W][C8]
-    TA* g1 = reinterpret_cast<TA*>(h->fg1.p);      // [NI][H1][W1][C1]
-    TA* g2 = reinterpret_cast<TA*>(h->fg2.p);      // [NI][H1][W1][C2]
+    Tape* tp = io.tape;
+    TA* g0 = tp ? TP<TA>(tp->f0act) : TP<TA>(h->fg0);      // [NI][H][W][C8]
+    TA* g1 = tp ? TP<TA>(tp->a1act) : TP<TA>(h->fg1);      // [NI][H1][W1][C1]
+    TA* g2 = tp ? TP<TA>(tp->a2act) : TP<TA>(h->fg2);      // [NI][H1][W1][C2]
+    TA* g0pre = tp ? TP<TA>(tp->f0pre) : nullptr;
+    TA* g1pre = tp ? TP<TA>(tp->a1pre) : nullptr;
+    TA* g2pre = tp ? TP<TA>(tp->a2pre) : nullptr;
+    float* v = tp ? FP(tp->v) : FP(h->qkv);                 // fp32 pre-embedding (inference: the QKV scratch)
+    float* x = tp ? FP(tp->ord[0].P[0]) : FP(h->x);
     fno_twiddles(h);
     // enc_spectral_1 + GELU on the (ring) frames  (enc_dec_fno.py:258-259)
     SpecView v0{io.input, 0, io.fcount, T};
-    run_spectral<TA>(h, h->fes1, v0, NI, H, W, 0, true, g0, nullptr, st);
+    spectral_act<TA>(h, h->fes1, v0, NI, H, W, 0, g0pre, g0, st);
     // enc_conv_1 + GELU (:260-261)
     EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-    conv_cl_gemm<TA>(h, EPI_BIAS_GELU_ERF, g0, H, W, C8, p0, h->enc_w[0], g1, C1, false, NI, e1, st, h->st[0]);
+    conv_cl_gemm<TA>(h, g1pre ? EPI_BIAS : EPI_BIAS_GELU_ERF, g0, H, W, C8, p0, h->enc_w[0], g1pre ? g1pre : g1, C1, false, NI, e1,
+                     st, h->st[0]);
+    if (g1pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, g1pre, g1, NI * H1 * W1 * C1, st);
     // enc_spectral_2 + GELU (:263-264)
     SpecView v1{g1, 1, nullptr, 1};
-    run_spectral<TA>(h, h->fes2, v1, NI, H1, W1, 1, true, g2, nullptr, st);
+    spectral_act<TA>(h, h->fes2, v1, NI, H1, W1, 1, g2pre, g2, st);
     // enc_conv_2 (:265) + t_encode FiLM + embeddings -> residual stream
     EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-    if ((sizeof(TA) == 2 && p1 * p1 * C2 > 1024) || h->st[1] != p1) {      // (split-K or pooled: fp32 pre-embedding, then the embed pass)
-        float* v = reinterpret_cast<float*>(h->qkv.p);
-        conv_cl_gemm<TA>(h, EPI_BIAS, g2, H1, W1, C2, p1, h->enc_w[1], v, C, true, NI, e2, st, h->st[1]);
-        embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(v, AF(h, h->film_t_off), AF(h, h->s_emb),
-                                                                                  AF(h, h->t_emb), x, tokens, T, L, C);
-        CK(cudaGetLastError());
-        h->launches++;
-    } else {
+    if (!tp && !(sizeof(TA) == 2 && p1 * p1 * C2 > 1024) && h->st[1] == p1) {      // the embed epilogue writes x directly
         e2.film = AF(h, h->film_t_off); e2.s_emb = AF(h, h->s_emb); e2.t_emb = AF(h, h->t_emb);
         e2.T = T; e2.L = L; e2.ldr = C;
         conv_cl_gemm<TA>(h, EPI_EMBED, g2, H1, W1, C2, p1, h->enc_w[1], x, C, true, NI, e2, st);
+        return;
     }
+    // (training, split-K or pooled: fp32 pre-embedding, then the embed pass)
+    conv_cl_gemm<TA>(h, EPI_BIAS, g2, H1, W1, C2, p1, h->enc_w[1], v, C, true, NI, e2, st, h->st[1]);
+    launch_embed(h, v, x, tokens, st);
 }
 
-// dec_FNO.forward (enc_dec_fno.py:303-323) of order o on the last-frame latent dmod [B*L][C] -> dfield[o] (B, D, H, W)
+// dec_FNO.forward (enc_dec_fno.py:303-323) of order o on the last-frame latent dmod [B*L][C] -> dfield[o] (B, D, H, W); the
+// stage grids go to the shared scratch (inference) or to the tape of the order (`ot`, training)
 template <typename TA>
-void run_decoder_fno(tante_handle_s* h, int o, const TA* dmod, int B, cudaStream_t st) {
+void run_decoder_fno(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape* ot, cudaStream_t st) {
     const OrderPlan& op = h->orders[o];
     const int C = h->C, C1 = h->C1, C2 = h->C2, C8 = h->C / 8, L = h->L, D = h->D, Hp = h->Hp, Wp = h->Wp;
     const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0;
-    TA* wb = reinterpret_cast<TA*>(h->wbuf.p);
-    TA* g0 = reinterpret_cast<TA*>(h->fg0.p);      // [B][H][W][C8]
-    TA* g1 = reinterpret_cast<TA*>(h->fg1.p);      // [B][H1][W1][C1]
-    TA* g2 = reinterpret_cast<TA*>(h->fg2.p);      // [B][H1][W1][C2]
-    float* field = reinterpret_cast<float*>(h->dfield.p) + (size_t)o * B * D * H * W;
-    auto post = [&](const TA* S, int ldS, int hi, int wi, int Cout, int k, int sd, const float* bias, TA* out) {
-        const long long total = (long long)B * (hi * k) * (wi * k) * Cout;
-        wide_deconv_post_kernel<TA, true, false><<<blocks_for(total, 256), 256, 0, st>>>(S, ldS, hi, wi, Cout, k, bias, out, nullptr, total, sd);
-        CK(cudaGetLastError());
-        h->launches++;
-    };
+    TA* wb = TP<TA>(h->wbuf);
+    TA* g2 = ot ? TP<TA>(ot->z1act) : TP<TA>(h->fg2);      // [B][H1][W1][C2]
+    TA* g1 = ot ? TP<TA>(ot->z2act) : TP<TA>(h->fg1);      // [B][H1][W1][C1]
+    TA* g0 = ot ? TP<TA>(ot->f0act) : TP<TA>(h->fg0);      // [B][H][W][C8]
+    TA* g2pre = ot ? TP<TA>(ot->z1pre) : nullptr;
+    TA* g1pre = ot ? TP<TA>(ot->z2pre) : nullptr;
+    TA* g0pre = ot ? TP<TA>(ot->f0pre) : nullptr;
+    float* field = FP(h->dfield) + (size_t)o * B * D * H * W;
     // (overlapped stages: bias-free GEMM, bias once per output sample in the resample pass -- see run_decoder_wide)
     const bool ov1 = h->st[1] != p1, ov0 = h->st[0] != p0;
     // dec_conv_1 (p1) + GELU
     const int N1 = p1 * p1 * C2, N2 = p0 * p0 * C8;
     EpiParams ed; ed.bias = ov1 ? AF(h, h->zero_off) : AF(h, op.decb[0]);
     gemm<TA>(h, EPI_BIAS, dmod, C, op.decw[0], wb, N1, false, B * L, N1, C, ed, st);
-    post(wb, N1, Hp, Wp, C2, p1, h->st[1], ov1 ? AF(h, op.decb[0]) : nullptr, g2);
+    post_act<TA>(h, wb, N1, B, Hp, Wp, C2, p1, h->st[1], ov1 ? AF(h, op.decb[0]) : nullptr, g2pre, g2, st);
     // dec_spectral_1 + GELU
     SpecView v2{g2, 1, nullptr, 1};
-    run_spectral<TA>(h, op.fs1, v2, B, H1, W1, 1, true, g1, nullptr, st);
+    spectral_act<TA>(h, op.fs1, v2, B, H1, W1, 1, g1pre, g1, st);
     // dec_conv_2 (p0) + GELU
     ed.bias = ov0 ? AF(h, h->zero_off) : AF(h, op.decb[1]);
     gemm<TA>(h, EPI_BIAS, g1, C1, op.decw[1], wb, N2, false, B * H1 * W1, N2, C1, ed, st);
-    post(wb, N2, H1, W1, C8, p0, h->st[0], ov0 ? AF(h, op.decb[1]) : nullptr, g0);
+    post_act<TA>(h, wb, N2, B, H1, W1, C8, p0, h->st[0], ov0 ? AF(h, op.decb[1]) : nullptr, g0pre, g0, st);
     // dec_spectral_2 -> derivative field
     SpecView v0{g0, 1, nullptr, 1};
     run_spectral<TA>(h, op.fs2, v0, B, H, W, 0, false, nullptr, field, st);
@@ -1208,190 +1276,246 @@ void launch_emit_wide(tante_handle_s* h, const StepIO& io, int B, const RolloutS
     h->launches++;
 }
 
-// One TANTE step (reference models/tante.py:125-176) as a launch sequence on `st`.
+// enc_CNN.forward (enc_dec_cnn.py:217-229) + t_encode FiLM + s_emb + t_emb (tante.py:132-141) -> residual stream
 template <typename TA>
-void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, cudaStream_t st) {
-    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L, K = h->K, Hm = h->Hm;
+void run_encoder_cnn(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, cudaStream_t st) {
+    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L;
     const PatchGeom& g = h->geom;
     const int tokens = B * T * L;
-    float* x = reinterpret_cast<float*>(h->x.p);
-    TA* ln = reinterpret_cast<TA*>(h->ln.p);
-    TA* qkv = reinterpret_cast<TA*>(h->qkv.p);
-    TA* att = reinterpret_cast<TA*>(h->att.p);
-    TA* hid = reinterpret_cast<TA*>(h->hid.p);
-    TA* a1 = reinterpret_cast<TA*>(h->a1.p);
-    TA* a2 = reinterpret_cast<TA*>(h->a2.p);
-
-    // --- encoder (enc_dec_cnn.py:217-229) + t_encode FiLM + s_emb + t_emb (tante.py:132-141) ---
-    if (h->fno) {
-        run_encoder_fno<TA>(h, io, B, st);
-    } else if (h->wide) {
-        run_encoder_wide<TA>(h, io, B, st);
-    } else {
+    const int K2 = g.k1 * g.k1 * C1, K3 = g.k2 * g.k2 * C2;
+    Tape* tp = io.tape;
+    TA* a1 = tp ? TP<TA>(tp->a1act) : TP<TA>(h->a1);
+    TA* a2 = tp ? TP<TA>(tp->a2act) : TP<TA>(h->a2);
+    TA* a1pre = tp ? TP<TA>(tp->a1pre) : nullptr;
+    TA* a2pre = tp ? TP<TA>(tp->a2pre) : nullptr;
+    float* x = tp ? FP(tp->ord[0].P[0]) : FP(h->x);
+    const bool cached = io.rollout && rs.enc_count != nullptr;
+    const bool prof = h->prof_on;
+    if (!tp && sizeof(TA) == 4 && C1 == 64) {
+        // fp32 inference: one FFMA kernel for enc_conv_1 + GELU (specialised for C/4 = 64)
         const int P = g.k0 * g.k1 * g.k2;
-        int WC = std::max(1, 128 / g.R1);
-        WC = std::min(WC, g.Wp);
+        const int WC = std::min(std::max(1, 128 / g.R1), g.Wp);
         const int K1 = g.k0 * g.k0 * g.D;
         const size_t smem = (size_t)(((g.D * P * (P * WC + 1) + 3) & ~3) + C1 * K1 + C1) * sizeof(float) +
                             (size_t)WC * g.R1 * C1 * sizeof(TA);
         dim3 grid(B * T * g.Hp, (g.Wp + WC - 1) / WC);
-        const bool cached = io.rollout && rs.enc_count != nullptr;
-        if (sizeof(TA) == 2 || C1 != 64) {      // (the FFMA patch kernel below is specialised for C/4 = 64)
-            // tensor mode: enc_conv_1 as im2col (coalesced tiles, bf16 -- what the reference's autocast feeds its conv) + a
-            // thin tcgen05 GEMM with the GELU in its epilogue; the FFMA kernel below is 64 erf-GELUs + 1024 FMAs per row
-            const long long rows_in = (long long)tokens * g.R1;
-            REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv GEMM");
-            TA* icols = reinterpret_cast<TA*>(h->icols.p);
-            const int* el = cached ? rs.enc_list : nullptr;
-            const int* ec = cached ? rs.enc_count : nullptr;
-            const int* fc = cached ? nullptr : io.fcount;
-            if (P >= 4) conv1_im2col_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(io.input, g, icols, rows_in, el, ec, fc);
-            else conv1_im2col_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(io.input, g, icols, rows_in, el, ec, fc);
-            CK(cudaGetLastError());
-            h->launches++;
-            EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-            const bool prof = h->prof_on;
-            if (cached) { e1.m_dev = rs.enc_count; e1.m_rows = L * g.R1; h->prof_on = false; }
-            gemm<TA>(h, EPI_BIAS_GELU_ERF, icols, kHeadPad, h->enc_w1pad, a1, C1, false, (int)rows_in, C1, kHeadPad, e1, st);
-            h->prof_on = prof;
-        } else {
-            patch_embed_conv1_kernel<TA><<<grid, 128, smem, st>>>(io.input, io.fcount, g, AF(h, h->enc_w[0]),
-                                                                  AF(h, h->enc_b[0]), WC, a1, cached ? rs.enc_list : nullptr,
-                                                                  cached ? rs.enc_count : nullptr);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
-        EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-        EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
-        if (cached) {
-            // Rollout: only the frames that entered the window are encoded (their count lives on the device: the
-            // GEMMs clip M to it); everything else comes out of the per-slot cache.  The encoder output of a frame
-            // does not depend on its window position -- FiLM(t) and the embeddings are applied afterwards.
-            e2.m_dev = rs.enc_count; e2.m_rows = L * g.R2;
-            e3.m_dev = rs.enc_count; e3.m_rows = L;
-            float* cnew = reinterpret_cast<float*>(h->qkv.p);       // scratch: free until the first QKV GEMM
-            const bool prof = h->prof_on;
-            h->prof_on = false;      // the row count of these two GEMMs lives on the device: keep them out of the FLOP tally
-            gemm<TA>(h, EPI_BIAS_GELU_ERF, a1, g.k1 * g.k1 * C1, h->enc_w[1], a2, C2, false, tokens * g.R2, C2, g.k1 * g.k1 * C1, e2, st);
-            gemm<TA>(h, EPI_BIAS, a2, g.k2 * g.k2 * C2, h->enc_w[2], cnew, C, true, tokens, C, g.k2 * g.k2 * C2, e3, st);
-            h->prof_on = prof;
-            const long long tot4 = (long long)tokens * (C / 4);
-            REQUIRE(tot4 < (1LL << 31), "latent too large for the 32-bit indexing of the cached embed pass");
-            embed_cached_kernel<<<(unsigned)std::min<long long>((tot4 + 255) / 256, 32LL * h->num_sms), 256, 0, st>>>(
-                cnew, reinterpret_cast<float*>(h->enc_cache.p), rs.enc_map, io.fcount, AF(h, h->film_t_off), AF(h, h->s_emb),
-                AF(h, h->t_emb), x, B, T, L, C, rs.act);
-            CK(cudaGetLastError());
-            h->launches++;
-        } else {
-            gemm<TA>(h, EPI_BIAS_GELU_ERF, a1, g.k1 * g.k1 * C1, h->enc_w[1], a2, C2, false, tokens * g.R2, C2, g.k1 * g.k1 * C1, e2, st);
-            e3.film = AF(h, h->film_t_off); e3.s_emb = AF(h, h->s_emb); e3.t_emb = AF(h, h->t_emb);
-            e3.T = T; e3.L = L; e3.ldr = C;
-            // the embed epilogue writes the fp32 residual stream directly
-            gemm<TA>(h, EPI_EMBED, a2, g.k2 * g.k2 * C2, h->enc_w[2], x, C, true, tokens, C, g.k2 * g.k2 * C2, e3, st);
-        }
+        patch_embed_conv1_kernel<TA><<<grid, 128, smem, st>>>(io.input, io.fcount, g, AF(h, h->enc_w[0]), AF(h, h->enc_b[0]), WC,
+                                                              a1, cached ? rs.enc_list : nullptr, cached ? rs.enc_count : nullptr);
+        CK(cudaGetLastError());
+        h->launches++;
+    } else {
+        // enc_conv_1 as im2col (coalesced tiles, bf16 -- what the reference's autocast feeds its conv; training keeps it for the
+        // weight gradient) + a thin GEMM over the zero-padded patch matrix; the FFMA kernel above is 64 erf-GELUs + 1024 FMAs
+        // per row
+        const long long rows_in = (long long)tokens * g.R1;
+        REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv GEMM");
+        TA* cols = tp ? TP<TA>(tp->cols) : TP<TA>(h->icols);
+        const int* el = cached ? rs.enc_list : nullptr;
+        const int* ec = cached ? rs.enc_count : nullptr;
+        const int* fc = cached ? nullptr : io.fcount;
+        if (g.k0 * g.k1 * g.k2 >= 4) conv1_im2col_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(io.input, g, cols, rows_in, el, ec, fc, io.ft);
+        else conv1_im2col_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(io.input, g, cols, rows_in, el, ec, fc, io.ft);
+        CK(cudaGetLastError());
+        h->launches++;
+        EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
+        if (cached) { e1.m_dev = rs.enc_count; e1.m_rows = L * g.R1; h->prof_on = false; }
+        gemm_act<TA, ACT_GELU_ERF>(h, cols, kHeadPad, h->enc_w1pad, a1pre, a1, (int)rows_in, C1, kHeadPad, e1, st);
+        h->prof_on = prof;
     }
-    if (h->debug) CK(cudaMemcpyAsync(h->dbg_in.p, x, (size_t)tokens * C * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
+    EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
+    if (cached) {
+        // Rollout: only the frames that entered the window are encoded (their count lives on the device: the
+        // GEMMs clip M to it); everything else comes out of the per-slot cache.  The encoder output of a frame
+        // does not depend on its window position -- FiLM(t) and the embeddings are applied afterwards.
+        e2.m_dev = rs.enc_count; e2.m_rows = L * g.R2;
+        e3.m_dev = rs.enc_count; e3.m_rows = L;
+        float* cnew = FP(h->qkv);       // scratch: free until the first QKV GEMM
+        h->prof_on = false;      // the row count of these two GEMMs lives on the device: keep them out of the FLOP tally
+        gemm<TA>(h, EPI_BIAS_GELU_ERF, a1, K2, h->enc_w[1], a2, C2, false, tokens * g.R2, C2, K2, e2, st);
+        gemm<TA>(h, EPI_BIAS, a2, K3, h->enc_w[2], cnew, C, true, tokens, C, K3, e3, st);
+        h->prof_on = prof;
+        const long long tot4 = (long long)tokens * (C / 4);
+        REQUIRE(tot4 < (1LL << 31), "latent too large for the 32-bit indexing of the cached embed pass");
+        embed_cached_kernel<<<(unsigned)std::min<long long>((tot4 + 255) / 256, 32LL * h->num_sms), 256, 0, st>>>(
+            cnew, FP(h->enc_cache), rs.enc_map, io.fcount, AF(h, h->film_t_off), AF(h, h->s_emb), AF(h, h->t_emb), x, B, T, L, C,
+            rs.act);
+        CK(cudaGetLastError());
+        h->launches++;
+        return;
+    }
+    gemm_act<TA, ACT_GELU_ERF>(h, a1, K2, h->enc_w[1], a2pre, a2, tokens * g.R2, C2, K2, e2, st);
+    if (tp) {      // training keeps the fp32 pre-embedding
+        gemm<TA>(h, EPI_BIAS, a2, K3, h->enc_w[2], tp->v.p, C, true, tokens, C, K3, e3, st);
+        launch_embed(h, FP(tp->v), x, tokens, st);
+    } else {       // the embed epilogue writes the fp32 residual stream directly
+        e3.film = AF(h, h->film_t_off); e3.s_emb = AF(h, h->s_emb); e3.t_emb = AF(h, h->t_emb);
+        e3.T = T; e3.L = L; e3.ldr = C;
+        gemm<TA>(h, EPI_EMBED, a2, K3, h->enc_w[2], x, C, true, tokens, C, K3, e3, st);
+    }
+}
 
-    float* rt = reinterpret_cast<float*>(h->rt.p);
+// One TANTE step (reference models/tante.py:125-176) as a launch sequence on `st`: tante_forward, the rollout (eager and the
+// captured step body) and, with io.tape set, the taped training calls.  Inference works in place on h->x and the shared
+// scratch buffers; a taped call runs the same kernels out of place into the tape slots, so that every input of a later
+// derivative survives, and keeps the GELU pre-activations next to the activations.
+template <typename TA>
+void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, cudaStream_t st) {
+    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L, K = h->K, Hm = h->Hm;
+    const int tokens = B * T * L;
+    Tape* tp = io.tape;
+    DropCfg drop;      // inference: none
+    if (tp) drop = tp->drop = make_drop_cfg(h->drop_p, h->drop_seed);
+    float* x = FP(h->x);
+
+    // --- encoder + t_encode FiLM + s_emb + t_emb ---
+    if (h->fno) run_encoder_fno<TA>(h, io, B, st);
+    else if (h->wide) run_encoder_wide<TA>(h, io, B, st);
+    else run_encoder_cnn<TA>(h, io, B, rs, st);
+    if (!tp && h->debug) CK(cudaMemcpyAsync(h->dbg_in.p, x, (size_t)tokens * C * sizeof(float), cudaMemcpyDeviceToDevice, st));
+
+    float* rt = FP(h->rt);
     for (int o = 0; o < K; ++o) {
         const OrderPlan& op = h->orders[o];
+        OrderTape* ot = tp ? &tp->ord[o] : nullptr;
         // --- Attn_Backbone.forward (attn_backbone.py:134-191) ---
-        launch_propagator(h, x, x, B, 0, op, st);
-        launch_propagator(h, x, x, B, 1, op, st);
-        launch_propagator(h, x, x, B, 2, op, st);
+        // propagators H, W, T: in place, or (encoder output | previous order's output) -> P[1] -> P[2] -> X[0]
+        float* px[4] = {x, x, x, x};
+        if (ot) {
+            px[0] = o == 0 ? FP(ot->P[0]) : FP(tp->ord[o - 1].X.back());
+            px[1] = FP(ot->P[1]); px[2] = FP(ot->P[2]); px[3] = FP(ot->X[0]);
+        }
+        for (int a = 0; a < 3; ++a) launch_propagator(h, px[a], px[a + 1], B, a, op, st);
         // In tensor mode every LayerNorm except the first one of an order is folded into the epilogue of the
         // residual GEMM that produces its input (EPI_BIAS_RESID_LN): the row is still on chip there.
         const bool kFuseLN = sizeof(TA) == 2 && C <= 256;      // (one CTA tile must hold the whole row)
         bool ln_ready = false;
-        for (size_t li = 0; li < op.layers.size(); ++li) {
+        const size_t nl = op.layers.size();
+        for (size_t li = 0; li < nl; ++li) {
             const LayerPlan& lp = op.layers[li];
-            if (lp.axis == 'C') {      // channel attention: its own width, its own LayerNorms (channel_axis.cuh)
-                run_channel_layer<TA>(h, lp, x, x, tokens, st);
+            const LayerBufs<TA> b = layer_bufs<TA>(h, ot, o, li);
+            if (lp.axis == 'C') {
+                // channel attention: its own width, its own LayerNorms (channel_axis.cuh); training keeps only the layer's fp32
+                // input -- the backward recomputes the block chunk by chunk
+                REQUIRE(drop.p <= 0.f, "dropout with an attention axis C layer is not implemented");
+                run_channel_layer<TA>(h, lp, b.x_in, b.x_out, tokens, st);
                 ln_ready = false;
                 continue;
             }
             // the next layer's LN1 rides in this layer's last epilogue -- unless that layer is a channel layer (other width)
-            const bool nx_ok = li + 1 < op.layers.size() && op.layers[li + 1].axis != 'C';
-            if (!ln_ready) launch_layernorm<TA>(h, x, lp.ln1w, lp.ln1b, ln, tokens, st);
+            const bool nx_ok = li + 1 < nl && op.layers[li + 1].axis != 'C';
+            if (!ln_ready) launch_layernorm<TA>(h, b.x_in, lp.ln1w, lp.ln1b, b.ln1, tokens, st);
             EpiParams eq; eq.bias = AF(h, lp.inb);
-            gemm<TA>(h, EPI_BIAS, ln, C, lp.inw, qkv, 3 * C, false, tokens, 3 * C, C, eq, st);
-            launch_attention<TA>(h, qkv, att, B, lp.axis, st);
+            gemm<TA>(h, EPI_BIAS, b.ln1, C, lp.inw, b.qkv, 3 * C, false, tokens, 3 * C, C, eq, st);
+            launch_attention<TA>(h, b.qkv, b.att, B, lp.axis, st, drop, b.site[0]);
             if constexpr (sizeof(TA) == 2) {
-                if (h->fuse_tail && C == kBtC && h->Hm == C) {
+                if (h->fuse_tail && C == kBtC && Hm == C) {
                     const LayerPlan* nx = nx_ok ? &op.layers[li + 1] : nullptr;
-                    launch_tail(h, lp, nx, att, x, x, ln, tokens, st);
+                    launch_tail(h, lp, nx, b, tokens, drop, st);
                     ln_ready = nx != nullptr;
                     continue;
                 }
             }
-            EpiParams eo; eo.bias = AF(h, lp.outb); eo.resid = x; eo.ldr = C;
+            if (sizeof(TA) == 2 && drop.p > 0.f) {
+                // Tensor mode with dropout outside the fused tail (mlp_ratio != 1, embed_dim 512, TANTE_FUSE_TAIL=0): the tcgen05 GEMM
+                // epilogues carry no mask generator, so each residual branch is a plain GEMM into a bf16 scratch followed by one
+                // pass  x <- x + mask * branch  (what autocast + nn.Dropout do in the reference); LayerNorms as their own passes.
+                TA* br = TP<TA>(h->hid);
+                const long long n4 = (long long)tokens * C / 4;
+                EpiParams eb; eb.bias = AF(h, lp.outb);
+                gemm<TA>(h, EPI_BIAS, b.att, C, lp.outw, br, C, false, tokens, C, C, eb, st);
+                resid_drop_kernel<TA><<<blocks_for(n4, 256), 256, 0, st>>>(br, b.x_in, b.x_mid, n4, drop, b.site[1]);
+                CK(cudaGetLastError());
+                h->launches++;
+                launch_layernorm<TA>(h, b.x_mid, lp.ln2w, lp.ln2b, b.ln2, tokens, st);
+                EpiParams eh; eh.bias = AF(h, lp.m0b);
+                gemm_act<TA, ACT_GELU_TANH>(h, b.ln2, C, lp.m0w, b.hpre, b.hact, tokens, Hm, C, eh, st);
+                eb.bias = AF(h, lp.m2b);
+                gemm<TA>(h, EPI_BIAS, b.hact, Hm, lp.m2w, br, C, false, tokens, C, Hm, eb, st);
+                resid_drop_kernel<TA><<<blocks_for(n4, 256), 256, 0, st>>>(br, b.x_mid, b.x_out, n4, drop, b.site[2]);
+                CK(cudaGetLastError());
+                h->launches++;
+                ln_ready = false;
+                continue;
+            }
+            EpiParams eo; eo.bias = AF(h, lp.outb); eo.resid = b.x_in; eo.ldr = C;
+            eo.drop = drop; eo.drop_site = b.site[1];
             if (kFuseLN) {
-                eo.ln_gamma = AF(h, lp.ln2w); eo.ln_beta = AF(h, lp.ln2b); eo.ln_out = ln;
-                gemm<TA>(h, EPI_BIAS_RESID_LN, att, C, lp.outw, x, C, true, tokens, C, C, eo, st);
+                eo.ln_gamma = AF(h, lp.ln2w); eo.ln_beta = AF(h, lp.ln2b); eo.ln_out = b.ln2;
+                gemm<TA>(h, EPI_BIAS_RESID_LN, b.att, C, lp.outw, b.x_mid, C, true, tokens, C, C, eo, st);
             } else {
-                gemm<TA>(h, EPI_BIAS_RESID, att, C, lp.outw, x, C, true, tokens, C, C, eo, st);
-                launch_layernorm<TA>(h, x, lp.ln2w, lp.ln2b, ln, tokens, st);
+                gemm<TA>(h, EPI_BIAS_RESID, b.att, C, lp.outw, b.x_mid, C, true, tokens, C, C, eo, st);
+                launch_layernorm<TA>(h, b.x_mid, lp.ln2w, lp.ln2b, b.ln2, tokens, st);
             }
             EpiParams e0; e0.bias = AF(h, lp.m0b);
-            gemm<TA>(h, EPI_BIAS_GELU_TANH, ln, C, lp.m0w, hid, Hm, false, tokens, Hm, C, e0, st);
-            EpiParams e2; e2.bias = AF(h, lp.m2b); e2.resid = x; e2.ldr = C;
+            gemm_act<TA, ACT_GELU_TANH>(h, b.ln2, C, lp.m0w, b.hpre, b.hact, tokens, Hm, C, e0, st);
+            EpiParams e2; e2.bias = AF(h, lp.m2b); e2.resid = b.x_mid; e2.ldr = C;
+            e2.drop = drop; e2.drop_site = b.site[2];
             if (kFuseLN && nx_ok && Hm == C) {      // (the LN-fused epilogue needs the K = C weight slice resident)
                 const LayerPlan& nx = op.layers[li + 1];
-                e2.ln_gamma = AF(h, nx.ln1w); e2.ln_beta = AF(h, nx.ln1b); e2.ln_out = ln;
-                gemm<TA>(h, EPI_BIAS_RESID_LN, hid, Hm, lp.m2w, x, C, true, tokens, C, Hm, e2, st);
+                e2.ln_gamma = AF(h, nx.ln1w); e2.ln_beta = AF(h, nx.ln1b); e2.ln_out = b.ln_next;
+                gemm<TA>(h, EPI_BIAS_RESID_LN, b.hact, Hm, lp.m2w, b.x_out, C, true, tokens, C, Hm, e2, st);
                 ln_ready = true;
             } else {
-                gemm<TA>(h, EPI_BIAS_RESID, hid, Hm, lp.m2w, x, C, true, tokens, C, Hm, e2, st);
+                gemm<TA>(h, EPI_BIAS_RESID, b.hact, Hm, lp.m2w, b.x_out, C, true, tokens, C, Hm, e2, st);
                 ln_ready = false;
             }
         }
-        // --- head of order o (tante.py:147-154) ---
-        float* d32 = reinterpret_cast<float*>(h->d32.p);
-        TA* dmod = reinterpret_cast<TA*>(h->dmod.p);
+        // --- head of order o (tante.py:147-154): last-frame latent -> interprator -> R_t -> FiLM modifier ---
         const long long LC = (long long)L * C;
         const long long tot = (long long)B * LC;
         const int eb = (int)((tot / 4 + 255) / 256);
-        last_frame_kernel<TA><<<eb, 256, 0, st>>>(x, dmod, d32, B, T, LC);
+        TA* dl = ot ? TP<TA>(ot->dl) : TP<TA>(h->dmod);      // (inference modulates it in place)
+        float* d32 = ot ? FP(ot->d32) : FP(h->d32);
+        last_frame_kernel<TA><<<eb, 256, 0, st>>>(ot ? FP(ot->X.back()) : x, dl, d32, B, T, LC);
         CK(cudaGetLastError());
         h->launches++;
+        TA* dmod = dl;
         if (!h->cfg.deg) {
-            TA* i1 = reinterpret_cast<TA*>(h->i1.p);
-            TA* i2 = reinterpret_cast<TA*>(h->i2.p);
+            TA* i1 = ot ? TP<TA>(ot->i1) : TP<TA>(h->i1);
+            TA* i2 = ot ? TP<TA>(ot->i2) : TP<TA>(h->i2);
+            float* film = ot ? FP(ot->film) : FP(h->filmbuf);
+            float* rt_o = rt + (size_t)o * h->max_batch;
+            if (ot) dmod = TP<TA>(ot->dmod);
             EpiParams ei; ei.bias = AF(h, op.intb[0]);
-            gemm<TA>(h, EPI_BIAS_RELU, dmod, C, op.intw[0], i1, C / 2, false, B * L, C / 2, C, ei, st);
+            gemm<TA>(h, EPI_BIAS_RELU, dl, C, op.intw[0], i1, C / 2, false, B * L, C / 2, C, ei, st);
             ei.bias = AF(h, op.intb[1]);
             gemm<TA>(h, EPI_BIAS_RELU, i1, C / 2, op.intw[1], i2, C / 4, false, B * L, C / 4, C / 2, ei, st);
-            rt_reduce_kernel<TA><<<B, 256, 0, st>>>(i2, AF(h, op.intw[2]), AF(h, op.intb[2]), L, C / 4, io.out_T,
-                                                    rt + (size_t)o * h->max_batch);
+            rt_reduce_kernel<TA><<<B, 256, 0, st>>>(i2, AF(h, op.intw[2]), AF(h, op.intb[2]), L, C / 4, io.out_T, rt_o);
             CK(cudaGetLastError());
             h->launches++;
-            float* fb = reinterpret_cast<float*>(h->filmbuf.p);
+            if (ot) CK(cudaMemcpyAsync(ot->rt.p, rt_o, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
             film_params_kernel<<<B, 256, C * sizeof(float), st>>>(
-                rt + (size_t)o * h->max_batch, 1.0f, AF(h, op.mod[0]), AF(h, op.mod[1]), AF(h, op.mod[2]),
-                AF(h, op.mod[3]), AF(h, op.mod[4]), AF(h, op.mod[5]), AF(h, op.mod[6]), AF(h, op.mod[7]), C, fb);
+                ot ? FP(ot->rt) : rt_o, 1.0f, AF(h, op.mod[0]), AF(h, op.mod[1]), AF(h, op.mod[2]), AF(h, op.mod[3]),
+                AF(h, op.mod[4]), AF(h, op.mod[5]), AF(h, op.mod[6]), AF(h, op.mod[7]), C, film);
             CK(cudaGetLastError());
             h->launches++;
-            film_apply_kernel<TA><<<eb, 256, 0, st>>>(d32, fb, dmod, LC, C, tot);
+            film_apply_kernel<TA><<<eb, 256, 0, st>>>(d32, film, dmod, LC, C, tot);
             CK(cudaGetLastError());
             h->launches++;
         }
-        if (h->fno) { run_decoder_fno<TA>(h, o, dmod, B, st); continue; }
-        if (h->wide) { run_decoder_wide<TA>(h, o, dmod, B, st); continue; }
-        TA* z1 = reinterpret_cast<TA*>(h->z1.p);
-        TA* z2 = reinterpret_cast<TA*>(h->z2[o].p);
+        // --- decoder of order o: the fields of the Horner emit, or the stage-1 activations the fused Taylor head reads ---
+        if (h->fno) { run_decoder_fno<TA>(h, o, dmod, B, ot, st); continue; }
+        if (h->wide) { run_decoder_wide<TA>(h, o, dmod, B, ot, st); continue; }
+        const PatchGeom& g = h->geom;
+        TA* z1 = ot ? TP<TA>(ot->z1act) : TP<TA>(h->z1);
+        TA* z2 = ot ? TP<TA>(ot->z2act) : TP<TA>(h->z2[o]);
+        TA* z1pre = ot ? TP<TA>(ot->z1pre) : nullptr;
+        TA* z2pre = ot ? TP<TA>(ot->z2pre) : nullptr;
         EpiParams ed; ed.bias = AF(h, op.decb[0]);
-        gemm<TA>(h, EPI_BIAS_GELU_ERF, dmod, C, op.decw[0], z1, g.k2 * g.k2 * C2, false, B * L, g.k2 * g.k2 * C2, C, ed, st);
+        gemm_act<TA, ACT_GELU_ERF>(h, dmod, C, op.decw[0], z1pre, z1, B * L, g.k2 * g.k2 * C2, C, ed, st);
         ed.bias = AF(h, op.decb[1]);
-        gemm<TA>(h, EPI_BIAS_GELU_ERF, z1, C2, op.decw[1], z2, g.k1 * g.k1 * C1, false, B * L * g.R2, g.k1 * g.k1 * C1, C2, ed, st);
+        gemm_act<TA, ACT_GELU_ERF>(h, z1, C2, op.decw[1], z2pre, z2, B * L * g.R2, g.k1 * g.k1 * C1, C2, ed, st);
     }
-    // --- step-size selection + fused Taylor head (tante.py:156-171) ---
+    // --- step-size selection + fused Taylor head / Horner emit (tante.py:156-171) ---
     select_step_kernel<<<(B + 127) / 128, 128, 0, st>>>(rt, K, h->max_batch, B, h->cfg.deg, h->cfg.output_length,
                                                         io.per_sample, io.rollout ? (1 << 30) : io.n_cap,
                                                         io.rollout ? nullptr : io.R_t,
                                                         io.rollout ? nullptr : reinterpret_cast<int*>(h->nbuf.p), rs,
-                                                        io.rollout ? 1 : 0);
+                                                        io.rollout ? 1 : 0, io.ft.cur, io.n_lim);
     CK(cudaGetLastError());
     h->launches++;
+    if (tp) CK(cudaMemcpyAsync(tp->n_arr.p, h->nbuf.p, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
     if (h->wide) launch_emit_wide(h, io, B, rs, st);
     else launch_head<TA>(h, io, B, rs, nullptr, st);
     if (io.rollout) {
@@ -1399,22 +1523,19 @@ void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs
         CK(cudaGetLastError());
         h->launches++;
     }
+    if (tp) {
+        tp->out_T = io.out_T;
+        tp->n_cap = io.n_cap;
+        tp->hist = io.ft.cur != nullptr;
+        tp->B_used = B;
+        tp->valid = true;
+    }
 }
 
 // ================================================================================================
 // Training: forward with an activation tape + full backward (what torch autograd does for the reference:
 // trainer/r_trainer.py:145-155, trainer/trainer.py:178-193).
 // ================================================================================================
-template <typename TA> inline TA* TP(DevBuf& b) { return reinterpret_cast<TA*>(b.p); }
-inline float* FP(DevBuf& b) { return reinterpret_cast<float*>(b.p); }
-
-
-template <typename TA, int ACT>
-void launch_act_fwd(tante_handle_s* h, const TA* pre, TA* out, long long n, cudaStream_t st) {
-    act_fwd_kernel<TA, ACT><<<blocks_for(n / 4, 256), 256, 0, st>>>(pre, out, n / 4);
-    CK(cudaGetLastError());
-    h->launches++;
-}
 template <typename TA, int ACT>
 void launch_act_bwd(tante_handle_s* h, TA* g, const TA* pre, long long n, cudaStream_t st) {
     act_bwd_kernel<TA, ACT><<<blocks_for(n / 4, 256), 256, 0, st>>>(g, pre, n / 4);
@@ -1845,369 +1966,6 @@ void backward_alloc(tante_handle_s* h, int B) {
         CK(cudaMemcpy(h->udesc_dev.p, ud.data(), ud.size() * sizeof(UnpackDesc), cudaMemcpyHostToDevice));
     }
     h->bw_batch = B;
-}
-
-// One TANTE step in training mode: same arithmetic as run_step, every activation the backward needs is kept.
-// Per-sample cursor mode (tante_train_forward_hist): the window frames relative to `input`; `frames` is the prediction buffer
-// (batch stride in.hbs) and a sample that has its n_lim frames emits nothing.
-struct TrainWin {
-    FrameTab in;
-    int n_lim;
-};
-
-template <typename TA>
-void run_step_train(tante_handle_s* h, Tape& tp, const float* input, int B, float out_T, int n_cap, float* frames,
-                    float* R_t, cudaStream_t st, const TrainWin* win = nullptr) {
-    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L, K = h->K, Hm = h->Hm;
-    const PatchGeom& g = h->geom;
-    const int tokens = B * T * L;
-    constexpr bool kTensor = sizeof(TA) == 2;
-    tp.drop = make_drop_cfg(h->drop_p, h->drop_seed);
-    const DropCfg& drop = tp.drop;
-    // --- encoder ---
-    if (h->fno) {
-        // enc_FNO.forward (enc_dec_fno.py:254-272): spectral layer -> GELU -> patch conv -> GELU -> spectral layer -> GELU -> patch conv;
-        // every pre-activation / activation grid is kept
-        REQUIRE(!win, "windowed BPTT is not available with enc_dec_type='fno'");
-        const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0, C8 = C / 8;
-        const long long NI = (long long)B * T;
-        SpecView v0{input, 0, nullptr, T};
-        run_spectral<TA>(h, h->fes1, v0, NI, H, W, 0, false, TP<TA>(tp.f0pre), nullptr, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.f0pre), TP<TA>(tp.f0act), NI * H * W * C8, st);
-        EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-        conv_cl_gemm<TA>(h, EPI_BIAS, TP<TA>(tp.f0act), H, W, C8, p0, h->enc_w[0], tp.a1pre.p, C1, false, NI, e1, st, h->st[0]);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a1pre), TP<TA>(tp.a1act), NI * H1 * W1 * C1, st);
-        SpecView v1{tp.a1act.p, 1, nullptr, 1};
-        run_spectral<TA>(h, h->fes2, v1, NI, H1, W1, 1, false, TP<TA>(tp.a2pre), nullptr, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a2pre), TP<TA>(tp.a2act), NI * H1 * W1 * C2, st);
-        EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-        conv_cl_gemm<TA>(h, EPI_BIAS, TP<TA>(tp.a2act), H1, W1, C2, p1, h->enc_w[1], tp.v.p, C, true, NI, e2, st, h->st[1]);
-        embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(
-            FP(tp.v), AF(h, h->film_t_off), AF(h, h->s_emb), AF(h, h->t_emb), FP(tp.ord[0].P[0]), tokens, T, L, C);
-        CK(cudaGetLastError());
-        h->launches++;
-    } else if (h->wide) {
-        // patch_scale 16 / 32 / 64 (wide_patch.cuh): natural-order stages, window gathers + GEMMs; the first patch matrix and every
-        // pre-activation / activation grid are kept for the backward
-        REQUIRE(!win, "windowed BPTT is not available at patch_scale >= 16 / with overlap");
-        const int H = h->cfg.H, W = h->cfg.W, D = h->D;
-        TA* wb = TP<TA>(h->wbuf);
-        TA* cg = TP<TA>(h->cgrid);
-        const WideDims wd = wide_dims(h, B);
-        const int H1 = wd.H1, W1 = wd.W1, H2 = wd.H2, W2 = wd.W2;
-        const long long NI = (long long)B * T;
-        REQUIRE(wd.rows1 < (1LL << 31) && wd.rows2 < (1LL << 31) && wd.rows3 < (1LL << 31), "input too large for the wide conv GEMMs");
-        auto pool = [&](const TA* in, int Hc, int Wc, int Cc, int Ho, int Wo, TA* out, float* out32) {
-            const long long total4 = NI * Ho * Wo * Cc / 4;
-            if (out32) wide_pool_kernel<TA, false, true><<<blocks_for(total4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, nullptr, out32, total4);
-            else wide_pool_kernel<TA, false, false><<<blocks_for(total4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, out, nullptr, total4);
-            CK(cudaGetLastError());
-            h->launches++;
-        };
-        const long long total = wd.rows1 * h->K1pad;
-        wide_im2col_cf_kernel<TA><<<blocks_for(total, 256), 256, 0, st>>>(input, nullptr, T, D, H, W, g.k0, (g.k0 - 1) / 2, h->K1pad,
-                                                                         TP<TA>(tp.cols), total, h->st[0], wd.Hc1, wd.Wc1);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-        gemm<TA>(h, EPI_BIAS, TP<TA>(tp.cols), h->K1pad, h->enc_w1wide, wd.pool1 ? (void*)cg : tp.a1pre.p, C1, false, (int)wd.rows1, C1,
-                 h->K1pad, e1, st);
-        if (wd.pool1) pool(cg, wd.Hc1, wd.Wc1, C1, H1, W1, TP<TA>(tp.a1pre), nullptr);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a1pre), TP<TA>(tp.a1act), NI * H1 * W1 * C1, st);
-        const int K2 = g.k1 * g.k1 * C1, K3 = g.k2 * g.k2 * C2;
-        wide_im2col_cl_kernel<TA><<<blocks_for(wd.rows2 * K2 / 4, 256), 256, 0, st>>>(TP<TA>(tp.a1act), H1, W1, C1, g.k1, (g.k1 - 1) / 2, wb,
-                                                                                     wd.rows2 * K2 / 4, h->st[1], wd.Hc2, wd.Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-        gemm<TA>(h, EPI_BIAS, wb, K2, h->enc_w[1], wd.pool2 ? (void*)cg : tp.a2pre.p, C2, false, (int)wd.rows2, C2, K2, e2, st);
-        if (wd.pool2) pool(cg, wd.Hc2, wd.Wc2, C2, H2, W2, TP<TA>(tp.a2pre), nullptr);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a2pre), TP<TA>(tp.a2act), NI * H2 * W2 * C2, st);
-        wide_im2col_cl_kernel<TA><<<blocks_for(wd.rows3 * K3 / 4, 256), 256, 0, st>>>(TP<TA>(tp.a2act), H2, W2, C2, g.k2, (g.k2 - 1) / 2, wb,
-                                                                                     wd.rows3 * K3 / 4, h->st[2], wd.Hc3, wd.Wc3);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
-        if (wd.pool3) {
-            if (kTensor && K3 > 1024) {      // (patch_scale 64: K blocks through the fp32 scratch of tante_reserve, as in run_encoder_wide)
-                REQUIRE((size_t)wd.rows3 * C * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
-                float* acc = FP(h->kscratch);
-                gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], acc, (int)wd.rows3, C, K3, e3.bias, st);
-                f32_to_ta_kernel<TA, false><<<blocks_for(wd.rows3 * C / 4, 256), 256, 0, st>>>(acc, cg, wd.rows3 * C / 4);
-                CK(cudaGetLastError());
-                h->launches++;
-            } else {
-                gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], cg, C, false, (int)wd.rows3, C, K3, e3, st);
-            }
-            pool(cg, wd.Hc3, wd.Wc3, C, h->Hp, h->Wp, nullptr, FP(tp.v));
-        } else if (kTensor && K3 > 1024) {      // (K = 2048 at patch_scale 64: K blocks, as in run_encoder_wide)
-            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], FP(tp.v), tokens, C, K3, e3.bias, st);
-        } else {
-            gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], tp.v.p, C, true, tokens, C, K3, e3, st);
-        }
-        embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(
-            FP(tp.v), AF(h, h->film_t_off), AF(h, h->s_emb), AF(h, h->t_emb), FP(tp.ord[0].P[0]), tokens, T, L, C);
-        CK(cudaGetLastError());
-        h->launches++;
-    } else {
-        // enc_conv_1 as im2col (kept for the weight gradient) + GEMM over the zero-padded patch matrix
-        const long long rows_in = (long long)tokens * g.R1;
-        REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv GEMM");
-        const FrameTab ft = win ? win->in : FrameTab();
-        if (g.k0 * g.k1 * g.k2 >= 4) conv1_im2col_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(input, g, TP<TA>(tp.cols), rows_in, nullptr, nullptr, nullptr, ft);
-        else conv1_im2col_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(input, g, TP<TA>(tp.cols), rows_in, nullptr, nullptr, nullptr, ft);
-        CK(cudaGetLastError());
-        h->launches++;
-        EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-        gemm<TA>(h, EPI_BIAS, TP<TA>(tp.cols), kHeadPad, h->enc_w1pad, tp.a1pre.p, C1, false, (int)rows_in, C1, kHeadPad, e1, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a1pre), TP<TA>(tp.a1act), (long long)tokens * g.R1 * C1, st);
-        EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
-        gemm<TA>(h, EPI_BIAS, TP<TA>(tp.a1act), g.k1 * g.k1 * C1, h->enc_w[1], tp.a2pre.p, C2, false, tokens * g.R2, C2,
-                 g.k1 * g.k1 * C1, e2, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(tp.a2pre), TP<TA>(tp.a2act), (long long)tokens * g.R2 * C2, st);
-        EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
-        gemm<TA>(h, EPI_BIAS, TP<TA>(tp.a2act), g.k2 * g.k2 * C2, h->enc_w[2], tp.v.p, C, true, tokens, C, g.k2 * g.k2 * C2, e3, st);
-        embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(
-            FP(tp.v), AF(h, h->film_t_off), AF(h, h->s_emb), AF(h, h->t_emb), FP(tp.ord[0].P[0]), tokens, T, L, C);
-        CK(cudaGetLastError());
-        h->launches++;
-    }
-    float* rt = reinterpret_cast<float*>(h->rt.p);
-    for (int o = 0; o < K; ++o) {
-        const OrderPlan& op = h->orders[o];
-        OrderTape& ot = tp.ord[o];
-        const float* pin = o == 0 ? FP(ot.P[0]) : FP(tp.ord[o - 1].X.back());
-        launch_propagator(h, pin, FP(ot.P[1]), B, 0, op, st);
-        launch_propagator(h, FP(ot.P[1]), FP(ot.P[2]), B, 1, op, st);
-        launch_propagator(h, FP(ot.P[2]), FP(ot.X[0]), B, 2, op, st);
-        bool ln_ready = false;
-        const size_t nl = op.layers.size();
-        for (size_t li = 0; li < nl; ++li) {
-            const LayerPlan& lp = op.layers[li];
-            float* x_in = FP(ot.X[2 * li]);
-            float* x_mid = FP(ot.X[2 * li + 1]);
-            float* x_out = FP(ot.X[2 * li + 2]);
-            if (lp.axis == 'C') {
-                // channel attention: only the layer's fp32 input is kept -- the backward recomputes the block chunk by chunk
-                REQUIRE(drop.p <= 0.f, "dropout with an attention axis C layer is not implemented");
-                run_channel_layer<TA>(h, lp, x_in, x_out, tokens, st);
-                ln_ready = false;
-                continue;
-            }
-            const bool nx_ok = li + 1 < nl && op.layers[li + 1].axis != 'C';
-            if (!ln_ready) launch_layernorm<TA>(h, x_in, lp.ln1w, lp.ln1b, TP<TA>(ot.ln1[li]), tokens, st);
-            EpiParams eq; eq.bias = AF(h, lp.inb);
-            gemm<TA>(h, EPI_BIAS, TP<TA>(ot.ln1[li]), C, lp.inw, ot.qkv[li].p, 3 * C, false, tokens, 3 * C, C, eq, st);
-            launch_attention<TA>(h, TP<TA>(ot.qkv[li]), TP<TA>(ot.att[li]), B, lp.axis, st, drop, drop_site(o, (int)li, 0));
-            if constexpr (kTensor) {
-                if (h->fuse_tail && C == kBtC && h->Hm == C) {
-                    const LayerPlan* nx = nx_ok ? &op.layers[li + 1] : nullptr;
-                    launch_tail(h, lp, nx, TP<TA>(ot.att[li]), x_in, x_out, nx ? TP<TA>(ot.ln1[li + 1]) : nullptr, tokens, st,
-                                x_mid, TP<TA>(ot.ln2[li]), TP<TA>(ot.hpre[li]), TP<TA>(ot.hact[li]), drop,
-                                drop_site(o, (int)li, 1), drop_site(o, (int)li, 2));
-                    ln_ready = nx != nullptr;
-                    continue;
-                }
-            }
-            if (kTensor && drop.p > 0.f) {
-                // Tensor mode with dropout outside the fused tail (mlp_ratio != 1, embed_dim 512, TANTE_FUSE_TAIL=0): the tcgen05 GEMM
-                // epilogues carry no mask generator, so each residual branch is a plain GEMM into a bf16 scratch followed by one
-                // pass  x <- x + mask * branch  (what autocast + nn.Dropout do in the reference); LayerNorms as their own passes.
-                TA* br = TP<TA>(h->hid);
-                const long long n4 = (long long)tokens * C / 4;
-                EpiParams eb; eb.bias = AF(h, lp.outb);
-                gemm<TA>(h, EPI_BIAS, TP<TA>(ot.att[li]), C, lp.outw, br, C, false, tokens, C, C, eb, st);
-                resid_drop_kernel<TA><<<blocks_for(n4, 256), 256, 0, st>>>(br, x_in, x_mid, n4, drop, drop_site(o, (int)li, 1));
-                CK(cudaGetLastError());
-                h->launches++;
-                launch_layernorm<TA>(h, x_mid, lp.ln2w, lp.ln2b, TP<TA>(ot.ln2[li]), tokens, st);
-                EpiParams eh; eh.bias = AF(h, lp.m0b);
-                gemm<TA>(h, EPI_BIAS, TP<TA>(ot.ln2[li]), C, lp.m0w, ot.hpre[li].p, Hm, false, tokens, Hm, C, eh, st);
-                launch_act_fwd<TA, ACT_GELU_TANH>(h, TP<TA>(ot.hpre[li]), TP<TA>(ot.hact[li]), (long long)tokens * Hm, st);
-                eb.bias = AF(h, lp.m2b);
-                gemm<TA>(h, EPI_BIAS, TP<TA>(ot.hact[li]), Hm, lp.m2w, br, C, false, tokens, C, Hm, eb, st);
-                resid_drop_kernel<TA><<<blocks_for(n4, 256), 256, 0, st>>>(br, x_mid, x_out, n4, drop, drop_site(o, (int)li, 2));
-                CK(cudaGetLastError());
-                h->launches++;
-                ln_ready = false;
-                continue;
-            }
-            EpiParams eo; eo.bias = AF(h, lp.outb); eo.resid = x_in; eo.ldr = C;
-            eo.drop = drop; eo.drop_site = drop_site(o, (int)li, 1);
-            if (kTensor && C <= 256) {
-                eo.ln_gamma = AF(h, lp.ln2w); eo.ln_beta = AF(h, lp.ln2b); eo.ln_out = ot.ln2[li].p;
-                gemm<TA>(h, EPI_BIAS_RESID_LN, TP<TA>(ot.att[li]), C, lp.outw, x_mid, C, true, tokens, C, C, eo, st);
-            } else {
-                gemm<TA>(h, EPI_BIAS_RESID, TP<TA>(ot.att[li]), C, lp.outw, x_mid, C, true, tokens, C, C, eo, st);
-                launch_layernorm<TA>(h, x_mid, lp.ln2w, lp.ln2b, TP<TA>(ot.ln2[li]), tokens, st);
-            }
-            EpiParams e0; e0.bias = AF(h, lp.m0b);
-            gemm<TA>(h, EPI_BIAS, TP<TA>(ot.ln2[li]), C, lp.m0w, ot.hpre[li].p, Hm, false, tokens, Hm, C, e0, st);
-            launch_act_fwd<TA, ACT_GELU_TANH>(h, TP<TA>(ot.hpre[li]), TP<TA>(ot.hact[li]), (long long)tokens * Hm, st);
-            EpiParams e2; e2.bias = AF(h, lp.m2b); e2.resid = x_mid; e2.ldr = C;
-            e2.drop = drop; e2.drop_site = drop_site(o, (int)li, 2);
-            if (kTensor && C <= 256 && nx_ok && Hm == C) {      // (the LN-fused epilogue needs the K = C weight slice resident)
-                const LayerPlan& nx = op.layers[li + 1];
-                e2.ln_gamma = AF(h, nx.ln1w); e2.ln_beta = AF(h, nx.ln1b); e2.ln_out = ot.ln1[li + 1].p;
-                gemm<TA>(h, EPI_BIAS_RESID_LN, TP<TA>(ot.hact[li]), Hm, lp.m2w, x_out, C, true, tokens, C, Hm, e2, st);
-                ln_ready = true;
-            } else {
-                gemm<TA>(h, EPI_BIAS_RESID, TP<TA>(ot.hact[li]), Hm, lp.m2w, x_out, C, true, tokens, C, Hm, e2, st);
-                ln_ready = false;
-            }
-        }
-        // --- head of order o ---
-        const long long LC = (long long)L * C;
-        const long long tot = (long long)B * LC;
-        const int eb = (int)((tot / 4 + 255) / 256);
-        last_frame_kernel<TA><<<eb, 256, 0, st>>>(FP(ot.X.back()), TP<TA>(ot.dl), FP(ot.d32), B, T, LC);
-        CK(cudaGetLastError());
-        h->launches++;
-        TA* dmod = TP<TA>(ot.dl);
-        if (!h->cfg.deg) {
-            EpiParams ei; ei.bias = AF(h, op.intb[0]);
-            gemm<TA>(h, EPI_BIAS_RELU, TP<TA>(ot.dl), C, op.intw[0], ot.i1.p, C / 2, false, B * L, C / 2, C, ei, st);
-            ei.bias = AF(h, op.intb[1]);
-            gemm<TA>(h, EPI_BIAS_RELU, TP<TA>(ot.i1), C / 2, op.intw[1], ot.i2.p, C / 4, false, B * L, C / 4, C / 2, ei, st);
-            rt_reduce_kernel<TA><<<B, 256, 0, st>>>(TP<TA>(ot.i2), AF(h, op.intw[2]), AF(h, op.intb[2]), L, C / 4, out_T,
-                                                    rt + (size_t)o * h->max_batch);
-            CK(cudaGetLastError());
-            h->launches++;
-            CK(cudaMemcpyAsync(ot.rt.p, rt + (size_t)o * h->max_batch, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
-            film_params_kernel<<<B, 256, C * sizeof(float), st>>>(
-                FP(ot.rt), 1.0f, AF(h, op.mod[0]), AF(h, op.mod[1]), AF(h, op.mod[2]), AF(h, op.mod[3]), AF(h, op.mod[4]),
-                AF(h, op.mod[5]), AF(h, op.mod[6]), AF(h, op.mod[7]), C, FP(ot.film));
-            CK(cudaGetLastError());
-            h->launches++;
-            film_apply_kernel<TA><<<eb, 256, 0, st>>>(FP(ot.d32), FP(ot.film), TP<TA>(ot.dmod), LC, C, tot);
-            CK(cudaGetLastError());
-            h->launches++;
-            dmod = TP<TA>(ot.dmod);
-        }
-        if (h->fno) {
-            // dec_FNO.forward (enc_dec_fno.py:303-323): deconv -> GELU -> spectral -> GELU -> deconv -> GELU -> spectral
-            TA* wb = TP<TA>(h->wbuf);
-            const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0, C8 = C / 8, D = h->D;
-            const int N1 = p1 * p1 * C2, N2 = p0 * p0 * C8;
-            float* field = FP(h->dfield) + (size_t)o * B * D * H * W;
-            const bool ovf1 = h->st[1] != p1, ovf0 = h->st[0] != p0;
-            EpiParams ew; ew.bias = ovf1 ? AF(h, h->zero_off) : AF(h, op.decb[0]);
-            gemm<TA>(h, EPI_BIAS, dmod, C, op.decw[0], wb, N1, false, B * L, N1, C, ew, st);
-            long long tot = (long long)B * H1 * W1 * C2;
-            wide_deconv_post_kernel<TA, false, false><<<blocks_for(tot, 256), 256, 0, st>>>(wb, N1, h->Hp, h->Wp, C2, p1, ovf1 ? AF(h, op.decb[0]) : nullptr,
-                                                                                          TP<TA>(ot.z1pre), nullptr, tot, h->st[1]);
-            CK(cudaGetLastError());
-            h->launches++;
-            launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z1pre), TP<TA>(ot.z1act), tot, st);
-            SpecView v2{ot.z1act.p, 1, nullptr, 1};
-            run_spectral<TA>(h, op.fs1, v2, B, H1, W1, 1, false, TP<TA>(ot.z2pre), nullptr, st);
-            launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z2pre), TP<TA>(ot.z2act), (long long)B * H1 * W1 * C1, st);
-            ew.bias = ovf0 ? AF(h, h->zero_off) : AF(h, op.decb[1]);
-            gemm<TA>(h, EPI_BIAS, TP<TA>(ot.z2act), C1, op.decw[1], wb, N2, false, B * H1 * W1, N2, C1, ew, st);
-            tot = (long long)B * H * W * C8;
-            wide_deconv_post_kernel<TA, false, false><<<blocks_for(tot, 256), 256, 0, st>>>(wb, N2, H1, W1, C8, p0, ovf0 ? AF(h, op.decb[1]) : nullptr,
-                                                                                          TP<TA>(ot.f0pre), nullptr, tot, h->st[0]);
-            CK(cudaGetLastError());
-            h->launches++;
-            launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.f0pre), TP<TA>(ot.f0act), tot, st);
-            SpecView v0{ot.f0act.p, 1, nullptr, 1};
-            run_spectral<TA>(h, op.fs2, v0, B, H, W, 0, false, nullptr, field, st);
-            continue;
-        }
-        if (h->wide) {
-            // decoder stage = GEMM to the sub-pixel matrix -> crop + bilinear resample to the grid (pre-activation kept) -> GELU
-            TA* wb = TP<TA>(h->wbuf);
-            const int Hp = h->Hp, Wp = h->Wp, D = h->D;
-            const int H2 = Hp * g.k2, W2 = Wp * g.k2, H1 = H2 * g.k1, W1 = W2 * g.k1;
-            const int N1 = g.k2 * g.k2 * C2, N2 = g.k1 * g.k1 * C1;
-            float* field = FP(h->dfield) + (size_t)o * B * D * h->cfg.H * h->cfg.W;
-            // (overlapped stages: bias-free GEMM, the bias once per output sample in the pass after it -- see run_decoder_wide)
-            const bool ov1 = h->st[2] != g.k2, ov2 = h->st[1] != g.k1;
-            EpiParams ew; ew.bias = ov1 ? AF(h, h->zero_off) : AF(h, op.decb[0]);
-            gemm<TA>(h, EPI_BIAS, dmod, C, op.decw[0], wb, N1, false, B * L, N1, C, ew, st);
-            long long tot = (long long)B * H2 * W2 * C2;
-            wide_deconv_post_kernel<TA, false, false><<<blocks_for(tot, 256), 256, 0, st>>>(wb, N1, Hp, Wp, C2, g.k2, ov1 ? AF(h, op.decb[0]) : nullptr,
-                                                                                          TP<TA>(ot.z1pre), nullptr, tot, h->st[2]);
-            CK(cudaGetLastError());
-            h->launches++;
-            launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z1pre), TP<TA>(ot.z1act), tot, st);
-            ew.bias = ov2 ? AF(h, h->zero_off) : AF(h, op.decb[1]);
-            gemm<TA>(h, EPI_BIAS, TP<TA>(ot.z1act), C2, op.decw[1], wb, N2, false, B * H2 * W2, N2, C2, ew, st);
-            tot = (long long)B * H1 * W1 * C1;
-            wide_deconv_post_kernel<TA, false, false><<<blocks_for(tot, 256), 256, 0, st>>>(wb, N2, H2, W2, C1, g.k1, ov2 ? AF(h, op.decb[1]) : nullptr,
-                                                                                          TP<TA>(ot.z2pre), nullptr, tot, h->st[1]);
-            CK(cudaGetLastError());
-            h->launches++;
-            launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z2pre), TP<TA>(ot.z2act), tot, st);
-            EpiParams e3; e3.bias = AF(h, h->zero_off);
-            gemm<TA>(h, EPI_BIAS, TP<TA>(ot.z2act), C1, op.w3nk, wb, h->NOpad, false, B * H1 * W1, h->NOpad, C1, e3, st);
-            tot = (long long)B * D * h->cfg.H * h->cfg.W;
-            wide_deconv_post_kernel<TA, false, true><<<blocks_for(tot, 256), 256, 0, st>>>(wb, h->NOpad, H1, W1, D, g.k0, AF(h, op.decb[2]), nullptr, field, tot, h->st[0]);
-            CK(cudaGetLastError());
-            h->launches++;
-            continue;
-        }
-        EpiParams ed; ed.bias = AF(h, op.decb[0]);
-        gemm<TA>(h, EPI_BIAS, dmod, C, op.decw[0], ot.z1pre.p, g.k2 * g.k2 * C2, false, B * L, g.k2 * g.k2 * C2, C, ed, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z1pre), TP<TA>(ot.z1act), (long long)B * L * g.R2 * C2, st);
-        ed.bias = AF(h, op.decb[1]);
-        gemm<TA>(h, EPI_BIAS, TP<TA>(ot.z1act), C2, op.decw[1], ot.z2pre.p, g.k1 * g.k1 * C1, false, B * L * g.R2,
-                 g.k1 * g.k1 * C1, C2, ed, st);
-        launch_act_fwd<TA, ACT_GELU_ERF>(h, TP<TA>(ot.z2pre), TP<TA>(ot.z2act), (long long)B * L * g.R1 * C1, st);
-    }
-    RolloutState rs{};
-    const int* cur = win ? win->in.cur : nullptr;
-    select_step_kernel<<<(B + 127) / 128, 128, 0, st>>>(rt, K, h->max_batch, B, h->cfg.deg, h->cfg.output_length, cur ? 1 : 0, n_cap,
-                                                        R_t, reinterpret_cast<int*>(h->nbuf.p), rs, 0, cur, win ? win->n_lim : 0);
-    CK(cudaGetLastError());
-    h->launches++;
-    CK(cudaMemcpyAsync(tp.n_arr.p, h->nbuf.p, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
-    if (h->wide) {      // Horner sum + residual over the decoded derivative fields (boundary C)
-        EmitParams ep{};
-        ep.dfield = FP(h->dfield);
-        ep.K = K; ep.fi = h->cfg.frame_interval;
-        ep.u_ring = input; ep.fcount = nullptr;
-        ep.n_arr = reinterpret_cast<int*>(h->nbuf.p);
-        ep.frames = frames; ep.n_cap = n_cap;
-        ep.B = B; ep.D = h->D; ep.T = T; ep.HW = (long long)h->cfg.H * h->cfg.W;
-        REQUIRE(ep.HW % 4 == 0, "H * W must be a multiple of 4");
-        taylor_emit_kernel<<<dim3(blocks_for(ep.HW / 4, 256), (unsigned)h->D, (unsigned)B), 256, 0, st>>>(ep);
-        CK(cudaGetLastError());
-        h->launches++;
-    } else
-    // fused Taylor head on the kept stage-1 activations
-    {
-        HeadParams hp{};
-        for (int k = 0; k < K; ++k) {
-            hp.z[k] = tp.ord[k].z2act.p;
-            hp.w3[k] = AF(h, h->orders[k].decw[2]);
-            hp.b3[k] = AF(h, h->orders[k].decb[2]);
-        }
-        hp.K = K; hp.fi = h->cfg.frame_interval; hp.u_ring = input; hp.fcount = nullptr;
-        hp.n_arr = reinterpret_cast<int*>(h->nbuf.p); hp.frames = frames; hp.n_cap = n_cap;
-        if (win) { hp.frames_bs = win->in.hbs; hp.cur = cur; }
-        const long long rows = (long long)B * L * g.R1;
-        bool done = false;
-        if (kTensor) {
-            cudaError_t e = cudaSuccess;
-            if (launch_head_mma(hp, g, C1, rows, B, h->num_sms, st, &e)) { CK(e); done = true; }
-        }
-        if (!done) {
-            const int NO = g.k0 * g.k0 * h->D;
-            const size_t smem = (size_t)(K * C1 * NO + K * h->D) * sizeof(float);
-            const int blocks = (int)((rows + 127) / 128);
-#define HEAD(KO) taylor_head_kernel<TA, 8, KO><<<blocks, 128, smem, st>>>(hp, g, C1, rows, B)
-            switch (K) { case 1: HEAD(1); break; case 2: HEAD(2); break; case 3: HEAD(3); break; default: HEAD(4); break; }
-#undef HEAD
-            CK(cudaGetLastError());
-        }
-        h->launches++;
-    }
-    tp.out_T = out_T;
-    tp.n_cap = n_cap;
-    tp.hist = cur != nullptr;
-    tp.B_used = B;
-    tp.valid = true;
 }
 
 // Backward of one taped step.  gframes: f32 (B, n_g, D, H, W) gradient of the emitted frames; gRt: f32 [B] or null;
@@ -3265,8 +3023,11 @@ int tante_train_forward(tante_handle_t h, int32_t slot, const float* input, int3
         cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
         Tape& tp = *h->tapes[slot];
         tape_alloc(h, tp, B);
-        if (h->cfg.precision == TANTE_PREC_FP32) run_step_train<float>(h, tp, input, B, out_T, n_cap, frames, R_t, st);
-        else run_step_train<__nv_bfloat16>(h, tp, input, B, out_T, n_cap, frames, R_t, st);
+        StepIO io;
+        io.input = input; io.frames = frames; io.n_cap = n_cap; io.R_t = R_t; io.out_T = out_T; io.tape = &tp;
+        RolloutState rs{};
+        if (h->cfg.precision == TANTE_PREC_FP32) run_step<float>(h, io, B, rs, st);
+        else run_step<__nv_bfloat16>(h, io, B, rs, st);
         h->last_B = B;
         if (n_host) {
             CK(cudaMemcpyAsync(h->h_flag + 8, h->nbuf.p, 4, cudaMemcpyDeviceToHost, st));
@@ -3322,11 +3083,14 @@ int tante_train_forward_hist(tante_handle_t h, int32_t slot, const float* input,
         Tape& tp = *h->tapes[slot];
         tape_alloc(h, tp, B);
         // the kernels of the call read the caller's cursor; the advance stores the value they saw in the tape
-        TrainWin win;
-        win.in = FrameTab{cursor, elem_offset(pred, input), pred_bstride, 0};
-        win.n_lim = n_steps;
-        if (h->cfg.precision == TANTE_PREC_FP32) run_step_train<float>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
-        else run_step_train<__nv_bfloat16>(h, tp, input, B, out_T, n_cap, pred, R_t, st, &win);
+        StepIO io;
+        io.input = input; io.frames = pred; io.n_cap = n_cap; io.R_t = R_t; io.out_T = out_T; io.tape = &tp;
+        io.per_sample = 1;
+        io.ft = FrameTab{cursor, elem_offset(pred, input), pred_bstride, 0};
+        io.n_lim = n_steps;
+        RolloutState rs{};
+        if (h->cfg.precision == TANTE_PREC_FP32) run_step<float>(h, io, B, rs, st);
+        else run_step<__nv_bfloat16>(h, io, B, rs, st);
         hist_advance_kernel<<<1, 256, 0, st>>>(reinterpret_cast<const int*>(tp.n_arr.p), cursor, reinterpret_cast<int*>(tp.cur.p), ns,
                                                steps, n_active, B, n_steps);
         CK(cudaGetLastError());
