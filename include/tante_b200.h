@@ -267,6 +267,35 @@ TANTE_API int tante_test_block_tail(const void* att, const void* Wo, const void*
 TANTE_API int tante_test_wgrad(int32_t use_tc, const void* A, const void* B, float* C, float* bias, int64_t M, int32_t N,
                      int32_t K, int32_t iters, void* stream);
 
+/* Kernel ids reported by tante_test_attention / tante_test_propagator (`*kernel`). */
+#define TANTE_AXK_FLASH 1      /* attention_flash_kernel                                                      */
+#define TANTE_AXK_MMA 2        /* axial_attention_(bwd_)mma_kernel, propagator_(bwd_)mma_kernel                */
+#define TANTE_AXK_SIMT 3       /* axial_attention_kernel, attention_bwd_kernel                                 */
+#define TANTE_AXK_LONG_MMA 4   /* attn_long_q_mma_kernel + attn_long_kv_mma_kernel (S > 64)                    */
+#define TANTE_AXK_LONG_FFMA 5  /* attn_long_stats_kernel + attn_long_dq_kernel + attn_long_dkv_kernel (S > 64) */
+#define TANTE_AXK_SMALL 6      /* propagator_small_kernel, propagator_small_bwd_kernel                         */
+#define TANTE_AXK_WIDE 7       /* propagator_bwd_wide_kernel                                                   */
+#define TANTE_AXK_GENERIC 8    /* propagator_kernel, propagator_bwd_kernel                                     */
+
+/* Test hook: the attention core of one axis through the model's own kernel choice.  nseq sequences of S tokens,
+ * token(seq, pos) = (outer * S + pos) * inner_sz + inner with seq = outer * inner_sz + inner; qkv packs rows of 3 * C
+ * (q | k | v), n_head heads of head_dim = C / n_head (16, 32 or 64).  precision: TANTE_PREC_FP32 (f32 buffers) or
+ * TANTE_PREC_BF16 (bf16 buffers).  dir 0: out_or_dqkv = out [tokens][C]; dir 1: out_or_dqkv = dqkv [tokens][3 C] from
+ * dout [tokens][C], stats = f32[2 * nseq * n_head * S] scratch (needed when S > 64).  causal masks keys after the query;
+ * drop_p > 0 drops attention probabilities with the masks of (seed, site).  `*kernel` receives a TANTE_AXK_* id. */
+TANTE_API int tante_test_attention(int32_t dir, int32_t precision, const void* qkv, const void* dout, void* out_or_dqkv,
+                                   float* stats, int64_t nseq, int32_t S, int32_t inner_sz, int32_t n_head, int32_t C,
+                                   int32_t causal, float drop_p, uint64_t seed, uint32_t site, int32_t* kernel, void* stream);
+
+/* Test hook: one axis propagator through the model's own kernel choice.  Element (outer, p, col) of the f32 latent lives at
+ * (outer * S + p) * IC + col, S in 1 .. 96, IC a multiple of 4; W1, W2 f32[S][S], b1, b2 f32[S].
+ * dir 0: x_or_dy = xin + W2 gelu(W1 xin + b1) + b2 along the axis (x_or_dy may alias xin);
+ * dir 1: x_or_dy holds the output gradient and is overwritten with the input gradient; gW1, gb1, gW2, gb2 are
+ * accumulated into (b2 is unused).  `*kernel` receives a TANTE_AXK_* id. */
+TANTE_API int tante_test_propagator(int32_t dir, int32_t precision, const float* xin, float* x_or_dy, const float* W1,
+                                    const float* b1, const float* W2, const float* b2, float* gW1, float* gb1, float* gW2,
+                                    float* gb2, int32_t S, int64_t IC, int64_t outer, int32_t* kernel, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -90,6 +90,11 @@ SIGNATURES = {
                                       C.c_void_p]),
     "tante_test_wgrad": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                    C.c_int32, C.c_int32, C.c_void_p]),
+    "tante_test_attention": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                       C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_uint64,
+                                       C.c_uint32, C.POINTER(C.c_int32), C.c_void_p]),
+    "tante_test_propagator": (C.c_int, [C.c_int32, C.c_int32] + [C.c_void_p] * 10 + [C.c_int32, C.c_int64, C.c_int64,
+                                                                                    C.POINTER(C.c_int32), C.c_void_p]),
     "tante_bench_head": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                    C.POINTER(C.c_float), C.c_void_p]),
 }

@@ -668,19 +668,21 @@ void launch_tail(tante_handle_s* h, const LayerPlan& lp, const LayerPlan* nx, co
     h->launches++;
 }
 
+// Launches behind one TANTE_AXK_* id (the S > 64 attention backwards are three kernels).
+inline int axial_launches(int kernel) { return kernel == TANTE_AXK_LONG_MMA || kernel == TANTE_AXK_LONG_FFMA ? 3 : 1; }
+
 // Attention core over n_seq sequences of S tokens addressed in place: token(pos) = (outer * S + pos) * inner + inner_idx, packed
-// qkv rows of 3 * Cw, n_head heads of HD = Cw / n_head features.
+// qkv rows of 3 * Cw, n_head heads of HD = Cw / n_head features.  Picks the kernel and launches it; returns its TANTE_AXK_* id.
 template <typename TA>
-void launch_attention_seq(tante_handle_s* h, const TA* qkv, TA* out, int nseq, int S, int inner, int n_head, int Cw, int HD,
-                          bool causal_b, cudaStream_t st, const DropCfg& drop = DropCfg(), uint32_t site = 0) {
+int dispatch_attention_fwd(const TA* qkv, TA* out, int nseq, int S, int inner, int n_head, int Cw, int HD, bool causal_b,
+                           const DropCfg& drop, uint32_t site, cudaStream_t st) {
     if (sizeof(TA) == 2 && drop.p <= 0.f) {
         // long sequences (composite axes, 65 .. 96-token axes, channel tokens): tiled online-softmax kernel
         cudaError_t e = cudaSuccess;
         if (launch_attention_flash(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<__nv_bfloat16*>(out), nseq, S,
                                    inner, n_head, Cw, HD, causal_b, st, &e)) {
             CK(e);
-            h->launches++;
-            return;
+            return TANTE_AXK_FLASH;
         }
     }
     if (sizeof(TA) == 2) {
@@ -688,8 +690,7 @@ void launch_attention_seq(tante_handle_s* h, const TA* qkv, TA* out, int nseq, i
         if (launch_attention_mma(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<__nv_bfloat16*>(out), nseq, S,
                                  inner, n_head, Cw, HD, causal_b, st, &e, drop, site)) {
             CK(e);
-            h->launches++;
-            return;
+            return TANTE_AXK_MMA;
         }
     }
     const long long total = (long long)nseq * n_head * S;
@@ -701,7 +702,13 @@ void launch_attention_seq(tante_handle_s* h, const TA* qkv, TA* out, int nseq, i
     if (HD == 32) ATT(32); else if (HD == 64) ATT(64); else ATT(16);
 #undef ATT
     CK(cudaGetLastError());
-    h->launches++;
+    return TANTE_AXK_SIMT;
+}
+
+template <typename TA>
+void launch_attention_seq(tante_handle_s* h, const TA* qkv, TA* out, int nseq, int S, int inner, int n_head, int Cw, int HD,
+                          bool causal_b, cudaStream_t st, const DropCfg& drop = DropCfg(), uint32_t site = 0) {
+    h->launches += axial_launches(dispatch_attention_fwd<TA>(qkv, out, nseq, S, inner, n_head, Cw, HD, causal_b, drop, site, st));
 }
 
 template <typename TA>
@@ -757,32 +764,24 @@ void run_channel_layer(tante_handle_s* h, const LayerPlan& lp, const float* x, f
     }
 }
 
-void launch_propagator(tante_handle_s* h, const float* xin, float* x, int B, int axis /*0=H,1=W,2=T*/,
-                       const OrderPlan& op, cudaStream_t st) {
-    int S; long long IC, outer;
-    const int T = h->T, L = h->L, Hp = h->Hp, Wp = h->Wp, C = h->C;
-    if (axis == 0) { S = Hp; IC = (long long)Wp * C; outer = (long long)B * T; }
-    else if (axis == 1) { S = Wp; IC = C; outer = (long long)B * T * Hp; }
-    else { S = T; IC = (long long)L * C; outer = B; }
+// Propagator of one axis: element (outer, p, col) at (outer * S + p) * IC + col; W1, W2 f32[S][S], b1, b2 f32[S].  xin == x
+// runs in place (inference), otherwise out of place (training).  Picks the kernel and launches it; returns its TANTE_AXK_* id.
+int dispatch_propagator(bool bf16, const float* xin, float* x, int S, long long IC, long long outer, const float* W1,
+                        const float* b1, const float* W2, const float* b2, int num_sms, cudaStream_t st) {
     if (S <= 4 && (IC & 3) == 0) {      // short axes (T = 4): per-column register mat-vecs, one pass over the latent
         const long long total = outer * (IC / 4);
-        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 16LL * h->num_sms);
-        const bool fast = h->cfg.precision == TANTE_PREC_BF16;
-#define PSMALL(TM, SM) propagator_small_kernel<TM, SM><<<grid, 256, 0, st>>>(xin, x, S, IC, outer, AF(h, op.prop[axis][0]), \
-            AF(h, op.prop[axis][1]), AF(h, op.prop[axis][2]), AF(h, op.prop[axis][3]))
-        if (fast) PSMALL(__nv_bfloat16, 4); else PSMALL(float, 4);
+        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 16LL * num_sms);
+#define PSMALL(TM, SM) propagator_small_kernel<TM, SM><<<grid, 256, 0, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2)
+        if (bf16) PSMALL(__nv_bfloat16, 4); else PSMALL(float, 4);
 #undef PSMALL
         CK(cudaGetLastError());
-        h->launches++;
-        return;
+        return TANTE_AXK_SMALL;
     }
-    if (h->cfg.precision == TANTE_PREC_BF16 && S > 8) {
+    if (bf16 && S > 8) {
         cudaError_t e = cudaSuccess;
-        if (launch_propagator_mma(xin, x, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]), AF(h, op.prop[axis][2]),
-                                  AF(h, op.prop[axis][3]), st, &e, h->num_sms)) {
+        if (launch_propagator_mma(xin, x, S, IC, outer, W1, b1, W2, b2, st, &e, num_sms)) {
             CK(e);
-            h->launches++;
-            return;
+            return TANTE_AXK_MMA;
         }
     }
     const int S4 = (S + 3) & ~3;
@@ -790,12 +789,22 @@ void launch_propagator(tante_handle_s* h, const float* xin, float* x, int B, int
     dim3 grid((unsigned)outer, (unsigned)((IC + 127) / 128));
     REQUIRE((IC + 127) / 128 <= 65535, "latent too large for the propagator grid");
     const int threads = 32 * std::min(8, S4 / 4);
-    if (h->cfg.precision == TANTE_PREC_BF16) propagator_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(xin, x, S, IC, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                               AF(h, op.prop[axis][2]), AF(h, op.prop[axis][3]));
-    else propagator_kernel<float><<<grid, threads, smem, st>>>(xin, x, S, IC, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                               AF(h, op.prop[axis][2]), AF(h, op.prop[axis][3]));
+    if (bf16) propagator_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(xin, x, S, IC, W1, b1, W2, b2);
+    else propagator_kernel<float><<<grid, threads, smem, st>>>(xin, x, S, IC, W1, b1, W2, b2);
     CK(cudaGetLastError());
-    h->launches++;
+    return TANTE_AXK_GENERIC;
+}
+
+void launch_propagator(tante_handle_s* h, const float* xin, float* x, int B, int axis /*0=H,1=W,2=T*/,
+                       const OrderPlan& op, cudaStream_t st) {
+    int S; long long IC, outer;
+    const int T = h->T, L = h->L, Hp = h->Hp, Wp = h->Wp, C = h->C;
+    if (axis == 0) { S = Hp; IC = (long long)Wp * C; outer = (long long)B * T; }
+    else if (axis == 1) { S = Wp; IC = C; outer = (long long)B * T * Hp; }
+    else { S = T; IC = (long long)L * C; outer = B; }
+    h->launches += axial_launches(dispatch_propagator(h->cfg.precision == TANTE_PREC_BF16, xin, x, S, IC, outer, AF(h, op.prop[axis][0]),
+                                                      AF(h, op.prop[axis][1]), AF(h, op.prop[axis][2]), AF(h, op.prop[axis][3]),
+                                                      h->num_sms, st));
 }
 
 inline unsigned blocks_for(long long n, int per) { return (unsigned)((n + per - 1) / per); }
@@ -1702,6 +1711,49 @@ void launch_ln_bwd(tante_handle_s* h, const TA* dy, const float* x, int64_t gamm
     h->launches++;
 }
 
+// Attention backward over the sequences of dispatch_attention_fwd: dqkv (packed like qkv) from qkv and the output gradient dout.
+// `stats` = f32[2 * nseq * n_head * S] scratch of the S > 64 kernels.  Returns the TANTE_AXK_* id of what it launched.
+template <typename TA>
+int dispatch_attention_bwd(const TA* qkv, const TA* dout, TA* dqkv, float* stats, long long nseq, int S, int inner, int n_head,
+                           int C, int HD, bool causal, const DropCfg& drop, uint32_t site, cudaStream_t st) {
+    if (S > 64) {
+        // composite axes and 65 .. 96-token axes: tiled recompute backward -- on mma.sync in the tensor mode without dropout
+        // (attention_long_bwd_mma.cuh), on FFMA tiles otherwise (attention_long_bwd.cuh)
+        cudaError_t e = cudaSuccess;
+        if constexpr (sizeof(TA) == 2) {
+            if (drop.p <= 0.f && launch_attention_long_bwd_mma(qkv, dout, dqkv, stats, nseq, S, inner, n_head, C, HD, causal, st, &e)) {
+                CK(e);
+                return TANTE_AXK_LONG_MMA;
+            }
+        }
+        REQUIRE(launch_attention_long_bwd<TA>(qkv, dout, dqkv, stats, nseq, S, inner, n_head, C, HD, causal, st, &e, drop, site),
+                "attention backward: sequence shape not covered");
+        CK(e);
+        return TANTE_AXK_LONG_FFMA;
+    }
+    if constexpr (sizeof(TA) == 2) {
+        cudaError_t e = cudaSuccess;
+        if (launch_attention_bwd_mma(qkv, dout, dqkv, nseq, S, inner, n_head, C, HD, causal, st, &e, drop, site)) {
+            CK(e);
+            return TANTE_AXK_MMA;
+        }
+    }
+    const int G = std::max(1, 64 / S);
+    const int R = G * S;
+    const float scale = 1.0f / sqrtf((float)HD);
+    dim3 grid((unsigned)((nseq + G - 1) / G), (unsigned)n_head);
+#define ATTB(HDv)                                                                                              \
+    do {                                                                                                       \
+        const size_t smem = (size_t)(4 * R * (HDv + 1) + 2 * R * (S + 1)) * sizeof(float);                     \
+        attention_bwd_kernel<TA, HDv><<<grid, 128, smem, st>>>(qkv, dout, dqkv, nseq, S, inner, n_head, C,      \
+                                                               causal, scale, G, drop, site);                  \
+    } while (0)
+    if (HD == 32) ATTB(32); else if (HD == 64) ATTB(64); else ATTB(16);
+#undef ATTB
+    CK(cudaGetLastError());
+    return TANTE_AXK_SIMT;
+}
+
 template <typename TA>
 void launch_attention_bwd(tante_handle_s* h, const TA* qkv, const TA* dout, TA* dqkv, int B, char axis, cudaStream_t st,
                           const DropCfg& drop = DropCfg(), uint32_t site = 0) {
@@ -1713,47 +1765,56 @@ void launch_attention_bwd(tante_handle_s* h, const TA* qkv, const TA* dout, TA* 
     else if (axis == 'L') { S = L; inner = 1; nseq = (long long)B * T; }               // (b t) (h w)
     else if (axis == 'Y') { S = T * Hp; inner = Wp; nseq = (long long)B * Wp; }        // (b w) (t h)
     else { S = T * L; inner = 1; nseq = B; }                                           // 'A': b (t h w)
-    if (S > 64) {
-        // composite axes and 65 .. 96-token axes: tiled recompute backward -- on mma.sync in the tensor mode without dropout
-        // (attention_long_bwd_mma.cuh), on FFMA tiles otherwise (attention_long_bwd.cuh)
-        cudaError_t e = cudaSuccess;
-        if constexpr (sizeof(TA) == 2) {
-            if (drop.p <= 0.f && launch_attention_long_bwd_mma(qkv, dout, dqkv, FP(h->att_stats), nseq, S, inner, h->cfg.n_head, h->C,
-                                                               h->HD, axis == 'T', st, &e)) {
-                CK(e);
-                h->launches += 3;
-                return;
-            }
-        }
-        REQUIRE(launch_attention_long_bwd<TA>(qkv, dout, dqkv, FP(h->att_stats), nseq, S, inner, h->cfg.n_head, h->C, h->HD,
-                                              axis == 'T', st, &e, drop, site),
-                "attention backward: sequence shape not covered");
-        CK(e);
-        h->launches += 3;
-        return;
+    h->launches += axial_launches(dispatch_attention_bwd<TA>(qkv, dout, dqkv, FP(h->att_stats), nseq, S, inner, h->cfg.n_head, h->C,
+                                                             h->HD, axis == 'T', drop, site, st));
+}
+
+// Backward of dispatch_propagator: dy (the gradient of its output) is overwritten in place by the gradient of its input xin;
+// gW1, gb1, gW2, gb2 are accumulated into.  Returns the TANTE_AXK_* id of what it launched.
+int dispatch_propagator_bwd(bool bf16, const float* xin, float* dy, int S, long long IC, long long outer, const float* W1,
+                            const float* b1, const float* W2, float* gW1, float* gb1, float* gW2, float* gb2, int num_sms,
+                            cudaStream_t st) {
+    if (S <= 4 && (IC & 3) == 0) {
+        const long long total = outer * (IC / 4);
+        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 2LL * num_sms);
+#define PSMALLB(TM, SM) propagator_small_bwd_kernel<TM, SM><<<grid, 256, 0, st>>>(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2)
+        if (bf16) PSMALLB(__nv_bfloat16, 4); else PSMALLB(float, 4);
+#undef PSMALLB
+        CK(cudaGetLastError());
+        return TANTE_AXK_SMALL;
     }
-    if constexpr (sizeof(TA) == 2) {
+    if (bf16) {
         cudaError_t e = cudaSuccess;
-        if (launch_attention_bwd_mma(qkv, dout, dqkv, nseq, S, inner, h->cfg.n_head, h->C, h->HD, axis == 'T', st, &e, drop, site)) {
+        if (launch_propagator_bwd_mma(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2, num_sms, st, &e)) {
             CK(e);
-            h->launches++;
-            return;
+            return TANTE_AXK_MMA;
         }
     }
-    const int G = std::max(1, 64 / S);
-    const int R = G * S;
-    const float scale = 1.0f / sqrtf((float)h->HD);
-    dim3 grid((unsigned)((nseq + G - 1) / G), (unsigned)h->cfg.n_head);
-#define ATTB(HDv)                                                                                              \
-    do {                                                                                                       \
-        const size_t smem = (size_t)(4 * R * (HDv + 1) + 2 * R * (S + 1)) * sizeof(float);                     \
-        attention_bwd_kernel<TA, HDv><<<grid, 128, smem, st>>>(qkv, dout, dqkv, nseq, S, inner, h->cfg.n_head, \
-                                                               h->C, axis == 'T', scale, G, drop, site);       \
-    } while (0)
-    if (h->HD == 32) ATTB(32); else if (h->HD == 64) ATTB(64); else ATTB(16);
-#undef ATTB
+    if (S > 64) {      // 65 .. 96-token axes: the one-lane-per-column kernel (both S x S matrices in shared memory)
+        REQUIRE(S <= kPropWideMaxS, "propagator backward: axis longer than 96 tokens");
+        const long long nslabw = outer * ((IC + kPropWideCols - 1) / kPropWideCols);
+        const unsigned gridw = (unsigned)std::min<long long>(nslabw, 2LL * num_sms);
+        const size_t smw = prop_bwd_wide_smem(S);
+        if (bf16) {
+            CK(cudaFuncSetAttribute(propagator_bwd_wide_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
+            propagator_bwd_wide_kernel<__nv_bfloat16><<<gridw, 256, smw, st>>>(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2);
+        } else {
+            CK(cudaFuncSetAttribute(propagator_bwd_wide_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
+            propagator_bwd_wide_kernel<float><<<gridw, 256, smw, st>>>(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2);
+        }
+        CK(cudaGetLastError());
+        return TANTE_AXK_WIDE;
+    }
+    int S4 = (S + 3) & ~3;
+    if (S4 > 4 && (S4 & (S4 - 1))) { int p2 = 8; while (p2 < S4) p2 <<= 1; S4 = p2; }
+    const int CW = kPropBwdSlab / S4;
+    const size_t smem = (size_t)(4 * (kPropBwdSlab + 4 * S4) + 3 * S4 * S4 + S4) * sizeof(float);
+    const long long nslab = outer * ((IC + CW - 1) / CW);
+    const unsigned grid = (unsigned)std::min<long long>(nslab, 2LL * num_sms);
+    if (bf16) propagator_bwd_kernel<__nv_bfloat16><<<grid, 256, smem, st>>>(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2);
+    else propagator_bwd_kernel<float><<<grid, 256, smem, st>>>(xin, dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2);
     CK(cudaGetLastError());
-    h->launches++;
+    return TANTE_AXK_GENERIC;
 }
 
 void launch_propagator_bwd(tante_handle_s* h, const float* xin, float* dy, int B, int axis, const OrderPlan& op, cudaStream_t st) {
@@ -1762,65 +1823,10 @@ void launch_propagator_bwd(tante_handle_s* h, const float* xin, float* dy, int B
     if (axis == 0) { S = Hp; IC = (long long)Wp * C; outer = (long long)B * T; }
     else if (axis == 1) { S = Wp; IC = C; outer = (long long)B * T * Hp; }
     else { S = T; IC = (long long)L * C; outer = B; }
-    if (S <= 4 && (IC & 3) == 0) {
-        const long long total = outer * (IC / 4);
-        const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 2LL * h->num_sms);
-        const bool fast = h->cfg.precision == TANTE_PREC_BF16;
-#define PSMALLB(TM, SM) propagator_small_bwd_kernel<TM, SM><<<grid, 256, 0, st>>>(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), \
-            AF(h, op.prop[axis][1]), AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),                \
-            GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]))
-        if (fast) PSMALLB(__nv_bfloat16, 4); else PSMALLB(float, 4);
-#undef PSMALLB
-        CK(cudaGetLastError());
-        h->launches++;
-        return;
-    }
-    if (h->cfg.precision == TANTE_PREC_BF16) {
-        cudaError_t e = cudaSuccess;
-        if (launch_propagator_bwd_mma(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                      AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),
-                                      GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]), h->num_sms, st, &e)) {
-            CK(e);
-            h->launches++;
-            return;
-        }
-    }
-    if (S > 64) {      // 65 .. 96-token axes: the one-lane-per-column kernel (both S x S matrices in shared memory)
-        REQUIRE(S <= kPropWideMaxS, "propagator backward: axis longer than 96 tokens");
-        const long long nslabw = outer * ((IC + kPropWideCols - 1) / kPropWideCols);
-        const unsigned gridw = (unsigned)std::min<long long>(nslabw, 2LL * h->num_sms);
-        const size_t smw = prop_bwd_wide_smem(S);
-        if (h->cfg.precision == TANTE_PREC_BF16) {
-            CK(cudaFuncSetAttribute(propagator_bwd_wide_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-            propagator_bwd_wide_kernel<__nv_bfloat16><<<gridw, 256, smw, st>>>(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                                                              AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),
-                                                                              GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]));
-        } else {
-            CK(cudaFuncSetAttribute(propagator_bwd_wide_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-            propagator_bwd_wide_kernel<float><<<gridw, 256, smw, st>>>(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                                                      AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),
-                                                                      GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]));
-        }
-        CK(cudaGetLastError());
-        h->launches++;
-        return;
-    }
-    int S4 = (S + 3) & ~3;
-    if (S4 > 4 && (S4 & (S4 - 1))) { int p2 = 8; while (p2 < S4) p2 <<= 1; S4 = p2; }
-    const int CW = kPropBwdSlab / S4;
-    const size_t smem = (size_t)(4 * (kPropBwdSlab + 4 * S4) + 3 * S4 * S4 + S4) * sizeof(float);
-    const long long nslab = outer * ((IC + CW - 1) / CW);
-    const unsigned grid = (unsigned)std::min<long long>(nslab, 2LL * h->num_sms);
-    if (h->cfg.precision == TANTE_PREC_BF16)
-        propagator_bwd_kernel<__nv_bfloat16><<<grid, 256, smem, st>>>(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                                                     AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),
-                                                                     GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]));
-    else
-        propagator_bwd_kernel<float><<<grid, 256, smem, st>>>(xin, dy, S, IC, outer, AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]),
-                                                             AF(h, op.prop[axis][2]), GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]),
-                                                             GA(h, op.prop[axis][2]), GA(h, op.prop[axis][3]));
-    CK(cudaGetLastError());
-    h->launches++;
+    h->launches += axial_launches(dispatch_propagator_bwd(h->cfg.precision == TANTE_PREC_BF16, xin, dy, S, IC, outer,
+                                                          AF(h, op.prop[axis][0]), AF(h, op.prop[axis][1]), AF(h, op.prop[axis][2]),
+                                                          GA(h, op.prop[axis][0]), GA(h, op.prop[axis][1]), GA(h, op.prop[axis][2]),
+                                                          GA(h, op.prop[axis][3]), h->num_sms, st));
 }
 
 void free_tape(Tape& tp) {
@@ -3445,6 +3451,69 @@ int tante_test_gemm(int32_t use_tc, int32_t epi, const void* A, const void* W, c
                 CK(launch_gemm_simt(epi, reinterpret_cast<const float*>(A), K, reinterpret_cast<const float*>(W), K,
                                     reinterpret_cast<float*>(C), N, M, N, K, ep, st));
         }
+    });
+}
+
+static bool aligned16(const void* p) { return reinterpret_cast<uintptr_t>(p) % 16 == 0; }
+
+int tante_test_attention(int32_t dir, int32_t precision, const void* qkv, const void* dout, void* out_or_dqkv, float* stats,
+                         int64_t nseq, int32_t S, int32_t inner_sz, int32_t n_head, int32_t C, int32_t causal, float drop_p,
+                         uint64_t seed, uint32_t site, int32_t* kernel, void* stream) {
+    return guarded([&] {
+        REQUIRE(dir == 0 || dir == 1, "dir: 0 forward, 1 backward");
+        REQUIRE(precision == TANTE_PREC_FP32 || precision == TANTE_PREC_BF16, "unknown precision");
+        REQUIRE(qkv && out_or_dqkv && kernel && (dir == 0 || dout) && (dir == 0 || S <= 64 || stats), "null argument");
+        REQUIRE(aligned16(qkv) && aligned16(dout) && aligned16(out_or_dqkv) && aligned16(stats), "buffers must be 16-byte aligned");
+        REQUIRE(S >= 1 && inner_sz >= 1 && nseq >= 1 && nseq <= 0x7fffffffLL, "S, inner_sz and nseq must be >= 1 (nseq < 2^31)");
+        REQUIRE(n_head >= 1 && C >= 1 && C % n_head == 0, "C must be n_head * head_dim");
+        const int HD = C / n_head;
+        REQUIRE(HD == 16 || HD == 32 || HD == 64, "head_dim must be 16, 32 or 64");
+        REQUIRE(causal == 0 || causal == 1, "causal must be 0 or 1");
+        REQUIRE(drop_p >= 0.f && drop_p < 1.f, "drop_p must be in [0, 1)");
+        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+        int dev = 0, sms = 148;
+        CK(cudaGetDevice(&dev));
+        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        set_smem_attrs();
+        const DropCfg drop = make_drop_cfg(drop_p, seed);
+        if (precision == TANTE_PREC_BF16) {
+            using B = __nv_bfloat16;
+            *kernel = dir == 0 ? dispatch_attention_fwd<B>(static_cast<const B*>(qkv), static_cast<B*>(out_or_dqkv), (int)nseq, S,
+                                                           inner_sz, n_head, C, HD, causal, drop, site, st)
+                               : dispatch_attention_bwd<B>(static_cast<const B*>(qkv), static_cast<const B*>(dout),
+                                                           static_cast<B*>(out_or_dqkv), stats, nseq, S, inner_sz, n_head, C, HD,
+                                                           causal, drop, site, st);
+        } else {
+            *kernel = dir == 0 ? dispatch_attention_fwd<float>(static_cast<const float*>(qkv), static_cast<float*>(out_or_dqkv),
+                                                               (int)nseq, S, inner_sz, n_head, C, HD, causal, drop, site, st)
+                               : dispatch_attention_bwd<float>(static_cast<const float*>(qkv), static_cast<const float*>(dout),
+                                                               static_cast<float*>(out_or_dqkv), stats, nseq, S, inner_sz, n_head,
+                                                               C, HD, causal, drop, site, st);
+        }
+    });
+}
+
+int tante_test_propagator(int32_t dir, int32_t precision, const float* xin, float* x_or_dy, const float* W1, const float* b1,
+                          const float* W2, const float* b2, float* gW1, float* gb1, float* gW2, float* gb2, int32_t S, int64_t IC,
+                          int64_t outer, int32_t* kernel, void* stream) {
+    return guarded([&] {
+        REQUIRE(dir == 0 || dir == 1, "dir: 0 forward, 1 backward");
+        REQUIRE(precision == TANTE_PREC_FP32 || precision == TANTE_PREC_BF16, "unknown precision");
+        REQUIRE(xin && x_or_dy && W1 && b1 && W2 && kernel, "null argument");
+        REQUIRE(dir == 1 || b2, "null argument");
+        REQUIRE(dir == 0 || (gW1 && gb1 && gW2 && gb2), "null argument");
+        REQUIRE(aligned16(xin) && aligned16(x_or_dy), "xin and x_or_dy must be 16-byte aligned");
+        REQUIRE(S >= 1 && S <= kPropWideMaxS, "S must be in 1 .. 96");
+        REQUIRE(IC >= 4 && IC % 4 == 0, "IC must be a positive multiple of 4");
+        REQUIRE(outer >= 1 && outer <= 0x7fffffffLL, "outer must be in 1 .. 2^31 - 1");
+        cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+        int dev = 0, sms = 148;
+        CK(cudaGetDevice(&dev));
+        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        set_smem_attrs();
+        const bool bf16 = precision == TANTE_PREC_BF16;
+        *kernel = dir == 0 ? dispatch_propagator(bf16, xin, x_or_dy, S, IC, outer, W1, b1, W2, b2, sms, st)
+                           : dispatch_propagator_bwd(bf16, xin, x_or_dy, S, IC, outer, W1, b1, W2, gW1, gb1, gW2, gb2, sms, st);
     });
 }
 

@@ -38,6 +38,50 @@ def test_library_is_sm100a_and_torch_free():
         assert "sm_100a" in cu.stdout
 
 
+def test_axial_test_hooks_reject_out_of_range_arguments():
+    """tante_test_attention / tante_test_propagator check their arguments before any device call (so this runs without
+    a GPU).  Every call below breaks exactly one rule of an otherwise valid call; the pointers are never dereferenced."""
+    lib = _abi.load()
+    P = 0x10000          # 16-byte aligned stand-in for a device buffer
+    kid = ctypes.c_int32(-1)
+
+    def att(**kw):
+        a = dict(dir=1, prec=_abi.PREC_BF16, qkv=P, dout=P, out=P, stats=P, nseq=8, S=80, inner=1, nh=8, C=256, causal=0,
+                 p=0.0)
+        a.update(kw)
+        return lib.tante_test_attention(a["dir"], a["prec"], a["qkv"], a["dout"], a["out"], a["stats"], a["nseq"], a["S"],
+                                        a["inner"], a["nh"], a["C"], a["causal"], a["p"], 1, 0, ctypes.byref(kid), None)
+
+    def prop(**kw):
+        a = dict(dir=1, prec=_abi.PREC_BF16, xin=P, x=P, W1=P, b1=P, W2=P, b2=P, gW1=P, gb1=P, gW2=P, gb2=P, S=32, IC=256,
+                 outer=4)
+        a.update(kw)
+        return lib.tante_test_propagator(a["dir"], a["prec"], a["xin"], a["x"], a["W1"], a["b1"], a["W2"], a["b2"], a["gW1"],
+                                         a["gb1"], a["gW2"], a["gb2"], a["S"], a["IC"], a["outer"], ctypes.byref(kid), None)
+
+    bad = [
+        (att, dict(qkv=None), "null argument"), (att, dict(out=None), "null argument"), (att, dict(dout=None), "null argument"),
+        (att, dict(stats=None), "null argument"), (att, dict(qkv=P + 2), "16-byte aligned"),
+        (att, dict(S=0), "must be >= 1"), (att, dict(nseq=0), "must be >= 1"), (att, dict(inner=0), "must be >= 1"),
+        (att, dict(nseq=1 << 31), "must be >= 1"),
+        (att, dict(C=256, nh=2), "head_dim must be 16, 32 or 64"), (att, dict(C=256, nh=32), "head_dim must be 16, 32 or 64"),
+        (att, dict(C=250, nh=8), "C must be n_head * head_dim"), (att, dict(nh=0), "C must be n_head * head_dim"),
+        (att, dict(p=1.0), "drop_p must be in [0, 1)"), (att, dict(p=-0.1), "drop_p must be in [0, 1)"),
+        (att, dict(p=float("nan")), "drop_p must be in [0, 1)"), (att, dict(causal=2), "causal must be 0 or 1"),
+        (att, dict(dir=2), "dir"), (att, dict(prec=7), "precision"),
+        (prop, dict(xin=None), "null argument"), (prop, dict(W2=None), "null argument"), (prop, dict(gW1=None), "null argument"),
+        (prop, dict(gb2=None), "null argument"), (prop, dict(dir=0, b2=None), "null argument"),
+        (prop, dict(x=P + 4), "16-byte aligned"),
+        (prop, dict(S=0), "S must be in 1 .. 96"), (prop, dict(S=97), "S must be in 1 .. 96"),
+        (prop, dict(IC=0), "IC must be a positive multiple of 4"), (prop, dict(IC=258), "IC must be a positive multiple of 4"),
+        (prop, dict(outer=0), "outer must be"), (prop, dict(dir=-1), "dir"), (prop, dict(prec=2), "precision"),
+    ]
+    for fn, kw, msg in bad:
+        assert fn(**kw) == 1, (fn.__name__, kw)
+        assert msg in lib.tante_last_error().decode(), (fn.__name__, kw, lib.tante_last_error())
+    assert kid.value == -1
+
+
 def _cfg(**kw):
     c = _abi.TanteConfig()
     base = dict(in_T=4, n_fields=4, H=128, W=384, taylor_order=1, n_head=8, embed_dim=256, patch_scale=8, deg=1,
