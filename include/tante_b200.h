@@ -252,6 +252,10 @@ TANTE_API int tante_test_gemm(int32_t use_tc, int32_t epi, const void* A, const 
                     const float* resid, void* C, int32_t out_bf16, int32_t M, int32_t N, int32_t K,
                     int32_t iters, const float* ln_gamma, const float* ln_beta, void* ln_out, void* stream);
 
+/* Test hook: the plan the tcgen05 GEMM (tante_test_gemm with use_tc = 1, and the model's own GEMMs) runs for C[M,N] with a
+ * K-long reduction on the current device: *ncta = CTAs that share one MMA (1, or 2 for a CTA pair). */
+TANTE_API int tante_test_gemm_plan(int32_t M, int32_t N, int32_t K, int32_t out_bf16, int32_t* ncta);
+
 /* Test hook: the fused block tail (block_tail_tc.cuh; reference attn_backbone.py:81-83 + the next layer's LayerNorm) stand-alone:
  *   x_mid = x_in + att Wo^T + bo;  h = gelu_tanh(LN(x_mid; g2, be2) W1^T + b1);  x_out = x_mid + h W2^T + b2;
  *   ln_out = LN(x_out; gn, ben)   (skipped when ln_out is NULL).

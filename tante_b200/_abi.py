@@ -70,6 +70,7 @@ SIGNATURES = {
     "tante_test_gemm": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_void_p]),
+    "tante_test_gemm_plan": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
     "tante_comm_unique_id": (C.c_int, [C.c_void_p]),
     "tante_comm_init": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "tante_allreduce_grads": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

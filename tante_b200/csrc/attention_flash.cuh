@@ -141,8 +141,7 @@ __global__ void __launch_bounds__(128) attention_flash_kernel(const __nv_bfloat1
 // Host launcher: sequences longer than 64 tokens, head_dim 32, no dropout.  Returns false otherwise (caller falls back).
 static bool launch_attention_flash(const __nv_bfloat16* qkv, __nv_bfloat16* out, long long n_seq, int S, int inner_sz, int n_head,
                                    int C, int head_dim, int causal, cudaStream_t st, cudaError_t* err) {
-    static const bool on = !(getenv("TANTE_ATT_FLASH") && atoi(getenv("TANTE_ATT_FLASH")) == 0);
-    if (!on || head_dim != 32 || S <= 64 || causal || n_seq * n_head > 0x7fffffffLL || (S + 63) / 64 > 65535) return false;
+    if (head_dim != 32 || S <= 64 || causal || n_seq * n_head > 0x7fffffffLL || (S + 63) / 64 > 65535) return false;
     dim3 grid((unsigned)(n_seq * n_head), (unsigned)((S + 63) / 64));
     const float sl2 = (1.0f / sqrtf((float)head_dim)) * 1.4426950408889634f;
     attention_flash_kernel<<<grid, 128, 0, st>>>(qkv, out, S, inner_sz, n_head, C, sl2);

@@ -297,10 +297,9 @@ __global__ void __launch_bounds__(128) attn_long_kv_mma_kernel(const __nv_bfloat
 static bool launch_attention_long_bwd_mma(const __nv_bfloat16* qkv, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, float* stats,
                                           long long n_seq, int S, int inner_sz, int n_head, int C, int head_dim, int causal,
                                           cudaStream_t st, cudaError_t* err) {
-    static const bool on = !(getenv("TANTE_ATT_LONG_MMA") && atoi(getenv("TANTE_ATT_LONG_MMA")) == 0);
     const long long gx = n_seq * n_head;
     const int tiles = (S + 63) / 64;
-    if (!on || head_dim != 32 || causal || gx > 0x7fffffffLL || tiles > 65535) return false;
+    if (head_dim != 32 || causal || gx > 0x7fffffffLL || tiles > 65535) return false;
     AlmGeom g{S, inner_sz, n_head, C, (1.0f / sqrtf((float)head_dim)) * 1.4426950408889634f, 1.0f / sqrtf((float)head_dim)};
     float* lse2 = stats;
     float* delta = stats + (size_t)gx * S;

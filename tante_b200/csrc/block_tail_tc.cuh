@@ -60,13 +60,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                   const __grid_constant__ CUtensorMap tmXin, const __grid_constant__ CUtensorMap tmXmid,
                   const __grid_constant__ CUtensorMap tmXout, const __grid_constant__ CUtensorMap tmLn2,
                   const __grid_constant__ CUtensorMap tmHpre, const __grid_constant__ CUtensorMap tmHact,
-                  const __grid_constant__ CUtensorMap tmLnOut, BtParams p, long long* trace) {
+                  const __grid_constant__ CUtensorMap tmLnOut, BtParams p) {
     constexpr bool TRAIN = MODE != 0;
-    // TANTE_TAIL_TRACE (debugging aid): CTA 0 records (event, clock64) pairs -- role 0 = MMA warp, 1 = first epilogue warp
-    int tr_n = 0;
-    auto TR = [&](int role, int ev) {
-        if (trace && blockIdx.x == 0 && tr_n < 1024) { trace[(role * 1024 + tr_n) * 2] = ev; trace[(role * 1024 + tr_n) * 2 + 1] = clock64(); ++tr_n; }
-    };
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment (SWIZZLE_128B) as an OFFSET into the shared array: a pointer -> integer -> pointer round trip would
     // lose the address space and turn every shared-memory access of the epilogue into a generic LD / ST
@@ -190,7 +185,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                     ++ar;
                 }
                 ptx::tc_fence_after();
-                if (lane == 0) TR(0, 100 + ph);
                 for (int kb = 0; kb < 4; ++kb) {
                     for (int nh = 0; nh < 2 / NCTA; ++nh) {
                         ptx::mbar_wait(&w_full[ws], wph);
@@ -211,7 +205,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                     }
                 }
                 if (lane == 0) {
-                    TR(0, 200 + ph);
                     if (NCTA == 2) {
                         ptx::umma_commit_pair(acc_full);
                         if (ph == 2) ptx::umma_commit_pair(a_empty);
@@ -300,10 +293,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                 ptx::mbar_arrive_expect_tx(&rb[0], kBtEbuf);
                 ptx::tma_load_2d(ebuf, &tmXin, &rb[0], cs * 32, row0);
             }
-            if (ew == 0 && lane == 0) TR(1, 10);
             ptx::mbar_wait(acc_full, af & 1u); ++af;
             ptx::tc_fence_after();
-            if (ew == 0 && lane == 0) TR(1, 11);
             if (lane == 0) {      // the A tile has been consumed by the first GEMM: its 4 KB slot takes the second chunk
                 ptx::mbar_arrive_expect_tx(&rb[1], kBtEbuf);
                 ptx::tma_load_2d(aslot, &tmXin, &rb[1], (cs + 4) * 32, row0);
@@ -354,11 +345,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             }
             {
                 float mean, rstd;
-                if (ew == 0 && lane == 0) TR(1, 12);
                 row_stats(0, rsum, rsq, mean, rstd);
-                if (ew == 0 && lane == 0) TR(1, 13);
                 ln_kblock(tm_x, mean, rstd, g2, be2, aown, lane);
-                if (ew == 0 && lane == 0) TR(1, 14);
                 if (TRAIN) {      // the saved LN2 output leaves straight from the A tile (same 32-row x 128-B swizzled box)
                     ptx::fence_proxy_async();
                     __syncwarp();
@@ -373,7 +361,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             // ---------------- phase 2: hidden = gelu_tanh(acc + b1) -> A tile ----------------
             ptx::mbar_wait(acc_full, af & 1u); ++af;
             ptx::tc_fence_after();
-            if (ew == 0 && lane == 0) TR(1, 21);
             if (lane == 0 && tile + ncl < tiles) {      // pull the next tile's residual rows into L2 (the loads themselves are issued late)
                 const int nrow0 = ((tile + ncl) * NCTA + crank) * 128 + q * 32;
                 ptx::tma_prefetch_l2_2d(&tmXin, cs * 32, nrow0);
@@ -427,10 +414,8 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             if (lane == 0) { if (NCTA == 2 && crank == 1 && kBtDirect) ptx::mbar_arrive_leader(a_ready); else ptx::mbar_arrive(a_ready); }
 
             // ---------------- phase 3: x_out = x_mid + drop(acc + b2) ; LN1' ----------------
-            if (ew == 0 && lane == 0) TR(1, 24);
             ptx::mbar_wait(acc_full, af & 1u); ++af;
             ptx::tc_fence_after();
-            if (ew == 0 && lane == 0) TR(1, 31);
             if (TRAIN) {      // hidden / pre-activation stores drained: the producer may refill the A tile
                 ebuf_free();
                 if (lane == 0) ptx::mbar_arrive(a_empty);
@@ -478,11 +463,9 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             if (lane == 0) {                                    // the next tile's first GEMM may overwrite the accumulator
                 if (NCTA == 2 && crank == 1 && kBtDirect) ptx::mbar_arrive_leader(acc_free); else ptx::mbar_arrive(acc_free);
             }
-            if (ew == 0 && lane == 0) TR(1, 32);
             if (p.has_ln_out) {
                 float mean, rstd;
                 row_stats(1, rsum, rsq, mean, rstd);
-                if (ew == 0 && lane == 0) TR(1, 33);
                 ebuf_free();
                 ln_kblock(tm_x, mean, rstd, gn, ben, ebuf, lane);
                 ptx::fence_proxy_async();
@@ -494,7 +477,6 @@ block_tail_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                 named_bar_sync(1 + q, 4 * 32);
                 ptx::tc_fence_after();
             }
-            if (ew == 0 && lane == 0) TR(1, 34);
         }
         if (lane == 0) ptx::bulk_wait_all<0>();
     }
@@ -556,9 +538,8 @@ static cudaError_t launch_block_tail(const BlockTailArgs& a, int M, bool train, 
     p.bo = a.bo; p.g2 = a.g2; p.be2 = a.be2; p.b1 = a.b1; p.b2 = a.b2; p.gn = a.gn; p.ben = a.ben;
     p.M = M; p.has_ln_out = a.ln_out != nullptr;
     p.drop = train ? a.drop : DropCfg(); p.site1 = a.site1; p.site2 = a.site2;
-    // CTA pairs (TANTE_TAIL_2CTA = 0 disables them) once there are enough 256-row units to fill the machine
-    static const int pair_mode = getenv("TANTE_TAIL_2CTA") ? atoi(getenv("TANTE_TAIL_2CTA")) : 1;
-    const int ncta = (pair_mode == 2 || (pair_mode == 1 && M >= 256 * (num_sms / 2))) ? 2 : 1;
+    // CTA pairs once there are enough 256-row units to fill the machine
+    const int ncta = M >= 256 * (num_sms / 2) ? 2 : 1;
     const int tiles = (M + 128 * ncta - 1) / (128 * ncta);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(ncta * std::min(tiles, num_sms / ncta))); cfg.blockDim = dim3(kBtThreads); cfg.dynamicSmemBytes = kBtSmem; cfg.stream = st;
@@ -575,27 +556,14 @@ static cudaError_t launch_block_tail(const BlockTailArgs& a, int M, bool train, 
         ++na;
     }
     cfg.attrs = at; cfg.numAttrs = (unsigned)na;
-    long long* trace = nullptr;
-    static const char* trace_path = getenv("TANTE_TAIL_TRACE");      // debugging aid: per-phase clock64 stamps of CTA 0
-    if (trace_path) {
-        if (cudaMalloc(&trace, 3 * 1024 * 2 * sizeof(long long)) != cudaSuccess) return cudaErrorMemoryAllocation;
-        cudaMemsetAsync(trace, 0, 3 * 1024 * 2 * sizeof(long long), st);
-    }
-    cudaError_t e;
 #define TANTE_BT_LAUNCH(MODE, NC) \
-    e = cudaLaunchKernelEx(&cfg, block_tail_kernel<MODE, NC>, tmA, tmWo, tmW1, tmW2, tmXin, tmXmid, tmXout, tmLn2, tmHpre, tmHact, tmLnOut, p, trace)
+    return cudaLaunchKernelEx(&cfg, block_tail_kernel<MODE, NC>, tmA, tmWo, tmW1, tmW2, tmXin, tmXmid, tmXout, tmLn2, tmHpre, tmHact, tmLnOut, p)
     const int mode = (train && p.drop.p > 0.f) ? 2 : (train ? 1 : 0);
-    if (ncta == 2) { if (mode == 2) TANTE_BT_LAUNCH(2, 2); else if (mode == 1) TANTE_BT_LAUNCH(1, 2); else TANTE_BT_LAUNCH(0, 2); }
-    else { if (mode == 2) TANTE_BT_LAUNCH(2, 1); else if (mode == 1) TANTE_BT_LAUNCH(1, 1); else TANTE_BT_LAUNCH(0, 1); }
+    if (ncta == 2) { if (mode == 2) TANTE_BT_LAUNCH(2, 2); if (mode == 1) TANTE_BT_LAUNCH(1, 2); TANTE_BT_LAUNCH(0, 2); }
+    if (mode == 2) TANTE_BT_LAUNCH(2, 1);
+    if (mode == 1) TANTE_BT_LAUNCH(1, 1);
+    TANTE_BT_LAUNCH(0, 1);
 #undef TANTE_BT_LAUNCH
-    if (trace) {
-        std::vector<long long> hbuf(3 * 1024 * 2);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(hbuf.data(), trace, hbuf.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        cudaFree(trace);
-        if (FILE* f = fopen(trace_path, "wb")) { fwrite(hbuf.data(), sizeof(long long), hbuf.size(), f); fclose(f); }
-    }
-    return e;
 }
 
 }  // namespace tante

@@ -181,10 +181,6 @@ enum Epilogue : int {
     EPI_BIAS_RESID = 4,  // C = resid + acc + bias   (fp32 residual stream, may alias C)
     EPI_EMBED = 5,       // encoder tail: v=acc+bias; v += v*scale[t]+shift[t]; v += s_emb[hw]; v += t_emb[t]
     EPI_BIAS_RESID_LN = 6,  // EPI_BIAS_RESID + LayerNorm of the updated row written to a second (bf16) output
-    // input-gradient GEMMs (tensor GEMM, bf16 output only): C = (acc + bias) * f'(pre[m][n]), pre = EpiParams::mul_pre
-    EPI_MULGRAD_RELU = 7,
-    EPI_MULGRAD_GELU_ERF = 8,
-    EPI_MULGRAD_GELU_TANH = 9,
 };
 
 struct EpiParams {
@@ -203,9 +199,11 @@ struct EpiParams {
     // optional device-side row count (rollout encoder cache): effective M = min(M, *m_dev * m_rows)
     const int* m_dev = nullptr;
     int m_rows = 0;
-    // EPI_MULGRAD_*: saved pre-activation (post-activation for ReLU), bf16 [M, ld_pre]
-    const void* mul_pre = nullptr;
-    int ld_pre = 0;
+    // Keeps the layout (and the 136-byte size) that the FP32 FFMA GEMM was tuned with: it takes EpiParams by value, and at
+    // 120 bytes nvcc keeps the fields in registers instead of re-reading the parameter space, which costs
+    // gemm_simt_kernel<128, *> its second CTA per SM (142 registers; residual epilogue at M = 65536 on a B200 at 1000 W:
+    // 245 -> 310 us).
+    uint32_t reserved[4] = {0u, 0u, 0u, 0u};
     // EPI_BIAS_RESID in training with dropout (SIMT GEMM): C = resid + drop(acc + bias), element index m * ldr + n
     DropCfg drop;
     uint32_t drop_site = 0;

@@ -43,19 +43,6 @@ __device__ __forceinline__ float act_rt(int epi, float v) {
     }
 }
 
-// derivative of the activation for the EPI_MULGRAD_* epilogues (bf16 mode: approximate transcendental units)
-__device__ __forceinline__ float act_grad_rt(int epi, float x) {
-    if (epi == EPI_MULGRAD_RELU) return x > 0.f ? 1.f : 0.f;
-    if (epi == EPI_MULGRAD_GELU_TANH) {
-        const float k = 0.79788456080286535588f;
-        const float x2 = x * x;
-        const float t = ptx::tanh_approx(k * fmaf(0.044715f * x, x2, x));
-        const float du = k * fmaf(3.0f * 0.044715f, x2, 1.0f);
-        return fmaf(0.5f * x * du, fmaf(-t, t, 1.0f), fmaf(0.5f, t, 0.5f));
-    }
-    return gelu_erf_grad_fast(x);
-}
-
 // byte offset of 16-byte chunk `c` of row `r` inside a SWIZZLE_128B staging buffer (1024-B aligned)
 __device__ __forceinline__ uint32_t sw128_off(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
 
@@ -105,7 +92,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int n0 = slice * BN;
     const bool has_ln = epi == EPI_BIAS_RESID_LN;          // requires BN == N (whole row in this CTA)
     const bool has_res = epi == EPI_BIAS_RESID || has_ln;
-    const bool has_mul = epi >= EPI_MULGRAD_RELU && epi <= EPI_MULGRAD_GELU_TANH;   // bf16 output only
 
     for (int i = threadIdx.x; i < BN; i += kTcThreads) {
         sBias[i] = ep.bias[n0 + i];
@@ -115,7 +101,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         ptx::prefetch_tmap(&tmA);
         ptx::prefetch_tmap(&tmW);
         ptx::prefetch_tmap(&tmC);
-        if (has_res || has_mul) ptx::prefetch_tmap(&tmR);
+        if (has_res) ptx::prefetch_tmap(&tmR);
         if (has_ln) ptx::prefetch_tmap(&tmL);
         for (int s = 0; s < nstage; ++s) { ptx::mbar_init(&full[s], 1); ptx::mbar_init(&empty[s], 1); }
         ptx::mbar_init(w_full, 1);
@@ -223,7 +209,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int half = ew >> 2;
         uint8_t* ebuf = sEpi + (size_t)ew * nebuf * kTcEpiBuf;
         uint64_t* rb = rbar + ew * 3;
-        uint32_t rphase0 = 0;       // bf16 (MULGRAD) path: phase of rb[0]
         uint32_t rph = 0;           // fp32 path: bit b = phase of rb[b]
         int nbuf = 0;        // staging buffer the next chunk uses (bf16 path with nebuf == 2 only)
         int t = 0;
@@ -232,13 +217,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const int row0 = (mt * NCTA + crank) * kTcBlockM + q * 32;
             const uint32_t tm = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
             if (out_bf16) {
-                // EPI_MULGRAD_*: the saved pre-activation tile is TMA-loaded into the staging buffer (first chunk
-                // before the accumulator is ready), multiplied in place and TMA-stored -- like the residual path.
-                if (has_mul && lane == 0 && half < BN / 64) {
-                    ptx::bulk_wait_read<0>();
-                    ptx::mbar_arrive_expect_tx(&rb[0], kTcEpiBuf);
-                    ptx::tma_load_2d(ebuf, &tmR, &rb[0], n0 + half * 64, row0);
-                }
                 ptx::mbar_wait(&tmem_full[acc], (t >> 1) & 1);
                 ptx::tc_fence_after();
 #pragma unroll 1
@@ -246,38 +224,22 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     uint32_t r0[32], r1[32];
                     ptx::tmem_ld_32x32(tm + (uint32_t)(ch * 64), r0);
                     ptx::tmem_ld_32x32(tm + (uint32_t)(ch * 64 + 32), r1);
-                    const bool alt = nebuf > 1 && !has_mul;      // alternate the two staging buffers (plain epilogues only)
+                    const bool alt = nebuf > 1;      // alternate the two staging buffers
                     uint8_t* buf = ebuf + (alt ? nbuf : 0) * kTcEpiBuf;
-                    if (lane == 0 && !(has_mul && ch == half)) {
+                    if (lane == 0) {
                         if (alt) ptx::bulk_wait_read<1>(); else ptx::bulk_wait_read<0>();
-                        if (has_mul) {
-                            ptx::mbar_arrive_expect_tx(&rb[0], kTcEpiBuf);
-                            ptx::tma_load_2d(buf, &tmR, &rb[0], n0 + ch * 64, row0);
-                        }
                     }
                     __syncwarp();
-                    if (has_mul) { ptx::mbar_wait(&rb[0], rphase0); rphase0 ^= 1; }
                     ptx::tc_wait_ld();
                     const float* bsm = sBias + ch * 64;
 #pragma unroll
                     for (int c = 0; c < 8; ++c) {                 // 8 x 16 B chunks = 64 bf16 columns
                         uint32_t pk[4];
-                        uint4 pre4 = make_uint4(0u, 0u, 0u, 0u);
-                        if (has_mul) pre4 = *reinterpret_cast<const uint4*>(buf + sw128_off(lane, c));
-                        const uint32_t prew[4] = {pre4.x, pre4.y, pre4.z, pre4.w};
 #pragma unroll
                         for (int j = 0; j < 4; ++j) {
                             const int col = c * 8 + j * 2;
-                            float a = __uint_as_float(col < 32 ? r0[col] : r1[col - 32]) + bsm[col];
-                            float b = __uint_as_float(col + 1 < 32 ? r0[col + 1] : r1[col + 1 - 32]) + bsm[col + 1];
-                            if (has_mul) {
-                                const float2 pv = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&prew[j]));
-                                a *= act_grad_rt(epi, pv.x);
-                                b *= act_grad_rt(epi, pv.y);
-                            } else {
-                                a = act_rt(epi, a);
-                                b = act_rt(epi, b);
-                            }
+                            const float a = act_rt(epi, __uint_as_float(col < 32 ? r0[col] : r1[col - 32]) + bsm[col]);
+                            const float b = act_rt(epi, __uint_as_float(col + 1 < 32 ? r0[col + 1] : r1[col + 1 - 32]) + bsm[col + 1]);
                             __nv_bfloat162 h2 = __floats2bfloat162_rn(a, b);
                             pk[j] = *reinterpret_cast<uint32_t*>(&h2);
                         }
@@ -480,15 +442,10 @@ static bool make_tmap_2d(CUtensorMap* m, CUtensorMapDataType dt, int esize, cons
 
 struct TcPlan { int BN, ncta, nkb, nstage, nebuf, grid; size_t smem; };
 
-// CTA pairs (cta_group::2): TANTE_GEMM_2CTA = 0 never, 1 (default) where they pay off, 2 everywhere they fit (tests).
-// Measured on B200 (tools/gemm_probe.py, M = 262144 / 65536, N = K = 256): the fp32 residual (+LayerNorm) epilogues gain
+// CTA pairs (cta_group::2) where they pay off.  Measured on B200 (tools/gemm_probe.py, M = 262144 / 65536, N = K = 256): the fp32 residual (+LayerNorm) epilogues gain
 // 16-19 % / 11-14 % from the second staging buffer the halved weight slice pays for (156.6 -> 126.9 us, 188.7 -> 158.2 us);
 // plain bf16 epilogues lose 4-19 % to the lock-step of the pair, so they stay on single CTAs unless the reduction is so
 // long (K = 768) that a single CTA could only keep a 64-wide weight slice resident.
-static int tc_pair_mode() {
-    static const int mode = getenv("TANTE_GEMM_2CTA") ? atoi(getenv("TANTE_GEMM_2CTA")) : 1;
-    return mode;
-}
 
 static bool tc_plan(int M, int N, int K, int num_sms, int out_bf16, TcPlan* p) {
     if (K % kTcBlockK != 0 || K > 1024 || N % 64 != 0) return false;
@@ -498,8 +455,7 @@ static bool tc_plan(int M, int N, int K, int num_sms, int out_bf16, TcPlan* p) {
     // pairs need >= 128 columns (64 per CTA) and enough 256-row tiles to fill the machine
     const bool narrow_single = (size_t)nkb * 128 * 128 > 128 * 1024;        // a single CTA would be down to 64-wide slices
     const bool pays = !out_bf16 || (narrow_single && N >= 128);
-    const int ncta = (tc_pair_mode() == 2 && N % 128 == 0) ? 2
-                     : (tc_pair_mode() == 1 && pays && N % 128 == 0 && M >= 256 * (num_sms / 2)) ? 2 : 1;
+    const int ncta = (pays && N % 128 == 0 && M >= 256 * (num_sms / 2)) ? 2 : 1;
     while ((size_t)nkb * (BN / ncta) * 128 > 128 * 1024 && BN > 64 * ncta) BN /= 2;   // keep the resident slice <= 128 KB
     if ((size_t)nkb * (BN / ncta) * 128 > 128 * 1024) return false;
     // pairs: the halved weight slice pays for a second staging buffer per epilogue warp (if >= 3 activation stages remain)
@@ -539,10 +495,8 @@ static cudaError_t tc_set_attrs() {
 }
 
 // Programmatic dependent launch for the tensor-core kernels (common.cuh): not inside stream capture (the rollout graphs keep
-// plain kernel nodes), TANTE_PDL=0 disables it.
+// plain kernel nodes).
 static bool pdl_enabled(cudaStream_t st) {
-    static const bool on = !(getenv("TANTE_PDL") && atoi(getenv("TANTE_PDL")) == 0);
-    if (!on) return false;
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) { (void)cudaGetLastError(); return false; }
     return cs == cudaStreamCaptureStatusNone;
@@ -568,10 +522,6 @@ static cudaError_t launch_gemm_tc(int epi, const __nv_bfloat16* A, int lda, cons
     tmR = tmC;
     tmL = tmC;
     if (is_ln && !make_tmap_2d(&tmL, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, ep.ln_out, M, N, N, 64, 32)) return cudaErrorInvalidValue;
-    if (epi >= EPI_MULGRAD_RELU && epi <= EPI_MULGRAD_GELU_TANH) {
-        if (!out_bf16 || !ep.mul_pre) return cudaErrorInvalidValue;
-        if (!make_tmap_2d(&tmR, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, ep.mul_pre, M, N, ep.ld_pre, 64, 32)) return cudaErrorInvalidValue;
-    }
     if (epi == EPI_BIAS_RESID || is_ln) {
         if (out_bf16) return cudaErrorInvalidValue;
         if (!make_tmap_2d(&tmR, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, ep.resid, M, N, ep.ldr, 32, 32)) return cudaErrorInvalidValue;

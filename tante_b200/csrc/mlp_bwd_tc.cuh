@@ -279,8 +279,7 @@ static cudaError_t launch_mlp_bwd(const __nv_bfloat16* dy, const __nv_bfloat16* 
                     make_tmap_2d(&tmDpre, BF, 2, dpre, M, kBtC, kBtC, 64, 32) &&
                     make_tmap_2d(&tmDln, BF, 2, dln, M, kBtC, kBtC, 64, 32);
     if (!ok) return cudaErrorInvalidValue;
-    static const int pair_mode = getenv("TANTE_TAIL_2CTA") ? atoi(getenv("TANTE_TAIL_2CTA")) : 1;
-    const int ncta = (pair_mode == 2 || (pair_mode == 1 && M >= 256 * (num_sms / 2))) ? 2 : 1;
+    const int ncta = M >= 256 * (num_sms / 2) ? 2 : 1;      // CTA pairs once 256-row units fill the machine
     const int tiles = (M + 128 * ncta - 1) / (128 * ncta);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(ncta * std::min(tiles, num_sms / ncta))); cfg.blockDim = dim3(kBtThreads);

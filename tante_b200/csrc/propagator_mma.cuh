@@ -14,17 +14,12 @@ namespace tante {
 // slab tile: row pitch 256 B (128 bf16), 16-byte chunk index XOR-swizzled with the row inside groups of 8
 __device__ __forceinline__ uint32_t slab_off(int r, int chunk) { return (uint32_t)(r * 256 + (((chunk & 8) | ((chunk ^ r) & 7)) << 4)); }
 
-// MH = 2 (TANTE_PROP_SPLIT=1, S > 48): eight warps, the two warps of a column group split the output rows (M blocks) between
-// them -- half the accumulator registers per thread, twice the warps per SM.  Measured SLOWER than the 4-warp variant (see the
-// launcher); kept as an opt-in experiment.
-template <int MB /* S_pad / 16 */, int MH = 1 /* warps per column group */>
-__global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kernel(const float* xin, float* x, int S, long long IC, long long n_outer,
+template <int MB /* S_pad / 16 */>
+__global__ void __launch_bounds__(128, 3) propagator_mma_kernel(const float* xin, float* x, int S, long long IC, long long n_outer,
                                                              const float* __restrict__ W1, const float* __restrict__ b1,
                                                              const float* __restrict__ W2, const float* __restrict__ b2) {
     constexpr int SP = MB * 16;
-    constexpr int THREADS = 128 * MH;
-    constexpr int MBH = MB / MH;                              // M blocks per warp
-    static_assert(MB % MH == 0, "M blocks must split evenly");
+    constexpr int THREADS = 128;
     constexpr int WPITCH = SP * 2 + 16;                       // bytes; odd number of 16-B chunks -> conflict-free ldmatrix
     extern __shared__ __align__(128) uint8_t pm_smem[];
     uint8_t* sV = pm_smem;
@@ -35,8 +30,7 @@ __global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kern
     float* sb2 = sb1 + SP;
 
     const int tid = threadIdx.x, lane = tid % 32;
-    const int warp = (tid / 32) & 3;                          // column group: 32 of the tile's 128 columns
-    const int mh = (tid / 32) >> 2;                           // which share of the M blocks
+    const int warp = tid / 32;                                // column group: 32 of the tile's 128 columns
     const long long ncb = (IC + 127) / 128;
 
     for (int i = tid; i < SP * SP; i += THREADS) {
@@ -77,9 +71,9 @@ __global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kern
     for (int pass = 0; pass < 2; ++pass) {
         const uint32_t aW = pass == 0 ? aW1 : aW2;
         const uint32_t aB = pass == 0 ? aV : aH;
-        float acc[MBH][4][4];
+        float acc[MB][4][4];
 #pragma unroll
-        for (int mb = 0; mb < MBH; ++mb)
+        for (int mb = 0; mb < MB; ++mb)
 #pragma unroll
             for (int nb = 0; nb < 4; ++nb) acc[mb][nb][0] = acc[mb][nb][1] = acc[mb][nb][2] = acc[mb][nb][3] = 0.f;
 #pragma unroll
@@ -90,17 +84,17 @@ __global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kern
                 ldsm_x4_t(aB + slab_off(kk * 16 + lrow, warp * 4 + 2 * j + lchk), bf[2 * j][0], bf[2 * j][1], bf[2 * j + 1][0],
                           bf[2 * j + 1][1]);
 #pragma unroll
-            for (int mb = 0; mb < MBH; ++mb) {
+            for (int mb = 0; mb < MB; ++mb) {
                 uint32_t af[4];
-                ldsm_x4(aW + (uint32_t)(((mh * MBH + mb) * 16 + lrow) * WPITCH + (kk * 2 + lchk) * 16), af[0], af[1], af[2], af[3]);
+                ldsm_x4(aW + (uint32_t)((mb * 16 + lrow) * WPITCH + (kk * 2 + lchk) * 16), af[0], af[1], af[2], af[3]);
 #pragma unroll
                 for (int nb = 0; nb < 4; ++nb) mma_bf16_16816(acc[mb][nb], af, bf[nb][0], bf[nb][1]);
             }
         }
         if (pass == 0) {
 #pragma unroll
-            for (int mb = 0; mb < MBH; ++mb) {
-                const int j0 = (mh * MBH + mb) * 16 + g, j1 = j0 + 8;
+            for (int mb = 0; mb < MB; ++mb) {
+                const int j0 = mb * 16 + g, j1 = j0 + 8;
                 const float bb0 = sb1[j0], bb1 = sb1[j1];
 #pragma unroll
                 for (int nb = 0; nb < 4; ++nb) {
@@ -111,16 +105,15 @@ __global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kern
                         pack_bf16x2(gelu_erf_fast(acc[mb][nb][2] + bb1), gelu_erf_fast(acc[mb][nb][3] + bb1));
                 }
             }
-            if (MH == 1) __syncwarp();     // the hidden columns of a warp are consumed only by the same warp
-            else __syncthreads();          // ... or by the warps of its column group (uniform: every thread runs both passes)
+            __syncwarp();     // the hidden columns of a warp are consumed only by the same warp
         } else {
             // residual add in two sweeps: all loads first (x may alias the output, so a load cannot be hoisted over
             // an earlier store and an interleaved loop would serialise 8*MB L2 round trips per thread)
 #pragma unroll
-            for (int mb = 0; mb < MBH; ++mb) {
+            for (int mb = 0; mb < MB; ++mb) {
 #pragma unroll
                 for (int hh = 0; hh < 2; ++hh) {
-                    const int p = (mh * MBH + mb) * 16 + g + 8 * hh;
+                    const int p = mb * 16 + g + 8 * hh;
                     const float bb = p < S ? sb2[p] : 0.f;
 #pragma unroll
                     for (int nb = 0; nb < 4; ++nb) {
@@ -134,10 +127,10 @@ __global__ void __launch_bounds__(128 * MH, MH == 2 ? 2 : 3) propagator_mma_kern
                 }
             }
 #pragma unroll
-            for (int mb = 0; mb < MBH; ++mb) {
+            for (int mb = 0; mb < MB; ++mb) {
 #pragma unroll
                 for (int hh = 0; hh < 2; ++hh) {
-                    const int p = (mh * MBH + mb) * 16 + g + 8 * hh;
+                    const int p = mb * 16 + g + 8 * hh;
 #pragma unroll
                     for (int nb = 0; nb < 4; ++nb) {
                         const int c = warp * 32 + nb * 8 + 2 * t;
@@ -155,7 +148,6 @@ static void prop_set_attrs() {
     static unsigned long long done = 0;
     if (!attrs_needed(done)) return;
     cudaFuncSetAttribute(propagator_mma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-    cudaFuncSetAttribute(propagator_mma_kernel<4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
 }
 
 static bool launch_propagator_mma(const float* xin, float* x, int S, long long IC, long long outer, const float* W1, const float* b1,
@@ -186,14 +178,7 @@ static bool launch_propagator_mma(const float* xin, float* x, int S, long long I
         case 1: propagator_mma_kernel<1><<<grid, 128, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2); break;
         case 2: propagator_mma_kernel<2><<<grid, 128, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2); break;
         case 3: propagator_mma_kernel<3><<<grid, 128, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2); break;
-        default: {
-            // measured on B200 (rollout, S = 64, 262144 tokens): 271 us with the row split vs 249 us without -- the doubled B-fragment
-            // ldmatrix traffic and the CTA-wide barrier between the passes cost more than the extra warps buy; opt-in experiment
-            static const bool split = getenv("TANTE_PROP_SPLIT") && atoi(getenv("TANTE_PROP_SPLIT")) != 0;
-            if (split) propagator_mma_kernel<4, 2><<<grid, 256, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2);
-            else propagator_mma_kernel<4><<<grid, 128, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2);
-            break;
-        }
+        default: propagator_mma_kernel<4><<<grid, 128, smem, st>>>(xin, x, S, IC, outer, W1, b1, W2, b2); break;
     }
     *err = cudaGetLastError();
     return true;

@@ -32,7 +32,6 @@
 #include "wgrad_tc.cuh"
 #include "metrics.cuh"
 #include "block_tail_tc.cuh"
-#include "block_tail2_tc.cuh"
 #include "mlp_bwd_tc.cuh"
 #include "wide_patch.cuh"
 #include "fno.cuh"
@@ -158,7 +157,7 @@ struct tante_handle_s {
     DevBuf icols;                       // tensor mode: im2col'ed input patches of the first conv, [B*T*L*R1][64] bf16
     DevBuf enc_cache;                   // rollout: encoder output per ring slot, fp32 [B*T*L][C]
     DevBuf enc_state;                   // rollout: [8] count, [B*T] list, [B*T] map
-    bool use_enc_cache = true;          // TANTE_ENC_CACHE=0 re-encodes the whole window every call
+    bool use_enc_cache = true;          // rollout: encode only the newest frame of a window (not with the wide / fno stages)
     bool axes_ok = true;                // Hp, Wp, T <= 64 (what the axial kernels cover)
     bool long_axes = false;             // an L / Y / A layer or an axis longer than 64 tokens: inference / rollout only
     bool chan = false;                  // an axis-'C' layer (channel_axis.cuh): inference / rollout only
@@ -179,9 +178,6 @@ struct tante_handle_s {
     DevBuf wbuf, dfield;                // wide: patch / sub-pixel matrix scratch; decoded derivative fields [K][B][D][H][W]
     float drop_p = 0.f;                 // tante_set_dropout: applies to the NEXT tante_train_forward calls
     unsigned long long drop_seed = 0;
-    bool fuse_mlp_bwd = true;           // tensor mode: MLP input-gradient chain as ONE kernel (TANTE_FUSE_MLP_BWD=0: GEMM + elementwise + GEMM)
-    bool no_switch = false;             // SWITCH conditional nodes unavailable on this driver: rollouts run without compaction
-    bool fuse_tail = true;              // tensor mode: out-proj + LN2 + MLP + LN1' of a block as ONE kernel (TANTE_FUSE_TAIL=0: three GEMMs)
 
     // workspace
     int max_batch = 0, max_roll = 0;
@@ -195,14 +191,12 @@ struct tante_handle_s {
     int last_B = 0;
     int num_sms = 148;
     // rollout graphs: key -> instantiated graph (WHILE node whose body is one model step)
-    struct RollGraph { cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr; bool while_node = false; int64_t launches_per_step = 0; };
+    struct RollGraph { cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr; int64_t launches_per_step = 0; };
     std::map<std::string, RollGraph> graphs;
     cudaStream_t cap_stream = nullptr;
-    int rollout_mode = 2;       // 0 = eager launches, 1 = one graph per step + host loop, 2 = device WHILE graph
     cudaGraphConditionalHandle cond_handle = 0;
     int use_cond = 0;
     cudaGraphConditionalHandle sw_handle = 0;   // SWITCH node of the compaction buckets
-    int last_graph_steps = 0;
     // live GEMM timing (tante_profile)
     bool prof_on = false;
     std::vector<cudaEvent_t> prof_ev;
@@ -664,7 +658,7 @@ void launch_tail(tante_handle_s* h, const LayerPlan& lp, const LayerPlan* nx, co
     a.x_in = b.x_in; a.x_out = b.x_out; a.ln_out = nx ? b.ln_next : nullptr;
     if (train) { a.x_mid = b.x_mid; a.ln2 = b.ln2; a.hpre = b.hpre; a.hact = b.hact; }
     a.drop = drop; a.site1 = b.site[1]; a.site2 = b.site[2];
-    CK(launch_block_tail_any(a, tokens, train, h->num_sms, st));
+    CK(launch_block_tail(a, tokens, train, h->num_sms, st));
     h->launches++;
 }
 
@@ -1418,7 +1412,7 @@ void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs
             gemm<TA>(h, EPI_BIAS, b.ln1, C, lp.inw, b.qkv, 3 * C, false, tokens, 3 * C, C, eq, st);
             launch_attention<TA>(h, b.qkv, b.att, B, lp.axis, st, drop, b.site[0]);
             if constexpr (sizeof(TA) == 2) {
-                if (h->fuse_tail && C == kBtC && Hm == C) {
+                if (C == kBtC && Hm == C) {
                     const LayerPlan* nx = nx_ok ? &op.layers[li + 1] : nullptr;
                     launch_tail(h, lp, nx, b, tokens, drop, st);
                     ln_ready = nx != nullptr;
@@ -1426,7 +1420,7 @@ void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs
                 }
             }
             if (sizeof(TA) == 2 && drop.p > 0.f) {
-                // Tensor mode with dropout outside the fused tail (mlp_ratio != 1, embed_dim 512, TANTE_FUSE_TAIL=0): the tcgen05 GEMM
+                // Tensor mode with dropout outside the fused tail (mlp_ratio != 1, embed_dim 512): the tcgen05 GEMM
                 // epilogues carry no mask generator, so each residual branch is a plain GEMM into a bf16 scratch followed by one
                 // pass  x <- x + mask * branch  (what autocast + nn.Dropout do in the reference); LayerNorms as their own passes.
                 TA* br = TP<TA>(h->hid);
@@ -1615,27 +1609,6 @@ void gemm_dx(tante_handle_s* h, const TA* A, int lda, int64_t wT_off, TA* out, i
         return;
     }
     gemm<TA>(h, EPI_BIAS, A, lda, wT_off, out, ldc, sizeof(TA) == 4, M, N, K, ep, st);
-}
-
-// dX = (dY * W) o f'(pre): in tensor mode the activation derivative is applied in the GEMM epilogue (the saved
-// pre-activation tile is TMA-loaded next to the accumulator); in the exact mode it is a separate elementwise pass.
-// `out` and `pre` are both [M][N] contiguous.
-template <typename TA, int ACT>
-void gemm_dx_act(tante_handle_s* h, const TA* A, int lda, int64_t wT_off, TA* out, const TA* pre, int M, int N, int K,
-                 cudaStream_t st) {
-    // measured on B200 (Active Matter, M = 65536): fused epilogue 60 us vs 17 us GEMM + 26 us elementwise pass -- the
-    // single 4 KB staging buffer per epilogue warp keeps too few bytes in flight, so the fusion is opt-in for now
-    static const bool fuse = getenv("TANTE_FUSE_ACTGRAD") && atoi(getenv("TANTE_FUSE_ACTGRAD")) != 0;
-    if (sizeof(TA) == 2 && fuse) {
-        EpiParams ep; ep.bias = AF(h, h->zero_off);
-        REQUIRE(N <= 8192, "input-gradient GEMM wider than the zero-bias vector");
-        ep.mul_pre = pre; ep.ld_pre = N;
-        const int epi = ACT == ACT_RELU ? EPI_MULGRAD_RELU : (ACT == ACT_GELU_ERF ? EPI_MULGRAD_GELU_ERF : EPI_MULGRAD_GELU_TANH);
-        gemm<TA>(h, epi, A, lda, wT_off, out, N, false, M, N, K, ep, st);
-    } else {
-        gemm_dx<TA>(h, A, lda, wT_off, out, N, M, N, K, st);
-        launch_act_bwd<TA, ACT>(h, out, pre, (long long)M * N, st);
-    }
 }
 
 // Backward of one SpectralLayer (fno.cuh, "training"): x = the layer's saved input, g = the gradient of its output (after the
@@ -2033,7 +2006,8 @@ void run_channel_layer_bwd(tante_handle_s* h, const LayerPlan& lp, const float* 
         CK(cudaGetLastError());
         h->launches++;
         wgrad<TA>(h, gxb, E, hact, Hc, GA(h, lp.m2w), rows, E, Hc, st, GA(h, lp.m2b));
-        gemm_dx_act<TA, ACT_GELU_TANH>(h, gxb, E, lp.m2wT, g1, hpre, rows, Hc, E, st);
+        gemm_dx<TA>(h, gxb, E, lp.m2wT, g1, Hc, rows, Hc, E, st);
+        launch_act_bwd<TA, ACT_GELU_TANH>(h, g1, hpre, (long long)rows * Hc, st);
         wgrad<TA>(h, g1, Hc, ln2, E, GA(h, lp.m0w), rows, Hc, E, st, GA(h, lp.m0b));
         gemm_dx<TA>(h, g1, Hc, lp.m0wT, g2, E, rows, E, Hc, st);
         launch_ln_bwd<TA>(h, g2, xm, lp.ln2w, gx, gxb_out, GA(h, lp.ln2w), GA(h, lp.ln2b), rows, st, DropCfg(), 0, E);
@@ -2146,7 +2120,8 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             CK(cudaGetLastError());
             h->launches++;
             wgrad<TA>(h, wb, NF2, TP<TA>(ot.z2act), C1, GA(h, op.decw[1]), MF2, NF2, C1, st, ovf0 ? nullptr : GA(h, op.decb[1]));
-            gemm_dx_act<TA, ACT_GELU_ERF>(h, wb, NF2, op.decwT[1], gr1, TP<TA>(ot.z2pre), (int)MF2, C1, NF2, st);
+            gemm_dx<TA>(h, wb, NF2, op.decwT[1], gr1, C1, (int)MF2, C1, NF2, st);
+            launch_act_bwd<TA, ACT_GELU_ERF>(h, gr1, TP<TA>(ot.z2pre), MF2 * C1, st);
             // dec_spectral_1
             SpecView xg1{ot.z1act.p, 1, nullptr, 1}, gv1{gr1, 1, nullptr, 1};
             run_spectral_bwd<TA>(h, op.fs1, xg1, gv1, B, H1, W1, 1, gr2, nullptr, st);
@@ -2184,14 +2159,16 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             } else {
                 launch_colsum<TA>(h, G, NP, rows1, NO, GA(h, op.decb[2]), st);
             }
-            gemm_dx_act<TA, ACT_GELU_ERF>(h, G, NP, op.w3pad, dz, TP<TA>(ot.z2pre), (int)rows1, C1, NP, st);
+            gemm_dx<TA>(h, G, NP, op.w3pad, dz, C1, (int)rows1, C1, NP, st);
+            launch_act_bwd<TA, ACT_GELU_ERF>(h, dz, TP<TA>(ot.z2pre), rows1 * C1, st);
             if (ov2) launch_colsum<TA>(h, dz, C1, rows1, C1, GA(h, op.decb[1]), st);
             tot = (long long)M2 * N2;
             wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(dz, nullptr, N2, H2, W2, C1, g.k1, wb, tot, h->st[1]);
             CK(cudaGetLastError());
             h->launches++;
             wgrad<TA>(h, wb, N2, TP<TA>(ot.z1act), C2, GA(h, op.decw[1]), M2, N2, C2, st, ov2 ? nullptr : GA(h, op.decb[1]));
-            gemm_dx_act<TA, ACT_GELU_ERF>(h, wb, N2, op.decwT[1], dz1, TP<TA>(ot.z1pre), M2, C2, N2, st);
+            gemm_dx<TA>(h, wb, N2, op.decwT[1], dz1, C2, M2, C2, N2, st);
+            launch_act_bwd<TA, ACT_GELU_ERF>(h, dz1, TP<TA>(ot.z1pre), (long long)M2 * C2, st);
             if (ov1) launch_colsum<TA>(h, dz1, C2, M2, C2, GA(h, op.decb[0]), st);
             tot = (long long)BL * N1;
             wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(dz1, nullptr, N1, Hp, Wp, C2, g.k2, wb, tot, h->st[2]);
@@ -2204,10 +2181,12 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
         // dec_conv_3: d_k = z2act * W3 + b3  ->  dW3 = z2act^T G, db3 = colsum(G), dz2 = (G W3^T) o gelu'(z2pre)
         wgrad_pad<TA>(h, TP<TA>(ot.z2act), C1, C1, G, kHeadPad, kHeadPad, GA(h, op.decw[2]), NO, NO, rows1, st);
         launch_colsum<TA>(h, G, kHeadPad, rows1, NO, GA(h, op.decb[2]), st);
-        gemm_dx_act<TA, ACT_GELU_ERF>(h, G, kHeadPad, op.w3pad, dz, TP<TA>(ot.z2pre), (int)rows1, C1, kHeadPad, st);
+        gemm_dx<TA>(h, G, kHeadPad, op.w3pad, dz, C1, (int)rows1, C1, kHeadPad, st);
+        launch_act_bwd<TA, ACT_GELU_ERF>(h, dz, TP<TA>(ot.z2pre), rows1 * C1, st);
         // dec_conv_2: z2pre[M2, N2] = z1act[M2, C2] * Wd2^T + b
         wgrad<TA>(h, dz, N2, TP<TA>(ot.z1act), C2, GA(h, op.decw[1]), M2, N2, C2, st, GA(h, op.decb[1]));
-        gemm_dx_act<TA, ACT_GELU_ERF>(h, dz, N2, op.decwT[1], dz1, TP<TA>(ot.z1pre), M2, C2, N2, st);
+        gemm_dx<TA>(h, dz, N2, op.decwT[1], dz1, C2, M2, C2, N2, st);
+        launch_act_bwd<TA, ACT_GELU_ERF>(h, dz1, TP<TA>(ot.z1pre), (long long)M2 * C2, st);
         // dec_conv_1: z1pre[BL, N1] = dmod[BL, C] * Wd1^T + b
         wgrad<TA>(h, dz1, N1, dmod, C, GA(h, op.decw[0]), BL, N1, C, st, GA(h, op.decb[0]));
         gemm_dx<TA>(h, dz1, N1, op.decwT[0], hd, C, BL, C, N1, st);
@@ -2236,7 +2215,8 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             CK(cudaGetLastError());
             h->launches++;
             wgrad<TA>(h, hi2, C / 4, TP<TA>(ot.i1), C / 2, GA(h, op.intw[1]), BL, C / 4, C / 2, st, GA(h, op.intb[1]));
-            gemm_dx_act<TA, ACT_RELU>(h, hi2, C / 4, op.intwT[1], hi1, TP<TA>(ot.i1), BL, C / 2, C / 4, st);
+            gemm_dx<TA>(h, hi2, C / 4, op.intwT[1], hi1, C / 2, BL, C / 2, C / 4, st);
+            launch_act_bwd<TA, ACT_RELU>(h, hi1, TP<TA>(ot.i1), (long long)BL * (C / 2), st);
             wgrad<TA>(h, hi1, C / 2, TP<TA>(ot.dl), C, GA(h, op.intw[0]), BL, C / 2, C, st, GA(h, op.intb[0]));
             gemm_dx<TA>(h, hi1, C / 2, op.intwT[0], hd, C, BL, C, C / 2, st);
         }
@@ -2266,7 +2246,7 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             }
             // MLP half: x_out = x_mid + W2 gelu_tanh(W0 ln2(x_mid) + b0) + b2
             wgrad<TA>(h, dxb, C, TP<TA>(ot.hact[li]), Hm, GA(h, lp.m2w), tokens, C, Hm, st, GA(h, lp.m2b));
-            if (kTensor && h->fuse_mlp_bwd && C == kBtC && h->Hm == C) {
+            if (kTensor && C == kBtC && h->Hm == C) {
                 // dpre = (dY W2) o gelu'(hpre) and dln2 = dpre W1 in one kernel (mlp_bwd_tc.cuh): dh never touches HBM
                 {
                     ProfScope ps(h, st, 2.0 * 2.0 * tokens * C * C, 4, (double)tokens * 4 * 2 * C);
@@ -2277,7 +2257,8 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
                 h->launches++;
                 wgrad<TA>(h, g1, C, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, C, C, st, GA(h, lp.m0b));
             } else {
-                gemm_dx_act<TA, ACT_GELU_TANH>(h, dxb, C, lp.m2wT, g1, TP<TA>(ot.hpre[li]), tokens, Hm, C, st);
+                gemm_dx<TA>(h, dxb, C, lp.m2wT, g1, Hm, tokens, Hm, C, st);
+                launch_act_bwd<TA, ACT_GELU_TANH>(h, g1, TP<TA>(ot.hpre[li]), (long long)tokens * Hm, st);
                 wgrad<TA>(h, g1, Hm, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, Hm, C, st, GA(h, lp.m0b));
                 gemm_dx<TA>(h, g1, Hm, lp.m0wT, g2, C, tokens, C, Hm, st);
             }
@@ -2435,10 +2416,12 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
         }
     } else {
     wgrad<TA>(h, g2, C, TP<TA>(tp.a2act), K3, GA(h, h->enc_w[2]), tokens, C, K3, st, GA(h, h->enc_b[2]));
-    gemm_dx_act<TA, ACT_GELU_ERF>(h, g2, C, h->enc_wT[2], gq, TP<TA>(tp.a2pre), tokens, K3, C, st);
+    gemm_dx<TA>(h, g2, C, h->enc_wT[2], gq, K3, tokens, K3, C, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, gq, TP<TA>(tp.a2pre), (long long)tokens * K3, st);
     wgrad<TA>(h, gq, C2, TP<TA>(tp.a1act), K2, GA(h, h->enc_w[1]), M2, C2, K2, st, GA(h, h->enc_b[1]));
     TA* ga1 = TP<TA>(h->ga1);
-    gemm_dx_act<TA, ACT_GELU_ERF>(h, gq, C2, h->enc_wT[1], ga1, TP<TA>(tp.a1pre), M2, K2, C2, st);
+    gemm_dx<TA>(h, gq, C2, h->enc_wT[1], ga1, K2, M2, K2, C2, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, ga1, TP<TA>(tp.a1pre), (long long)M2 * K2, st);
     (void)input;      // the patches were kept by the forward (tape im2col)
     TA* cols = TP<TA>(h->cols);
     wgrad_pad<TA>(h, ga1, C1, C1, TP<TA>(tp.cols), kHeadPad, kHeadPad, GA(h, h->enc_w[0]), NO, NO, rows_in, st, GA(h, h->enc_b[0]));
@@ -2529,70 +2512,51 @@ void destroy_graphs(tante_handle_s* h) {
     h->graphs.clear();
 }
 
-// Compaction buckets of a per-sample rollout (TANTE_ROLLOUT_COMPACT=0 disables): the step body is captured once per batch
-// size B, 3B/4, B/2, B/4 and a SWITCH node inside the WHILE body runs the smallest one that holds every running trajectory.
-// Needs the encoder cache (its frame lists already speak trajectory ids) and the patch-GEMM encoder.
-static bool compaction_wanted(const tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs) {
-    static const bool on = !(getenv("TANTE_ROLLOUT_COMPACT") && atoi(getenv("TANTE_ROLLOUT_COMPACT")) == 0);
-    return on && io.per_sample && B >= 8 && rs.enc_count && !h->wide && !h->fno && !h->cfg.deg;
+// Compaction buckets of a per-sample rollout: the step body is captured once per batch size B, 3B/4, B/2, B/4 and a SWITCH
+// node inside the WHILE body runs the smallest one that holds every running trajectory.  Needs the encoder cache (its frame
+// lists already speak trajectory ids) and the patch-GEMM encoder.
+static bool compaction_wanted(const tante_handle_s* h, bool per_sample, int B, const RolloutState& rs) {
+    return per_sample && B >= 8 && rs.enc_count && !h->wide && !h->fno && !h->cfg.deg;
 }
 
+// WHILE { step(B) }, or with compaction buckets WHILE { SWITCH(bucket) { step(B_0) | step(B_1) | ... } }
 template <typename TA>
-void build_roll_graph(tante_handle_s* h, tante_handle_s::RollGraph& rg, const StepIO& io, int B,
-                             const RolloutState& rs_in, bool while_node) {
+void build_roll_graph(tante_handle_s* h, tante_handle_s::RollGraph& rg, const StepIO& io, int B, const RolloutState& rs_in) {
     if (!h->cap_stream) CK(cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
     const int64_t launches0 = h->launches;
     RolloutState rs = rs_in;
-    if (while_node && rs.act && rs.n_buckets > 1) {
-        // WHILE { SWITCH(bucket) { step(B_0) | step(B_1) | ... } }
-        CK(cudaGraphCreate(&rg.graph, 0));
-        CK(cudaGraphConditionalHandleCreate(&h->cond_handle, rg.graph, 1, cudaGraphCondAssignDefault));
+    CK(cudaGraphCreate(&rg.graph, 0));
+    CK(cudaGraphConditionalHandleCreate(&h->cond_handle, rg.graph, 1, cudaGraphCondAssignDefault));
+    if (rs.act) {
         CK(cudaGraphConditionalHandleCreate(&h->sw_handle, rg.graph, 0, cudaGraphCondAssignDefault));
         rs.sw = h->sw_handle;
-        cudaGraphNodeParams np = {cudaGraphNodeTypeConditional};
-        np.conditional.handle = h->cond_handle;
-        np.conditional.type = cudaGraphCondTypeWhile;
-        np.conditional.size = 1;
-        cudaGraphNode_t node;
-        CK(cudaGraphAddNode(&node, rg.graph, nullptr, 0, &np));
-        cudaGraph_t body = np.conditional.phGraph_out[0];
-        cudaGraphNodeParams sp = {cudaGraphNodeTypeConditional};
+    }
+    cudaGraphNodeParams np = {cudaGraphNodeTypeConditional};
+    np.conditional.handle = h->cond_handle;
+    np.conditional.type = cudaGraphCondTypeWhile;
+    np.conditional.size = 1;
+    cudaGraphNode_t node;
+    CK(cudaGraphAddNode(&node, rg.graph, nullptr, 0, &np));
+    cudaGraph_t* bodies = np.conditional.phGraph_out;
+    int n_bodies = 1;
+    const int* body_B = &B;
+    cudaGraphNodeParams sp = {cudaGraphNodeTypeConditional};
+    if (rs.act) {
         sp.conditional.handle = h->sw_handle;
         sp.conditional.type = cudaGraphCondTypeSwitch;
         sp.conditional.size = (unsigned)rs.n_buckets;
         cudaGraphNode_t snode;
-        CK(cudaGraphAddNode(&snode, body, nullptr, 0, &sp));
-        h->use_cond = 1;
-        for (int k = 0; k < rs.n_buckets; ++k) {
-            CK(cudaStreamBeginCaptureToGraph(h->cap_stream, sp.conditional.phGraph_out[k], nullptr, nullptr, 0,
-                                             cudaStreamCaptureModeThreadLocal));
-            const int64_t l0 = h->launches;
-            try {
-                run_step<TA>(h, io, rs.bucket_sz[k], rs, h->cap_stream);
-            } catch (...) {
-                cudaGraph_t dummy = nullptr;
-                cudaStreamEndCapture(h->cap_stream, &dummy);
-                h->use_cond = 0;
-                throw;
-            }
-            CK(cudaStreamEndCapture(h->cap_stream, nullptr));
-            if (k > 0) h->launches = l0;      // the per-step launch count is that of the full bucket
-        }
-        h->use_cond = 0;
-    } else if (while_node) {
-        CK(cudaGraphCreate(&rg.graph, 0));
-        CK(cudaGraphConditionalHandleCreate(&h->cond_handle, rg.graph, 1, cudaGraphCondAssignDefault));
-        cudaGraphNodeParams np = {cudaGraphNodeTypeConditional};
-        np.conditional.handle = h->cond_handle;
-        np.conditional.type = cudaGraphCondTypeWhile;
-        np.conditional.size = 1;
-        cudaGraphNode_t node;
-        CK(cudaGraphAddNode(&node, rg.graph, nullptr, 0, &np));
-        cudaGraph_t body = np.conditional.phGraph_out[0];
-        h->use_cond = 1;
-        CK(cudaStreamBeginCaptureToGraph(h->cap_stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+        CK(cudaGraphAddNode(&snode, bodies[0], nullptr, 0, &sp));
+        bodies = sp.conditional.phGraph_out;
+        n_bodies = rs.n_buckets;
+        body_B = rs.bucket_sz;
+    }
+    h->use_cond = 1;
+    for (int k = 0; k < n_bodies; ++k) {
+        CK(cudaStreamBeginCaptureToGraph(h->cap_stream, bodies[k], nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+        const int64_t l0 = h->launches;
         try {
-            run_step<TA>(h, io, B, rs, h->cap_stream);
+            run_step<TA>(h, io, body_B[k], rs, h->cap_stream);
         } catch (...) {
             cudaGraph_t dummy = nullptr;
             cudaStreamEndCapture(h->cap_stream, &dummy);
@@ -2600,20 +2564,10 @@ void build_roll_graph(tante_handle_s* h, tante_handle_s::RollGraph& rg, const St
             throw;
         }
         CK(cudaStreamEndCapture(h->cap_stream, nullptr));
-        h->use_cond = 0;
-    } else {
-        CK(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-        try {
-            run_step<TA>(h, io, B, rs, h->cap_stream);
-        } catch (...) {
-            cudaGraph_t dummy = nullptr;
-            cudaStreamEndCapture(h->cap_stream, &dummy);
-            throw;
-        }
-        CK(cudaStreamEndCapture(h->cap_stream, &rg.graph));
+        if (k > 0) h->launches = l0;      // the per-step launch count is that of the full bucket
     }
+    h->use_cond = 0;
     CK(cudaGraphInstantiate(&rg.exec, rg.graph, 0));
-    rg.while_node = while_node;
     rg.launches_per_step = h->launches - launches0;
     h->launches = launches0;      // capture enqueued nothing
 }
@@ -2632,10 +2586,6 @@ int tante_create(const tante_config_t* cfg, int device, tante_handle_t* out) {
         h->cfg = *cfg;
         h->device = device;
         build_plan(h.get());
-        if (const char* m = getenv("TANTE_ROLLOUT_MODE")) h->rollout_mode = std::max(0, std::min(2, atoi(m)));
-        if (const char* m = getenv("TANTE_ENC_CACHE")) h->use_enc_cache = atoi(m) != 0;
-        if (const char* m = getenv("TANTE_FUSE_TAIL")) h->fuse_tail = atoi(m) != 0;
-        if (const char* m = getenv("TANTE_FUSE_MLP_BWD")) h->fuse_mlp_bwd = atoi(m) != 0;
         int sms = 0;   // stays at the B200 default when no device is visible (CPU-side plan checks)
         if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && sms > 0) h->num_sms = sms;
         else (void)cudaGetLastError();
@@ -2915,16 +2865,14 @@ int tante_rollout(tante_handle_t h, const float* window, int32_t B, int32_t n_ro
         const size_t wbytes = (size_t)B * h->T * h->D * h->cfg.H * h->cfg.W * 4;
         CK(cudaMemcpyAsync(h->ring.p, window, wbytes, cudaMemcpyDeviceToDevice, st));
         RolloutState rs = make_state(h, B, n_roll);
-        {
-            StepIO probe; probe.per_sample = per_sample;
-            const int mode0 = h->prof_on || h->debug ? 0 : h->rollout_mode;
-            if (mode0 == 2 && !h->no_switch && compaction_wanted(h, probe, B, rs)) {
-                rs.act = reinterpret_cast<int*>(h->state.p) + 4 * h->max_batch + 32;
-                const int cand[4] = {B, (3 * B + 3) / 4, (B + 1) / 2, (B + 3) / 4};
-                static const bool one_bucket = getenv("TANTE_ROLLOUT_COMPACT") && atoi(getenv("TANTE_ROLLOUT_COMPACT")) == 2;   // debug: reorder only
-                for (int c : cand)
-                    if (rs.n_buckets == 0 || (!one_bucket && c < rs.bucket_sz[rs.n_buckets - 1])) rs.bucket_sz[rs.n_buckets++] = c;
-            }
+        // While tante_profile or the stage capture is on, the rollout runs as eager launches: the per-launch event brackets
+        // and the stage copies cannot live inside a graph.
+        const bool eager = h->prof_on || h->debug;
+        if (!eager && compaction_wanted(h, per_sample, B, rs)) {
+            rs.act = reinterpret_cast<int*>(h->state.p) + 4 * h->max_batch + 32;
+            const int cand[4] = {B, (3 * B + 3) / 4, (B + 1) / 2, (B + 3) / 4};
+            for (int c : cand)
+                if (rs.n_buckets == 0 || c < rs.bucket_sz[rs.n_buckets - 1]) rs.bucket_sz[rs.n_buckets++] = c;
         }
         init_state_kernel<<<(B + 127) / 128, 128, 0, st>>>(rs, B, h->T);
         CK(cudaGetLastError());
@@ -2937,47 +2885,25 @@ int tante_rollout(tante_handle_t h, const float* window, int32_t B, int32_t n_ro
         io.ring_out = reinterpret_cast<float*>(h->ring.p); io.n_roll = n_roll;
         io.rollout = true; io.per_sample = per_sample; io.out_T = out_T;
 
-        int mode = h->prof_on || h->debug ? 0 : h->rollout_mode;
-        tante_handle_s::RollGraph* rg = nullptr;
-        if (mode > 0) {
+        if (!eager) {
             char key[96];
-            snprintf(key, sizeof(key), "%d/%d/%d/%.9g/%d", B, n_roll, per_sample, (double)out_T, mode);
+            snprintf(key, sizeof(key), "%d/%d/%d/%.9g", B, n_roll, per_sample, (double)out_T);
             auto it = h->graphs.find(key);
             if (it == h->graphs.end()) {
                 tante_handle_s::RollGraph g;
                 try {
-                    try {
-                        if (f32) build_roll_graph<float>(h, g, io, B, rs, mode == 2);
-                        else build_roll_graph<__nv_bfloat16>(h, g, io, B, rs, mode == 2);
-                    } catch (const Error&) {
-                        if (!(mode == 2 && rs.act)) throw;
-                        // SWITCH conditional nodes unavailable: same WHILE graph without the compaction buckets
-                        (void)cudaGetLastError();
-                        if (g.graph) { cudaGraphDestroy(g.graph); g.graph = nullptr; }
-                        h->no_switch = true;
-                        rs.act = nullptr; rs.n_buckets = 0;
-                        if (f32) build_roll_graph<float>(h, g, io, B, rs, true);
-                        else build_roll_graph<__nv_bfloat16>(h, g, io, B, rs, true);
-                    }
-                } catch (const Error& e) {
-                    if (mode != 2) throw;
-                    // conditional nodes unavailable: fall back to per-step graphs for this handle
-                    (void)cudaGetLastError();
-                    h->rollout_mode = mode = 1;
-                    snprintf(key, sizeof(key), "%d/%d/%d/%.9g/%d", B, n_roll, per_sample, (double)out_T, mode);
-                    if (f32) build_roll_graph<float>(h, g, io, B, rs, false);
-                    else build_roll_graph<__nv_bfloat16>(h, g, io, B, rs, false);
+                    if (f32) build_roll_graph<float>(h, g, io, B, rs);
+                    else build_roll_graph<__nv_bfloat16>(h, g, io, B, rs);
+                } catch (...) {
+                    if (g.graph) cudaGraphDestroy(g.graph);
+                    throw;
                 }
                 it = h->graphs.emplace(key, g).first;
             }
-            rg = &it->second;
-        }
-        if (mode == 2) {
             // the whole `while cumulative_length < n_steps_rollout` loop (r_evaler.py:94) is ONE graph launch:
             // a WHILE node re-runs the step body until the device-side counter of unfinished trajectories is 0
-            CK(cudaGraphLaunch(rg->exec, st));
-            h->launches += rg->launches_per_step;      // lower bound: the body runs >= 1 time (device decides)
-            h->last_graph_steps = -1;
+            CK(cudaGraphLaunch(it->second.exec, st));
+            h->launches += it->second.launches_per_step;      // lower bound: the body runs >= 1 time (device decides)
         } else {
             // host loop with a one-step-lagged look at the device's `remaining` counter (never stalls the stream)
             int pending[2] = {0, 0};
@@ -2988,8 +2914,7 @@ int tante_rollout(tante_handle_t h, const float* window, int32_t B, int32_t n_ro
                     pending[slot] = 0;
                     if (h->h_flag[slot] == 0) break;
                 }
-                if (mode == 1) { CK(cudaGraphLaunch(rg->exec, st)); h->launches += rg->launches_per_step; }
-                else if (f32) run_step<float>(h, io, B, rs, st);
+                if (f32) run_step<float>(h, io, B, rs, st);
                 else run_step<__nv_bfloat16>(h, io, B, rs, st);
                 CK(cudaMemcpyAsync(h->h_flag + slot, rs.remaining, 4, cudaMemcpyDeviceToHost, st));
                 CK(cudaEventRecord(h->ev[slot], st));
@@ -3321,7 +3246,7 @@ int tante_test_block_tail(const void* att, const void* Wo, const void* W1, const
         a.x_in = x_in; a.x_out = x_out; a.ln_out = reinterpret_cast<__nv_bfloat16*>(ln_out);
         a.x_mid = x_mid; a.ln2 = reinterpret_cast<__nv_bfloat16*>(ln2); a.hpre = reinterpret_cast<__nv_bfloat16*>(hpre);
         a.hact = reinterpret_cast<__nv_bfloat16*>(hact);
-        for (int i = 0; i < std::max(1, iters); ++i) CK(launch_block_tail_any(a, M, x_mid != nullptr, sms, st));
+        for (int i = 0; i < std::max(1, iters); ++i) CK(launch_block_tail(a, M, x_mid != nullptr, sms, st));
     });
 }
 
@@ -3451,6 +3376,19 @@ int tante_test_gemm(int32_t use_tc, int32_t epi, const void* A, const void* W, c
                 CK(launch_gemm_simt(epi, reinterpret_cast<const float*>(A), K, reinterpret_cast<const float*>(W), K,
                                     reinterpret_cast<float*>(C), N, M, N, K, ep, st));
         }
+    });
+}
+
+int tante_test_gemm_plan(int32_t M, int32_t N, int32_t K, int32_t out_bf16, int32_t* ncta) {
+    return guarded([&] {
+        REQUIRE(ncta, "null argument");
+        REQUIRE(M >= 1 && N >= 1 && K >= 1, "M, N and K must be >= 1");
+        int dev = 0, sms = 148;
+        CK(cudaGetDevice(&dev));
+        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        TcPlan plan;      // what launch_gemm_tc runs for this shape on this device
+        REQUIRE(tc_plan(M, N, K, sms, out_bf16, &plan), "no tcgen05 plan fits this shape");
+        *ncta = plan.ncta;
     });
 }
 

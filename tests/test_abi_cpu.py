@@ -82,6 +82,17 @@ def test_axial_test_hooks_reject_out_of_range_arguments():
     assert kid.value == -1
 
 
+def test_gemm_plan_hook_rejects_bad_arguments():
+    """tante_test_gemm_plan checks its arguments before any device call."""
+    lib = _abi.load()
+    n = ctypes.c_int32(-1)
+    for args, msg in (((256, 256, 256, 0, None), "null argument"), ((0, 256, 256, 0, ctypes.byref(n)), "must be >= 1"),
+                      ((256, 256, -64, 1, ctypes.byref(n)), "must be >= 1")):
+        assert lib.tante_test_gemm_plan(*args) == 1, args
+        assert msg in lib.tante_last_error().decode(), (args, lib.tante_last_error())
+    assert n.value == -1
+
+
 def _cfg(**kw):
     c = _abi.TanteConfig()
     base = dict(in_T=4, n_fields=4, H=128, W=384, taylor_order=1, n_head=8, embed_dim=256, patch_scale=8, deg=1,

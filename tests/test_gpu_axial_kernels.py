@@ -7,15 +7,12 @@ a whole-tensor rel-L2 is checked on top.  Every write-only output starts as NaN 
 band, so an element never written and a write out of bounds both fail."""
 import ctypes
 import math
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, rel_l2
+from conftest import rel_l2
 from dropout_ref import multipliers
 
 pytestmark = pytest.mark.gpu
@@ -426,19 +423,6 @@ def test_propagator_backward_matches_fp64(case):
     prec, S, IC, outer, _ = case
     kid, res = _run_propagator(1, prec, S, IC, outer, False)
     _check_prop(prec, S, kid, res)
-
-
-@pytest.mark.skipif(os.environ.get("TANTE_PROP_SPLIT") == "1", reason="already running under TANTE_PROP_SPLIT=1")
-def test_propagator_forward_split_variant_in_a_subprocess():
-    """TANTE_PROP_SPLIT=1 selects the eight-warp propagator_mma_kernel<4, 2> for 49 <= S <= 64; the switch is read once per
-    process, so the forward cases re-run in a child process.  Both variants report TANTE_AXK_MMA: that the child ran <4, 2>
-    rests on the switch, which launch_propagator_mma reads once into a static and then applies to every MB = 4 launch."""
-    env = dict(os.environ, TANTE_PROP_SPLIT="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", os.path.abspath(__file__),
-                        "-k", "test_propagator_forward_matches_fp64 and (S49 or S64)"], cwd=ROOT, env=env,
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-4000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout and "skipped" not in r.stdout.splitlines()[-1], r.stdout[-2000:]
 
 
 # ---------------------------------------------------------------------------------------------------------------------------

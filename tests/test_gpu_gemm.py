@@ -1,4 +1,6 @@
 """Unit parity of the two GEMM kernels (through the C-ABI test hook) against torch fp32 matmul."""
+import ctypes
+
 import pytest
 import torch
 
@@ -20,6 +22,21 @@ def _ref(epi, A, W, bias, resid):
     return y
 
 
+def _pair_expected(M, N, K, out_bf16):
+    """tc_plan's CTA-pair rule (gemm_tc.cuh): fp32-output epilogues, and bf16 output once K > 512 leaves a single CTA only a
+    64-wide weight slice, run on CTA pairs when N % 128 == 0 and there are enough 256-row tiles to fill the machine."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    pays = not out_bf16 or (K > 512 and N >= 128)
+    return 2 if pays and N % 128 == 0 and M >= 256 * (sms // 2) else 1
+
+
+def _plan_ncta(M, N, K, out_bf16):
+    """CTAs per MMA of the tcgen05 plan the library runs for this shape (tante_test_gemm_plan)."""
+    ncta = ctypes.c_int32(-1)
+    _abi.check(_abi.load().tante_test_gemm_plan(M, N, K, int(out_bf16), ctypes.byref(ncta)))
+    return ncta.value
+
+
 def _run(use_tc, epi, A, W, bias, resid, out_bf16):
     lib = _abi.load()
     M, K = A.shape
@@ -37,8 +54,10 @@ def _run(use_tc, epi, A, W, bias, resid, out_bf16):
     return C
 
 
+# CTA pairs run at M = 40000 and 40150 (above the threshold for any GPU of up to 312 SMs; the last 256-row pair tile is ragged:
+# 64 rows, all in the leader, and 214 rows, split 128 / 86) and single CTAs at the smaller M, both at K = 768 too.
 SHAPES = [(128, 256, 256), (4096, 768, 256), (1000, 256, 256), (333, 128, 256), (5000, 64, 128), (777, 256, 512),
-          (2048, 512, 256), (260, 128, 64), (40000, 768, 256), (3072, 256, 128)]
+          (2048, 512, 256), (260, 128, 64), (40000, 768, 256), (3072, 256, 128), (40150, 256, 768), (1000, 128, 768)]
 
 
 @pytest.mark.parametrize("M,N,K", SHAPES)
@@ -50,6 +69,7 @@ def test_tcgen05_gemm_matches_torch(M, N, K, epi):
     bias = torch.randn(N, device="cuda", generator=g)
     resid = torch.randn(M, N, device="cuda", generator=g)
     ref = _ref(epi, A, W, bias, resid)
+    assert _plan_ncta(M, N, K, False) == _pair_expected(M, N, K, out_bf16=False)
     out = _run(1, epi, A, W, bias, resid, out_bf16=False)
     err = float((out - ref).norm() / ref.norm())
     if epi == 2:
@@ -61,6 +81,7 @@ def test_tcgen05_gemm_matches_torch(M, N, K, epi):
         assert err < 2e-6, err                 # same bf16 inputs, fp32 accumulate: order-of-summation only
         assert float((out - ref).abs().max()) < 1e-4
     if epi != 4:
+        assert _plan_ncta(M, N, K, True) == _pair_expected(M, N, K, out_bf16=True)
         outb = _run(1, epi, A, W, bias, resid, out_bf16=True)
         errb = float((outb.float() - ref).norm() / ref.norm())
         assert errb < 4e-3, errb               # one bf16 rounding of the output
@@ -83,7 +104,7 @@ def test_ffma_gemm_matches_torch(M, N, K, epi):
     assert err < 1e-6, err
 
 
-@pytest.mark.parametrize("M,K", [(128, 256), (1000, 256), (4096, 128), (40000, 256), (333, 64)])
+@pytest.mark.parametrize("M,K", [(128, 256), (1000, 256), (4096, 128), (40000, 256), (40150, 256), (333, 64)])
 def test_tcgen05_gemm_residual_layernorm_epilogue(M, K):
     """x += A W^T + b fused with the next LayerNorm (EPI_BIAS_RESID_LN): both outputs vs torch."""
     lib = _abi.load()
@@ -99,6 +120,7 @@ def test_tcgen05_gemm_residual_layernorm_epilogue(M, K):
     ln_ref = torch.nn.functional.layer_norm(x_ref, (N,), gamma, beta, 1e-5)
     xc = x.clone()
     ln = torch.empty(M, N, device="cuda", dtype=torch.bfloat16)
+    assert _plan_ncta(M, N, K, False) == _pair_expected(M, N, K, out_bf16=False)
     _abi.check(lib.tante_test_gemm(1, 6, A.data_ptr(), W.data_ptr(), bias.data_ptr(), xc.data_ptr(), xc.data_ptr(), 0,
                                    M, N, K, 1, gamma.data_ptr(), beta.data_ptr(), ln.data_ptr(),
                                    torch.cuda.current_stream().cuda_stream))
@@ -107,13 +129,3 @@ def test_tcgen05_gemm_residual_layernorm_epilogue(M, K):
     assert float((ln.float() - ln_ref).norm() / ln_ref.norm()) < 4e-3      # one bf16 rounding
     assert float((ln.float() - ln_ref).abs().max()) < 0.05
 
-
-def test_cta_pair_gemm_on_every_shape_in_a_subprocess():
-    """The CTA-pair (cta_group::2) variant is only chosen where it pays off (fp32 epilogues / K = 768 at large M); force it
-    wherever it fits (TANTE_GEMM_2CTA=2, read once per process) and run this file's tcgen05 parity tests again."""
-    import os, subprocess, sys
-    env = dict(os.environ, TANTE_GEMM_2CTA="2")
-    here = os.path.abspath(__file__)
-    r = subprocess.run([sys.executable, "-m", "pytest", here, "-x", "-q", "-k", "tcgen05 and not subprocess"],
-                       env=env, capture_output=True, text=True, timeout=600, cwd=os.path.dirname(os.path.dirname(here)))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]

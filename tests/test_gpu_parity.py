@@ -418,3 +418,30 @@ def test_compacted_rollout_equals_single_trajectory_runs_bitwise(precision):
             assert ns1[: int(steps1[0]), 0].tolist() == seqs[b]
             assert torch.equal(y[b:b + 1], y1), f"trajectory {b}"
             assert torch.equal(R[: int(steps[b]), b], R1[: int(steps1[0]), 0])
+
+
+@pytest.mark.parametrize("per_sample", [False, True])
+def test_eager_rollout_equals_graph_rollout_bitwise(per_sample):
+    """While the GEMM profiler is on, a rollout runs as eager launches from a host loop (the per-launch event brackets cannot
+    live inside a graph); otherwise it is one device WHILE graph, which with per_sample and B >= 8 also compacts the batch
+    into smaller buckets as trajectories finish.  Both must produce the same frames, R_t, frames per call and calls per
+    sample, bit for bit."""
+    from gpu_util import make_model
+    cfg = O.OracleConfig(n_fields=2, H=32, W=48, taylor_order=2, attn_axes="THW-HWT", deg=False)
+    sd = O.make_state_dict(cfg, 5, rt_bias=3.0585)
+    B = 12
+    x = O.make_input(cfg, B, 6)
+    scale = torch.tensor([8.0, 0.05, 3.0, 1.0, 20.0, 8.0, 0.05, 1.0, 30.0, 8.0, 1.0, 50.0])
+    x = (x * scale.view(B, 1, 1, 1, 1)).cuda()
+    model = make_model(cfg, sd, precision="bf16")
+    with torch.inference_mode():
+        graph = model.rollout(x, 8, per_sample=per_sample)
+        model.profile_gemms(True)
+        try:
+            eager = model.rollout(x, 8, per_sample=per_sample)
+        finally:
+            model.profile_gemms(False)
+    if per_sample:
+        assert len({int(s) for s in graph[3].tolist()}) > 1, "test inputs should finish after different numbers of calls"
+    for name, g, e in zip(("y", "rts", "ns", "steps"), graph, eager):
+        assert torch.equal(g, e), name

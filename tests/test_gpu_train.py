@@ -160,6 +160,37 @@ def test_bf16_training_step_at_benchmarked_shape_vs_oracle():
     assert not bad, "bf16 gradients at the benchmarked shape differ from the oracle:\n" + "\n".join(bad)
 
 
+def test_bf16_training_on_cta_pairs_equals_single_cta_calls():
+    """At the benchmarked shape a call of 2 samples (8192 tokens) runs the block tail, the MLP backward and the fp32-epilogue
+    GEMMs on single CTAs; a call of 6 samples (24576 >= 256 * 74 tokens on a B200) runs them on CTA pairs.  Both see the same
+    rows, so the predictions and the gradient of a summed loss must agree up to the order of the weight-gradient reductions."""
+    from gpu_util import make_model
+    cfg = O.OracleConfig(n_fields=11, H=256, W=256, taylor_order=1, attn_axes="THWTHWTHW", deg=True)
+    sd = O.make_state_dict(cfg, 211)
+    x = O.make_input(cfg, 6, 214).cuda()
+    model = make_model(cfg, sd, "bf16").train()
+    assert 6 * cfg.in_T * cfg.Hp * cfg.Wp >= 256 * (torch.cuda.get_device_properties(0).multi_processor_count // 2)
+    assert 2 * cfg.in_T * cfg.Hp * cfg.Wp < 256 * (torch.cuda.get_device_properties(0).multi_processor_count // 2)
+
+    def run(chunks):
+        model.zero_grad(set_to_none=True)
+        ys = []
+        for xb in chunks:
+            y = model(xb)
+            y.float().square().sum().backward()
+            ys.append(y.detach().float())
+        return torch.cat(ys), {n: p.grad.detach().clone() for n, p in model.named_parameters()}
+    y6, g6 = run([x])
+    y2, g2 = run(x.split(2))
+    assert rel_l2(y6.cpu().numpy(), y2.cpu().numpy()) < 1e-6
+    flat6 = torch.cat([g.flatten() for g in g6.values()]).cpu().numpy()
+    flat2 = torch.cat([g.flatten() for g in g2.values()]).cpu().numpy()
+    assert rel_l2(flat6, flat2) < 1e-4
+    for n in g6:
+        if ".mlp." in n:      # downstream of the fused MLP backward
+            assert rel_l2(g6[n].cpu().numpy(), g2[n].cpu().numpy()) < 1e-3, n
+
+
 def _oracle_grads(cfg, sd, x, gy, grt, out_T, autocast=False):
     """autocast=True: the oracle under torch.autocast(bf16) -- the reference's own amp mode (r_trainer.py:71-74,145);
     its deviation from fp32 is the yardstick for the bf16 tensor mode on cancellation-dominated gradients."""
