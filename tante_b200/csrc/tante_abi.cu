@@ -539,6 +539,24 @@ struct StepIO {
     int n_lim = 0;
 };
 
+// Backward of one taped step (tante_backward, tante_backward_hist).  gframes: f32 (B, n_g, D, H, W) gradient of the emitted
+// frames, batch stride gf_bs; gRt: f32 [B] or null; grad_input: f32 (B, T, D, H, W) or null (written, not accumulated; but see
+// `gin`); flat: f32 [sum numel] parameter gradients in tante_param order (written, not accumulated).
+// Per-sample cursor mode (tante_backward_hist; gin.cur null: off): gframes is gpred, the gradient of the whole prediction buffer
+// (gf_bs == gin.hbs), and the window gradient is ACCUMULATED into it and into grad_input (nullable) through gin, whose
+// offsets are relative to grad_input, or to gpred when there is no grad_input (gin.skip_in).
+struct BackwardIO {
+    const float* input = nullptr;   // the window of the forward (B, T, D, H, W); null in the cursor mode
+    const float* gframes = nullptr;
+    long long gf_bs = 0;
+    int n_g = 1;
+    const float* gRt = nullptr;
+    float* grad_input = nullptr;
+    float* flat = nullptr;
+    FrameTab gin{};
+    float* gpred = nullptr;
+};
+
 RolloutState make_state(tante_handle_s* h, int B, int n_roll) {
     RolloutState rs;
     int* s = reinterpret_cast<int*>(h->state.p);
@@ -823,17 +841,6 @@ void gemm_act(tante_handle_s* h, const TA* A, int lda, int64_t w_off, TA* pre, T
     gemm<TA>(h, EPI_BIAS, A, lda, w_off, pre, N, false, M, N, K, ep, st);
     launch_act_fwd<TA, ACT>(h, pre, out, (long long)M * N, st);
 }
-// overlap: adaptive average pooling of a conv grid [n_img][Hc][Wc][Cc] to the patch grid [n_img][Ho][Wo][Cc], then GELU
-template <typename TA>
-void pool_act(tante_handle_s* h, const TA* in, long long n_img, int Hc, int Wc, int Cc, int Ho, int Wo, TA* pre, TA* out,
-              cudaStream_t st) {
-    const long long n4 = n_img * Ho * Wo * Cc / 4;
-    if (pre) wide_pool_kernel<TA, false, false><<<blocks_for(n4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, pre, nullptr, n4);
-    else wide_pool_kernel<TA, true, false><<<blocks_for(n4, 256), 256, 0, st>>>(in, Hc, Wc, Cc, Ho, Wo, out, nullptr, n4);
-    CK(cudaGetLastError());
-    h->launches++;
-    if (pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, out, n4 * 4, st);
-}
 // decoder stage: sub-pixel matrix S [B*hi*wi][ldS] -> crop + resample (+ bias) to the grid [B][hi*k][wi*k][Cout], then GELU
 template <typename TA>
 void post_act(tante_handle_s* h, const TA* S, int ldS, int B, int hi, int wi, int Cout, int k, int sd, const float* bias, TA* pre,
@@ -851,6 +858,24 @@ void launch_embed(tante_handle_s* h, const float* v, float* x, int tokens, cudaS
     const int C = h->C;
     embed_fwd_kernel<<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(v, AF(h, h->film_t_off), AF(h, h->s_emb),
                                                                               AF(h, h->t_emb), x, tokens, h->T, h->L, C);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+// backward of launch_embed (tante.py:136-141): gradient stream dxs -> gradient gv of the pre-embedding, s_emb / t_emb and the
+// t_encode FiLM parameters
+template <typename TA>
+void launch_embed_bwd(tante_handle_s* h, Tape& tp, TA* gv, cudaStream_t st) {
+    const int C = h->C, T = h->T, L = h->L;
+    CK(cudaMemsetAsync(h->dfilm.p, 0, (size_t)T * 2 * C * 4, st));
+    embed_bwd_kernel<TA><<<(L + (256 / (C / 4)) - 1) / (256 / (C / 4)), 256, 0, st>>>(FP(h->dxs), FP(tp.v), AF(h, h->film_t_off), gv,
+                                                                                     FP(h->dfilm), GA(h, h->s_emb), GA(h, h->t_emb),
+                                                                                     tp.B_used, T, L, C);
+    CK(cudaGetLastError());
+    h->launches++;
+    film_bwd_kernel<<<dim3(T, 16), 256, 3 * C * sizeof(float), st>>>(
+        AF(h, h->tseq_off), FP(h->dfilm), AF(h, h->tenc[0]), AF(h, h->tenc[1]), AF(h, h->tenc[2]), AF(h, h->tenc[4]),
+        AF(h, h->tenc[5]), AF(h, h->tenc[6]), GA(h, h->tenc[0]), GA(h, h->tenc[1]), GA(h, h->tenc[2]), GA(h, h->tenc[3]),
+        GA(h, h->tenc[4]), GA(h, h->tenc[5]), GA(h, h->tenc[6]), GA(h, h->tenc[7]), C, nullptr);
     CK(cudaGetLastError());
     h->launches++;
 }
@@ -896,26 +921,46 @@ void launch_head(tante_handle_s* h, const StepIO& io, int B, const RolloutState&
     CK(cudaGetLastError());
     h->launches++;
 }
+// backward of launch_head: all orders in one pass over the frame gradients -> the gradient G of every order's stage-3 output
+template <typename TA>
+void launch_head_bwd(tante_handle_s* h, Tape& tp, const BackwardIO& io, cudaStream_t st) {
+    const PatchGeom& g = h->geom;
+    const int K = h->K, T = h->T;
+    const long long rows1 = (long long)tp.B_used * h->L * g.R1;
+    const long long DHW = (long long)h->D * h->cfg.H * h->cfg.W;
+    HeadBwdParams hp{};
+    for (int k = 0; k < K; ++k) hp.G[k] = TP<TA>(h->hG) + (size_t)k * rows1 * kHeadPad;
+    hp.K = K; hp.fi = h->cfg.frame_interval; hp.gframes = io.gframes; hp.n_cap = io.n_g;
+    hp.gf_bs = io.gf_bs;
+    hp.n_arr = reinterpret_cast<const int*>(tp.n_arr.p);
+    hp.gi_last = io.grad_input ? io.grad_input + (size_t)(T - 1) * DHW : nullptr;
+    hp.gi_bs = (long long)T * DHW;
+    hp.cur = io.gin.cur; hp.gpred = io.gpred;
+    const size_t hsmem = (size_t)K * kPatchRows * kPatchPitch * sizeof(float);
+    if (g.k0 * g.k1 * g.k2 >= 4) head_gather_kernel<TA, 4><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
+    else head_gather_kernel<TA, 2><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
+    CK(cudaGetLastError());
+    h->launches++;
+}
 
 // ---- patch_scale >= 16 (wide_patch.cuh): encoder, decoder of one order, emit ----
 // Grids of the natural-order encoder stages for a batch of B windows: patch grids (H1 x W1, H2 x W2, Hp x Wp) and the conv grids in
 // front of them (kernel k, stride s, pad (k - 1) / 2); the two differ -- and an adaptive average pooling sits between -- only with
 // overlap_ratio != 0.
+inline int conv_dim(int n, int k, int s) { return (n + 2 * ((k - 1) / 2) - k) / s + 1; }
 struct WideDims {
     int H1, W1, H2, W2, Hc1, Wc1, Hc2, Wc2, Hc3, Wc3;
-    bool pool1, pool2, pool3;
+    bool pool1, pool3;
     long long rows1, rows2, rows3;
 };
 inline WideDims wide_dims(const tante_handle_s* h, int B) {
     const PatchGeom& g = h->geom;
-    auto cdim = [](int n, int k, int s) { return (n + 2 * ((k - 1) / 2) - k) / s + 1; };
     WideDims d;
     d.H1 = h->cfg.H / g.k0; d.W1 = h->cfg.W / g.k0; d.H2 = d.H1 / g.k1; d.W2 = d.W1 / g.k1;
-    d.Hc1 = cdim(h->cfg.H, g.k0, h->st[0]); d.Wc1 = cdim(h->cfg.W, g.k0, h->st[0]);
-    d.Hc2 = cdim(d.H1, g.k1, h->st[1]); d.Wc2 = cdim(d.W1, g.k1, h->st[1]);
-    d.Hc3 = cdim(d.H2, g.k2, h->st[2]); d.Wc3 = cdim(d.W2, g.k2, h->st[2]);
+    d.Hc1 = conv_dim(h->cfg.H, g.k0, h->st[0]); d.Wc1 = conv_dim(h->cfg.W, g.k0, h->st[0]);
+    d.Hc2 = conv_dim(d.H1, g.k1, h->st[1]); d.Wc2 = conv_dim(d.W1, g.k1, h->st[1]);
+    d.Hc3 = conv_dim(d.H2, g.k2, h->st[2]); d.Wc3 = conv_dim(d.W2, g.k2, h->st[2]);
     d.pool1 = d.Hc1 != d.H1 || d.Wc1 != d.W1;
-    d.pool2 = d.Hc2 != d.H2 || d.Wc2 != d.W2;
     d.pool3 = d.Hc3 != h->Hp || d.Wc3 != h->Wp;
     const long long NI = (long long)B * h->T;
     d.rows1 = NI * d.Hc1 * d.Wc1; d.rows2 = NI * d.Hc2 * d.Wc2; d.rows3 = NI * d.Hc3 * d.Wc3;
@@ -938,6 +983,208 @@ inline void gemm_bigk_f32(tante_handle_s* h, const __nv_bfloat16* A, int lda, in
     }
 }
 
+// ---- backward building blocks of the stage functions (each *_bwd sits beside its forward twin) ----
+template <typename TA, int ACT>
+void launch_act_bwd(tante_handle_s* h, TA* g, const TA* pre, long long n, cudaStream_t st) {
+    act_bwd_kernel<TA, ACT><<<blocks_for(n / 4, 256), 256, 0, st>>>(g, pre, n / 4);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+template <typename TA>
+void launch_colsum(tante_handle_s* h, const TA* x, int ld, long long M, int N, float* out, cudaStream_t st) {
+    const unsigned gx = (unsigned)((N + 127) / 128);
+    unsigned gy = (unsigned)std::max<long long>(1, std::min<long long>((M + 255) / 256, (4LL * h->num_sms + gx - 1) / gx));
+    colsum_kernel<TA><<<dim3(gx, gy), 256, 0, st>>>(x, ld, M, N, out);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+// dW[N][K] (+)= A[M][N]^T B[M][K] into the gradient arena
+// `bias_out` (nullable): also db[N] += column sums of A (fused into the tensor-core kernel, else a colsum launch)
+template <typename TA>
+void wgrad(tante_handle_s* h, const TA* A, int lda, const TA* Bm, int ldb, float* out, long long M, int N, int K,
+           cudaStream_t st, float* bias_out = nullptr) {
+    {
+        ProfScope ps(h, st, 2.0 * (double)M * N * K, 2, (double)M * (N + K) * sizeof(TA));
+        if constexpr (sizeof(TA) == 2) {
+            if (wgrad_tc_supported(M, N, K, K, lda, ldb, K)) {
+                CK(launch_wgrad_tc(A, lda, Bm, ldb, out, K, M, N, K, K, h->num_sms, st, bias_out));
+                h->launches++;
+                return;
+            }
+        }
+        CK((launch_wgrad_simt<TA, TA>(A, lda, Bm, ldb, out, K, M, N, K, h->num_sms, st)));
+        h->launches++;
+    }
+    if (bias_out) launch_colsum<TA>(h, A, lda, M, N, bias_out, st);
+}
+// same with a zero-padded B operand: B is stored [M][Kb] (Kb % 64 == 0), only the first Kc columns of dW are kept
+template <typename TA>
+void wgrad_pad(tante_handle_s* h, const TA* A, int lda, int N, const TA* Bm, int ldb, int Kb, float* out, int ldc, int Kc,
+               long long M, cudaStream_t st, float* bias_out = nullptr) {
+    {
+        ProfScope ps(h, st, 2.0 * (double)M * N * Kc, 2, (double)M * (N + Kb) * sizeof(TA));
+        if constexpr (sizeof(TA) == 2) {
+            if (wgrad_tc_supported(M, N, Kb, Kc, lda, ldb, ldc)) {
+                CK(launch_wgrad_tc(A, lda, Bm, ldb, out, ldc, M, N, Kb, Kc, h->num_sms, st, bias_out));
+                h->launches++;
+                return;
+            }
+        }
+        CK((launch_wgrad_simt<TA, TA>(A, lda, Bm, ldb, out, ldc, M, N, Kc, h->num_sms, st)));
+        h->launches++;
+    }
+    if (bias_out) launch_colsum<TA>(h, A, lda, M, N, bias_out, st);
+}
+// dX = dY * W via the transposed packed weight (no bias)
+template <typename TA>
+void gemm_dx(tante_handle_s* h, const TA* A, int lda, int64_t wT_off, TA* out, int ldc, int M, int N, int K, cudaStream_t st) {
+    EpiParams ep; ep.bias = AF(h, h->zero_off);
+    REQUIRE(N <= 8192, "input-gradient GEMM wider than the zero-bias vector");
+    if (sizeof(TA) == 2 && K > 1024) {
+        // the tcgen05 GEMM keeps a K <= 1024 weight slice resident (K = 2048: first deconv of patch_scale 64): two K halves
+        // accumulated through an fp32 scratch, then one conversion pass
+        REQUIRE(ldc == N, "input-gradient GEMM: K not covered");
+        if (h->kscratch.bytes < (size_t)M * N * 4) destroy_graphs(h);      // (a captured rollout may hold the old pointer)
+        dev_alloc(h, h->kscratch, (size_t)M * N * 4);      // (training only: never inside a stream capture)
+        float* v = FP(h->kscratch);
+        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(A), lda, wT_off, v, M, N, K, AF(h, h->zero_off), st);
+        convert_kernel<TA><<<blocks_for((long long)M * N / 4, 256), 256, 0, st>>>(v, out, (long long)M * N / 4);
+        CK(cudaGetLastError());
+        h->launches++;
+        return;
+    }
+    gemm<TA>(h, EPI_BIAS, A, lda, wT_off, out, ldc, sizeof(TA) == 4, M, N, K, ep, st);
+}
+
+// Natural-order patch stage as an activation producer (see gemm_act): the patch matrix A [n_img * Hc * Wc][K] times W^T + bias
+// onto the conv grid, in K blocks through the fp32 scratch when K exceeds the tcgen05 GEMM's resident slice (1024); with
+// overlap_ratio != 0 (conv grid != patch grid Ho x Wo) adaptive average pooling to the patch grid.  epi EPI_BIAS_GELU_ERF: GELU
+// into the TA grid `out` (with `pre` set through the pre-activation and act_fwd_kernel); EPI_BIAS: the fp32 grid `out`;
+// EPI_EMBED: the fp32 residual stream `out` (no pooling, no split-K).
+template <typename TA>
+void patch_gemm(tante_handle_s* h, int epi, const TA* A, int K, int64_t w_off, const EpiParams& ep, TA* pre, void* out, int Cout,
+                long long n_img, int Hc, int Wc, int Ho, int Wo, cudaStream_t st) {
+    const bool act = epi == EPI_BIAS_GELU_ERF;
+    const long long rows = n_img * Hc * Wc;
+    const bool pooled = Hc != Ho || Wc != Wo;
+    const bool bigk = sizeof(TA) == 2 && K > 1024;
+    REQUIRE(act || epi == EPI_BIAS || (epi == EPI_EMBED && !pooled && !bigk), "patch stage: epilogue not covered");
+    if (pooled) {
+        REQUIRE((size_t)rows * Cout * sizeof(TA) <= h->cgrid.bytes, "pooled conv: conv-grid scratch not reserved");
+        TA* cg = TP<TA>(h->cgrid);
+        if (bigk) {
+            REQUIRE((size_t)rows * Cout * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
+            float* v = FP(h->kscratch);
+            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(A), K, w_off, v, (int)rows, Cout, K, ep.bias, st);
+            f32_to_ta_kernel<TA, false><<<blocks_for(rows * Cout / 4, 256), 256, 0, st>>>(v, cg, rows * Cout / 4);
+            CK(cudaGetLastError());
+            h->launches++;
+        } else {
+            EpiParams eb; eb.bias = ep.bias;
+            gemm<TA>(h, EPI_BIAS, A, K, w_off, cg, Cout, false, (int)rows, Cout, K, eb, st);
+        }
+        const long long p4 = n_img * Ho * Wo * Cout / 4;
+        const unsigned nb = blocks_for(p4, 256);
+        if (!act) wide_pool_kernel<TA, false, true><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, nullptr, reinterpret_cast<float*>(out), p4);
+        else if (pre) wide_pool_kernel<TA, false, false><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, pre, nullptr, p4);
+        else wide_pool_kernel<TA, true, false><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, reinterpret_cast<TA*>(out), nullptr, p4);
+        CK(cudaGetLastError());
+        h->launches++;
+    } else if (bigk && !act) {
+        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(A), K, w_off, reinterpret_cast<float*>(out), (int)rows, Cout, K, ep.bias, st);
+    } else if (bigk) {
+        // 8x8 stages (K = 2048): accumulate in the fp32 scratch of tante_reserve, then bias-free activation + conversion
+        REQUIRE((size_t)rows * Cout * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
+        float* v = FP(h->kscratch);
+        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(A), K, w_off, v, (int)rows, Cout, K, ep.bias, st);
+        const long long n4 = rows * Cout / 4;
+        if (pre) f32_to_ta_kernel<TA, false><<<blocks_for(n4, 256), 256, 0, st>>>(v, pre, n4);
+        else f32_to_ta_kernel<TA, true><<<blocks_for(n4, 256), 256, 0, st>>>(v, reinterpret_cast<TA*>(out), n4);
+        CK(cudaGetLastError());
+        h->launches++;
+    } else {
+        gemm<TA>(h, act && pre ? EPI_BIAS : epi, A, K, w_off, act && pre ? pre : out, Cout, !act, (int)rows, Cout, K, ep, st);
+    }
+    if (act && pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, reinterpret_cast<TA*>(out), n_img * Ho * Wo * Cout, st);
+}
+
+// conv (kernel k, stride sd, default k) over a channels-last grid [n_img][Hs][Ws][Cin] as gather + patch_gemm
+template <typename TA>
+void conv_cl_gemm(tante_handle_s* h, int epi, const TA* grid, int Hs, int Ws, int Cin, int k, int64_t w_off, const EpiParams& ep,
+                  TA* pre, void* out, int Cout, long long n_img, cudaStream_t st, int sd = 0) {
+    TA* wb = TP<TA>(h->wbuf);
+    const int K = k * k * Cin;
+    const int se = sd > 0 ? sd : k, pad = (k - 1) / 2;
+    const int Hc = conv_dim(Hs, k, se), Wc = conv_dim(Ws, k, se);
+    const long long rows = n_img * Hc * Wc;
+    REQUIRE(rows < (1LL << 31), "input too large for the gather GEMM");
+    const long long total4 = rows * K / 4;
+    wide_im2col_cl_kernel<TA><<<blocks_for(total4, 256), 256, 0, st>>>(grid, Hs, Ws, Cin, k, pad, wb, total4, se, Hc, Wc);
+    CK(cudaGetLastError());
+    h->launches++;
+    patch_gemm<TA>(h, epi, wb, K, w_off, ep, pre, out, Cout, n_img, Hc, Wc, Hs / k, Ws / k, st);
+}
+
+// backward of the adaptive average pooling of an overlapped stage: gradient on the patch grid [n_img][Ho][Wo][Cc] -> on the conv
+// grid [n_img][Hc][Wc][Cc] (returned: the conv-grid scratch)
+template <typename TA>
+const TA* pool_bwd(tante_handle_s* h, const TA* g, long long n_img, int Hc, int Wc, int Cc, int Ho, int Wo, cudaStream_t st) {
+    TA* cg = TP<TA>(h->cgrid);
+    const long long total4 = n_img * Hc * Wc * Cc / 4;
+    wide_pool_bwd_kernel<TA, false><<<blocks_for(total4, 256), 256, 0, st>>>(g, nullptr, Hc, Wc, Cc, Ho, Wo, cg, total4);
+    CK(cudaGetLastError());
+    h->launches++;
+    return cg;
+}
+
+// backward of conv_cl_gemm for encoder stage i, then of the GELU that produced the stage input: gy = the gradient of the stage
+// output (patch grid [n_img][Hs / k][Ws / k][Cout]), x / xpre = the kept input grid [n_img][Hs][Ws][Cin] and its pre-activation.
+// Accumulates the gradients of enc_w[i] / enc_b[i]; the patch matrix is re-gathered from x (cheap, one pass) and its gradient
+// goes back to the grid through the transposed gather, into gx.
+template <typename TA>
+void conv_cl_gemm_bwd(tante_handle_s* h, int i, const TA* gy, const TA* x, const TA* xpre, TA* gx, int Hs, int Ws, int Cin, int k,
+                      int sd, int Cout, long long n_img, cudaStream_t st) {
+    TA* wb = TP<TA>(h->wbuf);
+    const int K = k * k * Cin, pad = (k - 1) / 2, Ho = Hs / k, Wo = Ws / k;
+    const int Hc = conv_dim(Hs, k, sd), Wc = conv_dim(Ws, k, sd);
+    const long long rows = n_img * Hc * Wc;
+    REQUIRE(rows < (1LL << 31), "input too large for the conv backward GEMMs");
+    const TA* dY = Hc != Ho || Wc != Wo ? pool_bwd<TA>(h, gy, n_img, Hc, Wc, Cout, Ho, Wo, st) : gy;
+    const long long k4 = rows * K / 4;
+    wide_im2col_cl_kernel<TA><<<blocks_for(k4, 256), 256, 0, st>>>(x, Hs, Ws, Cin, k, pad, wb, k4, sd, Hc, Wc);
+    CK(cudaGetLastError());
+    h->launches++;
+    wgrad<TA>(h, dY, Cout, wb, K, GA(h, h->enc_w[i]), rows, Cout, K, st, GA(h, h->enc_b[i]));
+    gemm_dx<TA>(h, dY, Cout, h->enc_wT[i], wb, K, (int)rows, K, Cout, st);
+    const long long n = n_img * Hs * Ws * Cin;
+    wide_col2im_cl_kernel<TA><<<blocks_for(n / 4, 256), 256, 0, st>>>(wb, Hs, Ws, Cin, k, pad, gx, n / 4, sd, Hc, Wc);
+    CK(cudaGetLastError());
+    h->launches++;
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, gx, xpre, n, st);
+}
+
+// backward of a natural-order decoder stage (GEMM onto the sub-pixel matrix, then post_act) of decoder layer i of order o: gy =
+// the gradient of the stage output grid [B][hi * k][wi * k][Cout], turned in place into that of its pre-activation `pre`.
+// Accumulates the gradients of decw[i] / decb[i] and writes the gradient of the stage input x [B * hi * wi][Cin] to gx.
+template <typename TA>
+void deconv_stage_bwd(tante_handle_s* h, const OrderPlan& op, int i, TA* gy, const TA* pre, const TA* x, TA* gx, int B, int hi,
+                      int wi, int Cin, int Cout, int k, int sd, cudaStream_t st) {
+    TA* wb = TP<TA>(h->wbuf);
+    const int N = k * k * Cout;
+    const long long Mo = (long long)B * (hi * k) * (wi * k), Mi = (long long)B * hi * wi;
+    // bias gradient: without overlap the replicated bias rode in the GEMM (column sums of the sub-pixel gradient, folded at
+    // unpack); an overlapped stage added bias[co] once per output sample, so its gradient is the sum of the OUTPUT gradient
+    const bool ov = sd != k;
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, gy, pre, Mo * Cout, st);
+    if (ov) launch_colsum<TA>(h, gy, Cout, Mo, Cout, GA(h, op.decb[i]), st);
+    const long long tot = Mi * N;
+    wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(gy, nullptr, N, hi, wi, Cout, k, wb, tot, sd);
+    CK(cudaGetLastError());
+    h->launches++;
+    wgrad<TA>(h, wb, N, x, Cin, GA(h, op.decw[i]), Mi, N, Cin, st, ov ? nullptr : GA(h, op.decb[i]));
+    gemm_dx<TA>(h, wb, N, op.decwT[i], gx, Cin, (int)Mi, Cin, N, st);
+}
+
 template <typename TA>
 void run_encoder_wide(tante_handle_s* h, const StepIO& io, int B, cudaStream_t st) {
     REQUIRE(!io.ft.cur, "windowed BPTT is not available at patch_scale >= 16 / with overlap");
@@ -948,77 +1195,64 @@ void run_encoder_wide(tante_handle_s* h, const StepIO& io, int B, cudaStream_t s
     const WideDims d = wide_dims(h, B);
     REQUIRE(d.rows1 * h->K1pad < (1LL << 40) && d.rows1 < (1LL << 31) && d.rows2 < (1LL << 31) && d.rows3 < (1LL << 31),
             "input too large for the wide conv GEMMs");
+    REQUIRE(sizeof(TA) == 4 || g.k1 * g.k1 * C1 <= 1024, "bf16 wide encoder: conv2 reduction k1 * k1 * embed_dim / 4 above 1024");
     Tape* tp = io.tape;
-    TA* wb = TP<TA>(h->wbuf);
-    TA* cg = TP<TA>(h->cgrid);
-    TA* cols = tp ? TP<TA>(tp->cols) : wb;      // first patch matrix (training keeps it for the weight gradient)
+    TA* cols = tp ? TP<TA>(tp->cols) : TP<TA>(h->wbuf);      // first patch matrix (training keeps it for the weight gradient)
     TA* a1 = tp ? TP<TA>(tp->a1act) : TP<TA>(h->a1);
     TA* a2 = tp ? TP<TA>(tp->a2act) : TP<TA>(h->a2);
     TA* a1pre = tp ? TP<TA>(tp->a1pre) : nullptr;
     TA* a2pre = tp ? TP<TA>(tp->a2pre) : nullptr;
     float* v = tp ? FP(tp->v) : FP(h->qkv);     // fp32 pre-embedding (inference: the QKV scratch, free until the first QKV GEMM)
     float* x = tp ? FP(tp->ord[0].P[0]) : FP(h->x);
-    // conv stage + GELU: GEMM over the patch matrix; with overlap onto the conv grid, then adaptive average pooling
-    auto stage = [&](const TA* A, int Kc, int64_t w_off, const float* bias, int Cc, long long rows, bool pooled, int Hc, int Wc,
-                     int Ho, int Wo, TA* pre, TA* out) {
-        EpiParams e; e.bias = bias;
-        if (!pooled) {
-            gemm_act<TA, ACT_GELU_ERF>(h, A, Kc, w_off, pre, out, (int)rows, Cc, Kc, e, st);
-            return;
-        }
-        gemm<TA>(h, EPI_BIAS, A, Kc, w_off, cg, Cc, false, (int)rows, Cc, Kc, e, st);
-        pool_act<TA>(h, cg, NI, Hc, Wc, Cc, Ho, Wo, pre, out, st);
-    };
-    // conv1: (shifted / strided) windows of the ring frames -> [rows1][K1pad] -> grid [BT][H1][W1][C1]
+    // conv1 + GELU: (shifted / strided) windows of the ring frames -> [rows1][K1pad] -> grid [BT][H1][W1][C1]
     const long long total = d.rows1 * h->K1pad;
     wide_im2col_cf_kernel<TA><<<blocks_for(total, 256), 256, 0, st>>>(io.input, io.fcount, T, h->D, h->cfg.H, h->cfg.W, g.k0,
                                                                      (g.k0 - 1) / 2, h->K1pad, cols, total, h->st[0], d.Hc1, d.Wc1);
     CK(cudaGetLastError());
     h->launches++;
-    stage(cols, h->K1pad, h->enc_w1wide, AF(h, h->enc_b[0]), C1, d.rows1, d.pool1, d.Hc1, d.Wc1, d.H1, d.W1, a1pre, a1);
-    // conv2
-    const int K2 = g.k1 * g.k1 * C1, K3 = g.k2 * g.k2 * C2;
-    wide_im2col_cl_kernel<TA><<<blocks_for(d.rows2 * K2 / 4, 256), 256, 0, st>>>(a1, d.H1, d.W1, C1, g.k1, (g.k1 - 1) / 2, wb,
-                                                                                d.rows2 * K2 / 4, h->st[1], d.Hc2, d.Wc2);
-    CK(cudaGetLastError());
-    h->launches++;
-    stage(wb, K2, h->enc_w[1], AF(h, h->enc_b[1]), C2, d.rows2, d.pool2, d.Hc2, d.Wc2, d.H2, d.W2, a2pre, a2);
+    EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
+    patch_gemm<TA>(h, EPI_BIAS_GELU_ERF, cols, h->K1pad, h->enc_w1wide, e1, a1pre, a1, C1, NI, d.Hc1, d.Wc1, d.H1, d.W1, st);
+    // conv2 + GELU
+    EpiParams e2; e2.bias = AF(h, h->enc_b[1]);
+    conv_cl_gemm<TA>(h, EPI_BIAS_GELU_ERF, a1, d.H1, d.W1, C1, g.k1, h->enc_w[1], e2, a2pre, a2, C2, NI, st, h->st[1]);
     // conv3 + t_encode FiLM + embeddings -> residual stream
-    wide_im2col_cl_kernel<TA><<<blocks_for(d.rows3 * K3 / 4, 256), 256, 0, st>>>(a2, d.H2, d.W2, C2, g.k2, (g.k2 - 1) / 2, wb,
-                                                                                d.rows3 * K3 / 4, h->st[2], d.Hc3, d.Wc3);
-    CK(cudaGetLastError());
-    h->launches++;
     EpiParams e3; e3.bias = AF(h, h->enc_b[2]);
-    // K = 2048 (patch_scale 64) exceeds the resident weight slice of the tcgen05 GEMM: K blocks through an fp32 scratch
-    const bool bigk = sizeof(TA) == 2 && K3 > 1024;
-    if (!d.pool3 && !bigk && !tp) {      // the embed epilogue writes the residual stream directly
+    if (!tp && !(sizeof(TA) == 2 && g.k2 * g.k2 * C2 > 1024) && !d.pool3) {      // the embed epilogue writes x directly
         e3.film = AF(h, h->film_t_off); e3.s_emb = AF(h, h->s_emb); e3.t_emb = AF(h, h->t_emb);
         e3.T = T; e3.L = h->L; e3.ldr = C;
-        gemm<TA>(h, EPI_EMBED, wb, K3, h->enc_w[2], x, C, true, tokens, C, K3, e3, st);
+        conv_cl_gemm<TA>(h, EPI_EMBED, a2, d.H2, d.W2, C2, g.k2, h->enc_w[2], e3, nullptr, x, C, NI, st, h->st[2]);
         return;
     }
-    if (d.pool3) {
-        // overlap: conv grid -> adaptive average pooling -> fp32 pre-embedding
-        if (bigk) {
-            REQUIRE((size_t)d.rows3 * C * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
-            float* acc = FP(h->kscratch);
-            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], acc, (int)d.rows3, C, K3, e3.bias, st);
-            f32_to_ta_kernel<TA, false><<<blocks_for(d.rows3 * C / 4, 256), 256, 0, st>>>(acc, cg, d.rows3 * C / 4);
-            CK(cudaGetLastError());
-            h->launches++;
-        } else {
-            gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], cg, C, false, (int)d.rows3, C, K3, e3, st);
-        }
-        const long long n4 = NI * h->Hp * h->Wp * C / 4;
-        wide_pool_kernel<TA, false, true><<<blocks_for(n4, 256), 256, 0, st>>>(cg, d.Hc3, d.Wc3, C, h->Hp, h->Wp, nullptr, v, n4);
+    // (training, split-K or pooled: fp32 pre-embedding, then the embed pass)
+    conv_cl_gemm<TA>(h, EPI_BIAS, a2, d.H2, d.W2, C2, g.k2, h->enc_w[2], e3, nullptr, v, C, NI, st, h->st[2]);
+    launch_embed(h, v, x, tokens, st);
+}
+
+// backward of run_encoder_wide from gv, the gradient of the fp32 pre-embedding
+template <typename TA>
+void run_encoder_wide_bwd(tante_handle_s* h, Tape& tp, const BackwardIO& io, const TA* gv, cudaStream_t st) {
+    const int C = h->C, C1 = h->C1, C2 = h->C2, D = h->D, H = h->cfg.H, W = h->cfg.W;
+    const PatchGeom& g = h->geom;
+    const WideDims wd = wide_dims(h, tp.B_used);
+    const long long NI = (long long)tp.B_used * h->T;
+    const int NO = g.k0 * g.k0 * D;
+    TA* ga2 = TP<TA>(h->gq);
+    TA* ga1 = TP<TA>(h->ga1);
+    conv_cl_gemm_bwd<TA>(h, 2, gv, TP<TA>(tp.a2act), TP<TA>(tp.a2pre), ga2, wd.H2, wd.W2, C2, g.k2, h->st[2], C, NI, st);
+    conv_cl_gemm_bwd<TA>(h, 1, ga2, TP<TA>(tp.a1act), TP<TA>(tp.a1pre), ga1, wd.H1, wd.W1, C1, g.k1, h->st[1], C2, NI, st);
+    // conv1: the forward kept its patch matrix; the input gradient goes back to the channels-first frames
+    const TA* dY1 = wd.pool1 ? pool_bwd<TA>(h, ga1, NI, wd.Hc1, wd.Wc1, C1, wd.H1, wd.W1, st) : ga1;
+    wgrad_pad<TA>(h, dY1, C1, C1, TP<TA>(tp.cols), h->K1pad, h->K1pad, GA(h, h->enc_w[0]), NO, NO, wd.rows1, st, GA(h, h->enc_b[0]));
+    if (io.grad_input) {
+        REQUIRE(wd.rows1 < (1LL << 31), "input too large for the first-conv backward GEMM");
+        TA* wb = TP<TA>(h->wbuf);
+        gemm_dx<TA>(h, dY1, C1, h->enc_wT[0], wb, h->K1pad, (int)wd.rows1, h->K1pad, C1, st);
+        const long long tot = NI * D * H * W;
+        wide_col2im_cf_kernel<TA><<<blocks_for(tot, 256), 256, 0, st>>>(wb, D, H, W, g.k0, (g.k0 - 1) / 2, h->K1pad, io.grad_input, tot,
+                                                                       h->st[0], wd.Hc1, wd.Wc1);
         CK(cudaGetLastError());
         h->launches++;
-    } else if (bigk) {
-        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K3, h->enc_w[2], v, tokens, C, K3, e3.bias, st);
-    } else {
-        gemm<TA>(h, EPI_BIAS, wb, K3, h->enc_w[2], v, C, true, tokens, C, K3, e3, st);
     }
-    launch_embed(h, v, x, tokens, st);
 }
 
 // decoder of order o on the (modified) last-frame latent dmod [B*L][C] -> derivative field dfield[o] (B, D, H, W); the stage
@@ -1056,6 +1290,38 @@ void run_decoder_wide(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape
                                                                                nullptr, field, n, h->st[0]);
     CK(cudaGetLastError());
     h->launches++;
+}
+
+// backward of run_decoder_wide of order o: the gradient of its derivative field (dfield, from the emit backward) -> the gradient of
+// dmod in h->hd
+template <typename TA>
+void run_decoder_wide_bwd(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape& ot, cudaStream_t st) {
+    const OrderPlan& op = h->orders[o];
+    const int C = h->C, C1 = h->C1, C2 = h->C2, D = h->D, Hp = h->Hp, Wp = h->Wp, NP = h->NOpad;
+    const PatchGeom& g = h->geom;
+    const int H2 = Hp * g.k2, W2 = Wp * g.k2, H1 = H2 * g.k1, W1 = W2 * g.k1, NO = g.k0 * g.k0 * D;
+    const long long rows1 = (long long)B * h->L * g.R1;
+    const long long HW = (long long)h->cfg.H * h->cfg.W;
+    const float* gf = FP(h->dfield) + (size_t)o * B * D * HW;
+    TA* G = TP<TA>(h->hG);                                   // dS3 [rows1][NOpad]
+    TA* dz = TP<TA>(h->hz) + (size_t)o * rows1 * C1;
+    TA* dz1 = TP<TA>(h->hz1);
+    // dec_conv_3: transpose of the crop + bilinear resample back to the sub-pixel matrix, then its weight / input gradients
+    const long long tot = rows1 * NP;
+    wide_deconv_post_bwd_kernel<TA, true><<<blocks_for(tot, 256), 256, 0, st>>>(nullptr, gf, NP, H1, W1, D, g.k0, G, tot, h->st[0]);
+    CK(cudaGetLastError());
+    h->launches++;
+    wgrad_pad<TA>(h, TP<TA>(ot.z2act), C1, C1, G, NP, NP, GA(h, op.decw[2]), NO, NO, rows1, st);
+    if (h->st[0] != g.k0) {      // overlapped stage: bias gradient = sum of the field gradient (see deconv_stage_bwd)
+        field_bias_grad_kernel<<<dim3((unsigned)D, 32), 256, 0, st>>>(gf, D, HW, B, GA(h, op.decb[2]));
+        CK(cudaGetLastError());
+        h->launches++;
+    } else {
+        launch_colsum<TA>(h, G, NP, rows1, NO, GA(h, op.decb[2]), st);
+    }
+    gemm_dx<TA>(h, G, NP, op.w3pad, dz, C1, (int)rows1, C1, NP, st);
+    deconv_stage_bwd<TA>(h, op, 1, dz, TP<TA>(ot.z2pre), TP<TA>(ot.z1act), dz1, B, H2, W2, C2, C1, g.k1, h->st[1], st);
+    deconv_stage_bwd<TA>(h, op, 0, dz1, TP<TA>(ot.z1pre), dmod, TP<TA>(h->hd), B, Hp, Wp, C, C2, g.k2, h->st[2], st);
 }
 
 // ---- enc_dec_type = 'fno' (fno.cuh) ----
@@ -1125,67 +1391,59 @@ void spectral_act(tante_handle_s* h, const SpecPlan& sp, const SpecView& in, lon
     if (pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, pre, out, N * H * W * sp.Cout, st);
 }
 
-// conv over a channels-last grid as gather + GEMM; K beyond the tcgen05 GEMM's resident slice (1024) runs in K blocks
+// Backward of one SpectralLayer (fno.cuh, "training"): x = the layer's saved input, g = the gradient of its output (after the
+// GELU backward).  Accumulates the gradients of weight / w0 / bias, and writes the input gradient to the channels-last grid
+// `dx` or accumulates it into the channels-first fp32 `gin` (first encoder layer); both null: parameters only.
 template <typename TA>
-void conv_cl_gemm(tante_handle_s* h, int epi, const TA* grid, int Hs, int Ws, int Cin, int k, int64_t w_off, void* out, int Cout,
-                  bool out_f32, long long n_img, EpiParams ep, cudaStream_t st, int sd = 0) {
-    TA* wb = reinterpret_cast<TA*>(h->wbuf.p);
-    const int K = k * k * Cin;
-    const int se = sd > 0 ? sd : k, pad = (k - 1) / 2;
-    const int Hc = (Hs + 2 * pad - k) / se + 1, Wc = (Ws + 2 * pad - k) / se + 1;      // conv grid; == the patch grid without overlap
-    const int Ho = Hs / k, Wo = Ws / k;
-    const bool pooled = Hc != Ho || Wc != Wo;
-    const long long rows = n_img * Hc * Wc;
-    REQUIRE(rows < (1LL << 31), "input too large for the gather GEMM");
-    const long long total4 = rows * K / 4;
-    wide_im2col_cl_kernel<TA><<<blocks_for(total4, 256), 256, 0, st>>>(grid, Hs, Ws, Cin, k, pad, wb, total4, se, Hc, Wc);
+void run_spectral_bwd(tante_handle_s* h, const SpecPlan& sp, const SpecView& x, const SpecView& g, long long N, int H, int W,
+                      int level, TA* dx, float* gin, cudaStream_t st) {
+    const int W0 = h->cfg.W, H0 = h->cfg.H, W1 = W0 / h->fp0;
+    const float2* tw = reinterpret_cast<const float2*>(h->ftw.p);
+    const float2* twW = level == 0 ? tw : tw + W0 + H0;
+    const float2* twH = level == 0 ? tw + W0 : tw + W0 + H0 + W1;
+    const int m1 = sp.wm1, m2 = sp.wm2, Cin = sp.Cin, Cout = sp.Cout;
+    float2* A = reinterpret_cast<float2*>(h->fA.p);
+    float2* Bc = reinterpret_cast<float2*>(h->fB.p);
+    float2* Cc = reinterpret_cast<float2*>(h->fC.p);
+    float2* Dd = reinterpret_cast<float2*>(h->fD.p);
+    // gY = dft_h(dft_w(g))  -> Bc
+    const long long rows_o = N * Cout * H, rows_i = N * Cin * H;
+    spec_dft_w_kernel<TA><<<blocks_for(rows_o, 4), 128, 0, st>>>(g, Cout, H, W, m2, twW, A, rows_o);
     CK(cudaGetLastError());
-    h->launches++;
-    const bool bigk = sizeof(TA) == 2 && K > 1024;
-    if (pooled) {
-        // overlap_ratio != 0: GEMM (+ bias) onto the conv grid, adaptive average pooling (+ GELU) to the patch grid
-        REQUIRE(epi == EPI_BIAS || epi == EPI_BIAS_GELU_ERF, "pooled conv: epilogue not covered");
-        REQUIRE((size_t)rows * Cout * sizeof(TA) <= h->cgrid.bytes, "pooled conv: conv-grid scratch not reserved");
-        TA* cg = reinterpret_cast<TA*>(h->cgrid.p);
-        if (bigk) {
-            REQUIRE((size_t)rows * Cout * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
-            float* v = reinterpret_cast<float*>(h->kscratch.p);
-            gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(wb), K, w_off, v, (int)rows, Cout, K, ep.bias, st);
-            f32_to_ta_kernel<TA, false><<<blocks_for(rows * Cout / 4, 256), 256, 0, st>>>(v, cg, rows * Cout / 4);
-            CK(cudaGetLastError());
-            h->launches++;
-        } else {
-            EpiParams eb; eb.bias = ep.bias;
-            gemm<TA>(h, EPI_BIAS, wb, K, w_off, cg, Cout, false, (int)rows, Cout, K, eb, st);
-        }
-        const long long p4 = n_img * Ho * Wo * Cout / 4;
-        const unsigned nb = blocks_for(p4, 256);
-        if (out_f32) wide_pool_kernel<TA, false, true><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, nullptr, reinterpret_cast<float*>(out), p4);
-        else if (epi == EPI_BIAS_GELU_ERF) wide_pool_kernel<TA, true, false><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, reinterpret_cast<TA*>(out), nullptr, p4);
-        else wide_pool_kernel<TA, false, false><<<nb, 256, 0, st>>>(cg, Hc, Wc, Cout, Ho, Wo, reinterpret_cast<TA*>(out), nullptr, p4);
+    const long long ty = N * Cout * 2 * m1 * m2, tx = N * Cin * 2 * m1 * m2;
+    spec_dft_h_kernel<<<blocks_for(ty, 256), 256, 0, st>>>(A, H, m1, m2, twH, Bc, ty);
+    CK(cudaGetLastError());
+    // X = dft_h(dft_w(x))  -> Cc (recomputed: two passes over the saved input)
+    spec_dft_w_kernel<TA><<<blocks_for(rows_i, 4), 128, 0, st>>>(x, Cin, H, W, m2, twW, A, rows_i);
+    CK(cudaGetLastError());
+    spec_dft_h_kernel<<<blocks_for(tx, 256), 256, 0, st>>>(A, H, m1, m2, twH, Cc, tx);
+    CK(cudaGetLastError());
+    const long long tw_ = (long long)Cin * Cout * m1 * m2;
+    spec_wt_grad_kernel<<<blocks_for(tw_, 256), 256, 0, st>>>(Cc, Bc, Cin, Cout, m1, m2, sp.wm2, sp.wm1, H, W, N,
+                                                             reinterpret_cast<float2*>(GA(h, sp.w)), tw_);
+    CK(cudaGetLastError());
+    h->launches += 5;
+    if (dx || gin) {
+        spec_mix_adj_kernel<<<blocks_for(tx, 256), 256, 0, st>>>(Bc, reinterpret_cast<const float2*>(AF(h, sp.w)), Cin, Cout, m1, m2,
+                                                                 sp.wm2, sp.wm1, H, W, A, tx);
+        CK(cudaGetLastError());
+        const long long ta = N * Cin * H * m2;
+        spec_idft_h_kernel<<<blocks_for(ta, 256), 256, 0, st>>>(A, H, m1, m2, twH, Dd, ta);
+        CK(cudaGetLastError());
+        const long long to = N * Cin * H * W;
+        if (gin) spec_in_bwd_kernel<TA, true><<<blocks_for(to, 256), 256, 0, st>>>(Dd, g, AF(h, sp.w0), Cin, Cout, H, W, m2, twW, nullptr, gin, to);
+        else spec_in_bwd_kernel<TA, false><<<blocks_for(to, 256), 256, 0, st>>>(Dd, g, AF(h, sp.w0), Cin, Cout, H, W, m2, twW, dx, nullptr, to);
+        CK(cudaGetLastError());
+        h->launches += 3;
+    }
+    // 1x1 conv: dw0 = g^T x, db = colsum(g)
+    if (x.mode == 1 && g.mode == 1 && Cin % 64 == 0 && Cout % 64 == 0) {
+        wgrad<TA>(h, reinterpret_cast<const TA*>(g.p), Cout, reinterpret_cast<const TA*>(x.p), Cin, GA(h, sp.w0), N * H * W, Cout, Cin, st,
+                  GA(h, sp.b0));
+    } else {
+        spec_w0_grad_kernel<TA><<<Cout * (Cin + 1), 256, 0, st>>>(g, x, Cin, Cout, H, W, N, GA(h, sp.w0), GA(h, sp.b0));
         CK(cudaGetLastError());
         h->launches++;
-        return;
-    }
-    if (bigk) {
-        const __nv_bfloat16* wbh = reinterpret_cast<const __nv_bfloat16*>(wb);
-        if (out_f32) {
-            REQUIRE(epi == EPI_BIAS, "the split-K path writes plain fp32 outputs");
-            gemm_bigk_f32(h, wbh, K, w_off, reinterpret_cast<float*>(out), (int)rows, Cout, K, ep.bias, st);
-        } else {
-            // 8x8 stages (K = 2048): accumulate in the fp32 scratch of tante_reserve, then bias-free activation + conversion
-            REQUIRE(epi == EPI_BIAS || epi == EPI_BIAS_GELU_ERF, "split-K conv: epilogue not covered");
-            REQUIRE((size_t)rows * Cout * 4 <= h->kscratch.bytes, "split-K conv: scratch not reserved");
-            float* v = reinterpret_cast<float*>(h->kscratch.p);
-            gemm_bigk_f32(h, wbh, K, w_off, v, (int)rows, Cout, K, ep.bias, st);
-            const long long n4 = rows * Cout / 4;
-            if (epi == EPI_BIAS_GELU_ERF) f32_to_ta_kernel<TA, true><<<blocks_for(n4, 256), 256, 0, st>>>(v, reinterpret_cast<TA*>(out), n4);
-            else f32_to_ta_kernel<TA, false><<<blocks_for(n4, 256), 256, 0, st>>>(v, reinterpret_cast<TA*>(out), n4);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
-    } else {
-        gemm<TA>(h, epi, wb, K, w_off, out, Cout, out_f32, (int)rows, Cout, K, ep, st);
     }
 }
 
@@ -1211,9 +1469,7 @@ void run_encoder_fno(tante_handle_s* h, const StepIO& io, int B, cudaStream_t st
     spectral_act<TA>(h, h->fes1, v0, NI, H, W, 0, g0pre, g0, st);
     // enc_conv_1 + GELU (:260-261)
     EpiParams e1; e1.bias = AF(h, h->enc_b[0]);
-    conv_cl_gemm<TA>(h, g1pre ? EPI_BIAS : EPI_BIAS_GELU_ERF, g0, H, W, C8, p0, h->enc_w[0], g1pre ? g1pre : g1, C1, false, NI, e1,
-                     st, h->st[0]);
-    if (g1pre) launch_act_fwd<TA, ACT_GELU_ERF>(h, g1pre, g1, NI * H1 * W1 * C1, st);
+    conv_cl_gemm<TA>(h, EPI_BIAS_GELU_ERF, g0, H, W, C8, p0, h->enc_w[0], e1, g1pre, g1, C1, NI, st, h->st[0]);
     // enc_spectral_2 + GELU (:263-264)
     SpecView v1{g1, 1, nullptr, 1};
     spectral_act<TA>(h, h->fes2, v1, NI, H1, W1, 1, g2pre, g2, st);
@@ -1222,12 +1478,34 @@ void run_encoder_fno(tante_handle_s* h, const StepIO& io, int B, cudaStream_t st
     if (!tp && !(sizeof(TA) == 2 && p1 * p1 * C2 > 1024) && h->st[1] == p1) {      // the embed epilogue writes x directly
         e2.film = AF(h, h->film_t_off); e2.s_emb = AF(h, h->s_emb); e2.t_emb = AF(h, h->t_emb);
         e2.T = T; e2.L = L; e2.ldr = C;
-        conv_cl_gemm<TA>(h, EPI_EMBED, g2, H1, W1, C2, p1, h->enc_w[1], x, C, true, NI, e2, st);
+        conv_cl_gemm<TA>(h, EPI_EMBED, g2, H1, W1, C2, p1, h->enc_w[1], e2, nullptr, x, C, NI, st);
         return;
     }
     // (training, split-K or pooled: fp32 pre-embedding, then the embed pass)
-    conv_cl_gemm<TA>(h, EPI_BIAS, g2, H1, W1, C2, p1, h->enc_w[1], v, C, true, NI, e2, st, h->st[1]);
+    conv_cl_gemm<TA>(h, EPI_BIAS, g2, H1, W1, C2, p1, h->enc_w[1], e2, nullptr, v, C, NI, st, h->st[1]);
     launch_embed(h, v, x, tokens, st);
+}
+
+// backward of run_encoder_fno from gv, the gradient of the fp32 pre-embedding
+template <typename TA>
+void run_encoder_fno_bwd(tante_handle_s* h, Tape& tp, const BackwardIO& io, const TA* gv, cudaStream_t st) {
+    const int C = h->C, C1 = h->C1, C2 = h->C2, C8 = h->C / 8, T = h->T;
+    const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0;
+    const long long NI = (long long)tp.B_used * T;
+    TA* gr0 = TP<TA>(h->fgr0);
+    TA* gr1 = TP<TA>(h->fgr1);
+    TA* gr2 = TP<TA>(h->fgr2);
+    // enc_conv_2 (p1): windows of the kept C/2 grid
+    conv_cl_gemm_bwd<TA>(h, 1, gv, TP<TA>(tp.a2act), TP<TA>(tp.a2pre), gr2, H1, W1, C2, p1, h->st[1], C, NI, st);
+    // enc_spectral_2
+    SpecView xs1{tp.a1act.p, 1, nullptr, 1}, gs1{gr2, 1, nullptr, 1};
+    run_spectral_bwd<TA>(h, h->fes2, xs1, gs1, NI, H1, W1, 1, gr1, nullptr, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, gr1, TP<TA>(tp.a1pre), NI * H1 * W1 * C1, st);
+    // enc_conv_1 (p0): windows of the kept C/8 grid
+    conv_cl_gemm_bwd<TA>(h, 0, gr1, TP<TA>(tp.f0act), TP<TA>(tp.f0pre), gr0, H, W, C8, p0, h->st[0], C1, NI, st);
+    // enc_spectral_1 on the input frames (input gradient accumulated on top of the u0 path)
+    SpecView xs0{io.input, 0, nullptr, T}, gs0{gr0, 1, nullptr, 1};
+    run_spectral_bwd<TA>(h, h->fes1, xs0, gs0, NI, H, W, 0, nullptr, io.grad_input, st);
 }
 
 // dec_FNO.forward (enc_dec_fno.py:303-323) of order o on the last-frame latent dmod [B*L][C] -> dfield[o] (B, D, H, W); the
@@ -1264,6 +1542,29 @@ void run_decoder_fno(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape*
     run_spectral<TA>(h, op.fs2, v0, B, H, W, 0, false, nullptr, field, st);
 }
 
+// backward of run_decoder_fno of order o: the gradient of its derivative field (dfield) -> the gradient of dmod in h->hd
+template <typename TA>
+void run_decoder_fno_bwd(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape& ot, cudaStream_t st) {
+    const OrderPlan& op = h->orders[o];
+    const int C = h->C, C1 = h->C1, C2 = h->C2, C8 = h->C / 8, D = h->D;
+    const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0;
+    TA* gr0 = TP<TA>(h->fgr0);
+    TA* gr1 = TP<TA>(h->fgr1);
+    TA* gr2 = TP<TA>(h->fgr2);
+    const float* gf = FP(h->dfield) + (size_t)o * B * D * H * W;
+    // dec_spectral_2 (field output, no activation)
+    SpecView xg0{ot.f0act.p, 1, nullptr, 1}, gv0{gf, 0, nullptr, 1};
+    run_spectral_bwd<TA>(h, op.fs2, xg0, gv0, B, H, W, 0, gr0, nullptr, st);
+    // dec_conv_2 (p0)
+    deconv_stage_bwd<TA>(h, op, 1, gr0, TP<TA>(ot.f0pre), TP<TA>(ot.z2act), gr1, B, H1, W1, C1, C8, p0, h->st[0], st);
+    // dec_spectral_1
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, gr1, TP<TA>(ot.z2pre), (long long)B * H1 * W1 * C1, st);
+    SpecView xg1{ot.z1act.p, 1, nullptr, 1}, gv1{gr1, 1, nullptr, 1};
+    run_spectral_bwd<TA>(h, op.fs1, xg1, gv1, B, H1, W1, 1, gr2, nullptr, st);
+    // dec_conv_1 (p1)
+    deconv_stage_bwd<TA>(h, op, 0, gr2, TP<TA>(ot.z1pre), dmod, TP<TA>(h->hd), B, h->Hp, h->Wp, C, C2, p1, h->st[1], st);
+}
+
 void launch_emit_wide(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, cudaStream_t st) {
     EmitParams ep{};
     ep.dfield = reinterpret_cast<const float*>(h->dfield.p);
@@ -1275,6 +1576,22 @@ void launch_emit_wide(tante_handle_s* h, const StepIO& io, int B, const RolloutS
     ep.B = B; ep.D = h->D; ep.T = h->T; ep.HW = (long long)h->cfg.H * h->cfg.W;
     REQUIRE(ep.HW % 4 == 0, "H * W must be a multiple of 4");
     taylor_emit_kernel<<<dim3(blocks_for(ep.HW / 4, 256), (unsigned)h->D, (unsigned)B), 256, 0, st>>>(ep);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+// backward of launch_emit_wide (field level): the gradient of every order's derivative field (dfield) and of u0, from the frame
+// gradients
+void launch_emit_wide_bwd(tante_handle_s* h, Tape& tp, const BackwardIO& io, cudaStream_t st) {
+    REQUIRE(!io.gin.cur, "windowed BPTT is not available at patch_scale >= 16");
+    const int T = h->T, D = h->D, B = tp.B_used;
+    EmitBwdParams ep{};
+    ep.gframes = io.gframes; ep.gf_bs = io.gf_bs;
+    ep.n_arr = reinterpret_cast<const int*>(tp.n_arr.p); ep.n_g = io.n_g;
+    ep.gfield = FP(h->dfield);
+    ep.gu0 = io.grad_input ? io.grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
+    ep.gu0_bs = (long long)T * D * h->cfg.H * h->cfg.W;
+    ep.K = h->K; ep.fi = h->cfg.frame_interval; ep.B = B; ep.D = D; ep.HW = (long long)h->cfg.H * h->cfg.W;
+    taylor_emit_bwd_kernel<<<dim3(blocks_for(ep.HW / 4, 256), (unsigned)D, (unsigned)B), 256, 0, st>>>(ep);
     CK(cudaGetLastError());
     h->launches++;
 }
@@ -1358,13 +1675,87 @@ void run_encoder_cnn(tante_handle_s* h, const StepIO& io, int B, const RolloutSt
     }
 }
 
+// backward of run_encoder_cnn from gv, the gradient of the fp32 pre-embedding
+template <typename TA>
+void run_encoder_cnn_bwd(tante_handle_s* h, Tape& tp, const BackwardIO& io, const TA* gv, cudaStream_t st) {
+    const int C = h->C, C1 = h->C1, C2 = h->C2;
+    const PatchGeom& g = h->geom;
+    const int tokens = tp.B_used * h->T * h->L;
+    const int K3 = g.k2 * g.k2 * C2, K2 = g.k1 * g.k1 * C1, M2 = tokens * g.R2, NO = g.k0 * g.k0 * h->D;
+    const long long rows_in = (long long)tokens * g.R1;
+    TA* ga2 = TP<TA>(h->gq);
+    TA* ga1 = TP<TA>(h->ga1);
+    wgrad<TA>(h, gv, C, TP<TA>(tp.a2act), K3, GA(h, h->enc_w[2]), tokens, C, K3, st, GA(h, h->enc_b[2]));
+    gemm_dx<TA>(h, gv, C, h->enc_wT[2], ga2, K3, tokens, K3, C, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, ga2, TP<TA>(tp.a2pre), (long long)tokens * K3, st);
+    wgrad<TA>(h, ga2, C2, TP<TA>(tp.a1act), K2, GA(h, h->enc_w[1]), M2, C2, K2, st, GA(h, h->enc_b[1]));
+    gemm_dx<TA>(h, ga2, C2, h->enc_wT[1], ga1, K2, M2, K2, C2, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, ga1, TP<TA>(tp.a1pre), (long long)M2 * K2, st);
+    // the patches were kept by the forward (tape im2col)
+    wgrad_pad<TA>(h, ga1, C1, C1, TP<TA>(tp.cols), kHeadPad, kHeadPad, GA(h, h->enc_w[0]), NO, NO, rows_in, st, GA(h, h->enc_b[0]));
+    if (io.grad_input || io.gin.cur) {
+        // dpatch[rows, 64 (K1 padded)] = da1[rows, C1] * W1[C1][K1]  (thin GEMM), then scatter-add into the pixels
+        REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv backward GEMM");
+        TA* cols = TP<TA>(h->cols);
+        gemm_dx<TA>(h, ga1, C1, h->enc_wT[0], cols, kHeadPad, (int)rows_in, kHeadPad, C1, st);
+        float* gbase = io.grad_input ? io.grad_input : io.gpred;
+        if (g.k0 * g.k1 * g.k2 >= 4) conv1_col2im_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, io.gin);
+        else conv1_col2im_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, io.gin);
+        CK(cudaGetLastError());
+        h->launches++;
+    }
+}
+
+// dec_CNN stages 1 and 2 of order o on the (modified) last-frame latent dmod [B*L][C] -> the stage-2 activations the fused Taylor
+// head reads (shared scratch in inference, the tape of the order `ot` in training)
+template <typename TA>
+void run_decoder_cnn(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape* ot, cudaStream_t st) {
+    const OrderPlan& op = h->orders[o];
+    const int C = h->C, C1 = h->C1, C2 = h->C2, L = h->L;
+    const PatchGeom& g = h->geom;
+    TA* z1 = ot ? TP<TA>(ot->z1act) : TP<TA>(h->z1);
+    TA* z2 = ot ? TP<TA>(ot->z2act) : TP<TA>(h->z2[o]);
+    TA* z1pre = ot ? TP<TA>(ot->z1pre) : nullptr;
+    TA* z2pre = ot ? TP<TA>(ot->z2pre) : nullptr;
+    EpiParams ed; ed.bias = AF(h, op.decb[0]);
+    gemm_act<TA, ACT_GELU_ERF>(h, dmod, C, op.decw[0], z1pre, z1, B * L, g.k2 * g.k2 * C2, C, ed, st);
+    ed.bias = AF(h, op.decb[1]);
+    gemm_act<TA, ACT_GELU_ERF>(h, z1, C2, op.decw[1], z2pre, z2, B * L * g.R2, g.k1 * g.k1 * C1, C2, ed, st);
+}
+
+// backward of dec_CNN of order o, stage 3 (the head's contraction) included: the head gradient G of the order -> the gradient of
+// dmod in h->hd
+template <typename TA>
+void run_decoder_cnn_bwd(tante_handle_s* h, int o, const TA* dmod, int B, OrderTape& ot, cudaStream_t st) {
+    const OrderPlan& op = h->orders[o];
+    const int C = h->C, C1 = h->C1, C2 = h->C2, BL = B * h->L;
+    const PatchGeom& g = h->geom;
+    const long long rows1 = (long long)BL * g.R1;       // stage-1 rows of the last frame (head)
+    const int M2 = BL * g.R2, N2 = g.k1 * g.k1 * C1, N1 = g.k2 * g.k2 * C2, NO = g.k0 * g.k0 * h->D;
+    TA* G = TP<TA>(h->hG) + (size_t)o * rows1 * kHeadPad;
+    TA* dz = TP<TA>(h->hz) + (size_t)o * rows1 * C1;
+    TA* dz1 = TP<TA>(h->hz1);
+    // dec_conv_3: d_k = z2act * W3 + b3  ->  dW3 = z2act^T G, db3 = colsum(G), dz2 = (G W3^T) o gelu'(z2pre)
+    wgrad_pad<TA>(h, TP<TA>(ot.z2act), C1, C1, G, kHeadPad, kHeadPad, GA(h, op.decw[2]), NO, NO, rows1, st);
+    launch_colsum<TA>(h, G, kHeadPad, rows1, NO, GA(h, op.decb[2]), st);
+    gemm_dx<TA>(h, G, kHeadPad, op.w3pad, dz, C1, (int)rows1, C1, kHeadPad, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, dz, TP<TA>(ot.z2pre), rows1 * C1, st);
+    // dec_conv_2: z2pre[M2, N2] = z1act[M2, C2] * Wd2^T + b
+    wgrad<TA>(h, dz, N2, TP<TA>(ot.z1act), C2, GA(h, op.decw[1]), M2, N2, C2, st, GA(h, op.decb[1]));
+    gemm_dx<TA>(h, dz, N2, op.decwT[1], dz1, C2, M2, C2, N2, st);
+    launch_act_bwd<TA, ACT_GELU_ERF>(h, dz1, TP<TA>(ot.z1pre), (long long)M2 * C2, st);
+    // dec_conv_1: z1pre[BL, N1] = dmod[BL, C] * Wd1^T + b
+    wgrad<TA>(h, dz1, N1, dmod, C, GA(h, op.decw[0]), BL, N1, C, st, GA(h, op.decb[0]));
+    gemm_dx<TA>(h, dz1, N1, op.decwT[0], TP<TA>(h->hd), C, BL, C, N1, st);
+}
+
 // One TANTE step (reference models/tante.py:125-176) as a launch sequence on `st`: tante_forward, the rollout (eager and the
 // captured step body) and, with io.tape set, the taped training calls.  Inference works in place on h->x and the shared
 // scratch buffers; a taped call runs the same kernels out of place into the tape slots, so that every input of a later
 // derivative survives, and keeps the GELU pre-activations next to the activations.
 template <typename TA>
 void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs, cudaStream_t st) {
-    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L, K = h->K, Hm = h->Hm;
+    const int C = h->C, T = h->T, L = h->L, K = h->K, Hm = h->Hm;
     const int tokens = B * T * L;
     Tape* tp = io.tape;
     DropCfg drop;      // inference: none
@@ -1498,17 +1889,9 @@ void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs
             h->launches++;
         }
         // --- decoder of order o: the fields of the Horner emit, or the stage-1 activations the fused Taylor head reads ---
-        if (h->fno) { run_decoder_fno<TA>(h, o, dmod, B, ot, st); continue; }
-        if (h->wide) { run_decoder_wide<TA>(h, o, dmod, B, ot, st); continue; }
-        const PatchGeom& g = h->geom;
-        TA* z1 = ot ? TP<TA>(ot->z1act) : TP<TA>(h->z1);
-        TA* z2 = ot ? TP<TA>(ot->z2act) : TP<TA>(h->z2[o]);
-        TA* z1pre = ot ? TP<TA>(ot->z1pre) : nullptr;
-        TA* z2pre = ot ? TP<TA>(ot->z2pre) : nullptr;
-        EpiParams ed; ed.bias = AF(h, op.decb[0]);
-        gemm_act<TA, ACT_GELU_ERF>(h, dmod, C, op.decw[0], z1pre, z1, B * L, g.k2 * g.k2 * C2, C, ed, st);
-        ed.bias = AF(h, op.decb[1]);
-        gemm_act<TA, ACT_GELU_ERF>(h, z1, C2, op.decw[1], z2pre, z2, B * L * g.R2, g.k1 * g.k1 * C1, C2, ed, st);
+        if (h->fno) run_decoder_fno<TA>(h, o, dmod, B, ot, st);
+        else if (h->wide) run_decoder_wide<TA>(h, o, dmod, B, ot, st);
+        else run_decoder_cnn<TA>(h, o, dmod, B, ot, st);
     }
     // --- step-size selection + fused Taylor head / Horner emit (tante.py:156-171) ---
     select_step_kernel<<<(B + 127) / 128, 128, 0, st>>>(rt, K, h->max_batch, B, h->cfg.deg, h->cfg.output_length,
@@ -1539,134 +1922,6 @@ void run_step(tante_handle_s* h, const StepIO& io, int B, const RolloutState& rs
 // Training: forward with an activation tape + full backward (what torch autograd does for the reference:
 // trainer/r_trainer.py:145-155, trainer/trainer.py:178-193).
 // ================================================================================================
-template <typename TA, int ACT>
-void launch_act_bwd(tante_handle_s* h, TA* g, const TA* pre, long long n, cudaStream_t st) {
-    act_bwd_kernel<TA, ACT><<<blocks_for(n / 4, 256), 256, 0, st>>>(g, pre, n / 4);
-    CK(cudaGetLastError());
-    h->launches++;
-}
-template <typename TA>
-void launch_colsum(tante_handle_s* h, const TA* x, int ld, long long M, int N, float* out, cudaStream_t st) {
-    const unsigned gx = (unsigned)((N + 127) / 128);
-    unsigned gy = (unsigned)std::max<long long>(1, std::min<long long>((M + 255) / 256, (4LL * h->num_sms + gx - 1) / gx));
-    colsum_kernel<TA><<<dim3(gx, gy), 256, 0, st>>>(x, ld, M, N, out);
-    CK(cudaGetLastError());
-    h->launches++;
-}
-// dW[N][K] (+)= A[M][N]^T B[M][K] into the gradient arena
-// `bias_out` (nullable): also db[N] += column sums of A (fused into the tensor-core kernel, else a colsum launch)
-template <typename TA>
-void wgrad(tante_handle_s* h, const TA* A, int lda, const TA* Bm, int ldb, float* out, long long M, int N, int K,
-           cudaStream_t st, float* bias_out = nullptr) {
-    {
-        ProfScope ps(h, st, 2.0 * (double)M * N * K, 2, (double)M * (N + K) * sizeof(TA));
-        if constexpr (sizeof(TA) == 2) {
-            if (wgrad_tc_supported(M, N, K, K, lda, ldb, K)) {
-                CK(launch_wgrad_tc(A, lda, Bm, ldb, out, K, M, N, K, K, h->num_sms, st, bias_out));
-                h->launches++;
-                return;
-            }
-        }
-        CK((launch_wgrad_simt<TA, TA>(A, lda, Bm, ldb, out, K, M, N, K, h->num_sms, st)));
-        h->launches++;
-    }
-    if (bias_out) launch_colsum<TA>(h, A, lda, M, N, bias_out, st);
-}
-// same with a zero-padded B operand: B is stored [M][Kb] (Kb % 64 == 0), only the first Kc columns of dW are kept
-template <typename TA>
-void wgrad_pad(tante_handle_s* h, const TA* A, int lda, int N, const TA* Bm, int ldb, int Kb, float* out, int ldc, int Kc,
-               long long M, cudaStream_t st, float* bias_out = nullptr) {
-    {
-        ProfScope ps(h, st, 2.0 * (double)M * N * Kc, 2, (double)M * (N + Kb) * sizeof(TA));
-        if constexpr (sizeof(TA) == 2) {
-            if (wgrad_tc_supported(M, N, Kb, Kc, lda, ldb, ldc)) {
-                CK(launch_wgrad_tc(A, lda, Bm, ldb, out, ldc, M, N, Kb, Kc, h->num_sms, st, bias_out));
-                h->launches++;
-                return;
-            }
-        }
-        CK((launch_wgrad_simt<TA, TA>(A, lda, Bm, ldb, out, ldc, M, N, Kc, h->num_sms, st)));
-        h->launches++;
-    }
-    if (bias_out) launch_colsum<TA>(h, A, lda, M, N, bias_out, st);
-}
-// dX = dY * W via the transposed packed weight (no bias)
-template <typename TA>
-void gemm_dx(tante_handle_s* h, const TA* A, int lda, int64_t wT_off, TA* out, int ldc, int M, int N, int K, cudaStream_t st) {
-    EpiParams ep; ep.bias = AF(h, h->zero_off);
-    REQUIRE(N <= 8192, "input-gradient GEMM wider than the zero-bias vector");
-    if (sizeof(TA) == 2 && K > 1024) {
-        // the tcgen05 GEMM keeps a K <= 1024 weight slice resident (K = 2048: first deconv of patch_scale 64): two K halves
-        // accumulated through an fp32 scratch, then one conversion pass
-        REQUIRE(ldc == N, "input-gradient GEMM: K not covered");
-        if (h->kscratch.bytes < (size_t)M * N * 4) destroy_graphs(h);      // (a captured rollout may hold the old pointer)
-        dev_alloc(h, h->kscratch, (size_t)M * N * 4);      // (training only: never inside a stream capture)
-        float* v = FP(h->kscratch);
-        gemm_bigk_f32(h, reinterpret_cast<const __nv_bfloat16*>(A), lda, wT_off, v, M, N, K, AF(h, h->zero_off), st);
-        convert_kernel<TA><<<blocks_for((long long)M * N / 4, 256), 256, 0, st>>>(v, out, (long long)M * N / 4);
-        CK(cudaGetLastError());
-        h->launches++;
-        return;
-    }
-    gemm<TA>(h, EPI_BIAS, A, lda, wT_off, out, ldc, sizeof(TA) == 4, M, N, K, ep, st);
-}
-
-// Backward of one SpectralLayer (fno.cuh, "training"): x = the layer's saved input, g = the gradient of its output (after the
-// GELU backward).  Accumulates the gradients of weight / w0 / bias, and writes the input gradient to the channels-last grid
-// `dx` or accumulates it into the channels-first fp32 `gin` (first encoder layer); both null: parameters only.
-template <typename TA>
-void run_spectral_bwd(tante_handle_s* h, const SpecPlan& sp, const SpecView& x, const SpecView& g, long long N, int H, int W,
-                      int level, TA* dx, float* gin, cudaStream_t st) {
-    const int W0 = h->cfg.W, H0 = h->cfg.H, W1 = W0 / h->fp0;
-    const float2* tw = reinterpret_cast<const float2*>(h->ftw.p);
-    const float2* twW = level == 0 ? tw : tw + W0 + H0;
-    const float2* twH = level == 0 ? tw + W0 : tw + W0 + H0 + W1;
-    const int m1 = sp.wm1, m2 = sp.wm2, Cin = sp.Cin, Cout = sp.Cout;
-    float2* A = reinterpret_cast<float2*>(h->fA.p);
-    float2* Bc = reinterpret_cast<float2*>(h->fB.p);
-    float2* Cc = reinterpret_cast<float2*>(h->fC.p);
-    float2* Dd = reinterpret_cast<float2*>(h->fD.p);
-    // gY = dft_h(dft_w(g))  -> Bc
-    const long long rows_o = N * Cout * H, rows_i = N * Cin * H;
-    spec_dft_w_kernel<TA><<<blocks_for(rows_o, 4), 128, 0, st>>>(g, Cout, H, W, m2, twW, A, rows_o);
-    CK(cudaGetLastError());
-    const long long ty = N * Cout * 2 * m1 * m2, tx = N * Cin * 2 * m1 * m2;
-    spec_dft_h_kernel<<<blocks_for(ty, 256), 256, 0, st>>>(A, H, m1, m2, twH, Bc, ty);
-    CK(cudaGetLastError());
-    // X = dft_h(dft_w(x))  -> Cc (recomputed: two passes over the saved input)
-    spec_dft_w_kernel<TA><<<blocks_for(rows_i, 4), 128, 0, st>>>(x, Cin, H, W, m2, twW, A, rows_i);
-    CK(cudaGetLastError());
-    spec_dft_h_kernel<<<blocks_for(tx, 256), 256, 0, st>>>(A, H, m1, m2, twH, Cc, tx);
-    CK(cudaGetLastError());
-    const long long tw_ = (long long)Cin * Cout * m1 * m2;
-    spec_wt_grad_kernel<<<blocks_for(tw_, 256), 256, 0, st>>>(Cc, Bc, Cin, Cout, m1, m2, sp.wm2, sp.wm1, H, W, N,
-                                                             reinterpret_cast<float2*>(GA(h, sp.w)), tw_);
-    CK(cudaGetLastError());
-    h->launches += 5;
-    if (dx || gin) {
-        spec_mix_adj_kernel<<<blocks_for(tx, 256), 256, 0, st>>>(Bc, reinterpret_cast<const float2*>(AF(h, sp.w)), Cin, Cout, m1, m2,
-                                                                 sp.wm2, sp.wm1, H, W, A, tx);
-        CK(cudaGetLastError());
-        const long long ta = N * Cin * H * m2;
-        spec_idft_h_kernel<<<blocks_for(ta, 256), 256, 0, st>>>(A, H, m1, m2, twH, Dd, ta);
-        CK(cudaGetLastError());
-        const long long to = N * Cin * H * W;
-        if (gin) spec_in_bwd_kernel<TA, true><<<blocks_for(to, 256), 256, 0, st>>>(Dd, g, AF(h, sp.w0), Cin, Cout, H, W, m2, twW, nullptr, gin, to);
-        else spec_in_bwd_kernel<TA, false><<<blocks_for(to, 256), 256, 0, st>>>(Dd, g, AF(h, sp.w0), Cin, Cout, H, W, m2, twW, dx, nullptr, to);
-        CK(cudaGetLastError());
-        h->launches += 3;
-    }
-    // 1x1 conv: dw0 = g^T x, db = colsum(g)
-    if (x.mode == 1 && g.mode == 1 && Cin % 64 == 0 && Cout % 64 == 0) {
-        wgrad<TA>(h, reinterpret_cast<const TA*>(g.p), Cout, reinterpret_cast<const TA*>(x.p), Cin, GA(h, sp.w0), N * H * W, Cout, Cin, st,
-                  GA(h, sp.b0));
-    } else {
-        spec_w0_grad_kernel<TA><<<Cout * (Cin + 1), 256, 0, st>>>(g, x, Cin, Cout, H, W, N, GA(h, sp.w0), GA(h, sp.b0));
-        CK(cudaGetLastError());
-        h->launches++;
-    }
-}
-
 template <typename TA>
 void launch_ln_bwd(tante_handle_s* h, const TA* dy, const float* x, int64_t gamma, float* dxs, TA* dxb, float* dg, float* db,
                    long long rows, cudaStream_t st, const DropCfg& drop = DropCfg(), uint32_t site = 0, int width = 0) {
@@ -1888,7 +2143,6 @@ void backward_alloc(tante_handle_s* h, int B) {
     const size_t BL = (size_t)B * h->L;
     const int C = h->C, C1 = h->C1, C2 = h->C2;
     const PatchGeom& g = h->geom;
-    const int NO = g.k0 * g.k0 * h->D;
     dev_alloc(h, h->garena, (size_t)h->garena_elems * 4);
     dev_alloc(h, h->dxs, tokens * C * 4);
     dev_alloc(h, h->dxb, tokens * C * es);      // bf16 mirror of the gradient stream; in the exact mode: its dropout-masked copy
@@ -1896,7 +2150,6 @@ void backward_alloc(tante_handle_s* h, int B) {
     dev_alloc(h, h->g2, tokens * C * es);
     dev_alloc(h, h->gq, tokens * std::max(3 * C, g.R2 * C2) * es);
     dev_alloc(h, h->ga1, tokens * g.R1 * C1 * es);
-    (void)NO;
     dev_alloc(h, h->cols, tokens * g.R1 * kHeadPad * es);
     dev_alloc(h, h->hz, (size_t)h->K * BL * g.R1 * C1 * es);
     dev_alloc(h, h->hG, (size_t)h->K * BL * g.R1 * (size_t)std::max(kHeadPad, h->wide ? h->NOpad : 0) * es);
@@ -1947,12 +2200,6 @@ void backward_alloc(tante_handle_s* h, int B) {
     h->bw_batch = B;
 }
 
-// Backward of one taped step.  gframes: f32 (B, n_g, D, H, W) gradient of the emitted frames; gRt: f32 [B] or null;
-// grad_input: f32 (B, T, D, H, W) or null (written, not accumulated; but see `win`); flat: f32 [sum numel] parameter gradients in
-// tante_param order (written, not accumulated).
-// win (per-sample cursor mode, tante_backward_hist): gframes is win->gpred, the gradient of the whole prediction buffer (batch
-// stride win->gin.hbs), and the window gradient is ACCUMULATED into it and into grad_input (nullable) through win->gin, whose
-// offsets are relative to grad_input, or to gpred when there is no grad_input (gin.skip_in).
 // Backward of one axis-'C' layer (channel_axis.cuh): dxs [tokens][C] holds the gradient of the layer output on entry and of its
 // input on return (the layer REPLACES the latent: no residual around it).  Per chunk of h->chanb_tokens latent tokens the block is
 // recomputed from the saved fp32 input (lift, LN1, QKV, attention, out-proj, LN2, MLP -- everything the backward reads stays in
@@ -2035,194 +2282,123 @@ void run_channel_layer_bwd(tante_handle_s* h, const LayerPlan& lp, const float* 
     }
 }
 
-struct BackwardWin { FrameTab gin; float* gpred; };
+// backward of the head of order o in run_step (tante.py:147-154): FiLM modifier and interprator (adaptive model; the R_t clamp
+// is straight-through), then the gradient of the last-frame latent (h->hd) goes into the last frame of the gradient stream
 template <typename TA>
-void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* gframes, int n_g, const float* gRt,
-                  float* grad_input, float* flat, cudaStream_t st, const BackwardWin* win = nullptr) {
+void run_interprator_bwd(tante_handle_s* h, int o, Tape& tp, const float* gRt, cudaStream_t st) {
+    const OrderPlan& op = h->orders[o];
+    OrderTape& ot = tp.ord[o];
+    const int B = tp.B_used, C = h->C, T = h->T, L = h->L, BL = B * L;
+    TA* hd = TP<TA>(h->hd);
+    float* dxs = FP(h->dxs);
+    if (!h->cfg.deg) {
+        // FiLM modifier (tante.py:151) and interprator (tante.py:149)
+        CK(cudaMemsetAsync(h->dfilm.p, 0, (size_t)B * 2 * C * 4, st));
+        {
+            const int chunks = std::max(1, std::min(L, (2 * h->num_sms + B - 1) / B));
+            film_apply_bwd_kernel<TA><<<dim3(B, chunks), C, 0, st>>>(hd, FP(ot.d32), FP(ot.film), dxs, FP(h->dfilm), T, L, C);
+            CK(cudaGetLastError());
+            h->launches++;
+        }
+        CK(cudaMemsetAsync(h->dcond.p, 0, (size_t)B * 4, st));
+        film_bwd_kernel<<<dim3(B, 16), 256, 3 * C * sizeof(float), st>>>(
+            FP(ot.rt), FP(h->dfilm), AF(h, op.mod[0]), AF(h, op.mod[1]), AF(h, op.mod[2]), AF(h, op.mod[4]),
+            AF(h, op.mod[5]), AF(h, op.mod[6]), GA(h, op.mod[0]), GA(h, op.mod[1]), GA(h, op.mod[2]), GA(h, op.mod[3]),
+            GA(h, op.mod[4]), GA(h, op.mod[5]), GA(h, op.mod[6]), GA(h, op.mod[7]), C, FP(h->dcond));
+        CK(cudaGetLastError());
+        h->launches++;
+        TA* hi2 = TP<TA>(h->hi2);
+        TA* hi1 = TP<TA>(h->hi1);
+        interp_tail_bwd_kernel<TA><<<B, 256, (C / 4) * sizeof(float), st>>>(
+            TP<TA>(ot.i2), AF(h, op.intw[2]), gRt, 1.0f / (float)h->K, FP(h->dcond), L, C / 4, hi2, GA(h, op.intw[2]),
+            GA(h, op.intb[2]));
+        CK(cudaGetLastError());
+        h->launches++;
+        wgrad<TA>(h, hi2, C / 4, TP<TA>(ot.i1), C / 2, GA(h, op.intw[1]), BL, C / 4, C / 2, st, GA(h, op.intb[1]));
+        gemm_dx<TA>(h, hi2, C / 4, op.intwT[1], hi1, C / 2, BL, C / 2, C / 4, st);
+        launch_act_bwd<TA, ACT_RELU>(h, hi1, TP<TA>(ot.i1), (long long)BL * (C / 2), st);
+        wgrad<TA>(h, hi1, C / 2, TP<TA>(ot.dl), C, GA(h, op.intw[0]), BL, C / 2, C, st, GA(h, op.intb[0]));
+        gemm_dx<TA>(h, hi1, C / 2, op.intwT[0], hd, C, BL, C, C / 2, st);
+    }
+    add_last_frame_kernel<TA><<<blocks_for((long long)BL * C / 4, 256), 256, 0, st>>>(hd, dxs, B, T, (long long)L * C);
+    CK(cudaGetLastError());
+    h->launches++;
+}
+
+// backward of transformer layer li of order o (the layer loop of run_step): takes the gradient stream h->dxs from the layer output
+// to its input.  dxb: the dY operand of the residual-branch GEMMs (the TA / dropout-masked copy of the stream, or the fp32 stream
+// itself); dxb_out: where the LayerNorm backwards write that copy (null: no copy).
+template <typename TA>
+void run_layer_bwd(tante_handle_s* h, Tape& tp, int o, int li, const TA* dxb, TA* dxb_out, cudaStream_t st) {
+    const LayerPlan& lp = h->orders[o].layers[li];
+    OrderTape& ot = tp.ord[o];
+    const int C = h->C, Hm = h->Hm, tokens = tp.B_used * h->T * h->L;
+    const DropCfg& drop = tp.drop;
+    float* dxs = FP(h->dxs);
+    TA* g1 = TP<TA>(h->g1);
+    TA* g2 = TP<TA>(h->g2);
+    TA* gq = TP<TA>(h->gq);
+    const float* x_in = FP(ot.X[2 * li]);
+    const float* x_mid = FP(ot.X[2 * li + 1]);
+    // MLP half: x_out = x_mid + W2 gelu_tanh(W0 ln2(x_mid) + b0) + b2
+    wgrad<TA>(h, dxb, C, TP<TA>(ot.hact[li]), Hm, GA(h, lp.m2w), tokens, C, Hm, st, GA(h, lp.m2b));
+    if (sizeof(TA) == 2 && C == kBtC && Hm == C) {
+        // dpre = (dY W2) o gelu'(hpre) and dln2 = dpre W1 in one kernel (mlp_bwd_tc.cuh): dh never touches HBM
+        {
+            ProfScope ps(h, st, 2.0 * 2.0 * tokens * C * C, 4, (double)tokens * 4 * 2 * C);
+            CK(launch_mlp_bwd(reinterpret_cast<const __nv_bfloat16*>(dxb), AH(h, lp.m2wT), AH(h, lp.m0wT),
+                              reinterpret_cast<const __nv_bfloat16*>(ot.hpre[li].p), reinterpret_cast<__nv_bfloat16*>(g1),
+                              reinterpret_cast<__nv_bfloat16*>(g2), tokens, h->num_sms, st));
+        }
+        h->launches++;
+        wgrad<TA>(h, g1, C, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, C, C, st, GA(h, lp.m0b));
+    } else {
+        gemm_dx<TA>(h, dxb, C, lp.m2wT, g1, Hm, tokens, Hm, C, st);
+        launch_act_bwd<TA, ACT_GELU_TANH>(h, g1, TP<TA>(ot.hpre[li]), (long long)tokens * Hm, st);
+        wgrad<TA>(h, g1, Hm, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, Hm, C, st, GA(h, lp.m0b));
+        gemm_dx<TA>(h, g1, Hm, lp.m0wT, g2, C, tokens, C, Hm, st);
+    }
+    launch_ln_bwd<TA>(h, g2, x_mid, lp.ln2w, dxs, dxb_out, GA(h, lp.ln2w), GA(h, lp.ln2b), tokens, st, drop, drop_site(o, li, 1));
+    // attention half: x_mid = x_in + Wo att(ln1(x_in)) + bo
+    wgrad<TA>(h, dxb, C, TP<TA>(ot.att[li]), C, GA(h, lp.outw), tokens, C, C, st, GA(h, lp.outb));
+    gemm_dx<TA>(h, dxb, C, lp.outwT, g2, C, tokens, C, C, st);
+    launch_attention_bwd<TA>(h, TP<TA>(ot.qkv[li]), g2, gq, tp.B_used, lp.axis, st, drop, drop_site(o, li, 0));
+    wgrad<TA>(h, gq, 3 * C, TP<TA>(ot.ln1[li]), C, GA(h, lp.inw), tokens, 3 * C, C, st, GA(h, lp.inb));
+    gemm_dx<TA>(h, gq, 3 * C, lp.inwT, g2, C, tokens, C, 3 * C, st);
+    // the copy written here is the dY of the layer below's MLP branch
+    launch_ln_bwd<TA>(h, g2, x_in, lp.ln1w, dxs, dxb_out, GA(h, lp.ln1w), GA(h, lp.ln1b), tokens, st, drop,
+                      drop_site(o, std::max(li - 1, 0), 2));
+}
+
+// Backward of one taped step (see BackwardIO): run_step in reverse, stage by stage.
+template <typename TA>
+void run_backward(tante_handle_s* h, Tape& tp, const BackwardIO& io, cudaStream_t st) {
     const int B = tp.B_used;
-    const int C = h->C, C1 = h->C1, C2 = h->C2, T = h->T, L = h->L, K = h->K, D = h->D, Hm = h->Hm;
-    const PatchGeom& g = h->geom;
-    const int tokens = B * T * L;
-    const int BL = B * L;
-    const int NO = g.k0 * g.k0 * D;
-    constexpr bool kTensor = sizeof(TA) == 2;
-    const long long rows1 = (long long)BL * g.R1;       // stage-1 rows of the last frame (head)
+    const int C = h->C, T = h->T, K = h->K;
+    const int tokens = B * T * h->L;
     float* dxs = FP(h->dxs);
     const DropCfg& drop = tp.drop;
     // dY operand of the residual-branch GEMMs: the bf16 copy of the gradient stream (tensor mode) and / or its
     // dropout-masked copy; the exact mode without dropout reads the fp32 stream itself
-    const bool mirror = kTensor || drop.p > 0.f;
+    const bool mirror = sizeof(TA) == 2 || drop.p > 0.f;
     TA* dxb = mirror ? TP<TA>(h->dxb) : reinterpret_cast<TA*>(dxs);
-    TA* g1 = TP<TA>(h->g1);
-    TA* g2 = TP<TA>(h->g2);
-    TA* gq = TP<TA>(h->gq);
+    TA* dxb_out = mirror ? dxb : nullptr;
     CK(cudaMemsetAsync(h->garena.p, 0, (size_t)h->garena_elems * 4, st));
     CK(cudaMemsetAsync(dxs, 0, (size_t)tokens * C * 4, st));
-    const size_t in_elems = (size_t)B * T * D * h->cfg.H * h->cfg.W;
-    if (grad_input && !win) CK(cudaMemsetAsync(grad_input, 0, in_elems * 4, st));
+    if (io.grad_input && !io.gin.cur) CK(cudaMemsetAsync(io.grad_input, 0, (size_t)B * T * h->D * h->cfg.H * h->cfg.W * 4, st));
 
-    // ---- Taylor head: all orders in one pass over the frame gradients ----
-    if (h->wide) {
-        // field-level emit (boundary C): gradient of every order's derivative field + of u0, from the frame gradients
-        REQUIRE(!win, "windowed BPTT is not available at patch_scale >= 16");
-        EmitBwdParams ep{};
-        ep.gframes = gframes; ep.gf_bs = (long long)n_g * D * h->cfg.H * h->cfg.W;
-        ep.n_arr = reinterpret_cast<const int*>(tp.n_arr.p); ep.n_g = n_g;
-        ep.gfield = FP(h->dfield);
-        ep.gu0 = grad_input ? grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
-        ep.gu0_bs = (long long)T * D * h->cfg.H * h->cfg.W;
-        ep.K = K; ep.fi = h->cfg.frame_interval; ep.B = B; ep.D = D; ep.HW = (long long)h->cfg.H * h->cfg.W;
-        taylor_emit_bwd_kernel<<<dim3(blocks_for(ep.HW / 4, 256), (unsigned)D, (unsigned)B), 256, 0, st>>>(ep);
-        CK(cudaGetLastError());
-        h->launches++;
-    } else {
-        HeadBwdParams hp{};
-        for (int k = 0; k < K; ++k) hp.G[k] = TP<TA>(h->hG) + (size_t)k * rows1 * kHeadPad;
-        hp.K = K; hp.fi = h->cfg.frame_interval; hp.gframes = gframes; hp.n_cap = n_g;
-        hp.gf_bs = win ? win->gin.hbs : (long long)n_g * D * h->cfg.H * h->cfg.W;
-        hp.n_arr = reinterpret_cast<const int*>(tp.n_arr.p);
-        hp.gi_last = grad_input ? grad_input + (size_t)(T - 1) * D * h->cfg.H * h->cfg.W : nullptr;
-        hp.gi_bs = (long long)T * D * h->cfg.H * h->cfg.W;
-        if (win) { hp.cur = win->gin.cur; hp.gpred = win->gpred; }
-        const size_t hsmem = (size_t)K * kPatchRows * kPatchPitch * sizeof(float);
-        if (g.k0 * g.k1 * g.k2 >= 4) head_gather_kernel<TA, 4><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
-        else head_gather_kernel<TA, 2><<<blocks_for(rows1, kPatchRows), 128, hsmem, st>>>(hp, g, rows1);
-        CK(cudaGetLastError());
-        h->launches++;
-    }
+    // ---- Taylor head / Horner emit: all orders in one pass over the frame gradients ----
+    if (h->wide) launch_emit_wide_bwd(h, tp, io, st);
+    else launch_head_bwd<TA>(h, tp, io, st);
     for (int o = K - 1; o >= 0; --o) {
         const OrderPlan& op = h->orders[o];
         OrderTape& ot = tp.ord[o];
-        TA* dz = TP<TA>(h->hz) + (size_t)o * rows1 * C1;
-        const int M2 = BL * g.R2, N2 = g.k1 * g.k1 * C1;
-        const int N1 = g.k2 * g.k2 * C2;
-        TA* dz1 = TP<TA>(h->hz1);
-        TA* dmod = h->cfg.deg ? TP<TA>(ot.dl) : TP<TA>(ot.dmod);
-        TA* hd = TP<TA>(h->hd);
-        if (h->fno) {
-            TA* wb = TP<TA>(h->wbuf);
-            const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0, C8 = C / 8;
-            const int NF1 = p1 * p1 * C2, NF2 = p0 * p0 * C8;
-            TA* gr0 = TP<TA>(h->fgr0);
-            TA* gr1 = TP<TA>(h->fgr1);
-            TA* gr2 = TP<TA>(h->fgr2);
-            const float* gf = FP(h->dfield) + (size_t)o * B * D * H * W;
-            // dec_spectral_2 (field output, no activation)
-            SpecView xg0{ot.f0act.p, 1, nullptr, 1}, gv0{gf, 0, nullptr, 1};
-            run_spectral_bwd<TA>(h, op.fs2, xg0, gv0, B, H, W, 0, gr0, nullptr, st);
-            launch_act_bwd<TA, ACT_GELU_ERF>(h, gr0, TP<TA>(ot.f0pre), (long long)B * H * W * C8, st);
-            // dec_conv_2 (p0)
-            const long long MF2 = (long long)B * H1 * W1;
-            const bool ovf1 = h->st[1] != p1, ovf0 = h->st[0] != p0;      // overlapped stage: bias gradient = sum of the stage-output gradient
-            if (ovf0) launch_colsum<TA>(h, gr0, C8, (long long)B * H * W, C8, GA(h, op.decb[1]), st);
-            long long tot = MF2 * NF2;
-            wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(gr0, nullptr, NF2, H1, W1, C8, p0, wb, tot, h->st[0]);
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad<TA>(h, wb, NF2, TP<TA>(ot.z2act), C1, GA(h, op.decw[1]), MF2, NF2, C1, st, ovf0 ? nullptr : GA(h, op.decb[1]));
-            gemm_dx<TA>(h, wb, NF2, op.decwT[1], gr1, C1, (int)MF2, C1, NF2, st);
-            launch_act_bwd<TA, ACT_GELU_ERF>(h, gr1, TP<TA>(ot.z2pre), MF2 * C1, st);
-            // dec_spectral_1
-            SpecView xg1{ot.z1act.p, 1, nullptr, 1}, gv1{gr1, 1, nullptr, 1};
-            run_spectral_bwd<TA>(h, op.fs1, xg1, gv1, B, H1, W1, 1, gr2, nullptr, st);
-            launch_act_bwd<TA, ACT_GELU_ERF>(h, gr2, TP<TA>(ot.z1pre), MF2 * C2, st);
-            // dec_conv_1 (p1)
-            if (ovf1) launch_colsum<TA>(h, gr2, C2, MF2, C2, GA(h, op.decb[0]), st);
-            tot = (long long)BL * NF1;
-            wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(gr2, nullptr, NF1, h->Hp, h->Wp, C2, p1, wb, tot, h->st[1]);
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad<TA>(h, wb, NF1, dmod, C, GA(h, op.decw[0]), BL, NF1, C, st, ovf1 ? nullptr : GA(h, op.decb[0]));
-            gemm_dx<TA>(h, wb, NF1, op.decwT[0], hd, C, BL, C, NF1, st);
-        } else if (h->wide) {
-            // natural-order stages (wide_patch.cuh): transpose of (crop + bilinear resample) back to the sub-pixel matrix, then the
-            // same weight / input gradient GEMMs as below, stage by stage
-            TA* wb = TP<TA>(h->wbuf);
-            TA* G = TP<TA>(h->hG);                                   // dS3 [rows1][NOpad]
-            const int NP = h->NOpad;
-            const int Hp = h->Hp, Wp = h->Wp;
-            const int H2 = Hp * g.k2, W2 = Wp * g.k2, H1 = H2 * g.k1, W1 = W2 * g.k1;
-            const float* gf = FP(h->dfield) + (size_t)o * B * D * h->cfg.H * h->cfg.W;
-            // bias gradients: without overlap the replicated bias rode in the GEMM (column sums of dS, folded at unpack); an overlapped
-            // stage added bias[co] once per output sample, so its gradient is the sum of the OUTPUT gradient (into the first Cout entries)
-            const bool ov0 = h->st[0] != g.k0, ov1 = h->st[2] != g.k2, ov2 = h->st[1] != g.k1;
-            long long tot = rows1 * NP;
-            wide_deconv_post_bwd_kernel<TA, true><<<blocks_for(tot, 256), 256, 0, st>>>(nullptr, gf, NP, H1, W1, D, g.k0, G, tot, h->st[0]);
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad_pad<TA>(h, TP<TA>(ot.z2act), C1, C1, G, NP, NP, GA(h, op.decw[2]), NO, NO, rows1, st);
-            if (ov0) {
-                const long long HWp = (long long)h->cfg.H * h->cfg.W;
-                field_bias_grad_kernel<<<dim3((unsigned)D, 32), 256, 0, st>>>(gf, D, HWp, B, GA(h, op.decb[2]));
-                CK(cudaGetLastError());
-                h->launches++;
-            } else {
-                launch_colsum<TA>(h, G, NP, rows1, NO, GA(h, op.decb[2]), st);
-            }
-            gemm_dx<TA>(h, G, NP, op.w3pad, dz, C1, (int)rows1, C1, NP, st);
-            launch_act_bwd<TA, ACT_GELU_ERF>(h, dz, TP<TA>(ot.z2pre), rows1 * C1, st);
-            if (ov2) launch_colsum<TA>(h, dz, C1, rows1, C1, GA(h, op.decb[1]), st);
-            tot = (long long)M2 * N2;
-            wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(dz, nullptr, N2, H2, W2, C1, g.k1, wb, tot, h->st[1]);
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad<TA>(h, wb, N2, TP<TA>(ot.z1act), C2, GA(h, op.decw[1]), M2, N2, C2, st, ov2 ? nullptr : GA(h, op.decb[1]));
-            gemm_dx<TA>(h, wb, N2, op.decwT[1], dz1, C2, M2, C2, N2, st);
-            launch_act_bwd<TA, ACT_GELU_ERF>(h, dz1, TP<TA>(ot.z1pre), (long long)M2 * C2, st);
-            if (ov1) launch_colsum<TA>(h, dz1, C2, M2, C2, GA(h, op.decb[0]), st);
-            tot = (long long)BL * N1;
-            wide_deconv_post_bwd_kernel<TA, false><<<blocks_for(tot, 256), 256, 0, st>>>(dz1, nullptr, N1, Hp, Wp, C2, g.k2, wb, tot, h->st[2]);
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad<TA>(h, wb, N1, dmod, C, GA(h, op.decw[0]), BL, N1, C, st, ov1 ? nullptr : GA(h, op.decb[0]));
-            gemm_dx<TA>(h, wb, N1, op.decwT[0], hd, C, BL, C, N1, st);
-        } else {
-        TA* G = TP<TA>(h->hG) + (size_t)o * rows1 * kHeadPad;
-        // dec_conv_3: d_k = z2act * W3 + b3  ->  dW3 = z2act^T G, db3 = colsum(G), dz2 = (G W3^T) o gelu'(z2pre)
-        wgrad_pad<TA>(h, TP<TA>(ot.z2act), C1, C1, G, kHeadPad, kHeadPad, GA(h, op.decw[2]), NO, NO, rows1, st);
-        launch_colsum<TA>(h, G, kHeadPad, rows1, NO, GA(h, op.decb[2]), st);
-        gemm_dx<TA>(h, G, kHeadPad, op.w3pad, dz, C1, (int)rows1, C1, kHeadPad, st);
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, dz, TP<TA>(ot.z2pre), rows1 * C1, st);
-        // dec_conv_2: z2pre[M2, N2] = z1act[M2, C2] * Wd2^T + b
-        wgrad<TA>(h, dz, N2, TP<TA>(ot.z1act), C2, GA(h, op.decw[1]), M2, N2, C2, st, GA(h, op.decb[1]));
-        gemm_dx<TA>(h, dz, N2, op.decwT[1], dz1, C2, M2, C2, N2, st);
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, dz1, TP<TA>(ot.z1pre), (long long)M2 * C2, st);
-        // dec_conv_1: z1pre[BL, N1] = dmod[BL, C] * Wd1^T + b
-        wgrad<TA>(h, dz1, N1, dmod, C, GA(h, op.decw[0]), BL, N1, C, st, GA(h, op.decb[0]));
-        gemm_dx<TA>(h, dz1, N1, op.decwT[0], hd, C, BL, C, N1, st);
-        }
-        if (!h->cfg.deg) {
-            // FiLM modifier (tante.py:151) and interprator (tante.py:149)
-            CK(cudaMemsetAsync(h->dfilm.p, 0, (size_t)B * 2 * C * 4, st));
-            {
-                const int chunks = std::max(1, std::min(L, (2 * h->num_sms + B - 1) / B));
-                film_apply_bwd_kernel<TA><<<dim3(B, chunks), C, 0, st>>>(hd, FP(ot.d32), FP(ot.film), dxs, FP(h->dfilm), T, L, C);
-                CK(cudaGetLastError());
-                h->launches++;
-            }
-            CK(cudaMemsetAsync(h->dcond.p, 0, (size_t)B * 4, st));
-            film_bwd_kernel<<<dim3(B, 16), 256, 3 * C * sizeof(float), st>>>(
-                FP(ot.rt), FP(h->dfilm), AF(h, op.mod[0]), AF(h, op.mod[1]), AF(h, op.mod[2]), AF(h, op.mod[4]),
-                AF(h, op.mod[5]), AF(h, op.mod[6]), GA(h, op.mod[0]), GA(h, op.mod[1]), GA(h, op.mod[2]), GA(h, op.mod[3]),
-                GA(h, op.mod[4]), GA(h, op.mod[5]), GA(h, op.mod[6]), GA(h, op.mod[7]), C, FP(h->dcond));
-            CK(cudaGetLastError());
-            h->launches++;
-            TA* hi2 = TP<TA>(h->hi2);
-            TA* hi1 = TP<TA>(h->hi1);
-            interp_tail_bwd_kernel<TA><<<B, 256, (C / 4) * sizeof(float), st>>>(
-                TP<TA>(ot.i2), AF(h, op.intw[2]), gRt, 1.0f / (float)K, FP(h->dcond), L, C / 4, hi2, GA(h, op.intw[2]),
-                GA(h, op.intb[2]));
-            CK(cudaGetLastError());
-            h->launches++;
-            wgrad<TA>(h, hi2, C / 4, TP<TA>(ot.i1), C / 2, GA(h, op.intw[1]), BL, C / 4, C / 2, st, GA(h, op.intb[1]));
-            gemm_dx<TA>(h, hi2, C / 4, op.intwT[1], hi1, C / 2, BL, C / 2, C / 4, st);
-            launch_act_bwd<TA, ACT_RELU>(h, hi1, TP<TA>(ot.i1), (long long)BL * (C / 2), st);
-            wgrad<TA>(h, hi1, C / 2, TP<TA>(ot.dl), C, GA(h, op.intw[0]), BL, C / 2, C, st, GA(h, op.intb[0]));
-            gemm_dx<TA>(h, hi1, C / 2, op.intwT[0], hd, C, BL, C, C / 2, st);
-        }
-        add_last_frame_kernel<TA><<<blocks_for((long long)BL * C / 4, 256), 256, 0, st>>>(hd, dxs, B, T, (long long)L * C);
-        CK(cudaGetLastError());
-        h->launches++;
+        // ---- decoder and head of order o ----
+        const TA* dmod = h->cfg.deg ? TP<TA>(ot.dl) : TP<TA>(ot.dmod);
+        if (h->fno) run_decoder_fno_bwd<TA>(h, o, dmod, B, ot, st);
+        else if (h->wide) run_decoder_wide_bwd<TA>(h, o, dmod, B, ot, st);
+        else run_decoder_cnn_bwd<TA>(h, o, dmod, B, ot, st);
+        run_interprator_bwd<TA>(h, o, tp, io.gRt, st);
         // ---- backbone of order o ----
         if (mirror) {
             convert_kernel<TA><<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(
@@ -2230,13 +2406,10 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
             CK(cudaGetLastError());
             h->launches++;
         }
-        TA* dxb_out = mirror ? dxb : nullptr;
         for (int li = (int)op.layers.size() - 1; li >= 0; --li) {
             const LayerPlan& lp = op.layers[li];
-            const float* x_in = FP(ot.X[2 * li]);
-            const float* x_mid = FP(ot.X[2 * li + 1]);
             if (lp.axis == 'C') {
-                run_channel_layer_bwd<TA>(h, lp, x_in, dxs, tokens, st);
+                run_channel_layer_bwd<TA>(h, lp, FP(ot.X[2 * li]), dxs, tokens, st);
                 if (mirror) {      // the layer below reads the TA mirror of the gradient stream as its dY
                     convert_kernel<TA><<<blocks_for((long long)tokens * C / 4, 256), 256, 0, st>>>(dxs, dxb, (long long)tokens * C / 4);
                     CK(cudaGetLastError());
@@ -2244,205 +2417,25 @@ void run_backward(tante_handle_s* h, Tape& tp, const float* input, const float* 
                 }
                 continue;
             }
-            // MLP half: x_out = x_mid + W2 gelu_tanh(W0 ln2(x_mid) + b0) + b2
-            wgrad<TA>(h, dxb, C, TP<TA>(ot.hact[li]), Hm, GA(h, lp.m2w), tokens, C, Hm, st, GA(h, lp.m2b));
-            if (kTensor && C == kBtC && h->Hm == C) {
-                // dpre = (dY W2) o gelu'(hpre) and dln2 = dpre W1 in one kernel (mlp_bwd_tc.cuh): dh never touches HBM
-                {
-                    ProfScope ps(h, st, 2.0 * 2.0 * tokens * C * C, 4, (double)tokens * 4 * 2 * C);
-                    CK(launch_mlp_bwd(reinterpret_cast<const __nv_bfloat16*>(dxb), AH(h, lp.m2wT), AH(h, lp.m0wT),
-                                      reinterpret_cast<const __nv_bfloat16*>(ot.hpre[li].p), reinterpret_cast<__nv_bfloat16*>(g1),
-                                      reinterpret_cast<__nv_bfloat16*>(g2), tokens, h->num_sms, st));
-                }
-                h->launches++;
-                wgrad<TA>(h, g1, C, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, C, C, st, GA(h, lp.m0b));
-            } else {
-                gemm_dx<TA>(h, dxb, C, lp.m2wT, g1, Hm, tokens, Hm, C, st);
-                launch_act_bwd<TA, ACT_GELU_TANH>(h, g1, TP<TA>(ot.hpre[li]), (long long)tokens * Hm, st);
-                wgrad<TA>(h, g1, Hm, TP<TA>(ot.ln2[li]), C, GA(h, lp.m0w), tokens, Hm, C, st, GA(h, lp.m0b));
-                gemm_dx<TA>(h, g1, Hm, lp.m0wT, g2, C, tokens, C, Hm, st);
-            }
-            launch_ln_bwd<TA>(h, g2, x_mid, lp.ln2w, dxs, dxb_out, GA(h, lp.ln2w), GA(h, lp.ln2b), tokens, st, drop,
-                              drop_site(o, li, 1));
-            // attention half: x_mid = x_in + Wo att(ln1(x_in)) + bo
-            wgrad<TA>(h, dxb, C, TP<TA>(ot.att[li]), C, GA(h, lp.outw), tokens, C, C, st, GA(h, lp.outb));
-            gemm_dx<TA>(h, dxb, C, lp.outwT, g2, C, tokens, C, C, st);
-            launch_attention_bwd<TA>(h, TP<TA>(ot.qkv[li]), g2, gq, B, lp.axis, st, drop, drop_site(o, li, 0));
-            wgrad<TA>(h, gq, 3 * C, TP<TA>(ot.ln1[li]), C, GA(h, lp.inw), tokens, 3 * C, C, st, GA(h, lp.inb));
-            gemm_dx<TA>(h, gq, 3 * C, lp.inwT, g2, C, tokens, C, 3 * C, st);
-            // the copy written here is the dY of the layer below's MLP branch
-            launch_ln_bwd<TA>(h, g2, x_in, lp.ln1w, dxs, dxb_out, GA(h, lp.ln1w), GA(h, lp.ln1b), tokens, st, drop,
-                              drop_site(o, std::max(li - 1, 0), 2));
+            run_layer_bwd<TA>(h, tp, o, li, dxb, dxb_out, st);
         }
         const float* pin = o == 0 ? FP(ot.P[0]) : FP(tp.ord[o - 1].X.back());
         launch_propagator_bwd(h, FP(ot.P[2]), dxs, B, 2, op, st);
         launch_propagator_bwd(h, FP(ot.P[1]), dxs, B, 1, op, st);
         launch_propagator_bwd(h, pin, dxs, B, 0, op, st);
     }
-    // ---- embeddings + t_encode FiLM (tante.py:136-141) ----
-    CK(cudaMemsetAsync(h->dfilm.p, 0, (size_t)T * 2 * C * 4, st));
-    embed_bwd_kernel<TA><<<(L + (256 / (C / 4)) - 1) / (256 / (C / 4)), 256, 0, st>>>(dxs, FP(tp.v), AF(h, h->film_t_off), g2, FP(h->dfilm), GA(h, h->s_emb),
-                                          GA(h, h->t_emb), B, T, L, C);
-    CK(cudaGetLastError());
-    h->launches++;
-    film_bwd_kernel<<<dim3(T, 16), 256, 3 * C * sizeof(float), st>>>(
-        AF(h, h->tseq_off), FP(h->dfilm), AF(h, h->tenc[0]), AF(h, h->tenc[1]), AF(h, h->tenc[2]), AF(h, h->tenc[4]),
-        AF(h, h->tenc[5]), AF(h, h->tenc[6]), GA(h, h->tenc[0]), GA(h, h->tenc[1]), GA(h, h->tenc[2]), GA(h, h->tenc[3]),
-        GA(h, h->tenc[4]), GA(h, h->tenc[5]), GA(h, h->tenc[6]), GA(h, h->tenc[7]), C, nullptr);
-    CK(cudaGetLastError());
-    h->launches++;
-    // ---- encoder (enc_dec_cnn.py:217-229) ----
-    const int K3 = g.k2 * g.k2 * C2, K2 = g.k1 * g.k1 * C1;
-    const int M2 = tokens * g.R2;
-    const long long rows_in = (long long)tokens * g.R1;
-    if (h->fno) {
-        TA* wb = TP<TA>(h->wbuf);
-        const int H = h->cfg.H, W = h->cfg.W, p0 = h->fp0, p1 = h->fp1, H1 = H / p0, W1 = W / p0, C8 = C / 8;
-        const long long NI = (long long)B * T, MF1 = NI * H1 * W1;
-        const int KF2 = p1 * p1 * C2, KF1 = p0 * p0 * C8;
-        TA* gr0 = TP<TA>(h->fgr0);
-        TA* gr1 = TP<TA>(h->fgr1);
-        TA* gr2 = TP<TA>(h->fgr2);
-        // conv grids (== the patch grids without overlap); with overlap the gradient of a pooled output first goes back to its conv grid
-        auto cdimf = [](int n, int k, int sdv) { return (n + 2 * ((k - 1) / 2) - k) / sdv + 1; };
-        const int Hc2 = cdimf(H1, p1, h->st[1]), Wc2 = cdimf(W1, p1, h->st[1]), Hc1 = cdimf(H, p0, h->st[0]), Wc1 = cdimf(W, p0, h->st[0]);
-        const bool pool2 = Hc2 != h->Hp || Wc2 != h->Wp, pool1 = Hc1 != H1 || Wc1 != W1;
-        const long long rows2 = NI * Hc2 * Wc2, rows1 = NI * Hc1 * Wc1;
-        REQUIRE(rows1 < (1LL << 31) && rows2 < (1LL << 31), "input too large for the conv backward GEMMs");
-        TA* cg = TP<TA>(h->cgrid);
-        // enc_conv_2 (p1): windows of the kept C/2 grid
-        const TA* dY2 = g2;
-        if (pool2) {
-            const long long t4 = rows2 * C / 4;
-            wide_pool_bwd_kernel<TA, false><<<blocks_for(t4, 256), 256, 0, st>>>(g2, nullptr, Hc2, Wc2, C, h->Hp, h->Wp, cg, t4);
-            CK(cudaGetLastError());
-            h->launches++;
-            dY2 = cg;
-        }
-        wide_im2col_cl_kernel<TA><<<blocks_for(rows2 * KF2 / 4, 256), 256, 0, st>>>(TP<TA>(tp.a2act), H1, W1, C2, p1, (p1 - 1) / 2, wb,
-                                                                                   rows2 * KF2 / 4, h->st[1], Hc2, Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        wgrad<TA>(h, dY2, C, wb, KF2, GA(h, h->enc_w[1]), rows2, C, KF2, st, GA(h, h->enc_b[1]));
-        gemm_dx<TA>(h, dY2, C, h->enc_wT[1], wb, KF2, (int)rows2, KF2, C, st);
-        wide_col2im_cl_kernel<TA><<<blocks_for(MF1 * C2 / 4, 256), 256, 0, st>>>(wb, H1, W1, C2, p1, (p1 - 1) / 2, gr2, MF1 * C2 / 4, h->st[1], Hc2, Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, gr2, TP<TA>(tp.a2pre), MF1 * C2, st);
-        // enc_spectral_2
-        SpecView xs1{tp.a1act.p, 1, nullptr, 1}, gs1{gr2, 1, nullptr, 1};
-        run_spectral_bwd<TA>(h, h->fes2, xs1, gs1, NI, H1, W1, 1, gr1, nullptr, st);
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, gr1, TP<TA>(tp.a1pre), MF1 * C1, st);
-        // enc_conv_1 (p0): windows of the kept C/8 grid
-        const TA* dY1 = gr1;
-        if (pool1) {
-            const long long t4 = rows1 * C1 / 4;
-            wide_pool_bwd_kernel<TA, false><<<blocks_for(t4, 256), 256, 0, st>>>(gr1, nullptr, Hc1, Wc1, C1, H1, W1, cg, t4);
-            CK(cudaGetLastError());
-            h->launches++;
-            dY1 = cg;
-        }
-        wide_im2col_cl_kernel<TA><<<blocks_for(rows1 * KF1 / 4, 256), 256, 0, st>>>(TP<TA>(tp.f0act), H, W, C8, p0, (p0 - 1) / 2, wb, rows1 * KF1 / 4,
-                                                                                   h->st[0], Hc1, Wc1);
-        CK(cudaGetLastError());
-        h->launches++;
-        wgrad<TA>(h, dY1, C1, wb, KF1, GA(h, h->enc_w[0]), rows1, C1, KF1, st, GA(h, h->enc_b[0]));
-        gemm_dx<TA>(h, dY1, C1, h->enc_wT[0], wb, KF1, (int)rows1, KF1, C1, st);
-        wide_col2im_cl_kernel<TA><<<blocks_for(NI * H * W * C8 / 4, 256), 256, 0, st>>>(wb, H, W, C8, p0, (p0 - 1) / 2, gr0, NI * H * W * C8 / 4,
-                                                                                       h->st[0], Hc1, Wc1);
-        CK(cudaGetLastError());
-        h->launches++;
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, gr0, TP<TA>(tp.f0pre), NI * H * W * C8, st);
-        // enc_spectral_1 on the input frames (input gradient accumulated on top of the u0 path)
-        SpecView xs0{input, 0, nullptr, T}, gs0{gr0, 1, nullptr, 1};
-        run_spectral_bwd<TA>(h, h->fes1, xs0, gs0, NI, H, W, 0, nullptr, grad_input, st);
-    } else if (h->wide) {
-        // natural-order stages: the patch matrices of conv3 / conv2 are re-gathered from the kept activation grids (cheap, one
-        // pass), their gradients go back to the grids through the transposed gather; with overlap_ratio != 0 the gradient of a
-        // stage's (pooled) output first goes back to its conv grid (wide_pool_bwd_kernel)
-        TA* wb = TP<TA>(h->wbuf);
-        TA* cg = TP<TA>(h->cgrid);
-        const int H = h->cfg.H, W = h->cfg.W;
-        const WideDims wd = wide_dims(h, B);
-        const int H1 = wd.H1, W1 = wd.W1, H2 = wd.H2, W2 = wd.W2;
-        const long long NI = (long long)B * T;
-        auto pool_bwd = [&](const TA* gp, int Hc, int Wc, int Cc, int Ho, int Wo) {
-            const long long total4 = NI * Hc * Wc * Cc / 4;
-            wide_pool_bwd_kernel<TA, false><<<blocks_for(total4, 256), 256, 0, st>>>(gp, nullptr, Hc, Wc, Cc, Ho, Wo, cg, total4);
-            CK(cudaGetLastError());
-            h->launches++;
-        };
-        // stage 3
-        const TA* dY3 = g2;
-        if (wd.pool3) { pool_bwd(g2, wd.Hc3, wd.Wc3, C, h->Hp, h->Wp); dY3 = cg; }
-        wide_im2col_cl_kernel<TA><<<blocks_for(wd.rows3 * K3 / 4, 256), 256, 0, st>>>(TP<TA>(tp.a2act), H2, W2, C2, g.k2, (g.k2 - 1) / 2, wb,
-                                                                                     wd.rows3 * K3 / 4, h->st[2], wd.Hc3, wd.Wc3);
-        CK(cudaGetLastError());
-        h->launches++;
-        wgrad<TA>(h, dY3, C, wb, K3, GA(h, h->enc_w[2]), wd.rows3, C, K3, st, GA(h, h->enc_b[2]));
-        gemm_dx<TA>(h, dY3, C, h->enc_wT[2], wb, K3, (int)wd.rows3, K3, C, st);
-        wide_col2im_cl_kernel<TA><<<blocks_for(NI * H2 * W2 * C2 / 4, 256), 256, 0, st>>>(wb, H2, W2, C2, g.k2, (g.k2 - 1) / 2, gq,
-                                                                                         NI * H2 * W2 * C2 / 4, h->st[2], wd.Hc3, wd.Wc3);
-        CK(cudaGetLastError());
-        h->launches++;
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, gq, TP<TA>(tp.a2pre), NI * H2 * W2 * C2, st);
-        // stage 2
-        const TA* dY2 = gq;
-        if (wd.pool2) { pool_bwd(gq, wd.Hc2, wd.Wc2, C2, H2, W2); dY2 = cg; }
-        wide_im2col_cl_kernel<TA><<<blocks_for(wd.rows2 * K2 / 4, 256), 256, 0, st>>>(TP<TA>(tp.a1act), H1, W1, C1, g.k1, (g.k1 - 1) / 2, wb,
-                                                                                     wd.rows2 * K2 / 4, h->st[1], wd.Hc2, wd.Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        wgrad<TA>(h, dY2, C2, wb, K2, GA(h, h->enc_w[1]), wd.rows2, C2, K2, st, GA(h, h->enc_b[1]));
-        gemm_dx<TA>(h, dY2, C2, h->enc_wT[1], wb, K2, (int)wd.rows2, K2, C2, st);
-        TA* ga1 = TP<TA>(h->ga1);
-        wide_col2im_cl_kernel<TA><<<blocks_for(NI * H1 * W1 * C1 / 4, 256), 256, 0, st>>>(wb, H1, W1, C1, g.k1, (g.k1 - 1) / 2, ga1,
-                                                                                         NI * H1 * W1 * C1 / 4, h->st[1], wd.Hc2, wd.Wc2);
-        CK(cudaGetLastError());
-        h->launches++;
-        launch_act_bwd<TA, ACT_GELU_ERF>(h, ga1, TP<TA>(tp.a1pre), NI * H1 * W1 * C1, st);
-        // stage 1
-        const TA* dY1 = ga1;
-        if (wd.pool1) { pool_bwd(ga1, wd.Hc1, wd.Wc1, C1, H1, W1); dY1 = cg; }
-        wgrad_pad<TA>(h, dY1, C1, C1, TP<TA>(tp.cols), h->K1pad, h->K1pad, GA(h, h->enc_w[0]), NO, NO, wd.rows1, st, GA(h, h->enc_b[0]));
-        if (grad_input) {
-            REQUIRE(wd.rows1 < (1LL << 31), "input too large for the first-conv backward GEMM");
-            gemm_dx<TA>(h, dY1, C1, h->enc_wT[0], wb, h->K1pad, (int)wd.rows1, h->K1pad, C1, st);
-            const long long tot = (long long)in_elems;
-            wide_col2im_cf_kernel<TA><<<blocks_for(tot, 256), 256, 0, st>>>(wb, D, H, W, g.k0, (g.k0 - 1) / 2, h->K1pad, grad_input, tot,
-                                                                           h->st[0], wd.Hc1, wd.Wc1);
-            CK(cudaGetLastError());
-            h->launches++;
-        }
-    } else {
-    wgrad<TA>(h, g2, C, TP<TA>(tp.a2act), K3, GA(h, h->enc_w[2]), tokens, C, K3, st, GA(h, h->enc_b[2]));
-    gemm_dx<TA>(h, g2, C, h->enc_wT[2], gq, K3, tokens, K3, C, st);
-    launch_act_bwd<TA, ACT_GELU_ERF>(h, gq, TP<TA>(tp.a2pre), (long long)tokens * K3, st);
-    wgrad<TA>(h, gq, C2, TP<TA>(tp.a1act), K2, GA(h, h->enc_w[1]), M2, C2, K2, st, GA(h, h->enc_b[1]));
-    TA* ga1 = TP<TA>(h->ga1);
-    gemm_dx<TA>(h, gq, C2, h->enc_wT[1], ga1, K2, M2, K2, C2, st);
-    launch_act_bwd<TA, ACT_GELU_ERF>(h, ga1, TP<TA>(tp.a1pre), (long long)M2 * K2, st);
-    (void)input;      // the patches were kept by the forward (tape im2col)
-    TA* cols = TP<TA>(h->cols);
-    wgrad_pad<TA>(h, ga1, C1, C1, TP<TA>(tp.cols), kHeadPad, kHeadPad, GA(h, h->enc_w[0]), NO, NO, rows_in, st, GA(h, h->enc_b[0]));
-    if (grad_input || win) {
-        // dpatch[rows, 64 (K1 padded)] = da1[rows, C1] * W1[C1][K1]  (thin GEMM), then scatter-add into the pixels
-        REQUIRE(rows_in < (1LL << 31), "input too large for the first-conv backward GEMM");
-        gemm_dx<TA>(h, ga1, C1, h->enc_wT[0], cols, kHeadPad, (int)rows_in, kHeadPad, C1, st);
-        const FrameTab gt = win ? win->gin : FrameTab();
-        float* gbase = grad_input ? grad_input : win->gpred;
-        if (g.k0 * g.k1 * g.k2 >= 4) conv1_col2im_kernel<TA, 4><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, gt);
-        else conv1_col2im_kernel<TA, 2><<<blocks_for(rows_in, kPatchRows), 128, 0, st>>>(cols, g, gbase, rows_in, gt);
-        CK(cudaGetLastError());
-        h->launches++;
-    }
-    }
+    // ---- embeddings + t_encode FiLM, then the encoder ----
+    TA* gv = TP<TA>(h->g2);
+    launch_embed_bwd<TA>(h, tp, gv, st);
+    if (h->fno) run_encoder_fno_bwd<TA>(h, tp, io, gv, st);
+    else if (h->wide) run_encoder_wide_bwd<TA>(h, tp, io, gv, st);
+    else run_encoder_cnn_bwd<TA>(h, tp, io, gv, st);
     // ---- packed gradient arena -> flat state_dict-layout buffer ----
     {
         int64_t max_numel = 0;
         for (const Param& p : h->params) max_numel = std::max(max_numel, p.numel);
         dim3 grid((unsigned)std::min<int64_t>((max_numel + 255) / 256, 64), (unsigned)h->params.size());
-        unpack_grads_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const UnpackDesc*>(h->udesc_dev.p), FP(h->garena), flat);
+        unpack_grads_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const UnpackDesc*>(h->udesc_dev.p), FP(h->garena), io.flat);
         CK(cudaGetLastError());
         h->launches++;
     }
@@ -2779,10 +2772,9 @@ int tante_reserve(tante_handle_t h, int32_t max_batch, int32_t max_roll, int32_t
             dev_alloc(h, h->fB, ca * 8);
             h->f_ca = ca;
             if (es == 2 && h->fp0 * h->fp0 * C8 > 1024) dev_alloc(h, h->kscratch, NI * HW1 * C1 * 4);      // split-K enc_conv_1 (8x8 windows)
-            auto cdimf = [](int n, int k, int sdv) { return (size_t)((n + 2 * ((k - 1) / 2) - k) / sdv + 1); };
             const int H1f = h->cfg.H / h->fp0, W1f = h->cfg.W / h->fp0;
-            const size_t rc1 = NI * cdimf(h->cfg.H, h->fp0, h->st[0]) * cdimf(h->cfg.W, h->fp0, h->st[0]);      // conv grids (== patch grids
-            const size_t rc2 = NI * cdimf(H1f, h->fp1, h->st[1]) * cdimf(W1f, h->fp1, h->st[1]);                // without overlap)
+            const size_t rc1 = NI * conv_dim(h->cfg.H, h->fp0, h->st[0]) * conv_dim(h->cfg.W, h->fp0, h->st[0]);      // conv grids (== patch
+            const size_t rc2 = NI * conv_dim(H1f, h->fp1, h->st[1]) * conv_dim(W1f, h->fp1, h->st[1]);                // grids without overlap)
             size_t m = rc1 * (size_t)(h->fp0 * h->fp0 * C8);                          // conv_1 windows
             m = std::max(m, rc2 * (size_t)(h->fp1 * h->fp1 * C2));                    // conv_2 windows
             if (h->overlap) {
@@ -2797,12 +2789,11 @@ int tante_reserve(tante_handle_t h, int32_t max_batch, int32_t max_roll, int32_t
         } else if (h->wide) {
             const size_t BLs = BL;
             // conv grids of the three encoder stages (== the patch grids without overlap)
-            auto cdim = [](int n, int k, int s) { return (size_t)((n + 2 * ((k - 1) / 2) - k) / s + 1); };
             const size_t NIw = (size_t)max_batch * h->T;
             const int Hh1 = h->cfg.H / g.k0, Ww1 = h->cfg.W / g.k0, Hh2 = Hh1 / g.k1, Ww2 = Ww1 / g.k1;
-            const size_t r1 = NIw * cdim(h->cfg.H, g.k0, h->st[0]) * cdim(h->cfg.W, g.k0, h->st[0]);
-            const size_t r2 = NIw * cdim(Hh1, g.k1, h->st[1]) * cdim(Ww1, g.k1, h->st[1]);
-            const size_t r3 = NIw * cdim(Hh2, g.k2, h->st[2]) * cdim(Ww2, g.k2, h->st[2]);
+            const size_t r1 = NIw * conv_dim(h->cfg.H, g.k0, h->st[0]) * conv_dim(h->cfg.W, g.k0, h->st[0]);
+            const size_t r2 = NIw * conv_dim(Hh1, g.k1, h->st[1]) * conv_dim(Ww1, g.k1, h->st[1]);
+            const size_t r3 = NIw * conv_dim(Hh2, g.k2, h->st[2]) * conv_dim(Ww2, g.k2, h->st[2]);
             size_t m = r1 * (size_t)h->K1pad;                                              // conv1 windows
             m = std::max(m, r2 * (size_t)(g.k1 * g.k1 * C1));                               // conv2 windows
             m = std::max(m, r3 * (size_t)(g.k2 * g.k2 * C2));                               // conv3 windows
@@ -2979,10 +2970,12 @@ int tante_backward(tante_handle_t h, int32_t slot, const float* input, const flo
         CK(cudaSetDevice(h->device));
         cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
         backward_alloc(h, tp.B_used);
-        if (h->cfg.precision == TANTE_PREC_FP32)
-            run_backward<float>(h, tp, input, grad_frames, n_frames, grad_Rt, grad_input, grad_params, st);
-        else
-            run_backward<__nv_bfloat16>(h, tp, input, grad_frames, n_frames, grad_Rt, grad_input, grad_params, st);
+        BackwardIO io;
+        io.input = input; io.gframes = grad_frames; io.n_g = n_frames;
+        io.gf_bs = (long long)n_frames * h->D * h->cfg.H * h->cfg.W;
+        io.gRt = grad_Rt; io.grad_input = grad_input; io.flat = grad_params;
+        if (h->cfg.precision == TANTE_PREC_FP32) run_backward<float>(h, tp, io, st);
+        else run_backward<__nv_bfloat16>(h, tp, io, st);
         tp.valid = false;
     });
 }
@@ -3042,14 +3035,14 @@ int tante_backward_hist(tante_handle_t h, int32_t slot, float* grad_pred, int64_
         CK(cudaSetDevice(h->device));
         cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
         backward_alloc(h, tp.B_used);
-        BackwardWin win;
-        win.gin = FrameTab{reinterpret_cast<const int*>(tp.cur.p), grad_input ? elem_offset(grad_pred, grad_input) : 0, gp_bstride,
-                           grad_input ? 0 : 1};
-        win.gpred = grad_pred;
-        if (h->cfg.precision == TANTE_PREC_FP32)
-            run_backward<float>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_input, grad_params, st, &win);
-        else
-            run_backward<__nv_bfloat16>(h, tp, nullptr, grad_pred, tp.n_cap, grad_Rt, grad_input, grad_params, st, &win);
+        BackwardIO io;
+        io.gframes = grad_pred; io.gf_bs = gp_bstride; io.n_g = tp.n_cap;
+        io.gRt = grad_Rt; io.grad_input = grad_input; io.flat = grad_params;
+        io.gin = FrameTab{reinterpret_cast<const int*>(tp.cur.p), grad_input ? elem_offset(grad_pred, grad_input) : 0, gp_bstride,
+                          grad_input ? 0 : 1};
+        io.gpred = grad_pred;
+        if (h->cfg.precision == TANTE_PREC_FP32) run_backward<float>(h, tp, io, st);
+        else run_backward<__nv_bfloat16>(h, tp, io, st);
         tp.valid = false;
     });
 }
